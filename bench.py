@@ -11,6 +11,7 @@ reduce of step k overlaps the rendering of step k+1) and the addition into rank 
     python bench.py --gpus 1 --steps K --warmup W                     (one JSON line)
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...     the reference's algorithm on the host cores (CPU oracle)
+    python bench.py ... --dump-outputs DIR   also writes the frame of the timed steps as DIR/*.npy (same arguments, same inputs)
 
 Besides the contract's keys the line carries: `reduce_check` (the reduced frame's weights and an oracle crop),
 `strong` (one fixed-size frame, --total-spp samples split over the ranks), `e2e_ref_signature` (the reference's own
@@ -54,7 +55,35 @@ def parse():
                     help="f64 = the reference's type (parity path, the headline); f32 = VRJ_PRECISION_F32_FAST, reported separately")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip strong / e2e_ref_signature / sharded_check / extra_configs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frame they left (colour_sum, weight) to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 64 * 10 ** 6  # at most this much .npy data from --dump-outputs
+
+
+def dump_outputs(out_dir, frame, H, W):
+    """The timed path's result as its caller holds it after the last step: the frame's per-pixel XYZ sums (float64) and
+    sample weights (float32: whole sample counts, exact).  A frame too large for DUMP_BYTES is reduced to a fixed, seeded
+    sample of pixels, whose row-major indices go to pixel_index.npy."""
+    import numpy as np
+    npix = H * W
+    f = frame.cpu().numpy()
+    colour_sum, weight = f[:npix * 3].reshape(npix, 3), f[npix * 3:].astype(np.float32)
+    per_pixel = colour_sum.itemsize * 3 + weight.itemsize
+    if npix * per_pixel <= DUMP_BYTES:
+        arrays = {"colour_sum": colour_sum.reshape(H, W, 3), "weight": weight.reshape(H, W)}
+    else:
+        n = (DUMP_BYTES - 4096) // (per_pixel + 8)  # 4 KB left for the .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(npix, n, replace=False))
+        arrays = {"colour_sum": colour_sum[idx], "weight": weight[idx], "pixel_index": idx.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def peaks():
@@ -328,6 +357,8 @@ def main():
     fence()
     wall = time.perf_counter() - t0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, frame, H, W)
 
     # ---- reduce_check (outside the timed region): the frame on rank 0 holds every sample of every rank exactly once
     reduce_check = None
@@ -398,8 +429,7 @@ def main():
     pinned = {"colour": pinned_array(capi, np, npix * 3), "weight": pinned_array(capi, np, npix)}
     host_frame = torch.empty(npix * 4, dtype=torch.float64).pin_memory() if (world > 1 and rank == 0) else None
     fence()
-    n_e2e = max(10, min(args.steps, 20))
-    for k in range(n_e2e + 1):
+    for k in range(args.steps + 1):
         if world > 1:
             dist.barrier()
             torch.cuda.synchronize()

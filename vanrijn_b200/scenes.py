@@ -9,7 +9,10 @@ a Git-LFS pointer in the reference snapshot, so until the real 4.86 MB file is d
 (path given by $VANRIJN_BUNNY_OBJ) every "bunny" configuration uses the displaced
 icosphere of SURVEY.md 8(d): 6 subdivisions = 81 920 triangles / 40 962 vertices.
 """
+import atexit
 import os
+import shutil
+import tempfile
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -113,13 +116,25 @@ def write_obj(path, pos, nrm, faces):
                    fmt="f %d//%d %d//%d %d//%d")
 
 
+_MESH_DIR = None
+
+
+def _mesh_dir():
+    """A temporary directory of this process for generated meshes, removed at exit: the source tree may be read-only."""
+    global _MESH_DIR
+    if _MESH_DIR is None:
+        _MESH_DIR = tempfile.mkdtemp(prefix="vanrijn_b200_meshes_")
+        atexit.register(shutil.rmtree, _MESH_DIR, True)
+    return _MESH_DIR
+
+
 def bunny_obj_path(cache_dir=None, subdivisions=6):
     """Path of the bunny OBJ: the real file when $VANRIJN_BUNNY_OBJ points at one, else the proxy
-    (generated once into cache_dir)."""
+    (generated once into cache_dir, by default a temporary directory of this process)."""
     real = os.environ.get("VANRIJN_BUNNY_OBJ")
     if real and os.path.exists(real) and os.path.getsize(real) > 1000:
         return real, "stanford_bunny"
-    cache_dir = cache_dir or os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "build", "meshes")
+    cache_dir = cache_dir or _mesh_dir()
     os.makedirs(cache_dir, exist_ok=True)
     path = os.path.join(cache_dir, "bunny_proxy_s%d.obj" % subdivisions)
     if not os.path.exists(path):

@@ -280,6 +280,49 @@ VRJ_API VrjStatus vrj_copy_to_host(int32_t device, void *host_dst, const void *d
 VRJ_API VrjStatus vrj_render_tile(const VrjScene *scene, const VrjTile *tile, uint64_t height, uint64_t width,
                           const VrjRenderParams *params, VrjAccumOut *out);
 
+/* ---- adaptive sampling: per-pixel sample counts set by an on-device noise estimate ----
+ * vrj_render_adaptive renders `tile` in passes and stops sampling a pixel once the estimated error of its mean Y is small.
+ * A pixel that ends with n samples holds, bit for bit, what vrj_render_tile with spp = n (same seed, sample_offset,
+ * sample_stride) gives it: its k-th sample has index sample_offset + k * stride, and samples are applied in sample order.
+ *
+ * Passes.  Pass 0 gives every pixel samples 0 .. min_samples-1.  After each pass every active pixel is judged; the active
+ * pixels that have not converged and hold fewer than max_samples take min(pass_samples, max_samples - n) more in the next
+ * pass.  All active pixels hold the same n, so every count is min_samples + j * pass_samples, capped at max_samples.
+ *
+ * Stopping rule, in binary64 in exactly this order (n = weight, s = colour_sum.y, q = y_sq_sum):
+ *     m = s * (1.0 / n);   v = (q - s * m) / (n - 1.0);   if (v < 0) v = 0;
+ *     t = rel_error * (m > abs_floor ? m : abs_floor);   converged  iff  v <= t * t * n
+ * i.e. the standard error of the mean, sqrt(v / n), is at most rel_error * max(m, abs_floor).  A NaN anywhere fails the
+ * test: such a pixel samples until max_samples.
+ *
+ * y_sq_sum (optional, NULL: not returned): one double per pixel, memory of the kind out->memory says; q = q + y * y over the
+ * pixel's samples in sample order, y being exactly the Y value the sample adds to colour_sum.
+ * out: the arrays, layout and memory kinds of vrj_render_tile, srgb8 included; out->stats sums the passes (device_ms spans
+ * the first to the last kernel, the per-pass readback of the active count -- 4 bytes -- included).  out->accumulate and
+ * out->photons: VRJ_ERR_UNSUPPORTED.  params: every field keeps its meaning (integrators, lights, filters, precisions,
+ * sample_stride, count_traversal) except spp, which must be 0 (the counts come from `ap`).  astats may be NULL.
+ * Scheduling: the call is never coalesced with others; it takes the device's render turn like any other call and uses a
+ * scratch block from the pool (16 bytes per pixel more than vrj_render_tile: y_sq_sum and two pixel lists). */
+typedef struct VrjAdaptiveParams {
+    uint32_t min_samples;   /* every pixel first takes samples 0..min_samples-1; >= 2 */
+    uint32_t max_samples;   /* no pixel takes more; >= min_samples */
+    uint32_t pass_samples;  /* samples each still-active pixel takes per further pass; >= 1 */
+    uint32_t pad;
+    double rel_error;       /* > 0, finite */
+    double abs_floor;       /* >= 0, finite */
+} VrjAdaptiveParams;
+
+typedef struct VrjAdaptiveStats {
+    uint64_t passes;              /* including the first (min_samples) pass */
+    uint64_t samples;             /* sum over pixels of the samples each received (= sum of weight) */
+    uint64_t pixels_converged;    /* stopped by the error rule */
+    uint64_t pixels_unconverged;  /* reached max_samples without meeting it */
+} VrjAdaptiveStats;
+
+VRJ_API VrjStatus vrj_render_adaptive(const VrjScene *scene, const VrjTile *tile, uint64_t height, uint64_t width,
+                                      const VrjRenderParams *params, const VrjAdaptiveParams *ap, VrjAccumOut *out,
+                                      double *y_sq_sum, VrjAdaptiveStats *astats);
+
 /* Sampler::sample on n rays (host arrays, 3 doubles each; directions are normalised like Ray::new).
  * object_id / prim_id are -1 and t is +inf on a miss. */
 /* ---- one box, several GPUs (SURVEY 8e): shard by sample index, one NCCL reduce into the first device ----

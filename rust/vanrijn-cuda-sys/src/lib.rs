@@ -114,6 +114,28 @@ pub struct VrjBvhBuildStats {
     pub pad: u32,
 }
 
+/// Sample counts and error target of `vrj_render_adaptive` (see the header for the passes and the stopping rule).
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct VrjAdaptiveParams {
+    pub min_samples: u32,
+    pub max_samples: u32,
+    pub pass_samples: u32,
+    pub pad: u32,
+    pub rel_error: f64,
+    pub abs_floor: f64,
+}
+
+/// What `vrj_render_adaptive` did: passes, samples over all pixels, pixels stopped by the rule / at `max_samples`.
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct VrjAdaptiveStats {
+    pub passes: u64,
+    pub samples: u64,
+    pub pixels_converged: u64,
+    pub pixels_unconverged: u64,
+}
+
 extern "C" {
     pub fn vrj_last_error() -> *const c_char;
     pub fn vrj_abi_version() -> i32;
@@ -130,6 +152,11 @@ extern "C" {
     pub fn vrj_copy_to_host(device: i32, host_dst: *mut c_void, device_src: *const c_void, bytes: u64) -> i32;
     pub fn vrj_render_tile(scene: *const VrjScene, tile: *const VrjTile, height: u64, width: u64,
                            params: *const VrjRenderParams, out: *mut VrjAccumOut) -> i32;
+    /// Per-pixel sample counts from an on-device noise estimate; a pixel with n samples holds what
+    /// `vrj_render_tile` with spp = n gives it.  `params.spp` must be 0; `y_sq_sum` may be NULL.
+    pub fn vrj_render_adaptive(scene: *const VrjScene, tile: *const VrjTile, height: u64, width: u64,
+                               params: *const VrjRenderParams, ap: *const VrjAdaptiveParams, out: *mut VrjAccumOut,
+                               y_sq_sum: *mut f64, astats: *mut VrjAdaptiveStats) -> i32;
     pub fn vrj_comm_create(n_devices: i32, devices: *const i32, out: *mut *mut VrjComm) -> i32;
     pub fn vrj_comm_destroy(comm: *mut VrjComm);
     pub fn vrj_comm_scene_create(comm: *mut VrjComm, desc: *const VrjSceneDesc, out: *mut *mut VrjMultiScene) -> i32;

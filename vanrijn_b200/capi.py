@@ -27,7 +27,7 @@ OK = 0
 CUDA_SYMBOLS = ["vrj_last_error", "vrj_abi_version", "vrj_device_count", "vrj_scene_create", "vrj_scene_destroy",
                 "vrj_scene_device_bytes", "vrj_scene_upload_bytes", "vrj_render_tile", "vrj_trace_rays", "vrj_release_scratch", "vrj_alloc_host",
                 "vrj_free_host", "vrj_alloc_device", "vrj_free_device", "vrj_copy_to_host", "vrj_comm_create", "vrj_comm_destroy", "vrj_comm_scene_create", "vrj_comm_scene_destroy",
-                "vrj_render_sharded", "vrj_tone_map", "vrj_bvh_build"]
+                "vrj_render_sharded", "vrj_tone_map", "vrj_bvh_build", "vrj_render_adaptive"]
 
 
 class VrjError(RuntimeError):
@@ -123,6 +123,18 @@ class AccumOut(C.Structure):
                 ("stats", C.POINTER(Stats)), ("srgb8", C.c_void_p)]
 
 
+class AdaptiveParams(C.Structure):
+    _fields_ = [("min_samples", C.c_uint32), ("max_samples", C.c_uint32), ("pass_samples", C.c_uint32), ("pad", C.c_uint32),
+                ("rel_error", C.c_double), ("abs_floor", C.c_double)]
+
+
+class AdaptiveStats(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("passes", "samples", "pixels_converged", "pixels_unconverged")]
+
+    def as_dict(self):
+        return {n: int(getattr(self, n)) for n, _ in self._fields_}
+
+
 _cuda = None
 _host = None
 
@@ -161,6 +173,9 @@ def cuda():
         L.vrj_render_tile.restype = C.c_int32
         L.vrj_render_tile.argtypes = [C.c_void_p, C.POINTER(Tile), C.c_uint64, C.c_uint64, C.POINTER(RenderParams),
                                       C.POINTER(AccumOut)]
+        L.vrj_render_adaptive.restype = C.c_int32
+        L.vrj_render_adaptive.argtypes = [C.c_void_p, C.POINTER(Tile), C.c_uint64, C.c_uint64, C.POINTER(RenderParams),
+                                          C.POINTER(AdaptiveParams), C.POINTER(AccumOut), C.c_void_p, C.POINTER(AdaptiveStats)]
         L.vrj_comm_create.restype = C.c_int32
         L.vrj_comm_create.argtypes = [C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_void_p)]
         L.vrj_comm_destroy.argtypes = [C.c_void_p]

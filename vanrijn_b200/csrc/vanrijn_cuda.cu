@@ -32,12 +32,12 @@ thread_local std::string g_error;
 
 // the six instantiations live in vrj_batch_inst.cu (one object file each)
 namespace vrjimpl {
-extern template VrjStatus run_batch<float, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *);
-extern template VrjStatus run_batch<float, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *);
-extern template VrjStatus run_batch<double, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *);
-extern template VrjStatus run_batch<double, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *);
-extern template VrjStatus run_batch<float, float, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *);
-extern template VrjStatus run_batch<float, float, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *);
+extern template VrjStatus run_batch<float, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
+extern template VrjStatus run_batch<float, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
+extern template VrjStatus run_batch<double, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
+extern template VrjStatus run_batch<double, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
+extern template VrjStatus run_batch<float, float, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
+extern template VrjStatus run_batch<float, float, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
 } // namespace vrjimpl
 // NVTX ranges (SURVEY section 5) through the header-only NVTX 3: no library to link or load -- the calls are no-ops until a
 // tool (ncu --nvtx, nsys) injects itself
@@ -311,7 +311,7 @@ std::unordered_map<void *, size_t> g_host_pool_live;
 // Blocks are kept for concurrent callers (main.rs:197-209 drives the entry point from a pool of workers, each call needing
 // its own block): up to 16 per device as long as what the pool holds stays under 48 GB -- sixteen 1-spp 1080p blocks are
 // 14 GB, one 64-spp block is 45 GB.  A caller is handed the smallest pooled block that is large enough, else the largest.
-size_t scratch_bytes(const Scratch *s) { return s->capacity * 240 + s->rec_capacity * sizeof(TraceRec) + s->npix * 88; }
+size_t scratch_bytes(const Scratch *s) { return s->capacity * 240 + s->rec_capacity * sizeof(TraceRec) + s->npix * 88 + s->adapt_npix * 16; }
 std::atomic<int> g_active_calls[64];
 
 // Render gate: how many calls may have their wavefronts on one device at the same moment.  main.rs:197-209 drives the entry
@@ -399,6 +399,29 @@ void release_scratch(VrjScene *sc, Scratch *s) {
     else delete s;
 }
 
+// A group of a block's buffers is all-or-nothing: a failed allocation leaves the group empty with its size field at 0 (never
+// half-sized or stale), so the block can go back to the pool and the caller can retry
+// ... and ONE allocation: cudaMalloc waits for a gap in the device's work, so with another caller's persistent kernels
+// running the 25 buffers of a block cost 30 ms each (measured: 840 ms for the second block of a worker pool)
+VrjStatus alloc_group(DeviceBuffer &slab, std::vector<std::pair<DeviceBuffer *, size_t>> &want, const char *what) {
+    for (auto &w : want) w.first->release();
+    slab.release();
+    size_t total = 0;
+    for (auto &w : want) total += (w.second + 255) & ~size_t(255);
+    cudaError_t e = slab.alloc(total);
+    if (e != cudaSuccess) {
+        slab.release();
+        cudaGetLastError();
+        return fail(e == cudaErrorMemoryAllocation ? VRJ_ERR_OUT_OF_MEMORY : VRJ_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
+    }
+    size_t at = 0;
+    for (auto &w : want) {
+        w.first->borrow(static_cast<char *>(slab.p) + at, w.second);
+        at += (w.second + 255) & ~size_t(255);
+    }
+    return VRJ_OK;
+}
+
 // `queue_oom` (optional): set when the allocation that failed was the path queues -- the only part a smaller batch shrinks
 VrjStatus ensure_scratch(Scratch *s, size_t capacity, size_t rec_capacity, size_t npix, uint32_t steps, uint32_t n_lights, size_t n_light_samples, bool *queue_oom = nullptr) {
     if (queue_oom) *queue_oom = false;
@@ -414,28 +437,7 @@ VrjStatus ensure_scratch(Scratch *s, size_t capacity, size_t rec_capacity, size_
         for (cudaEvent_t &e : s->drain_ev) VRJ_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         VRJ_CUDA(cudaMallocHost(&s->host_count, 256 * sizeof(uint32_t))); // drain-check slots + the sample table of coalesced calls
     }
-    // every group below is all-or-nothing: a failed allocation leaves the group empty with its size field at 0 (never
-    // half-sized or stale), so the block can go back to the pool and the caller can retry
-    // ... and ONE allocation: cudaMalloc waits for a gap in the device's work, so with another caller's persistent kernels
-    // running the 25 buffers of a block cost 30 ms each (measured: 840 ms for the second block of a worker pool)
-    auto alloc_group = [](DeviceBuffer &slab, std::vector<std::pair<DeviceBuffer *, size_t>> &want, const char *what) -> VrjStatus {
-        for (auto &w : want) w.first->release();
-        slab.release();
-        size_t total = 0;
-        for (auto &w : want) total += (w.second + 255) & ~size_t(255);
-        cudaError_t e = slab.alloc(total);
-        if (e != cudaSuccess) {
-            slab.release();
-            cudaGetLastError();
-            return fail(e == cudaErrorMemoryAllocation ? VRJ_ERR_OUT_OF_MEMORY : VRJ_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
-        }
-        size_t at = 0;
-        for (auto &w : want) {
-            w.first->borrow(static_cast<char *>(slab.p) + at, w.second);
-            at += (w.second + 255) & ~size_t(255);
-        }
-        return VRJ_OK;
-    };
+    // every group below is all-or-nothing (alloc_group)
     if (s->capacity < capacity) {
         s->capacity = 0;
         std::vector<std::pair<DeviceBuffer *, size_t>> want;
@@ -773,6 +775,141 @@ VrjStatus render_coalesced(const VrjScene *scene, const VrjTile *tile, uint64_t 
         co.cv.notify_all();
     }
     return st;
+}
+
+// ---------------------------------------------------------------------------------------------- shared by the render calls
+// a call in flight on a device: the path budget is shared between such calls, and wait_event sleeps instead of spinning
+struct ActiveCall {
+    std::atomic<int> &n;
+    int others;
+    explicit ActiveCall(std::atomic<int> &c) : n(c), others(c.fetch_add(1)) {}
+    ~ActiveCall() { n.fetch_sub(1); }
+};
+
+// the argument checks of vrj_render_tile and vrj_render_adaptive; *n_light_samples: samples of the call's light spectra
+VrjStatus check_render_args(const VrjScene *scene, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p,
+                            const VrjAccumOut *out, size_t *n_light_samples) {
+    if (!scene || !tile || !p || !out) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (tile->end_column < tile->start_column || tile->end_row < tile->start_row || tile->end_column > width || tile->end_row > height)
+        return fail(VRJ_ERR_INVALID_ARGUMENT, "tile outside the image");
+    if (width * height > 0xffffffffull) return fail(VRJ_ERR_UNSUPPORTED, "image larger than 2^32 pixels");
+    if (p->integrator > VRJ_INTEGRATOR_WHITTED) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown integrator");
+    if (p->bvh_filter > VRJ_FILTER_Q16) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown bvh_filter");
+    if (p->precision > VRJ_PRECISION_F32_FAST) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown precision");
+    if (p->max_depth > 65535) return fail(VRJ_ERR_INVALID_ARGUMENT, "max_depth exceeds u16 (RECURSION_LIMIT is a u16)");
+    if (p->n_lights && !p->lights) return fail(VRJ_ERR_INVALID_ARGUMENT, "lights is NULL");
+    size_t n = 0;
+    for (uint32_t i = 0; i < p->n_lights; i++) {
+        if (p->lights[i].spectrum.n_samples < 2 || !p->lights[i].spectrum.samples) return fail(VRJ_ERR_INVALID_ARGUMENT, "light spectrum needs >= 2 samples");
+        n += p->lights[i].spectrum.n_samples;
+    }
+    if (p->ambient_light) {
+        if (p->ambient_light->n_samples < 2 || !p->ambient_light->samples) return fail(VRJ_ERR_INVALID_ARGUMENT, "ambient spectrum needs >= 2 samples");
+        n += p->ambient_light->n_samples;
+    }
+    *n_light_samples = n;
+    return VRJ_OK;
+}
+
+// Paths in flight per batch: 128 Mi by default = 45 GB of queue state (sized for 180 GB of HBM), shared between the calls
+// running on this device right now, so several callers asking for many samples each do not have to find out through failed
+// allocations that they cannot all have a full budget
+uint64_t call_path_budget(const VrjScene *scene, const ActiveCall &active) {
+    return std::max<uint64_t>(scene->path_budget / (uint64_t)(active.others + 1), std::min<uint64_t>(scene->path_budget, uint64_t(1) << 22));
+}
+
+// TraceRec records: only the calls that walk them need the extra 96 bytes per path in flight
+bool call_wants_records(const VrjScene *scene, const VrjRenderParams *p, uint32_t filter) {
+    return p->precision == VRJ_PRECISION_F64 && filter == VRJ_FILTER_F32 && scene->trace_records && scene->dev.n_bvh_items > 0;
+}
+
+// the block for batches of *batch samples of npix pixels
+VrjStatus ensure_call_scratch(Scratch *s, const VrjRenderParams *p, bool records, uint64_t npix, uint32_t *batch, size_t n_light_samples) {
+    bool queue_oom = false;
+    auto ensure = [&] {
+        return ensure_scratch(s, npix * *batch, records ? npix * *batch : 0, npix, p->max_depth + 3, p->n_lights, n_light_samples, &queue_oom);
+    };
+    VrjStatus st = ensure();
+    while (st == VRJ_ERR_OUT_OF_MEMORY && queue_oom && *batch > 1) { // 240 bytes per path in flight: halve the batch until the queues fit
+        vrj_pool_trim();
+        *batch = (*batch + 1) / 2;
+        st = ensure();
+    }
+    if (st == VRJ_ERR_OUT_OF_MEMORY && !queue_oom) { // the accumulators do not shrink with the batch: give cached blocks back, once
+        vrj_pool_trim();
+        st = ensure();
+    }
+    return st;
+}
+
+// the call's lights and ambient spectrum into the block (RenderConst::lights / light_samples)
+VrjStatus stage_lights(Scratch *s, const VrjRenderParams *p) {
+    if (!p->n_lights && !p->ambient_light) return VRJ_OK;
+    std::vector<LightDev> lights(p->n_lights + 1);
+    std::vector<double> lsamples;
+    auto put = [&lsamples](const VrjSpectrumData &sd) {
+        SpectrumDev d{sd.shortest_wavelength, sd.longest_wavelength, (uint32_t)lsamples.size(), sd.n_samples};
+        lsamples.insert(lsamples.end(), sd.samples, sd.samples + sd.n_samples);
+        return d;
+    };
+    for (uint32_t i = 0; i < p->n_lights; i++) {
+        for (int k = 0; k < 3; k++) lights[i].dir[k] = p->lights[i].direction[k];
+        lights[i].spectrum = put(p->lights[i].spectrum);
+    }
+    lights[p->n_lights] = LightDev{};
+    if (p->ambient_light) lights[p->n_lights].spectrum = put(*p->ambient_light);
+    VRJ_CUDA(cudaMemcpyAsync(s->lights.p, lights.data(), lights.size() * sizeof(LightDev), cudaMemcpyHostToDevice, s->stream));
+    if (!lsamples.empty())
+        VRJ_CUDA(cudaMemcpyAsync(s->light_samples.p, lsamples.data(), lsamples.size() * sizeof(double), cudaMemcpyHostToDevice, s->stream));
+    VRJ_CUDA(cudaStreamSynchronize(s->stream)); // the staging vectors are locals
+    return VRJ_OK;
+}
+
+// one batch in the kernel variant the call's precision, walk and counting select
+VrjStatus dispatch_batch(const VrjScene *scene, Scratch *s, const RenderConst &rc, const VrjRenderParams *p, uint32_t filter, uint64_t *launches,
+                         const ResolveCopy *copy, double *ysq) {
+    const bool whitted = p->integrator == VRJ_INTEGRATOR_WHITTED;
+    // F32X4: the staged rays walk the 4-wide tree; inline any-hit queries (Whitted shadow rays, k_tail) use the 2-wide f32 tree
+    const int quad = filter == VRJ_FILTER_F32X4 ? 1 : filter == VRJ_FILTER_Q16 ? 2 : 0;
+    // VRJ_PRECISION_F32_FAST: the whole sample in binary32 over the 2-wide f32 tree (no reference counterpart; not a parity mode)
+    const bool fast = p->precision == VRJ_PRECISION_F32_FAST;
+    if (p->count_traversal)
+        return fast ? run_batch<float, float, true>(scene, s, rc, whitted, 0, launches, nullptr, copy, ysq)
+             : filter == VRJ_FILTER_F64 ? run_batch<double, double, true>(scene, s, rc, whitted, 0, launches, nullptr, copy, ysq)
+                                        : run_batch<float, double, true>(scene, s, rc, whitted, quad, launches, nullptr, copy, ysq);
+    return fast ? run_batch<float, float, false>(scene, s, rc, whitted, 0, launches, nullptr, copy, ysq)
+         : filter == VRJ_FILTER_F64 ? run_batch<double, double, false>(scene, s, rc, whitted, 0, launches, nullptr, copy, ysq)
+                                    : run_batch<float, double, false>(scene, s, rc, whitted, quad, launches, nullptr, copy, ysq);
+}
+
+// VrjStats of a call from its counters and the boundary events run_levels recorded
+void fill_call_stats(VrjStats *st, const Scratch *s, const unsigned long long *hstats, uint64_t launches, float ms) {
+    fill_stats(st, hstats, launches, ms);
+    double cls_ms[6] = {0, 0, 0, 0, 0, 0}; // 0 T (camera rays), 1 T (bounce rays), 2 resolve, 3 shade, 4 raygen, 5 tail
+    uint64_t cls_n[6] = {0, 0, 0, 0, 0, 0};
+    for (size_t i = 1; i < s->n_marks; i++) {
+        int c = s->mark_class[i];
+        if (c < 0) continue;
+        float seg = 0.f;
+        if (cudaEventElapsedTime(&seg, s->marks[i - 1], s->marks[i]) == cudaSuccess) cls_ms[c] += seg, cls_n[c]++;
+    }
+    st->primary_ms = cls_ms[0], st->bounce_ms = cls_ms[1], st->resolve_ms = cls_ms[2];
+    st->primary_launches = cls_n[0], st->bounce_launches = cls_n[1], st->resolve_launches = cls_n[2];
+    st->shade_ms = cls_ms[3] + cls_ms[4], st->shade_launches = cls_n[3] + cls_n[4];
+    st->tail_ms = cls_ms[5], st->tail_launches = cls_n[5];
+    st->coalesced_calls = 1;
+}
+
+// the tone-mapped colours of the block's accumulators to out->srgb8
+VrjStatus copy_srgb8(Scratch *s, uint64_t npix, uint8_t *dst, cudaMemcpyKind kind, uint64_t *launches) {
+    if (s->srgb8.bytes < npix * 3) {
+        s->srgb8.release();
+        VRJ_CUDA(s->srgb8.alloc(npix * 3));
+    }
+    k_tone_map<<<(unsigned)((npix + 255) / 256), 256, 0, s->stream>>>(s->acc_colour.as<double>(), s->srgb8.as<unsigned char>(), npix, 0);
+    (*launches)++;
+    VRJ_CUDA(cudaMemcpyAsync(dst, s->srgb8.p, npix * 3, kind, s->stream));
+    return VRJ_OK;
 }
 
 } // namespace
@@ -1229,24 +1366,9 @@ VrjStatus vrj_copy_to_host(int32_t device, void *host_dst, const void *device_sr
 VrjStatus vrj_render_tile(const VrjScene *scene_c, const VrjTile *tile, uint64_t height, uint64_t width,
                           const VrjRenderParams *p, VrjAccumOut *out) {
     VrjScene *scene = const_cast<VrjScene *>(scene_c);
-    if (!scene || !tile || !p || !out) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
-    if (tile->end_column < tile->start_column || tile->end_row < tile->start_row || tile->end_column > width || tile->end_row > height)
-        return fail(VRJ_ERR_INVALID_ARGUMENT, "tile outside the image");
-    if (width * height > 0xffffffffull) return fail(VRJ_ERR_UNSUPPORTED, "image larger than 2^32 pixels");
-    if (p->integrator > VRJ_INTEGRATOR_WHITTED) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown integrator");
-    if (p->bvh_filter > VRJ_FILTER_Q16) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown bvh_filter");
-    if (p->precision > VRJ_PRECISION_F32_FAST) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown precision");
-    if (p->max_depth > 65535) return fail(VRJ_ERR_INVALID_ARGUMENT, "max_depth exceeds u16 (RECURSION_LIMIT is a u16)");
-    if (p->n_lights && !p->lights) return fail(VRJ_ERR_INVALID_ARGUMENT, "lights is NULL");
     size_t n_light_samples = 0;
-    for (uint32_t i = 0; i < p->n_lights; i++) {
-        if (p->lights[i].spectrum.n_samples < 2 || !p->lights[i].spectrum.samples) return fail(VRJ_ERR_INVALID_ARGUMENT, "light spectrum needs >= 2 samples");
-        n_light_samples += p->lights[i].spectrum.n_samples;
-    }
-    if (p->ambient_light) {
-        if (p->ambient_light->n_samples < 2 || !p->ambient_light->samples) return fail(VRJ_ERR_INVALID_ARGUMENT, "ambient spectrum needs >= 2 samples");
-        n_light_samples += p->ambient_light->n_samples;
-    }
+    VrjStatus st = check_render_args(scene, tile, height, width, p, out, &n_light_samples);
+    if (st != VRJ_OK) return st;
     const uint64_t tw = tile->end_column - tile->start_column, th = tile->end_row - tile->start_row;
     const uint64_t npix = tw * th;
     DeviceGuard device_guard;
@@ -1257,20 +1379,11 @@ VrjStatus vrj_render_tile(const VrjScene *scene_c, const VrjTile *tile, uint64_t
     if (npix == 0 || p->spp == 0) return VRJ_OK;
     VRJ_CUDA(cudaSetDevice(scene->device));
 
-    // batch: as many samples of the whole tile in flight as fit the path budget -- 128 Mi paths by default = 45 GB of queue
-    // state (sized for 180 GB of HBM) -- shared between the calls running on this device right now, so several callers asking
-    // for many samples each do not have to find out through failed allocations that they cannot all have a full budget
-    struct ActiveCall {
-        std::atomic<int> &n;
-        int others;
-        explicit ActiveCall(std::atomic<int> &c) : n(c), others(c.fetch_add(1)) {}
-        ~ActiveCall() { n.fetch_sub(1); }
-    } active(g_active_calls[(unsigned)scene->device % 64]);
+    // batch: as many samples of the whole tile in flight as fit the path budget
+    ActiveCall active(g_active_calls[(unsigned)scene->device % 64]);
     if (coalescable(p, out, npix)) return render_coalesced(scene, tile, height, width, p, out);
-    const uint64_t path_budget = std::max<uint64_t>(scene->path_budget / (uint64_t)(active.others + 1), std::min<uint64_t>(scene->path_budget, uint64_t(1) << 22));
-    uint32_t batch = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(p->spp, path_budget / npix));
+    uint32_t batch = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(p->spp, call_path_budget(scene, active) / npix));
     if (npix * (uint64_t)batch > 0xfffffff0ull) return fail(VRJ_ERR_UNSUPPORTED, "tile too large");
-    const bool whitted = p->integrator == VRJ_INTEGRATOR_WHITTED;
     Scratch *s = acquire_scratch(scene, npix * batch);
     struct Releaser {
         VrjScene *sc;
@@ -1283,20 +1396,8 @@ VrjStatus vrj_render_tile(const VrjScene *scene_c, const VrjTile *tile, uint64_t
             release_scratch(sc, s);
         }
     } releaser{scene, s};
-    bool queue_oom = false;
-    // TraceRec records: only the calls that walk them need the extra 96 bytes per path in flight
     const uint32_t filter = effective_filter(scene, p);
-    const bool records = p->precision == VRJ_PRECISION_F64 && filter == VRJ_FILTER_F32 && scene->trace_records && scene->dev.n_bvh_items > 0;
-    VrjStatus st = ensure_scratch(s, npix * batch, records ? npix * batch : 0, npix, p->max_depth + 3, p->n_lights, n_light_samples, &queue_oom);
-    while (st == VRJ_ERR_OUT_OF_MEMORY && queue_oom && batch > 1) { // 240 bytes per path in flight: halve the batch until the queues fit
-        vrj_pool_trim();
-        batch = (batch + 1) / 2;
-        st = ensure_scratch(s, npix * batch, records ? npix * batch : 0, npix, p->max_depth + 3, p->n_lights, n_light_samples, &queue_oom);
-    }
-    if (st == VRJ_ERR_OUT_OF_MEMORY && !queue_oom) { // the accumulators do not shrink with the batch: give cached blocks back, once
-        vrj_pool_trim();
-        st = ensure_scratch(s, npix * batch, records ? npix * batch : 0, npix, p->max_depth + 3, p->n_lights, n_light_samples, &queue_oom);
-    }
+    st = ensure_call_scratch(s, p, call_wants_records(scene, p, filter), npix, &batch, n_light_samples);
     if (st != VRJ_OK) return st;
 
     const cudaMemcpyKind in_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
@@ -1314,34 +1415,13 @@ VrjStatus vrj_render_tile(const VrjScene *scene_c, const VrjTile *tile, uint64_t
             VRJ_CUDA(cudaMemsetAsync(arrs[i].dev->p, 0, npix * arrs[i].per * sizeof(double), s->stream));
     }
     VRJ_CUDA(cudaMemsetAsync(s->stats.p, 0, ST_COUNT * sizeof(unsigned long long), s->stream));
-    if (p->n_lights || p->ambient_light) {
-        std::vector<LightDev> lights(p->n_lights + 1);
-        std::vector<double> lsamples;
-        auto put = [&lsamples](const VrjSpectrumData &sd) {
-            SpectrumDev d{sd.shortest_wavelength, sd.longest_wavelength, (uint32_t)lsamples.size(), sd.n_samples};
-            lsamples.insert(lsamples.end(), sd.samples, sd.samples + sd.n_samples);
-            return d;
-        };
-        for (uint32_t i = 0; i < p->n_lights; i++) {
-            for (int k = 0; k < 3; k++) lights[i].dir[k] = p->lights[i].direction[k];
-            lights[i].spectrum = put(p->lights[i].spectrum);
-        }
-        lights[p->n_lights] = LightDev{};
-        if (p->ambient_light) lights[p->n_lights].spectrum = put(*p->ambient_light);
-        VRJ_CUDA(cudaMemcpyAsync(s->lights.p, lights.data(), lights.size() * sizeof(LightDev), cudaMemcpyHostToDevice, s->stream));
-        if (!lsamples.empty())
-            VRJ_CUDA(cudaMemcpyAsync(s->light_samples.p, lsamples.data(), lsamples.size() * sizeof(double), cudaMemcpyHostToDevice, s->stream));
-        VRJ_CUDA(cudaStreamSynchronize(s->stream)); // the staging vectors are locals
-    }
+    st = stage_lights(s, p);
+    if (st != VRJ_OK) return st;
 
     RenderConst rc = make_render_const(tile, height, width, p);
     rc.lights = s->lights.as<LightDev>();
     rc.light_samples = s->light_samples.as<double>();
 
-    // F32X4: the staged rays walk the 4-wide tree; inline any-hit queries (Whitted shadow rays, k_tail) use the 2-wide f32 tree
-    const int quad = filter == VRJ_FILTER_F32X4 ? 1 : filter == VRJ_FILTER_Q16 ? 2 : 0;
-    // VRJ_PRECISION_F32_FAST: the whole sample in binary32 over the 2-wide f32 tree (no reference counterpart; not a parity mode)
-    const bool fast = p->precision == VRJ_PRECISION_F32_FAST;
     uint64_t launches = 0;
     s->n_marks = 0;
     RenderTurn turn(scene->device); // declared after `releaser`: an early return gives the turn back before the block
@@ -1365,15 +1445,7 @@ VrjStatus vrj_render_tile(const VrjScene *scene_c, const VrjTile *tile, uint64_t
         copied = copied || copy != nullptr;
         rc.div_batch = FastDiv::make(rc.batch_samples), rc.div_tile_w = FastDiv::make(rc.tile_w);
         rc.first_sample = p->sample_offset + (uint64_t)done * rc.sample_stride;
-        if (p->count_traversal) {
-            st = fast ? run_batch<float, float, true>(scene, s, rc, whitted, 0, &launches, nullptr, copy)
-                 : filter == VRJ_FILTER_F64 ? run_batch<double, double, true>(scene, s, rc, whitted, 0, &launches, nullptr, copy)
-                                            : run_batch<float, double, true>(scene, s, rc, whitted, quad, &launches, nullptr, copy);
-        } else {
-            st = fast ? run_batch<float, float, false>(scene, s, rc, whitted, 0, &launches, nullptr, copy)
-                 : filter == VRJ_FILTER_F64 ? run_batch<double, double, false>(scene, s, rc, whitted, 0, &launches, nullptr, copy)
-                                            : run_batch<float, double, false>(scene, s, rc, whitted, quad, &launches, nullptr, copy);
-        }
+        st = dispatch_batch(scene, s, rc, p, filter, &launches, copy, nullptr);
         if (st != VRJ_OK) return st;
         if (out->photons) {
             // debug output, batch-major: [(sample * npix + pixel) * 2]; the device keeps the batch pixel-major, so transpose
@@ -1398,13 +1470,8 @@ VrjStatus vrj_render_tile(const VrjScene *scene_c, const VrjTile *tile, uint64_t
                 VRJ_CUDA(cudaMemcpyAsync(arrs[i].user, arrs[i].dev->p, npix * arrs[i].per * sizeof(double), out_kind, s->stream));
     }
     if (out->srgb8) {
-        if (s->srgb8.bytes < npix * 3) {
-            s->srgb8.release();
-            VRJ_CUDA(s->srgb8.alloc(npix * 3));
-        }
-        k_tone_map<<<(unsigned)((npix + 255) / 256), 256, 0, s->stream>>>(s->acc_colour.as<double>(), s->srgb8.as<unsigned char>(), npix, 0);
-        launches++;
-        VRJ_CUDA(cudaMemcpyAsync(out->srgb8, s->srgb8.p, npix * 3, out_kind, s->stream));
+        st = copy_srgb8(s, npix, out->srgb8, out_kind, &launches);
+        if (st != VRJ_OK) return st;
     }
     const auto t_call2 = std::chrono::steady_clock::now();
     VRJ_CUDA(cudaEventRecord(s->ev_done, s->stream));
@@ -1421,21 +1488,145 @@ VrjStatus vrj_render_tile(const VrjScene *scene_c, const VrjTile *tile, uint64_t
         std::fprintf(stderr, "vrj_render_tile: setup %.3f ms, enqueue %.3f ms, wait %.3f ms (device %.3f ms, %llu launches)\n",
                      msd(t_call0, t_call1), msd(t_call1, t_call2), msd(t_call2, t_call3), ms, (unsigned long long)launches);
     }
-    if (out->stats) {
-        fill_stats(out->stats, hstats, launches, ms);
-        double cls_ms[6] = {0, 0, 0, 0, 0, 0}; // 0 T (camera rays), 1 T (bounce rays), 2 resolve, 3 shade, 4 raygen, 5 tail
-        uint64_t cls_n[6] = {0, 0, 0, 0, 0, 0};
-        for (size_t i = 1; i < s->n_marks; i++) {
-            int c = s->mark_class[i];
-            if (c < 0) continue;
-            float seg = 0.f;
-            if (cudaEventElapsedTime(&seg, s->marks[i - 1], s->marks[i]) == cudaSuccess) cls_ms[c] += seg, cls_n[c]++;
+    if (out->stats) fill_call_stats(out->stats, s, hstats, launches, ms);
+    return VRJ_OK;
+}
+
+// Adaptive sampling (the header states the passes and the stopping rule).  Pass j renders its `count` samples for the pixels of
+// its list -- the whole tile in pass 0, RenderConst::pixel_list after that -- in batches split to the path budget like
+// vrj_render_tile's, and k_resolve_adaptive applies them to the tile's accumulators and y_sq_sum.  k_adaptive_select then
+// judges the list's pixels, an exclusive scan (vrj_build::exclusive_scan_u32) of its flags gives every continuing pixel its
+// place, and k_adaptive_compact writes the next list in tile order.  The host reads back one count per pass and copies the
+// arrays out once, at the end.
+VrjStatus vrj_render_adaptive(const VrjScene *scene_c, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p,
+                              const VrjAdaptiveParams *ap, VrjAccumOut *out, double *y_sq_sum, VrjAdaptiveStats *astats) {
+    VrjScene *scene = const_cast<VrjScene *>(scene_c);
+    size_t n_light_samples = 0;
+    VrjStatus st = check_render_args(scene, tile, height, width, p, out, &n_light_samples);
+    if (st != VRJ_OK) return st;
+    if (!ap) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (p->spp != 0) return fail(VRJ_ERR_INVALID_ARGUMENT, "params->spp must be 0: vrj_render_adaptive takes its sample counts from VrjAdaptiveParams");
+    if (ap->min_samples < 2) return fail(VRJ_ERR_INVALID_ARGUMENT, "min_samples must be >= 2 (the variance needs two samples)");
+    if (ap->max_samples < ap->min_samples) return fail(VRJ_ERR_INVALID_ARGUMENT, "max_samples must be >= min_samples");
+    if (ap->pass_samples < 1) return fail(VRJ_ERR_INVALID_ARGUMENT, "pass_samples must be >= 1");
+    if (!(ap->rel_error > 0.0) || !std::isfinite(ap->rel_error)) return fail(VRJ_ERR_INVALID_ARGUMENT, "rel_error must be > 0 and finite");
+    if (!(ap->abs_floor >= 0.0) || !std::isfinite(ap->abs_floor)) return fail(VRJ_ERR_INVALID_ARGUMENT, "abs_floor must be >= 0 and finite");
+    if (out->accumulate) return fail(VRJ_ERR_UNSUPPORTED, "vrj_render_adaptive does not continue from a previous state (accumulate)");
+    if (out->photons) return fail(VRJ_ERR_UNSUPPORTED, "vrj_render_adaptive has no photons output");
+    const uint64_t npix = (tile->end_column - tile->start_column) * (tile->end_row - tile->start_row);
+    DeviceGuard device_guard;
+    VRJ_NVTX_RANGE(call_range, "vrj_render_adaptive");
+    if (out->stats) std::memset(out->stats, 0, sizeof(VrjStats));
+    if (astats) std::memset(astats, 0, sizeof(VrjAdaptiveStats));
+    if (npix == 0) return VRJ_OK;
+    VRJ_CUDA(cudaSetDevice(scene->device));
+
+    ActiveCall active(g_active_calls[(unsigned)scene->device % 64]);
+    // the largest pass renders every pixel (min_samples) or a subset (pass_samples): the block is sized for the larger of the two
+    const uint32_t widest = std::min(ap->max_samples, std::max(ap->min_samples, ap->pass_samples));
+    uint32_t batch = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(widest, call_path_budget(scene, active) / npix));
+    if (npix * (uint64_t)batch > 0xfffffff0ull) return fail(VRJ_ERR_UNSUPPORTED, "tile too large");
+    Scratch *s = acquire_scratch(scene, npix * batch);
+    struct Releaser {
+        VrjScene *sc;
+        Scratch *s;
+        ~Releaser() {
+            if (s->stream) cudaStreamSynchronize(s->stream);
+            release_scratch(sc, s);
         }
-        out->stats->primary_ms = cls_ms[0], out->stats->bounce_ms = cls_ms[1], out->stats->resolve_ms = cls_ms[2];
-        out->stats->primary_launches = cls_n[0], out->stats->bounce_launches = cls_n[1], out->stats->resolve_launches = cls_n[2];
-        out->stats->shade_ms = cls_ms[3] + cls_ms[4], out->stats->shade_launches = cls_n[3] + cls_n[4];
-        out->stats->tail_ms = cls_ms[5], out->stats->tail_launches = cls_n[5];
-        out->stats->coalesced_calls = 1;
+    } releaser{scene, s};
+    const uint32_t filter = effective_filter(scene, p);
+    st = ensure_call_scratch(s, p, call_wants_records(scene, p, filter), npix, &batch, n_light_samples);
+    if (st != VRJ_OK) return st;
+    if (s->adapt_npix < npix) {
+        s->adapt_npix = 0;
+        std::vector<std::pair<DeviceBuffer *, size_t>> want = {{&s->ysq, npix * 8}, {&s->alist[0], npix * 4}, {&s->alist[1], npix * 4},
+                                                               {&s->aconverged, 8}};
+        st = alloc_group(s->adapt_slab, want, "adaptive sampling buffers");
+        if (st != VRJ_OK) return st;
+        s->adapt_npix = npix;
+    }
+    const size_t capacity = npix * batch; // paths per batch
+    DeviceBuffer *zero[5] = {&s->acc_sum, &s->acc_bias, &s->acc_weight, &s->acc_wbias, &s->ysq};
+    const size_t per[5] = {3, 3, 1, 1, 1};
+    for (int i = 0; i < 5; i++) VRJ_CUDA(cudaMemsetAsync(zero[i]->p, 0, npix * per[i] * sizeof(double), s->stream));
+    VRJ_CUDA(cudaMemsetAsync(s->aconverged.p, 0, sizeof(unsigned long long), s->stream));
+    VRJ_CUDA(cudaMemsetAsync(s->stats.p, 0, ST_COUNT * sizeof(unsigned long long), s->stream));
+    st = stage_lights(s, p);
+    if (st != VRJ_OK) return st;
+
+    RenderConst rc = make_render_const(tile, height, width, p);
+    rc.lights = s->lights.as<LightDev>();
+    rc.light_samples = s->light_samples.as<double>();
+    rc.div_tile_w = FastDiv::make(rc.tile_w);
+    // the flags and the scan's tile totals live in the photon buffer, which is free between a pass's resolve and the next
+    // batch: (n + 1) + (n / 2048 + 2) uint32 fit the 16 bytes per path of a block that holds at least one path per pixel
+    uint32_t *flags = s->photons.as<uint32_t>();
+    uint32_t *host_active = s->host_count + 192; // pinned slots (host_count: 0..3 drain check, 8.. sample table, 160.. stats)
+    unsigned long long *host_converged = reinterpret_cast<unsigned long long *>(s->host_count + 194);
+    uint64_t launches = 0, passes = 0, samples = 0;
+    uint32_t n_active = (uint32_t)npix, held = 0, count = ap->min_samples, cur = 0;
+    const uint32_t *list = nullptr; // pass 0: the whole tile
+    s->n_marks = 0;
+    RenderTurn turn(scene->device); // declared after `releaser`: an early return gives the turn back before the block
+    turn.acquire();
+    VRJ_CUDA(cudaEventRecord(s->ev0, s->stream));
+    for (;;) {
+        const uint32_t b = (uint32_t)std::max<size_t>(1, std::min<size_t>(count, capacity / n_active));
+        rc.npix = n_active, rc.pixel_list = list;
+        for (uint32_t done = 0; done < count; done += b) {
+            rc.batch_samples = std::min(b, count - done);
+            rc.div_batch = FastDiv::make(rc.batch_samples);
+            rc.first_sample = p->sample_offset + (uint64_t)(held + done) * rc.sample_stride;
+            st = dispatch_batch(scene, s, rc, p, filter, &launches, nullptr, s->ysq.as<double>());
+            if (st != VRJ_OK) return st;
+        }
+        held += count, passes++, samples += (uint64_t)n_active * count;
+        const uint32_t more = held < ap->max_samples ? 1u : 0u;
+        k_adaptive_select<<<(n_active + 1 + 255) / 256, 256, 0, s->stream>>>(s->acc_sum.as<double>(), s->acc_weight.as<double>(), s->ysq.as<double>(), list, n_active,
+                                                                          ap->rel_error, ap->abs_floor, more, flags, s->aconverged.as<unsigned long long>());
+        launches++;
+        VRJ_CUDA(cudaGetLastError());
+        if (!more) break;
+        st = vrj_build::exclusive_scan_u32(flags, n_active + 1, flags + n_active + 1, s->stream);
+        if (st != VRJ_OK) return st;
+        launches += 3;
+        k_adaptive_compact<<<(n_active + 255) / 256, 256, 0, s->stream>>>(list, flags, n_active, s->alist[cur].as<uint32_t>());
+        launches++;
+        VRJ_CUDA(cudaGetLastError());
+        VRJ_CUDA(cudaMemcpyAsync(host_active, flags + n_active, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
+        VRJ_CUDA(cudaStreamSynchronize(s->stream));
+        if (*host_active == 0) break;
+        n_active = *host_active, list = s->alist[cur].as<uint32_t>(), cur ^= 1u;
+        count = std::min(ap->pass_samples, ap->max_samples - held);
+    }
+    unsigned long long *hstats = reinterpret_cast<unsigned long long *>(s->host_count + 160);
+    VRJ_CUDA(cudaEventRecord(s->ev1, s->stream));
+    VRJ_CUDA(cudaMemcpyAsync(hstats, s->stats.p, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+    VRJ_CUDA(cudaMemcpyAsync(host_converged, s->aconverged.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+    const cudaMemcpyKind out_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    struct Arr {
+        double *user;
+        DeviceBuffer *dev;
+        size_t per;
+    } arrs[6] = {{out->colour, &s->acc_colour, 3}, {out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3},
+                 {out->weight, &s->acc_weight, 1}, {out->weight_bias, &s->acc_wbias, 1}, {y_sq_sum, &s->ysq, 1}};
+    for (const Arr &a : arrs)
+        if (a.user) VRJ_CUDA(cudaMemcpyAsync(a.user, a.dev->p, npix * a.per * sizeof(double), out_kind, s->stream));
+    if (out->srgb8) {
+        st = copy_srgb8(s, npix, out->srgb8, out_kind, &launches);
+        if (st != VRJ_OK) return st;
+    }
+    VRJ_CUDA(cudaEventRecord(s->ev_done, s->stream));
+    VRJ_CUDA(wait_event(s->ev1, scene->device)); // the last kernel is done: the next caller may render while this one's copies run
+    turn.release();
+    VRJ_CUDA(wait_event(s->ev_done, scene->device));
+    float ms = 0.f;
+    VRJ_CUDA(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+    if (out->stats) fill_call_stats(out->stats, s, hstats, launches, ms);
+    if (astats) {
+        astats->passes = passes, astats->samples = samples;
+        astats->pixels_converged = *host_converged, astats->pixels_unconverged = npix - *host_converged;
     }
     return VRJ_OK;
 }

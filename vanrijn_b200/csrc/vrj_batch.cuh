@@ -81,6 +81,8 @@ struct Scratch {
     DeviceBuffer queue_slab, rec_slab, acc_slab; // the groups above live in one allocation each (see ensure_scratch)
     DeviceBuffer multi_out, sample_table; // coalesced calls: their output arrays (call-major pieces) and the batch's sample indices
     DeviceBuffer lights, light_samples, srgb8;
+    DeviceBuffer ysq, alist[2], aconverged, adapt_slab; // vrj_render_adaptive: y_sq_sum, this / next pass's pixel list, a counter
+    size_t adapt_npix = 0;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr; // first / last kernel of a call
     cudaEvent_t ev_done = nullptr;             // behind the call's last copy
@@ -183,9 +185,9 @@ inline bool wants_records(const VrjScene *sc, int walk) {
 }
 
 // One batch with the integrator (WHITTED) and the scene's material kinds (MM, see vrj_device.cuh) fixed at compile time.
-template <typename NT, typename R, bool COUNT, bool WHITTED, int MM>
+template <typename NT, typename R, bool COUNT, bool WHITTED, int MM, bool LIST>
 VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int walk, uint64_t *launches, const MultiCalls *multi,
-                     const ResolveCopy *copy) {
+                     const ResolveCopy *copy, double *ysq) {
     const bool quad = walk == 1, q16 = walk == 2; // 0: the 2-wide tree in NT boxes; 1: 4-wide f32; 2: 2-wide on the 16-bit grid
     // launch sequence: G T S_0 [X_k T_k S_k]*, k = 1..levels (X = k_tail, a no-op until the queue is short);
     // SimpleRandom needs max_depth levels, Whitted one more (its limit-0 level still shades and traces);
@@ -200,14 +202,14 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
     VRJ_CUDA(cudaMemsetAsync(qcount, 0, ((size_t)stride * 5 + 2) * sizeof(uint32_t), s->stream));
     unsigned long long *stats = s->stats.as<unsigned long long>();
     double2 *photons = s->photons.as<double2>();
-    const int g_gen = persistent_grid(sc, k_raygen<R, COUNT>), g_t = quad ? persistent_grid(sc, k_trace4<COUNT, false>) : q16 ? persistent_grid(sc, k_traceq<COUNT, false>) : persistent_grid(sc, k_trace<NT, R, COUNT>);
-    const int g_t0 = quad ? persistent_grid(sc, k_trace4<COUNT, true>) : q16 ? persistent_grid(sc, k_traceq<COUNT, true>) : persistent_grid(sc, k_trace_primary<NT, R, COUNT>);
-    const int g_s0 = persistent_grid(sc, k_shade<NT, R, COUNT, WHITTED, true, MM>);
-    const int g_s = persistent_grid(sc, k_shade<NT, R, COUNT, WHITTED, false, MM>);
+    const int g_gen = persistent_grid(sc, k_raygen<R, COUNT, LIST>), g_t = quad ? persistent_grid(sc, k_trace4<COUNT, false>) : q16 ? persistent_grid(sc, k_traceq<COUNT, false>) : persistent_grid(sc, k_trace<NT, R, COUNT>);
+    const int g_t0 = quad ? persistent_grid(sc, k_trace4<COUNT, true, LIST>) : q16 ? persistent_grid(sc, k_traceq<COUNT, true, LIST>) : persistent_grid(sc, k_trace_primary<NT, R, COUNT, LIST>);
+    const int g_s0 = persistent_grid(sc, k_shade<NT, R, COUNT, WHITTED, true, MM, LIST>);
+    const int g_s = persistent_grid(sc, k_shade<NT, R, COUNT, WHITTED, false, MM, LIST>);
     // k_tail pays off for deep recursion limits (the reference's 128: 260 launches -> 28); at depth <= 12 the
     // per-level latency it removes is smaller than what its one-thread-per-path traversal costs (measured)
     const uint32_t tail_max = levels > 12 ? sc->tail_max : sc->tail_max_shallow;
-    const int g_x = tail_max ? persistent_grid(sc, k_tail<NT, R, COUNT, WHITTED, MM>) : 0; // persistent warps, per-lane refill
+    const int g_x = tail_max ? persistent_grid(sc, k_tail<NT, R, COUNT, WHITTED, MM, LIST>) : 0; // persistent warps, per-lane refill
     uint32_t *tail_work = tail_done + 1 + stride;   // k_tail's work-fetch counter (after the k_stage counters)
     const bool has_bvh = sc->dev.n_bvh_items > 0;
     // the default walk of the parity path takes its rays as ready-to-walk records (TraceRec); the other walks form the
@@ -218,19 +220,19 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
     VRJ_NVTX_RANGE(batch_range, "vrj batch");
     VRJ_CUDA(s->mark(-1));
     // the raygen kernel uses work_s[0]; S_0 uses work_t[stride-1] (never used by a T)
-    k_raygen<R, COUNT><<<g_gen, 128, 0, s->stream>>>(sc->dev, rc, s->queue(0), tb0, lcount + 0, work_s + 0, stats);
+    k_raygen<R, COUNT, LIST><<<g_gen, 128, 0, s->stream>>>(sc->dev, rc, s->queue(0), tb0, lcount + 0, work_s + 0, stats);
     (*launches)++;
     VRJ_CUDA(s->mark(4));
     if (has_bvh) {
         if (rec) k_trace_rec<COUNT><<<g_tr, 128, 0, s->stream>>>(sc->dev, tb0, lcount + 0, work_t + 0, stats, tail_done);
-        else if (quad) k_trace4<COUNT, true><<<g_t0, 128, 0, s->stream>>>(sc->dev, rc, s->queue(0), tb0, lcount + 0, work_t + 0, stats, tail_done);
-        else if (q16) k_traceq<COUNT, true><<<g_t0, 128, 0, s->stream>>>(sc->dev, rc, s->queue(0), tb0, lcount + 0, work_t + 0, stats, tail_done);
-        else k_trace_primary<NT, R, COUNT><<<g_t0, 128, 0, s->stream>>>(sc->dev, rc, tb0, lcount + 0, work_t + 0, stats);
+        else if (quad) k_trace4<COUNT, true, LIST><<<g_t0, 128, 0, s->stream>>>(sc->dev, rc, s->queue(0), tb0, lcount + 0, work_t + 0, stats, tail_done);
+        else if (q16) k_traceq<COUNT, true, LIST><<<g_t0, 128, 0, s->stream>>>(sc->dev, rc, s->queue(0), tb0, lcount + 0, work_t + 0, stats, tail_done);
+        else k_trace_primary<NT, R, COUNT, LIST><<<g_t0, 128, 0, s->stream>>>(sc->dev, rc, tb0, lcount + 0, work_t + 0, stats);
         (*launches)++;
         VRJ_CUDA(s->mark(0));
     }
     uint32_t *work_s0 = work_t + (stride - 1);
-    k_shade<NT, R, COUNT, WHITTED, true, MM><<<g_s0, 128, 0, s->stream>>>(sc->dev, rc, s->queue(0), nullptr, tb0, s->queue(1), qcount + 1, tb1, lcount + 1, work_s0, photons, stats, tail_done);
+    k_shade<NT, R, COUNT, WHITTED, true, MM, LIST><<<g_s0, 128, 0, s->stream>>>(sc->dev, rc, s->queue(0), nullptr, tb0, s->queue(1), qcount + 1, tb1, lcount + 1, work_s0, photons, stats, tail_done);
     (*launches)++;
     VRJ_CUDA(s->mark(3));
     bool drain_pending = false;
@@ -247,7 +249,7 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
         VRJ_CUDA(s->mark(4));
 #endif
         if (tail_max) {
-            k_tail<NT, R, COUNT, WHITTED, MM><<<g_x, 128, 0, s->stream>>>(sc->dev, rc, s->queue(ci), qcount + k, tail_max, photons, stats, tail_done, tail_work);
+            k_tail<NT, R, COUNT, WHITTED, MM, LIST><<<g_x, 128, 0, s->stream>>>(sc->dev, rc, s->queue(ci), qcount + k, tail_max, photons, stats, tail_done, tail_work);
             (*launches)++;
             VRJ_CUDA(s->mark(5));
         }
@@ -260,7 +262,7 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
             (*launches)++;
             VRJ_CUDA(s->mark(1));
         }
-        k_shade<NT, R, COUNT, WHITTED, false, MM><<<g_s, 128, 0, s->stream>>>(sc->dev, rc, s->queue(ci), qcount + k, ci ? tb1 : tb0, s->queue(ni), qcount + k + 1, ni ? tb1 : tb0, lcount + k + 1, work_s + k, photons, stats, tail_done);
+        k_shade<NT, R, COUNT, WHITTED, false, MM, LIST><<<g_s, 128, 0, s->stream>>>(sc->dev, rc, s->queue(ci), qcount + k, ci ? tb1 : tb0, s->queue(ni), qcount + k + 1, ni ? tb1 : tb0, lcount + k + 1, work_s + k, photons, stats, tail_done);
         (*launches)++;
         VRJ_CUDA(s->mark(3));
         // Deep recursion limits (the reference's 128): stop launching once the batch has drained (queue empty, or finished
@@ -286,6 +288,9 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
     acc.weight = s->acc_weight.as<double>(), acc.weight_bias = s->acc_wbias.as<double>();
     if (multi) {
         k_resolve_multi<R><<<(rc.npix * multi->n + 255) / 256, 256, 0, s->stream>>>(*multi, photons, rc.npix, rc.batch_samples);
+        (*launches)++;
+    } else if (ysq) {
+        k_resolve_adaptive<R><<<(rc.npix + 255) / 256, 256, 0, s->stream>>>(acc, ysq, rc.pixel_list, photons, rc.npix, rc.batch_samples);
         (*launches)++;
     } else if (copy && copy->pieces > 1) {
         const double *dev[5] = {acc.colour, acc.sum, acc.bias, acc.weight, acc.weight_bias};
@@ -315,15 +320,23 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
 
 // kernel variants exist for "Lambertian only" (the reference's own scenes: main.rs, benches/simple_scene.rs) and for
 // "any material"; VRJ_MATERIAL_MASK=15 in the environment forces the general variant (experiments)
-template <typename NT, typename R, bool COUNT>
-VrjStatus run_batch(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches, const MultiCalls *multi = nullptr,
-                    const ResolveCopy *copy = nullptr) {
+template <typename NT, typename R, bool COUNT, bool LIST>
+VrjStatus run_materials(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches, const MultiCalls *multi,
+                        const ResolveCopy *copy, double *ysq) {
     const bool lambert_only = sc->kernel_material_mask == 1u;
     if (whitted)
-        return lambert_only ? run_levels<NT, R, COUNT, true, 1>(sc, s, rc, walk, launches, multi, copy)
-                            : run_levels<NT, R, COUNT, true, VRJ_MM_ALL>(sc, s, rc, walk, launches, multi, copy);
-    return lambert_only ? run_levels<NT, R, COUNT, false, 1>(sc, s, rc, walk, launches, multi, copy)
-                        : run_levels<NT, R, COUNT, false, VRJ_MM_ALL>(sc, s, rc, walk, launches, multi, copy);
+        return lambert_only ? run_levels<NT, R, COUNT, true, 1, LIST>(sc, s, rc, walk, launches, multi, copy, ysq)
+                            : run_levels<NT, R, COUNT, true, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches, multi, copy, ysq);
+    return lambert_only ? run_levels<NT, R, COUNT, false, 1, LIST>(sc, s, rc, walk, launches, multi, copy, ysq)
+                        : run_levels<NT, R, COUNT, false, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches, multi, copy, ysq);
+}
+// `ysq` (vrj_render_adaptive): the batch is resolved by k_resolve_adaptive, which also keeps y_sq_sum; a batch over
+// rc.pixel_list runs the LIST variants of the kernels
+template <typename NT, typename R, bool COUNT>
+VrjStatus run_batch(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches, const MultiCalls *multi = nullptr,
+                    const ResolveCopy *copy = nullptr, double *ysq = nullptr) {
+    return rc.pixel_list ? run_materials<NT, R, COUNT, true>(sc, s, rc, whitted, walk, launches, multi, copy, ysq)
+                         : run_materials<NT, R, COUNT, false>(sc, s, rc, whitted, walk, launches, multi, copy, ysq);
 }
 
 } // namespace vrjimpl

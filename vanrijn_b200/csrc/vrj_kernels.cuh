@@ -118,6 +118,9 @@ struct RenderConst {
     double film_w, film_h;
     const LightDev *lights;      // n_lights entries, then (if has_ambient) the ambient light's spectrum in entry n_lights
     const double *light_samples;
+    const uint32_t *pixel_list;  // kernels with LIST = true: batch position p renders tile pixel pixel_list[p] and npix is the
+                                 // list's length (the still-active pixels of an adaptive pass, vrj_render_adaptive); slots and
+                                 // photons stay indexed by list position
 };
 
 template <typename R>
@@ -183,9 +186,12 @@ __device__ __forceinline__ void biased_ray(V3<R> origin, V3<R> direction, R amou
 // same nodes (broadcast loads), hits the same primitive class, and the first bounces leave from neighbouring points
 // (k_trace on camera rays 3.5 -> 2.5 ms per 32-spp step, measured).  A sample is still a pure function of
 // (seed, pixel, sample index), so the order changes no result.
+// LIST: the batch covers the pixels of rc.pixel_list (a compile-time switch, so the tile's kernels carry no trace of it).
+template <bool LIST = false>
 __device__ __forceinline__ void slot_to_pixel(const RenderConst &rc, uint32_t slot, uint32_t &pixel_global,
                                               uint64_t &sample, uint64_t &grow, uint64_t &gcol) {
     uint32_t p = rc.div_batch.div(slot), s = slot - p * rc.batch_samples;
+    if (LIST) p = __ldg(rc.pixel_list + p);
     uint32_t row = rc.div_tile_w.div(p), col = p - row * rc.tile_w;
     grow = rc.start_row + row, gcol = rc.start_column + col;
     pixel_global = (uint32_t)(grow * rc.width + gcol);
@@ -225,11 +231,11 @@ __device__ __forceinline__ void stage_ray(const DevScene &sc, bool have_ray, uin
 // The camera ray of a result slot (camera.rs:45-66): two Philox draws, the film point, Ray::new.  It is a pure function of
 // the slot, so the primary level never stores it: k_raygen, k_trace on camera rays and the first k_shade each form it again
 // (one Philox block + one normalisation) instead of moving 48 bytes per ray through HBM three times.
-template <typename R>
+template <typename R, bool LIST = false>
 __device__ __forceinline__ void camera_ray(const DevScene &sc, const RenderConst &rc, uint32_t slot, V3<R> &o, V3<R> &d) {
     uint32_t pixel;
     uint64_t sample, grow, gcol;
-    slot_to_pixel(rc, slot, pixel, sample, grow, gcol);
+    slot_to_pixel<LIST>(rc, slot, pixel, sample, grow, gcol);
     Rng rng;
     rng.init(rc.seed, pixel, sample, 0);
     R ux = rng.uniform<R>(), uy = rng.uniform<R>();
@@ -241,7 +247,7 @@ __device__ __forceinline__ void camera_ray(const DevScene &sc, const RenderConst
 }
 
 // ---- k_raygen: camera rays (camera.rs:45-66), staged for traversal ----
-template <typename R, bool COUNT>
+template <typename R, bool COUNT, bool LIST = false>
 __global__ void __launch_bounds__(128, sizeof(R) == 4 ? VRJ_SHADE_MINB_F32 : VRJ_RAYGEN_MINB) k_raygen(DevScene sc, RenderConst rc, PathQueue q, TraceBuffers tb, uint32_t *list_count,
                                                 uint32_t *work, unsigned long long *stats) {
     const uint32_t n = rc.npix * rc.batch_samples;
@@ -261,7 +267,7 @@ __global__ void __launch_bounds__(128, sizeof(R) == 4 ? VRJ_SHADE_MINB_F32 : VRJ
             if (base + (k & ~31u) >= n) break; // the whole warp is past the end
             V3<R> o = V3<R>{R(0), R(0), R(0)}, d = V3<R>{R(0), R(0), R(1)};
             if (j < n) {
-                camera_ray(sc, rc, j, o, d);
+                camera_ray<R, LIST>(sc, rc, j, o, d);
                 ls.v[ST_PRIMARY]++;
             }
             stage_ray<COUNT>(sc, j < n, j, o, d, tb, list_count, ls);
@@ -306,6 +312,7 @@ struct RecHitSink {
     }
 };
 // the same for the camera rays of a batch: the ray is formed from its slot, nothing is read from the queue
+template <bool LIST = false>
 struct PrimaryRaySource {
     const DevScene &sc;
     const RenderConst &rc;
@@ -313,7 +320,7 @@ struct PrimaryRaySource {
     template <typename R>
     __device__ __forceinline__ void load(uint32_t r, V3<R> &o, V3<R> &d, HitT<R> &best) {
         uint32_t j = tb.list[r];
-        camera_ray(sc, rc, j, o, d);
+        camera_ray<R, LIST>(sc, rc, j, o, d);
         int2 h = tb.hits[j];
         best.item = h.x, best.tri = h.y, best.t = (R)tb.tbest[j];
     }
@@ -355,11 +362,11 @@ __global__ void VRJ_TRACE_BOUNDS(R) k_trace(DevScene sc, PathQueue q, TraceBuffe
 }
 
 // k_trace for the camera rays of a batch
-template <typename NT, typename R, bool COUNT>
+template <typename NT, typename R, bool COUNT, bool LIST = false>
 __global__ void VRJ_TRACE_BOUNDS(R) k_trace_primary(DevScene sc, RenderConst rc, TraceBuffers tb, const uint32_t *list_count, uint32_t *work,
                                                     unsigned long long *stats) {
     const uint32_t n = *list_count;
-    PrimaryRaySource source{sc, rc, tb};
+    PrimaryRaySource<LIST> source{sc, rc, tb};
     ListHitSink sink{tb};
     TraceCounters tc = {0, 0};
     trace_persistent<NT, R, COUNT>(sc, n, work, source, sink, tc);
@@ -390,7 +397,7 @@ __global__ void VRJ_TRACE_BOUNDS(double) k_trace_rec(DevScene sc, TraceBuffers t
 }
 
 // the same launch over the 4-wide form of the tree (VRJ_FILTER_F32X4)
-template <bool COUNT, bool PRIMARY>
+template <bool COUNT, bool PRIMARY, bool LIST = false>
 __global__ void __launch_bounds__(128, VRJ_TRACE4_MINB) k_trace4(DevScene sc, RenderConst rc, PathQueue q, TraceBuffers tb, const uint32_t *list_count,
                                                                  uint32_t *work, unsigned long long *stats, const uint32_t *tail_done) {
     if (tail_done && *tail_done) return;
@@ -398,7 +405,7 @@ __global__ void __launch_bounds__(128, VRJ_TRACE4_MINB) k_trace4(DevScene sc, Re
     ListHitSink sink{tb};
     TraceCounters tc = {0, 0};
     if (PRIMARY) {
-        PrimaryRaySource source{sc, rc, tb};
+        PrimaryRaySource<LIST> source{sc, rc, tb};
         trace_persistent_quad<COUNT>(sc, n, work, source, sink, tc);
     } else {
         ListRaySource source{q, tb};
@@ -413,7 +420,7 @@ __global__ void __launch_bounds__(128, VRJ_TRACE4_MINB) k_trace4(DevScene sc, Re
 }
 
 // the same launch over 16-bit nodes (VRJ_FILTER_Q16)
-template <bool COUNT, bool PRIMARY>
+template <bool COUNT, bool PRIMARY, bool LIST = false>
 __global__ void __launch_bounds__(128, VRJ_TRACE_MINB) k_traceq(DevScene sc, RenderConst rc, PathQueue q, TraceBuffers tb, const uint32_t *list_count,
                                                                 uint32_t *work, unsigned long long *stats, const uint32_t *tail_done) {
     if (tail_done && *tail_done) return;
@@ -421,7 +428,7 @@ __global__ void __launch_bounds__(128, VRJ_TRACE_MINB) k_traceq(DevScene sc, Ren
     ListHitSink sink{tb};
     TraceCounters tc = {0, 0};
     if (PRIMARY) {
-        PrimaryRaySource source{sc, rc, tb};
+        PrimaryRaySource<LIST> source{sc, rc, tb};
         trace_persistent_q16<COUNT>(sc, n, work, source, sink, tc);
     } else {
         ListRaySource source{q, tb};
@@ -451,7 +458,7 @@ __device__ __forceinline__ double2 photon_out(R wavelength, R intensity) { retur
 // shadow rays), update the affine accumulator -- leaves the bounce ray and the new state in p and returns true.
 // `first`: p.slot is set, the rest of the state is initialised here (camera.rs:108-119).
 // `load_ray(o, d)` fetches the ray only when it is needed.
-template <typename NT, bool COUNT, bool WHITTED, int MM, typename R, typename RayLoader>
+template <typename NT, bool COUNT, bool WHITTED, int MM, bool LIST, typename R, typename RayLoader>
 __device__ __forceinline__ bool shade_entry(const DevScene &sc, const RenderConst &rc, PathRegsT<R> &p, int2 hit, R hit_t, bool first,
                                             RayLoader load_ray, double2 *photons, LocalStats &ls) {
     const R span = R(740.0) - R(380.0); // photon.rs:18-24, colour/mod.rs:13-14
@@ -463,7 +470,7 @@ __device__ __forceinline__ bool shade_entry(const DevScene &sc, const RenderCons
         }
         uint32_t pixel;
         uint64_t sample, grow, gcol;
-        slot_to_pixel(rc, p.slot, pixel, sample, grow, gcol);
+        slot_to_pixel<LIST>(rc, p.slot, pixel, sample, grow, gcol);
         Rng rng;
         rng.init(rc.seed, pixel, sample, 2);
         p.wl = R(380.0) + span * rng.uniform<R>(); // photon.rs:18-24
@@ -535,7 +542,7 @@ __device__ __forceinline__ bool shade_entry(const DevScene &sc, const RenderCons
     Rng rng;
     uint32_t pixel;
     uint64_t sample, grow, gcol;
-    slot_to_pixel(rc, p.slot, pixel, sample, grow, gcol);
+    slot_to_pixel<LIST>(rc, p.slot, pixel, sample, grow, gcol);
     rng.init(rc.seed, pixel, sample, p.ordinal);
     V3<R> w_s;
     R pdf;
@@ -566,7 +573,7 @@ __device__ __forceinline__ bool shade_entry(const DevScene &sc, const RenderCons
 }
 
 // ---- k_shade: consume the hits of a queue; survivors are enqueued warp-ballot compacted and staged ----
-template <typename NT, typename R, bool COUNT, bool WHITTED, bool FIRST, int MM>
+template <typename NT, typename R, bool COUNT, bool WHITTED, bool FIRST, int MM, bool LIST = false>
 __global__ void VRJ_SHADE_BOUNDS(R) k_shade(DevScene sc, RenderConst rc, PathQueue in, const uint32_t *in_count,
                                                TraceBuffers tb_in, PathQueue out, uint32_t *out_count, TraceBuffers tb_out,
                                                uint32_t *list_count, uint32_t *work, double2 *photons,
@@ -627,10 +634,10 @@ __global__ void VRJ_SHADE_BOUNDS(R) k_shade(DevScene sc, RenderConst rc, PathQue
                     p.wl = (R)a3.x, p.A = (R)a3.y, p.B = (R)a4.x, p.aux = (R)a4.y;
                     p.slot = a5.x, p.ordinal = a5.y, p.limit = a5.z, p.flags = a5.w;
                 }
-                alive = shade_entry<NT, COUNT, WHITTED, MM>(
+                alive = shade_entry<NT, COUNT, WHITTED, MM, LIST>(
                     sc, rc, p, hit, hit.x >= 0 ? (R)tb_in.tbest[j] : R(0), FIRST,
                     [&in, &sc, &rc, j](V3<R> &o, V3<R> &d) {
-                        if (FIRST) camera_ray(sc, rc, j, o, d); // never stored: see camera_ray
+                        if (FIRST) camera_ray<R, LIST>(sc, rc, j, o, d); // never stored: see camera_ray
                         else queue_load_ray(in, j, o, d);
                     },
                     photons, ls);
@@ -682,7 +689,7 @@ __global__ void __launch_bounds__(128, VRJ_STAGE_MINB) k_stage(DevScene sc, Path
 // run for dozens), so a lane whose path has ended takes the next queue entry at once (one warp-aggregated atomic) instead
 // of idling until the longest path of its warp is done -- in the one-path-per-thread form a warp ran ~6 bounces for ~1.7
 // useful ones per lane.
-template <typename NT, typename R, bool COUNT, bool WHITTED, int MM>
+template <typename NT, typename R, bool COUNT, bool WHITTED, int MM, bool LIST = false>
 __global__ void __launch_bounds__(128, 2) k_tail(DevScene sc, RenderConst rc, PathQueue in, const uint32_t *in_count,
                                               uint32_t tail_max, double2 *photons, unsigned long long *stats,
                                               uint32_t *tail_done, uint32_t *work) {
@@ -726,7 +733,7 @@ __global__ void __launch_bounds__(128, 2) k_tail(DevScene sc, RenderConst rc, Pa
             // one lane, one path: what it waits on is the chain of dependent node fetches, and the 4-wide tree halves it
             HitT<R> h = trace_closest<NT, COUNT, false, R, VRJ_TAIL_QUAD != 0>(sc, p.o, p.d, tc);
             if (COUNT) ls.v[ST_NODES] += tc.node_visits, ls.v[ST_TRIS] += tc.tri_tests;
-            alive = shade_entry<NT, COUNT, WHITTED, MM>(sc, rc, p, make_int2(h.item, h.tri), h.t, false, [](V3<R> &, V3<R> &) {}, photons, ls);
+            alive = shade_entry<NT, COUNT, WHITTED, MM, LIST>(sc, rc, p, make_int2(h.item, h.tri), h.t, false, [](V3<R> &, V3<R> &) {}, photons, ls);
         }
     }
     ls.flush(stats);
@@ -770,6 +777,73 @@ __global__ void k_resolve(AccumDev acc, const double2 *photons, uint32_t first, 
     acc.weight[p] = w, acc.weight_bias[p] = wb;
     double inv = 1.0 / w;
     acc.colour[3 * p] = sx * inv, acc.colour[3 * p + 1] = sy * inv, acc.colour[3 * p + 2] = sz * inv;
+}
+
+// k_resolve for one pass of an adaptive render (vrj_render_adaptive): list position i holds tile pixel list[i] (pixel i when
+// `list` is NULL) and its samples are the batch's slots i * batch_samples + s.  Besides the Kahan update it keeps
+// ysq[pixel] = ysq + y * y in sample order, y being the sample's Y exactly as it enters colour_sum (the noise estimate of
+// k_adaptive_select).
+template <typename R>
+__global__ void k_resolve_adaptive(AccumDev acc, double *ysq, const uint32_t *list, const double2 *photons, uint32_t n, uint32_t batch_samples) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t p = list ? list[i] : i;
+    double sx = acc.sum[3 * p], sy = acc.sum[3 * p + 1], sz = acc.sum[3 * p + 2];
+    double bx = acc.bias[3 * p], by = acc.bias[3 * p + 1], bz = acc.bias[3 * p + 2];
+    double w = acc.weight[p], wb = acc.weight_bias[p], q = ysq[p];
+    for (uint32_t s = 0; s < batch_samples; s++) { // accumulation_buffer.rs:44-60, as in k_resolve
+        double2 ph = photons[(size_t)i * batch_samples + s];
+        D3 c = d3(0.0, 0.0, 0.0);
+        if (__double_as_longlong(ph.y) != 0ll) c = convert<double>(cmf<R>((R)ph.x) * (R)ph.y);
+        const double weight = 1.0;
+        double wy = weight - wb;
+        double wt = w + wy;
+        wb = (wt - w) - wy;
+        w = wt;
+        double yx = c.x * weight - bx, yy = c.y * weight - by, yz = c.z * weight - bz;
+        double tx = sx + yx, ty = sy + yy, tz = sz + yz;
+        bx = (tx - sx) - yx, by = (ty - sy) - yy, bz = (tz - sz) - yz;
+        sx = tx, sy = ty, sz = tz;
+        q = q + c.y * c.y;
+    }
+    acc.sum[3 * p] = sx, acc.sum[3 * p + 1] = sy, acc.sum[3 * p + 2] = sz;
+    acc.bias[3 * p] = bx, acc.bias[3 * p + 1] = by, acc.bias[3 * p + 2] = bz;
+    acc.weight[p] = w, acc.weight_bias[p] = wb;
+    ysq[p] = q;
+    double inv = 1.0 / w;
+    acc.colour[3 * p] = sx * inv, acc.colour[3 * p + 1] = sy * inv, acc.colour[3 * p + 2] = sz * inv;
+}
+
+// The stopping rule of vrj_render_adaptive on the n pixels of the pass just resolved (list as in k_resolve_adaptive), in the
+// order the header states it so a caller can replay it bit for bit: n = weight, s = colour_sum.y, q = y_sq_sum,
+// m = s / n (as s * (1/n)), v = max(0, (q - s m) / (n - 1)), t = rel_error * max(m, abs_floor); converged iff v <= t t n.
+// A NaN anywhere fails the comparison: such a pixel keeps sampling.  flag[i] = 1 if pixel i takes another pass (`more` is 0
+// when the pass reached max_samples); flag[n] = 0, so the exclusive scan of flag[0..n] ends in the next pass's length.
+static __global__ void k_adaptive_select(const double *sum, const double *weight, const double *ysq, const uint32_t *list, uint32_t n,
+                                         double rel_error, double abs_floor, uint32_t more, uint32_t *flag, unsigned long long *converged) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    bool conv = false;
+    if (i < n) {
+        const uint32_t p = list ? list[i] : i;
+        const double w = weight[p], s = sum[3 * p + 1], q = ysq[p];
+        const double m = s * (1.0 / w);
+        double v = (q - s * m) / (w - 1.0);
+        if (v < 0.0) v = 0.0;
+        const double t = rel_error * (m > abs_floor ? m : abs_floor);
+        conv = v <= t * t * w;
+        flag[i] = !conv && more ? 1u : 0u;
+    } else if (i == n) {
+        flag[n] = 0u;
+    }
+    const uint32_t c = __reduce_add_sync(0xffffffffu, conv ? 1u : 0u);
+    if ((threadIdx.x & 31) == 0 && c) atomicAdd(converged, (unsigned long long)c);
+}
+
+// order-preserving compaction behind the scan of k_adaptive_select's flags: the next pass's list stays row-major, so its
+// camera rays stay as coherent as the tile's
+static __global__ void k_adaptive_compact(const uint32_t *list, const uint32_t *offset, uint32_t n, uint32_t *next) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n && offset[i + 1] != offset[i]) next[offset[i]] = list ? list[i] : i;
 }
 
 // Several calls rendered as ONE wavefront (vanrijn_cuda.cu, "coalesced calls"): the batch's samples [first[c], first[c] +

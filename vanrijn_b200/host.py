@@ -181,6 +181,39 @@ class HostScene:
         out["stats"] = st
         return out
 
+    def render_adaptive(self, tile, height, width, min_samples, max_samples, pass_samples, rel_error, abs_floor=0.0,
+                        want=("colour", "colour_sum", "colour_bias", "weight", "weight_bias", "y_sq_sum"), device=0, **kw):
+        """vrj_render_adaptive with host output buffers: every pixel takes min_samples, then pass_samples more per pass until
+        the standard error of its mean Y is at most rel_error * max(mean, abs_floor) or it holds max_samples.  `kw` are the
+        render parameters of make_params (spp excepted; pass spp=... to check the call refuses it).  Returns a dict of numpy
+        arrays (those in `want`, "srgb8" included if asked for) + 'stats' (VrjStats) + 'adaptive' (VrjAdaptiveStats)."""
+        sc, ec, sr, er = tile
+        npix = (ec - sc) * (er - sr)
+        kw.setdefault("spp", 0)
+        p, keep = self.make_params(**kw)
+        ap = capi.AdaptiveParams(min_samples=min_samples, max_samples=max_samples, pass_samples=pass_samples,
+                                 rel_error=rel_error, abs_floor=abs_floor)
+        out = {}
+        ao = capi.AccumOut(memory=capi.MEM_HOST, accumulate=0)
+        for name, per in (("colour", 3), ("colour_sum", 3), ("colour_bias", 3), ("weight", 1), ("weight_bias", 1)):
+            if name in want:
+                out[name] = np.zeros(npix * per)
+                setattr(ao, name, out[name].ctypes.data)
+        if "srgb8" in want:
+            out["srgb8"] = np.zeros(npix * 3, np.uint8)
+            ao.srgb8 = out["srgb8"].ctypes.data
+        ysq = None
+        if "y_sq_sum" in want:
+            out["y_sq_sum"] = np.zeros(npix)
+            ysq = out["y_sq_sum"].ctypes.data
+        st, ast = capi.Stats(), capi.AdaptiveStats()
+        ao.stats = C.pointer(st)
+        t = capi.Tile(sc, ec, sr, er)
+        capi.check(capi.cuda().vrj_render_adaptive(self.device_scene(device), C.byref(t), height, width, C.byref(p), C.byref(ap),
+                                                   C.byref(ao), ysq, C.byref(ast)))
+        out["stats"], out["adaptive"] = st, ast
+        return out
+
     def render_device(self, tile, height, width, sum_ptr, weight_ptr, device=0, accumulate=False, colour_ptr=None, **kw):
         """vrj_render_tile writing colour_sum / weight straight into caller-owned DEVICE memory
         (e.g. torch tensors that torch.distributed then reduces).  Returns the stats."""

@@ -22,7 +22,7 @@ all: $(LIBDIR)/libvanrijn_cuda.so $(LIBDIR)/libvanrijn_host.so oracle examples t
 OBJDIR ?= build/obj
 BATCH_OBJS = $(OBJDIR)/vrj_batch_0.o $(OBJDIR)/vrj_batch_1.o $(OBJDIR)/vrj_batch_2.o $(OBJDIR)/vrj_batch_3.o \
              $(OBJDIR)/vrj_batch_4.o $(OBJDIR)/vrj_batch_5.o
-$(OBJDIR)/vanrijn_cuda.o: $(CSRC)/vanrijn_cuda.cu $(CSRC)/vrj_scene_prep.cuh $(CUDA_DEPS)
+$(OBJDIR)/vanrijn_cuda.o: $(CSRC)/vanrijn_cuda.cu $(CSRC)/vrj_scene_prep.cuh $(CSRC)/vrj_denoise.cuh $(CUDA_DEPS)
 	mkdir -p $(OBJDIR)
 	$(NVCC) $(NVFLAGS) $(EXTRA) -c -o $@ $(CSRC)/vanrijn_cuda.cu
 $(OBJDIR)/vrj_batch_%.o: $(CSRC)/vrj_batch_inst.cu $(CUDA_DEPS)

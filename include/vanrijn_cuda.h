@@ -323,6 +323,80 @@ VRJ_API VrjStatus vrj_render_adaptive(const VrjScene *scene, const VrjTile *tile
                                       const VrjRenderParams *params, const VrjAdaptiveParams *ap, VrjAccumOut *out,
                                       double *y_sq_sum, VrjAdaptiveStats *astats);
 
+/* ---- first-hit features for a denoiser ----
+ * vrj_render_aux traces params->spp (>= 1) camera rays per pixel of `tile`: the rays of samples sample_offset + k * stride,
+ * k = 0 .. spp-1, with params->seed -- exactly the camera rays vrj_render_tile / vrj_render_adaptive trace with the same
+ * params.  Of params only spp, seed, sample_offset and sample_stride are read; the features are always those of the binary64
+ * (parity) path's hits, whatever `precision` says.
+ * Per pixel, over the samples whose ray hit, in sample order (n_k: the shading normal of the hit, as the integrator sees
+ * it; t_k: its distance; hits: their number):
+ *     normal    = normalize(sum n_k)   (the sum starts from (0,0,0); normalize multiplies by 1/norm); (0,0,0) if hits == 0
+ *     depth     = (sum t_k) * (1.0 / hits);   +inf if hits == 0
+ *     object_id = VrjItem.object_id of the first sample (in sample order) that hit; -1 if none
+ *     material  = index into VrjSceneDesc.materials of that same hit; -1 if none
+ * Arrays are tile-local and row-major like VrjAccumOut's; every pointer may be NULL (not returned) and is memory of the
+ * kind `memory` says (device: the scene's GPU).  stats (host memory, may be NULL) reports primary_rays, kernel_launches and
+ * device_ms.  Runs on a stream of its own; safe to call concurrently with renders on the same scene. */
+typedef struct VrjAuxOut {
+    uint32_t memory, pad;   /* VRJ_MEM_*: all four pointers */
+    double *normal;         /* 3 per pixel */
+    double *depth;          /* 1 per pixel */
+    int32_t *object_id;     /* 1 per pixel (VrjItem.object_id) */
+    int32_t *material;      /* 1 per pixel (index into VrjSceneDesc.materials) */
+    VrjStats *stats;        /* host memory, may be NULL: primary_rays, kernel_launches, device_ms */
+} VrjAuxOut;
+VRJ_API VrjStatus vrj_render_aux(const VrjScene *scene, const VrjTile *tile, uint64_t height, uint64_t width,
+                                 const VrjRenderParams *params, VrjAuxOut *out);
+
+/* ---- vrj_denoise: edge-avoiding a-trous filter guided by the per-pixel variance (SVGF-style) ----
+ * Inputs: one tile's arrays as vrj_render_adaptive (colour_sum, weight, y_sq_sum) and vrj_render_aux (normal, depth,
+ * material) return them, tile_height rows of tile_width pixels.  All pointers are memory of the kind `memory` says, on
+ * `device`.  colour (3 per pixel) receives the filtered XYZ; srgb8 (optional, 3 bytes per pixel) is vrj_tone_map
+ * (VRJ_TONEMAP_XYZ) of that colour; device_ms (optional, host) is the CUDA-event time of the call's kernels.
+ * The filter sees only this tile: separately denoised tiles show seams at their borders, so a caller who wants none
+ * denoises the whole frame as one tile.
+ *
+ * The filter, in binary64 in exactly this order (CUDA's exp, pow and sqrt):
+ *   per pixel p:  n = weight, s = colour_sum, q = y_sq_sum;
+ *                 c = s * (1/n)  (per component: VrjAccumOut.colour's bits);  m = s.y * (1/n);
+ *                 v = (q - s.y*m) / (n - 1);  if (v < 0) v = 0;  var = v * (1/n)   (the variance of the mean Y)
+ *   p is INVALID if n < 2, or a component of c, or var, is not finite (decided once, from the inputs).  An invalid pixel
+ *   keeps its input c through every iteration and gives weight to no neighbour.
+ *   iteration i = 0 .. iterations-1, step = 1 << i; c, var: the previous iteration's output (the above for i = 0); the
+ *   guides N = normal, z = depth, id = material never change.  For every valid p:
+ *     W = 0, C = (0,0,0), V = 0
+ *     for dy = -2..2 (outer), dx = -2..2 (inner): tap q = p + step * (dx, dy); skip q outside the tile or invalid
+ *       w = h[dx] * h[dy],  h = {1/16, 1/4, 3/8, 1/4, 1/16}   (the centre tap keeps exactly 9/64)
+ *       if q != p:
+ *         if id_p != id_q: skip the tap
+ *         if id_p >= 0:  w = w * pow(max(0, dot(N_p, N_q)), sigma_normal)         dot = (x*x' + y*y') + z*z'
+ *                        w = w * exp(-|z_p - z_q| / (((sigma_depth * z_p) * step) * max(|dx|, |dy|)))
+ *         w = w * exp(-|Y_p - Y_q| / (sigma_luminance * sqrt(var_p) + 1e-10))     Y = c.y
+ *       W = W + w;  C = C + w * c_q (per component);  V = V + (w * w) * var_q
+ *     c' = C * (1/W) (per component);  var' = V * (1/(W * W))
+ *   W >= 9/64 because the centre tap always counts.  Pixels that both missed share id -1 and blend without the geometric
+ *   terms.  iterations == 0 returns c: colour_sum * (1/weight) unchanged.
+ * Defaults chosen with tools/denoise_quality.py on C3 / C5 at 1080p (DESIGN.md section 3.7): VRJ_DENOISE_DEFAULT_*.
+ * Limitation: on mirror and glass first hits the guides describe the surface, not what is seen in it; there only the
+ * luminance term keeps reflections sharp.
+ * Errors: NULL required pointers, an unknown memory kind, iterations > 10, sigma_luminance or sigma_depth not > 0 and
+ * finite, sigma_normal not >= 0 and finite: VRJ_ERR_INVALID_ARGUMENT.  tile_width * tile_height == 0: VRJ_OK, no work. */
+typedef struct VrjDenoiseParams {
+    uint32_t iterations;      /* 0..10; 0 returns colour_sum * (1/weight) unchanged */
+    uint32_t pad;
+    double sigma_luminance;   /* > 0, finite */
+    double sigma_normal;      /* >= 0, finite (exponent) */
+    double sigma_depth;       /* > 0, finite */
+} VrjDenoiseParams;
+#define VRJ_DENOISE_DEFAULT_ITERATIONS 4
+#define VRJ_DENOISE_DEFAULT_SIGMA_LUMINANCE 32.0
+#define VRJ_DENOISE_DEFAULT_SIGMA_NORMAL 128.0
+#define VRJ_DENOISE_DEFAULT_SIGMA_DEPTH 0.5
+VRJ_API VrjStatus vrj_denoise(int32_t device, uint32_t memory, uint64_t tile_width, uint64_t tile_height,
+                              const double *colour_sum, const double *weight, const double *y_sq_sum,
+                              const double *normal, const double *depth, const int32_t *material,
+                              const VrjDenoiseParams *dp, double *colour, uint8_t *srgb8, double *device_ms);
+
 /* Sampler::sample on n rays (host arrays, 3 doubles each; directions are normalised like Ray::new).
  * object_id / prim_id are -1 and t is +inf on a miss. */
 /* ---- one box, several GPUs (SURVEY 8e): shard by sample index, one NCCL reduce into the first device ----

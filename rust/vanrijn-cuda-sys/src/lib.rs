@@ -136,6 +136,36 @@ pub struct VrjAdaptiveStats {
     pub pixels_unconverged: u64,
 }
 
+/// Outputs of `vrj_render_aux`: per-pixel first-hit features (see the header for the sums); any pointer may be NULL.
+#[repr(C)]
+pub struct VrjAuxOut {
+    pub memory: u32,
+    pub pad: u32,
+    pub normal: *mut f64,
+    pub depth: *mut f64,
+    pub object_id: *mut i32,
+    pub material: *mut i32,
+    pub stats: *mut VrjStats,
+}
+
+/// Parameters of `vrj_denoise` (the header states the filter operation by operation).
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct VrjDenoiseParams {
+    pub iterations: u32,
+    pub pad: u32,
+    pub sigma_luminance: f64,
+    pub sigma_normal: f64,
+    pub sigma_depth: f64,
+}
+
+impl Default for VrjDenoiseParams {
+    /// `VRJ_DENOISE_DEFAULT_*` of the header
+    fn default() -> Self {
+        VrjDenoiseParams { iterations: 4, pad: 0, sigma_luminance: 32.0, sigma_normal: 128.0, sigma_depth: 0.5 }
+    }
+}
+
 extern "C" {
     pub fn vrj_last_error() -> *const c_char;
     pub fn vrj_abi_version() -> i32;
@@ -157,6 +187,15 @@ extern "C" {
     pub fn vrj_render_adaptive(scene: *const VrjScene, tile: *const VrjTile, height: u64, width: u64,
                                params: *const VrjRenderParams, ap: *const VrjAdaptiveParams, out: *mut VrjAccumOut,
                                y_sq_sum: *mut f64, astats: *mut VrjAdaptiveStats) -> i32;
+    /// First-hit normal, depth, object id and material of the camera rays a render with the same
+    /// spp / seed / sample_offset / sample_stride traces.
+    pub fn vrj_render_aux(scene: *const VrjScene, tile: *const VrjTile, height: u64, width: u64,
+                          params: *const VrjRenderParams, out: *mut VrjAuxOut) -> i32;
+    /// Variance-guided a-trous filter over one tile of `vrj_render_adaptive` + `vrj_render_aux` outputs.
+    pub fn vrj_denoise(device: i32, memory: u32, tile_width: u64, tile_height: u64, colour_sum: *const f64,
+                       weight: *const f64, y_sq_sum: *const f64, normal: *const f64, depth: *const f64,
+                       material: *const i32, dp: *const VrjDenoiseParams, colour: *mut f64, srgb8: *mut u8,
+                       device_ms: *mut f64) -> i32;
     pub fn vrj_comm_create(n_devices: i32, devices: *const i32, out: *mut *mut VrjComm) -> i32;
     pub fn vrj_comm_destroy(comm: *mut VrjComm);
     pub fn vrj_comm_scene_create(comm: *mut VrjComm, desc: *const VrjSceneDesc, out: *mut *mut VrjMultiScene) -> i32;

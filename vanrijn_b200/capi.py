@@ -27,7 +27,7 @@ OK = 0
 CUDA_SYMBOLS = ["vrj_last_error", "vrj_abi_version", "vrj_device_count", "vrj_scene_create", "vrj_scene_destroy",
                 "vrj_scene_device_bytes", "vrj_scene_upload_bytes", "vrj_render_tile", "vrj_trace_rays", "vrj_release_scratch", "vrj_alloc_host",
                 "vrj_free_host", "vrj_alloc_device", "vrj_free_device", "vrj_copy_to_host", "vrj_comm_create", "vrj_comm_destroy", "vrj_comm_scene_create", "vrj_comm_scene_destroy",
-                "vrj_render_sharded", "vrj_tone_map", "vrj_bvh_build", "vrj_render_adaptive"]
+                "vrj_render_sharded", "vrj_tone_map", "vrj_bvh_build", "vrj_render_adaptive", "vrj_render_aux", "vrj_denoise"]
 
 
 class VrjError(RuntimeError):
@@ -135,6 +135,16 @@ class AdaptiveStats(C.Structure):
         return {n: int(getattr(self, n)) for n, _ in self._fields_}
 
 
+class AuxOut(C.Structure):
+    _fields_ = [("memory", C.c_uint32), ("pad", C.c_uint32), ("normal", C.c_void_p), ("depth", C.c_void_p),
+                ("object_id", C.c_void_p), ("material", C.c_void_p), ("stats", C.POINTER(Stats))]
+
+
+class DenoiseParams(C.Structure):
+    _fields_ = [("iterations", C.c_uint32), ("pad", C.c_uint32), ("sigma_luminance", C.c_double), ("sigma_normal", C.c_double),
+                ("sigma_depth", C.c_double)]
+
+
 _cuda = None
 _host = None
 
@@ -176,6 +186,11 @@ def cuda():
         L.vrj_render_adaptive.restype = C.c_int32
         L.vrj_render_adaptive.argtypes = [C.c_void_p, C.POINTER(Tile), C.c_uint64, C.c_uint64, C.POINTER(RenderParams),
                                           C.POINTER(AdaptiveParams), C.POINTER(AccumOut), C.c_void_p, C.POINTER(AdaptiveStats)]
+        L.vrj_render_aux.restype = C.c_int32
+        L.vrj_render_aux.argtypes = [C.c_void_p, C.POINTER(Tile), C.c_uint64, C.c_uint64, C.POINTER(RenderParams), C.POINTER(AuxOut)]
+        L.vrj_denoise.restype = C.c_int32
+        L.vrj_denoise.argtypes = [C.c_int32, C.c_uint32, C.c_uint64, C.c_uint64] + [C.c_void_p] * 6 + \
+                                 [C.POINTER(DenoiseParams), C.c_void_p, C.c_void_p, dp]
         L.vrj_comm_create.restype = C.c_int32
         L.vrj_comm_create.argtypes = [C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_void_p)]
         L.vrj_comm_destroy.argtypes = [C.c_void_p]

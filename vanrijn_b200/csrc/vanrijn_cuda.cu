@@ -3,6 +3,7 @@
 // point that computes returns VRJ_ERR_CUDA.
 #include "../../include/vanrijn_cuda.h"
 #include "vrj_batch.cuh"
+#include "vrj_denoise.cuh"
 #include "vrj_scene_prep.cuh"
 #include "vrj_internal.h"
 
@@ -786,13 +787,20 @@ struct ActiveCall {
     ~ActiveCall() { n.fetch_sub(1); }
 };
 
+// the tile lies inside the image, and the image's pixel indices fit 32 bits
+VrjStatus check_tile(const VrjTile *tile, uint64_t height, uint64_t width) {
+    if (tile->end_column < tile->start_column || tile->end_row < tile->start_row || tile->end_column > width || tile->end_row > height)
+        return fail(VRJ_ERR_INVALID_ARGUMENT, "tile outside the image");
+    if (width * height > 0xffffffffull) return fail(VRJ_ERR_UNSUPPORTED, "image larger than 2^32 pixels");
+    return VRJ_OK;
+}
+
 // the argument checks of vrj_render_tile and vrj_render_adaptive; *n_light_samples: samples of the call's light spectra
 VrjStatus check_render_args(const VrjScene *scene, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p,
                             const VrjAccumOut *out, size_t *n_light_samples) {
     if (!scene || !tile || !p || !out) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
-    if (tile->end_column < tile->start_column || tile->end_row < tile->start_row || tile->end_column > width || tile->end_row > height)
-        return fail(VRJ_ERR_INVALID_ARGUMENT, "tile outside the image");
-    if (width * height > 0xffffffffull) return fail(VRJ_ERR_UNSUPPORTED, "image larger than 2^32 pixels");
+    const VrjStatus st = check_tile(tile, height, width);
+    if (st != VRJ_OK) return st;
     if (p->integrator > VRJ_INTEGRATOR_WHITTED) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown integrator");
     if (p->bvh_filter > VRJ_FILTER_Q16) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown bvh_filter");
     if (p->precision > VRJ_PRECISION_F32_FAST) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown precision");
@@ -1628,6 +1636,153 @@ VrjStatus vrj_render_adaptive(const VrjScene *scene_c, const VrjTile *tile, uint
         astats->passes = passes, astats->samples = samples;
         astats->pixels_converged = *host_converged, astats->pixels_unconverged = npix - *host_converged;
     }
+    return VRJ_OK;
+}
+
+// a stream and two events of a call's own (vrj_render_aux, vrj_denoise: short calls that take no render turn and no scratch
+// block).  Declared after the call's DeviceBuffers: nothing may still use them when they return to the pool.
+struct CallStream {
+    cudaStream_t s = nullptr;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    cudaError_t create() {
+        cudaError_t e = cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking);
+        if (e == cudaSuccess) e = cudaEventCreate(&e0);
+        if (e == cudaSuccess) e = cudaEventCreate(&e1);
+        return e;
+    }
+    ~CallStream() {
+        if (s) cudaStreamSynchronize(s), cudaStreamDestroy(s);
+        if (e0) cudaEventDestroy(e0);
+        if (e1) cudaEventDestroy(e1);
+    }
+};
+
+// First-hit features (the header states them): k_aux, one thread per pixel, forms each pixel's camera rays from the render's
+// RenderConst.  Like vrj_trace_rays it runs on a stream of its own and takes no render turn.
+VrjStatus vrj_render_aux(const VrjScene *scene_c, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p,
+                         VrjAuxOut *out) {
+    VrjScene *scene = const_cast<VrjScene *>(scene_c);
+    if (!scene || !tile || !p || !out) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
+    VrjStatus st = check_tile(tile, height, width);
+    if (st != VRJ_OK) return st;
+    if (p->spp == 0) return fail(VRJ_ERR_INVALID_ARGUMENT, "params->spp must be >= 1");
+    if (out->memory > VRJ_MEM_DEVICE) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown memory kind");
+    if (out->stats) std::memset(out->stats, 0, sizeof(VrjStats));
+    const uint64_t npix = (tile->end_column - tile->start_column) * (tile->end_row - tile->start_row);
+    if (npix == 0) return VRJ_OK;
+    if (npix * (uint64_t)p->spp > 0xffffffffull) return fail(VRJ_ERR_UNSUPPORTED, "more than 2^32 camera rays in one call");
+    DeviceGuard device_guard;
+    VRJ_NVTX_RANGE(call_range, "vrj_render_aux");
+    VRJ_CUDA(cudaSetDevice(scene->device));
+    RenderConst rc = make_render_const(tile, height, width, p);
+    rc.batch_samples = p->spp, rc.first_sample = p->sample_offset;
+    rc.div_batch = FastDiv::make(p->spp), rc.div_tile_w = FastDiv::make(rc.tile_w);
+    AuxDev a{out->normal, out->depth, out->object_id, out->material};
+    DeviceBuffer d_normal, d_depth, d_obj, d_mat;
+    const bool host = out->memory == VRJ_MEM_HOST;
+    if (host) { // the kernel writes device buffers, copied back below
+        if (a.normal) {
+            VRJ_CUDA(d_normal.alloc(npix * 24));
+            a.normal = d_normal.as<double>();
+        }
+        if (a.depth) {
+            VRJ_CUDA(d_depth.alloc(npix * 8));
+            a.depth = d_depth.as<double>();
+        }
+        if (a.object_id) {
+            VRJ_CUDA(d_obj.alloc(npix * 4));
+            a.object_id = d_obj.as<int32_t>();
+        }
+        if (a.material) {
+            VRJ_CUDA(d_mat.alloc(npix * 4));
+            a.material = d_mat.as<int32_t>();
+        }
+    }
+    CallStream cs;
+    VRJ_CUDA(cs.create());
+    VRJ_CUDA(cudaEventRecord(cs.e0, cs.s));
+    k_aux<float><<<(unsigned)((npix + 127) / 128), 128, 0, cs.s>>>(scene->dev, rc, a);
+    VRJ_CUDA(cudaGetLastError());
+    VRJ_CUDA(cudaEventRecord(cs.e1, cs.s));
+    if (host) {
+        if (out->normal) VRJ_CUDA(cudaMemcpyAsync(out->normal, a.normal, npix * 24, cudaMemcpyDeviceToHost, cs.s));
+        if (out->depth) VRJ_CUDA(cudaMemcpyAsync(out->depth, a.depth, npix * 8, cudaMemcpyDeviceToHost, cs.s));
+        if (out->object_id) VRJ_CUDA(cudaMemcpyAsync(out->object_id, a.object_id, npix * 4, cudaMemcpyDeviceToHost, cs.s));
+        if (out->material) VRJ_CUDA(cudaMemcpyAsync(out->material, a.material, npix * 4, cudaMemcpyDeviceToHost, cs.s));
+    }
+    VRJ_CUDA(cudaStreamSynchronize(cs.s));
+    float ms = 0.f;
+    VRJ_CUDA(cudaEventElapsedTime(&ms, cs.e0, cs.e1));
+    if (out->stats) out->stats->primary_rays = npix * p->spp, out->stats->kernel_launches = 1, out->stats->device_ms = ms;
+    return VRJ_OK;
+}
+
+// The variance-guided a-trous filter (the header states it; vrj_denoise.cuh): k_denoise_init forms (c, var) per pixel,
+// `iterations` launches of k_denoise_step ping-pong two pooled buffers of 32 bytes per pixel, k_denoise_colour writes the last
+// one out and k_tone_map makes the optional preview.  Host-memory inputs go through pooled device copies.
+VrjStatus vrj_denoise(int32_t device, uint32_t memory, uint64_t tile_width, uint64_t tile_height, const double *colour_sum,
+                      const double *weight, const double *y_sq_sum, const double *normal, const double *depth, const int32_t *material,
+                      const VrjDenoiseParams *dp, double *colour, uint8_t *srgb8, double *device_ms) {
+    if (!dp) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (memory > VRJ_MEM_DEVICE) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown memory kind");
+    if (dp->iterations > 10) return fail(VRJ_ERR_INVALID_ARGUMENT, "iterations must be <= 10");
+    if (!(dp->sigma_luminance > 0.0) || !std::isfinite(dp->sigma_luminance)) return fail(VRJ_ERR_INVALID_ARGUMENT, "sigma_luminance must be > 0 and finite");
+    if (!(dp->sigma_normal >= 0.0) || !std::isfinite(dp->sigma_normal)) return fail(VRJ_ERR_INVALID_ARGUMENT, "sigma_normal must be >= 0 and finite");
+    if (!(dp->sigma_depth > 0.0) || !std::isfinite(dp->sigma_depth)) return fail(VRJ_ERR_INVALID_ARGUMENT, "sigma_depth must be > 0 and finite");
+    if (device_ms) *device_ms = 0.0;
+    if (tile_width == 0 || tile_height == 0) return VRJ_OK;
+    if (!colour_sum || !weight || !y_sq_sum || !normal || !depth || !material || !colour) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (tile_width > 0xffffffffull || tile_height > 0xffffffffull || tile_width * tile_height > 0xffffffffull)
+        return fail(VRJ_ERR_UNSUPPORTED, "tile larger than 2^32 pixels");
+    const uint64_t npix = tile_width * tile_height;
+    const uint32_t n32 = (uint32_t)npix;
+    DeviceGuard device_guard;
+    VRJ_NVTX_RANGE(call_range, "vrj_denoise");
+    VRJ_CUDA(cudaSetDevice(device));
+    DeviceBuffer ping, d_in[6], d_colour, d_srgb8;
+    VRJ_CUDA(ping.alloc(npix * 64));
+    double4 *buf[2] = {ping.as<double4>(), ping.as<double4>() + npix};
+    const void *src[6] = {colour_sum, weight, y_sq_sum, normal, depth, material};
+    const size_t per[6] = {24, 8, 8, 24, 8, 4};
+    double *out_colour = colour;
+    uint8_t *out_srgb8 = srgb8;
+    const bool host = memory == VRJ_MEM_HOST;
+    if (host) {
+        for (int i = 0; i < 6; i++) VRJ_CUDA(d_in[i].alloc(npix * per[i]));
+        VRJ_CUDA(d_colour.alloc(npix * 24));
+        out_colour = d_colour.as<double>();
+        if (srgb8) {
+            VRJ_CUDA(d_srgb8.alloc(npix * 3));
+            out_srgb8 = d_srgb8.as<uint8_t>();
+        }
+    }
+    CallStream cs;
+    VRJ_CUDA(cs.create());
+    if (host) {
+        for (int i = 0; i < 6; i++) VRJ_CUDA(cudaMemcpyAsync(d_in[i].p, src[i], npix * per[i], cudaMemcpyHostToDevice, cs.s));
+        for (int i = 0; i < 6; i++) src[i] = d_in[i].p;
+    }
+    const DenoiseGuides g{static_cast<const double *>(src[3]), static_cast<const double *>(src[4]), static_cast<const int32_t *>(src[5])};
+    const unsigned blocks = (unsigned)((npix + 255) / 256);
+    VRJ_CUDA(cudaEventRecord(cs.e0, cs.s));
+    k_denoise_init<<<blocks, 256, 0, cs.s>>>(static_cast<const double *>(src[0]), static_cast<const double *>(src[1]),
+                                             static_cast<const double *>(src[2]), n32, buf[0]);
+    const uint32_t bx = (uint32_t)((tile_width + 31) / 32), by = (uint32_t)((tile_height + 7) / 8);
+    for (uint32_t i = 0; i < dp->iterations; i++)
+        k_denoise_step<<<bx * by, 256, 0, cs.s>>>(buf[i & 1], buf[(i + 1) & 1], g, (uint32_t)tile_width, (uint32_t)tile_height, bx,
+                                                   1 << i, dp->sigma_luminance, dp->sigma_normal, dp->sigma_depth);
+    k_denoise_colour<<<blocks, 256, 0, cs.s>>>(buf[dp->iterations & 1], n32, out_colour);
+    if (srgb8) k_tone_map<<<blocks, 256, 0, cs.s>>>(out_colour, out_srgb8, npix, VRJ_TONEMAP_XYZ);
+    VRJ_CUDA(cudaGetLastError());
+    VRJ_CUDA(cudaEventRecord(cs.e1, cs.s));
+    if (host) {
+        VRJ_CUDA(cudaMemcpyAsync(colour, out_colour, npix * 24, cudaMemcpyDeviceToHost, cs.s));
+        if (srgb8) VRJ_CUDA(cudaMemcpyAsync(srgb8, out_srgb8, npix * 3, cudaMemcpyDeviceToHost, cs.s));
+    }
+    VRJ_CUDA(cudaStreamSynchronize(cs.s));
+    float ms = 0.f;
+    VRJ_CUDA(cudaEventElapsedTime(&ms, cs.e0, cs.e1));
+    if (device_ms) *device_ms = ms;
     return VRJ_OK;
 }
 

@@ -963,4 +963,40 @@ static __global__ void k_hit_ids(DevScene sc, uint32_t n, TraceBuffers tb, int32
     t[i] = tb.tbest[i];
 }
 
+// ---- k_aux: first-hit features of a render's camera rays (vrj_render_aux; the header states the per-pixel sums) ----
+// One thread per tile pixel.  rc is the render's RenderConst with batch_samples = spp, so slot p * spp + k is sample k of
+// pixel p and camera_ray forms exactly the ray the render traced; the closest hit and its frame come from the code the
+// integrator uses (trace_closest with a full walk, rebuild_hit), always in binary64.  A template so that only the
+// translation unit that launches it compiles it.
+struct AuxDev {
+    double *normal, *depth;
+    int32_t *object_id, *material;
+};
+template <typename NT>
+__global__ void __launch_bounds__(128) k_aux(DevScene sc, RenderConst rc, AuxDev out) {
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= rc.npix) return;
+    D3 nsum = d3(0.0, 0.0, 0.0);
+    double tsum = 0.0;
+    uint32_t hits = 0;
+    int32_t obj = -1, mat = -1;
+    for (uint32_t k = 0; k < rc.batch_samples; k++) {
+        D3 o, d;
+        camera_ray<double>(sc, rc, p * rc.batch_samples + k, o, d);
+        TraceCounters tc = {0, 0};
+        const Hit h = trace_closest<NT, false, false, double>(sc, o, d, tc);
+        HitFrame f;
+        // rebuild_hit repeats the test that found the hit, so it cannot fail here; a failure would count as a miss
+        if (h.item < 0 || !rebuild_hit(sc, o, d, h.item, h.tri, h.t, f)) continue;
+        nsum = nsum + f.normal;
+        tsum = tsum + h.t;
+        if (hits++ == 0) obj = (int32_t)sc.items[h.item].object_id, mat = (int32_t)f.material;
+    }
+    const D3 n = hits ? normalize(nsum) : d3(0.0, 0.0, 0.0);
+    if (out.normal) out.normal[3 * (size_t)p] = n.x, out.normal[3 * (size_t)p + 1] = n.y, out.normal[3 * (size_t)p + 2] = n.z;
+    if (out.depth) out.depth[p] = hits ? tsum * (1.0 / (double)hits) : CUDART_INF;
+    if (out.object_id) out.object_id[p] = obj;
+    if (out.material) out.material[p] = mat;
+}
+
 } // namespace vrj

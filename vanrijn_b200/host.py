@@ -214,6 +214,26 @@ class HostScene:
         out["stats"], out["adaptive"] = st, ast
         return out
 
+    def render_aux(self, tile, height, width, spp=1, want=("normal", "depth", "object_id", "material"), device=0, **kw):
+        """vrj_render_aux with host output buffers: the first-hit features of the camera rays that a render with the same
+        spp, seed, sample_offset and sample_stride traces (`kw`: the other keywords of make_params).  Returns a dict of numpy
+        arrays (those in `want`: normal, 3 per pixel; depth; object_id and material, int32) + 'stats'."""
+        sc, ec, sr, er = tile
+        npix = (ec - sc) * (er - sr)
+        p, keep = self.make_params(spp=spp, **kw)
+        ao = capi.AuxOut(memory=capi.MEM_HOST)
+        out = {}
+        for name, per, dtype in (("normal", 3, np.float64), ("depth", 1, np.float64), ("object_id", 1, np.int32), ("material", 1, np.int32)):
+            if name in want:
+                out[name] = np.zeros(npix * per, dtype)
+                setattr(ao, name, out[name].ctypes.data)
+        st = capi.Stats()
+        ao.stats = C.pointer(st)
+        t = capi.Tile(sc, ec, sr, er)
+        capi.check(capi.cuda().vrj_render_aux(self.device_scene(device), C.byref(t), height, width, C.byref(p), C.byref(ao)))
+        out["stats"] = st
+        return out
+
     def render_device(self, tile, height, width, sum_ptr, weight_ptr, device=0, accumulate=False, colour_ptr=None, **kw):
         """vrj_render_tile writing colour_sum / weight straight into caller-owned DEVICE memory
         (e.g. torch tensors that torch.distributed then reduces).  Returns the stats."""
@@ -302,6 +322,34 @@ def tone_map(colour, source=capi.TONEMAP_XYZ, device=0):
     c = np.ascontiguousarray(colour, dtype=np.float64).reshape(-1, 3)
     out = np.zeros((c.shape[0], 3), np.uint8)
     capi.check(capi.cuda().vrj_tone_map(device, capi.MEM_HOST, source, c.ctypes.data_as(dp), c.shape[0], out.ctypes.data))
+    return out
+
+
+# vrj_denoise's defaults (VRJ_DENOISE_DEFAULT_* in include/vanrijn_cuda.h), chosen with tools/denoise_quality.py
+DENOISE_ITERATIONS, DENOISE_SIGMA_LUMINANCE, DENOISE_SIGMA_NORMAL, DENOISE_SIGMA_DEPTH = 4, 32.0, 128.0, 0.5
+
+
+def denoise(colour_sum, weight, y_sq_sum, aux, tile_width, tile_height, iterations=DENOISE_ITERATIONS,
+            sigma_luminance=DENOISE_SIGMA_LUMINANCE, sigma_normal=DENOISE_SIGMA_NORMAL, sigma_depth=DENOISE_SIGMA_DEPTH,
+            want_srgb8=False, device=0):
+    """vrj_denoise on host arrays: one tile's colour_sum / weight / y_sq_sum (HostScene.render_adaptive) and the normal /
+    depth / material of `aux` (HostScene.render_aux).  Returns a dict: colour (npix * 3 float64), srgb8 (npix * 3 uint8, if
+    asked for) and device_ms."""
+    npix = tile_width * tile_height
+    ins = [np.ascontiguousarray(colour_sum, np.float64), np.ascontiguousarray(weight, np.float64),
+           np.ascontiguousarray(y_sq_sum, np.float64), np.ascontiguousarray(aux["normal"], np.float64),
+           np.ascontiguousarray(aux["depth"], np.float64), np.ascontiguousarray(aux["material"], np.int32)]
+    for a, per in zip(ins, (3, 1, 1, 3, 1, 1)):
+        assert a.size == npix * per, (a.size, npix, per)
+    out = {"colour": np.zeros(npix * 3)}
+    if want_srgb8:
+        out["srgb8"] = np.zeros(npix * 3, np.uint8)
+    ms = C.c_double(0.0)
+    params = capi.DenoiseParams(iterations=iterations, sigma_luminance=sigma_luminance, sigma_normal=sigma_normal,
+                                sigma_depth=sigma_depth)
+    capi.check(capi.cuda().vrj_denoise(device, capi.MEM_HOST, tile_width, tile_height, *[a.ctypes.data for a in ins], C.byref(params),
+                                       out["colour"].ctypes.data, out["srgb8"].ctypes.data if want_srgb8 else None, C.byref(ms)))
+    out["device_ms"] = ms.value
     return out
 
 

@@ -12,6 +12,10 @@
 // --cache FILE: the flattened scene on disk (load_scene_cache if FILE exists, else build the scene and save_scene_cache),
 // --resident: keep the frame's AccumulationBuffer on the GPU (DeviceAccumulationBuffer) instead of downloading a
 // buffer per tile and merging on the host; previews then move 3 bytes per pixel.
+// --rel-error E (with --resident): sample adaptively instead (DeviceProgressiveBuffer, vrj_render_progressive), one pass
+// of --spp samples per loop iteration: every pixel first takes --min-spp (default 4), then pixels whose mean Y is not yet
+// within E take --spp more, up to --max-spp (default 64); the loop also ends when no pixel is active.
+// --denoise (with --rel-error): previews and --out are the denoised frame (vrj_render_aux once, vrj_denoise per preview).
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -30,13 +34,16 @@ struct CommandLineParameters {
     double time = 0.0;
     uint32_t spp = 1, passes = 0, depth = 128, preview_every = 0;
     uint64_t seed = 1;
-    bool resident = false;
+    bool resident = false, denoise = false;
+    double rel_error = 0.0; // > 0: adaptive progressive passes (--rel-error)
+    uint32_t min_spp = 4, max_spp = 64;
     BoundingVolumeHierarchy::Builder builder = BoundingVolumeHierarchy::Builder::AtUpload;
 };
 
 [[noreturn]] void usage(const char *why) {
     std::fprintf(stderr, "error: %s\nUSAGE: vanrijn --size <WIDTH> <HEIGHT> [--out <FILENAME>] [--time <SECONDS>] [--obj <FILE>] [--spp N] "
-                         "[--passes N] [--depth N] [--builder host|device|upload] [--seed N] [--preview-every N] [--resident] [--cache FILE]\n", why);
+                         "[--passes N] [--depth N] [--builder host|device|upload] [--seed N] [--preview-every N] [--resident] [--cache FILE]\n"
+                         "       [--rel-error E [--min-spp N] [--max-spp N] [--denoise]]\n", why);
     std::exit(2);
 }
 
@@ -60,6 +67,10 @@ CommandLineParameters parse_args(int argc, char **argv) {
         else if (a == "--seed") p.seed = std::strtoull(value(), nullptr, 10), i++;
         else if (a == "--preview-every") p.preview_every = (uint32_t)std::strtoul(value(), nullptr, 10), i++;
         else if (a == "--resident") p.resident = true;
+        else if (a == "--rel-error") p.rel_error = std::strtod(value(), nullptr), i++;
+        else if (a == "--min-spp") p.min_spp = (uint32_t)std::strtoul(value(), nullptr, 10), i++;
+        else if (a == "--max-spp") p.max_spp = (uint32_t)std::strtoul(value(), nullptr, 10), i++;
+        else if (a == "--denoise") p.denoise = true;
         else if (a == "--builder") {
             const std::string b = value();
             i++;
@@ -71,6 +82,9 @@ CommandLineParameters parse_args(int argc, char **argv) {
     }
     if (p.width == 0 || p.height == 0) usage("--size <WIDTH> <HEIGHT> is required");
     if (p.spp == 0) usage("--spp must be positive");
+    if (p.rel_error > 0.0 && !p.resident) usage("--rel-error needs --resident");
+    if (p.rel_error < 0.0 || p.min_spp < 2 || p.max_spp < p.min_spp) usage("--rel-error must be > 0, --min-spp >= 2, --max-spp >= --min-spp");
+    if (p.denoise && p.rel_error <= 0.0) usage("--denoise needs --rel-error");
     return p;
 }
 
@@ -130,9 +144,39 @@ int main(int argc, char **argv) {
         uint32_t pass = 0;
         const auto t0 = std::chrono::steady_clock::now();
         std::unique_ptr<DeviceAccumulationBuffer> resident;
-        if (parameters.resident) resident.reset(new DeviceAccumulationBuffer(image_width, image_height));
+        std::unique_ptr<DeviceProgressiveBuffer> progressive;
+        if (parameters.resident && parameters.rel_error > 0.0) progressive.reset(new DeviceProgressiveBuffer(image_width, image_height));
+        else if (parameters.resident) resident.reset(new DeviceAccumulationBuffer(image_width, image_height));
+        RenderOptions progressive_options;
+        progressive_options.spp = parameters.spp, progressive_options.max_depth = parameters.depth, progressive_options.seed = parameters.seed;
+        auto progressive_image = [&] {
+            return parameters.denoise ? progressive->denoised_image_rgb_u8(scene, progressive_options) : progressive->to_image_rgb_u8();
+        };
         for (; pass < passes_wanted; pass++) {
             if (parameters.time > 0.0 && pass > 0 && seconds_since(t0) >= parameters.time) break;
+            if (progressive) {
+                ProgressiveOptions pp;
+                VrjProgressiveStats pstats{};
+                VrjStats stats{};
+                pp.min_samples = parameters.min_spp, pp.max_samples = parameters.max_spp, pp.pass_samples = parameters.spp;
+                pp.rel_error = parameters.rel_error, pp.stats = &pstats;
+                progressive_options.stats = &stats;
+                const auto t_call = std::chrono::steady_clock::now();
+                progressive->render(scene, progressive_options, pp);
+                call_s += seconds_since(t_call);
+                rays += stats.primary_rays + stats.bounce_rays + stats.shadow_rays;
+                device_ms += stats.device_ms;
+                std::printf("pass %u: %llu samples, %llu pixels active, %llu converged, %llu at --max-spp\n", pass + 1,
+                            (unsigned long long)pstats.samples, (unsigned long long)pstats.pixels_active,
+                            (unsigned long long)pstats.pixels_converged, (unsigned long long)pstats.pixels_at_max);
+                if (parameters.preview_every && !parameters.output_file.empty() && (pass + 1) % parameters.preview_every == 0)
+                    progressive_image().write_png(parameters.output_file);
+                if (pstats.pixels_active == 0) {
+                    pass++;
+                    break;
+                }
+                continue;
+            }
             if (resident) {
                 RenderOptions o;
                 VrjStats stats{};
@@ -173,7 +217,8 @@ int main(int argc, char **argv) {
                     pass * (double)parameters.spp / wall);
         std::printf("host time: partial_render_scene %.3f s (device %.3f s), merge_tile %.3f s\n", call_s, device_ms / 1e3, merge_s);
         if (!parameters.output_file.empty()) {
-            if (resident) resident->to_image_rgb_u8().write_png(parameters.output_file);
+            if (progressive) progressive_image().write_png(parameters.output_file);
+            else if (resident) resident->to_image_rgb_u8().write_png(parameters.output_file);
             else rendered_image.to_image_rgb_u8().write_png(parameters.output_file); // main.rs:222-225
             std::printf("wrote %s\n", parameters.output_file.c_str());
         }

@@ -299,6 +299,7 @@ class AccumulationBuffer {
   private:
     friend AccumulationBuffer partial_render_scene(const Scene &, Tile, size_t, size_t, const struct RenderOptions &);
     friend class DeviceAccumulationBuffer;
+    friend class DeviceProgressiveBuffer;
     friend struct MainLoopStats render_like_main(const struct Scene &, size_t, size_t, size_t, uint64_t, unsigned, const struct RenderOptions &, bool,
                                                  AccumulationBuffer &);
     struct Uninitialized {};
@@ -383,6 +384,44 @@ class DeviceAccumulationBuffer {
     size_t width_, height_;
     int device_;
     uint64_t samples_ = 0;
+};
+
+// The schedule of vrj_render_progressive (include/vanrijn_cuda.h): pixels below min_samples, and pixels below max_samples
+// whose mean Y is not yet within rel_error, take samples; max_passes passes per render() call (0: until none is active).
+struct ProgressiveOptions {
+    uint32_t min_samples = 4, max_samples = 64, pass_samples = 4;
+    uint32_t max_passes = 1;
+    double rel_error = 0.05, abs_floor = 0.0;
+    VrjProgressiveStats *stats = nullptr; // optional: what the last call did and the state it left
+};
+
+// A progressive frame kept on the GPU, sampled adaptively: the AccumulationBuffer's arrays plus the per-pixel sum of
+// squared Y (y_sq_sum) that vrj_denoise needs.  Keep options.seed, sample_offset and sample_stride fixed across calls.
+class DeviceProgressiveBuffer {
+  public:
+    DeviceProgressiveBuffer(size_t width, size_t height, int device = 0);
+    ~DeviceProgressiveBuffer();
+    DeviceProgressiveBuffer(const DeviceProgressiveBuffer &) = delete;
+    DeviceProgressiveBuffer &operator=(const DeviceProgressiveBuffer &) = delete;
+    size_t width() const { return width_; }
+    size_t height() const { return height_; }
+    // continues the frame's state with up to pp.max_passes passes (options.spp is ignored: the counts come from pp)
+    void render(const Scene &scene, const RenderOptions &options, const ProgressiveOptions &pp);
+    ImageRgbU8 to_image_rgb_u8() const; // ClampingToneMapper on the device
+    // vrj_denoise (the header's defaults) of the frame as it stands, on the device; the first-hit features come from one
+    // vrj_render_aux of options.spp camera rays per pixel, traced at the first call and kept for the frame
+    ImageRgbU8 denoised_image_rgb_u8(const Scene &scene, const RenderOptions &options);
+    AccumulationBuffer download() const; // the five arrays
+    std::vector<double> download_y_sq_sum() const;
+
+  private:
+    double *colour_ = nullptr, *sum_ = nullptr, *bias_ = nullptr, *weight_ = nullptr, *weight_bias_ = nullptr, *y_sq_sum_ = nullptr;
+    double *normal_ = nullptr, *depth_ = nullptr, *denoised_ = nullptr;
+    int32_t *material_ = nullptr;
+    uint8_t *srgb8_ = nullptr;
+    size_t width_, height_;
+    int device_;
+    bool started_ = false, have_aux_ = false;
 };
 
 // Collects the flattened SoA arrays and exposes them as a VrjSceneDesc.

@@ -323,6 +323,59 @@ VRJ_API VrjStatus vrj_render_adaptive(const VrjScene *scene, const VrjTile *tile
                                       const VrjRenderParams *params, const VrjAdaptiveParams *ap, VrjAccumOut *out,
                                       double *y_sq_sum, VrjAdaptiveStats *astats);
 
+/* ---- progressive rendering: adaptive or uniform sampling continued from a saved frame state ----
+ * vrj_render_progressive runs the passes of vrj_render_adaptive on a state the caller keeps between calls, so a frame can be
+ * previewed (and denoised: the state includes y_sq_sum) while it is sampled, and a rendered frame can be refined further.
+ *
+ * State: out->colour_sum, colour_bias, weight, weight_bias and y_sq_sum, all five required, memory of the kind out->memory
+ * says.  out->accumulate == 0: the state starts at zero; != 0: the arrays hold the state to continue.  On return they hold
+ * the new state.  out->colour and out->srgb8 (optional) are computed for EVERY pixel of the tile at return (colour =
+ * colour_sum * (1/weight)).  out->photons: VRJ_ERR_UNSUPPORTED.  params: as vrj_render_adaptive; spp must be 0.
+ *
+ * Sample indices.  Pixel p holds n = weight[p] samples: its samples sample_offset + k * stride for k < n.  Keep seed,
+ * sample_offset and sample_stride fixed across the calls that continue one state.  A weight that is negative, not an
+ * integer, not finite or >= 2^32 is VRJ_ERR_INVALID_ARGUMENT (the state is left as it was).
+ *
+ * Schedule.  Before each pass every pixel is judged on its current (n, s = colour_sum.y, q = y_sq_sum) with
+ * vrj_render_adaptive's stopping rule, bit for bit (the rule above).  Pixel p is ACTIVE if n < min_samples, or if
+ * n < max_samples and the rule fails.  An active pixel takes c samples in the pass -- c = min_samples - n if n < min_samples,
+ * else c = min(pass_samples, max_samples - n) -- its samples n .. n + c - 1, applied in sample order.  The call stops after
+ * max_passes passes, or earlier when no pixel is active; a state with no active pixel comes back unchanged, bit for bit,
+ * with passes = 0.
+ *
+ * Guarantees:
+ *  (a) a pixel that ends with n samples holds, bit for bit, the colour_sum, colour_bias, weight and weight_bias that
+ *      vrj_render_tile with spp = n gives it, and the y_sq_sum of vrj_render_adaptive (q = q + y * y in sample order);
+ *  (b) accumulate == 0 and max_passes == 0 equals vrj_render_adaptive with the same min / max / pass samples, rel_error and
+ *      abs_floor: every array, passes, samples, and pixels_converged / pixels_at_max = pixels_converged / _unconverged;
+ *  (c) the schedule depends only on the state, so any split of the passes into calls ends in the same state;
+ *  (d) a state vrj_render_adaptive returned can be continued (with a larger max_samples, a smaller rel_error, ...);
+ *  (e) calls with min_samples == max_samples = 4, 8, 12, ... are a uniform progressive frame, y_sq_sum included.
+ * pstats (host, may be NULL): passes and samples run by this call; the three pixel counts describe the state at return and
+ * add up to the tile's pixels.  out->stats sums the call's passes like vrj_render_adaptive's.
+ * Scheduling: never coalesced; takes the device's render turn; uses a scratch block from the pool (y_sq_sum, two pixel
+ * lists and a per-pixel count: 20 bytes per pixel more than vrj_render_tile).  Pixels of one pass that take different
+ * counts are rendered in one sub-pass per distinct count. */
+typedef struct VrjProgressiveParams {
+    uint32_t min_samples;   /* as VrjAdaptiveParams: >= 2 */
+    uint32_t max_samples;   /* >= min_samples */
+    uint32_t pass_samples;  /* >= 1 */
+    uint32_t max_passes;    /* passes this call may run; 0 = until no pixel is active */
+    double rel_error;       /* > 0, finite */
+    double abs_floor;       /* >= 0, finite */
+} VrjProgressiveParams;
+
+typedef struct VrjProgressiveStats {
+    uint64_t passes, samples;   /* run by this call */
+    uint64_t pixels_converged;  /* at return: not active, and the rule holds (n >= min_samples >= 2) */
+    uint64_t pixels_at_max;     /* at return: not active, n >= max_samples, and the rule does not hold */
+    uint64_t pixels_active;     /* at return: the rest, which would take samples in another pass */
+} VrjProgressiveStats;
+
+VRJ_API VrjStatus vrj_render_progressive(const VrjScene *scene, const VrjTile *tile, uint64_t height, uint64_t width,
+                                         const VrjRenderParams *params, const VrjProgressiveParams *pp,
+                                         VrjAccumOut *out, double *y_sq_sum, VrjProgressiveStats *pstats);
+
 /* ---- first-hit features for a denoiser ----
  * vrj_render_aux traces params->spp (>= 1) camera rays per pixel of `tile`: the rays of samples sample_offset + k * stride,
  * k = 0 .. spp-1, with params->seed -- exactly the camera rays vrj_render_tile / vrj_render_adaptive trace with the same

@@ -136,6 +136,36 @@ pub struct VrjAdaptiveStats {
     pub pixels_unconverged: u64,
 }
 
+/// Sample counts, pass limit and error target of `vrj_render_progressive` (the header states the schedule).
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct VrjProgressiveParams {
+    pub min_samples: u32,
+    pub max_samples: u32,
+    pub pass_samples: u32,
+    pub max_passes: u32,
+    pub rel_error: f64,
+    pub abs_floor: f64,
+}
+
+impl Default for VrjProgressiveParams {
+    /// A preview loop's: one pass of 4 samples per call, at most 64 per pixel, 5 % relative error of the mean Y
+    fn default() -> Self {
+        VrjProgressiveParams { min_samples: 4, max_samples: 64, pass_samples: 4, max_passes: 1, rel_error: 0.05, abs_floor: 0.0 }
+    }
+}
+
+/// What `vrj_render_progressive` did (passes, samples) and the state it left: pixels converged / at `max_samples` / active.
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct VrjProgressiveStats {
+    pub passes: u64,
+    pub samples: u64,
+    pub pixels_converged: u64,
+    pub pixels_at_max: u64,
+    pub pixels_active: u64,
+}
+
 /// Outputs of `vrj_render_aux`: per-pixel first-hit features (see the header for the sums); any pointer may be NULL.
 #[repr(C)]
 pub struct VrjAuxOut {
@@ -187,6 +217,11 @@ extern "C" {
     pub fn vrj_render_adaptive(scene: *const VrjScene, tile: *const VrjTile, height: u64, width: u64,
                                params: *const VrjRenderParams, ap: *const VrjAdaptiveParams, out: *mut VrjAccumOut,
                                y_sq_sum: *mut f64, astats: *mut VrjAdaptiveStats) -> i32;
+    /// Continues the state in `out` (colour_sum, colour_bias, weight, weight_bias) and `y_sq_sum`, all required, with
+    /// the adaptive schedule for at most `pp.max_passes` passes; `params.spp` must be 0.
+    pub fn vrj_render_progressive(scene: *const VrjScene, tile: *const VrjTile, height: u64, width: u64,
+                                  params: *const VrjRenderParams, pp: *const VrjProgressiveParams, out: *mut VrjAccumOut,
+                                  y_sq_sum: *mut f64, pstats: *mut VrjProgressiveStats) -> i32;
     /// First-hit normal, depth, object id and material of the camera rays a render with the same
     /// spp / seed / sample_offset / sample_stride traces.
     pub fn vrj_render_aux(scene: *const VrjScene, tile: *const VrjTile, height: u64, width: u64,

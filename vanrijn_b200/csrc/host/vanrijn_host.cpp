@@ -1053,24 +1053,35 @@ DeviceAccumulationBuffer::~DeviceAccumulationBuffer() {
     for (void *p : {(void *)colour_, (void *)sum_, (void *)bias_, (void *)weight_, (void *)weight_bias_, (void *)srgb8_}) vrj_free_device(p);
     colour_ = sum_ = bias_ = weight_ = weight_bias_ = nullptr, srgb8_ = nullptr;
 }
-void DeviceAccumulationBuffer::render(const Scene &scene, RenderOptions o) {
+// VrjRenderParams of RenderOptions for the device-resident buffers; the lights it points to live in this object
+struct DeviceRenderParams {
     VrjRenderParams p{};
-    p.spp = o.spp, p.max_depth = o.max_depth, p.sample_offset = o.sample_offset + samples_ * o.sample_stride, p.seed = o.seed;
-    p.integrator = o.integrator, p.bvh_filter = o.bvh_filter, p.bias = 0.0000001, p.sample_stride = o.sample_stride;
-    auto as_data = [](const Spectrum &s) {
-        return VrjSpectrumData{s.shortest_wavelength, s.longest_wavelength, (uint32_t)s.samples.size(), 0u, s.samples.data()};
-    };
     std::vector<VrjLight> lights;
-    VrjSpectrumData ambient = as_data(o.ambient_light);
-    if (o.integrator == VRJ_INTEGRATOR_WHITTED) {
-        for (const DirectionalLight &l : o.lights) {
-            VrjLight d{};
-            d.direction[0] = l.direction.x, d.direction[1] = l.direction.y, d.direction[2] = l.direction.z;
-            d.spectrum = as_data(l.spectrum);
-            lights.push_back(d);
+    VrjSpectrumData ambient{};
+    explicit DeviceRenderParams(const RenderOptions &o) {
+        p.spp = o.spp, p.max_depth = o.max_depth, p.sample_offset = o.sample_offset, p.seed = o.seed;
+        p.integrator = o.integrator, p.bvh_filter = o.bvh_filter, p.bias = 0.0000001, p.sample_stride = o.sample_stride;
+        auto as_data = [](const Spectrum &s) {
+            return VrjSpectrumData{s.shortest_wavelength, s.longest_wavelength, (uint32_t)s.samples.size(), 0u, s.samples.data()};
+        };
+        ambient = as_data(o.ambient_light);
+        if (o.integrator == VRJ_INTEGRATOR_WHITTED) {
+            for (const DirectionalLight &l : o.lights) {
+                VrjLight d{};
+                d.direction[0] = l.direction.x, d.direction[1] = l.direction.y, d.direction[2] = l.direction.z;
+                d.spectrum = as_data(l.spectrum);
+                lights.push_back(d);
+            }
+            p.lights = lights.data(), p.n_lights = (uint32_t)lights.size(), p.ambient_light = &ambient;
         }
-        p.lights = lights.data(), p.n_lights = (uint32_t)lights.size(), p.ambient_light = &ambient;
     }
+    DeviceRenderParams(const DeviceRenderParams &) = delete;
+};
+
+void DeviceAccumulationBuffer::render(const Scene &scene, RenderOptions o) {
+    DeviceRenderParams dp(o);
+    VrjRenderParams &p = dp.p;
+    p.sample_offset = o.sample_offset + samples_ * o.sample_stride;
     VrjTile t{0, width_, 0, height_};
     VrjAccumOut out{};
     out.memory = VRJ_MEM_DEVICE, out.accumulate = 1; // continue the Kahan state left by the previous pass (zero at first)
@@ -1100,6 +1111,84 @@ AccumulationBuffer DeviceAccumulationBuffer::download() const {
     for (const auto &c : copies)
         if (vrj_copy_to_host(device_, c.dst, c.src, c.count * 8) != VRJ_OK) throw std::runtime_error(std::string("vrj_copy_to_host: ") + vrj_last_error());
     return b;
+}
+
+DeviceProgressiveBuffer::DeviceProgressiveBuffer(size_t width, size_t height, int device) : width_(width), height_(height), device_(device) {
+    const size_t n = width * height;
+    auto f64 = [device](size_t count) { return static_cast<double *>(vrj_alloc_device(device, count * 8)); };
+    colour_ = f64(3 * n), sum_ = f64(3 * n), bias_ = f64(3 * n), weight_ = f64(n), weight_bias_ = f64(n), y_sq_sum_ = f64(n);
+    normal_ = f64(3 * n), depth_ = f64(n), denoised_ = f64(3 * n);
+    material_ = static_cast<int32_t *>(vrj_alloc_device(device, n * 4)), srgb8_ = static_cast<uint8_t *>(vrj_alloc_device(device, 3 * n));
+    if (!colour_ || !sum_ || !bias_ || !weight_ || !weight_bias_ || !y_sq_sum_ || !normal_ || !depth_ || !denoised_ || !material_ || !srgb8_) {
+        const std::string why = vrj_last_error();
+        this->~DeviceProgressiveBuffer();
+        throw std::runtime_error("DeviceProgressiveBuffer: " + why);
+    }
+}
+DeviceProgressiveBuffer::~DeviceProgressiveBuffer() {
+    for (void *p : {(void *)colour_, (void *)sum_, (void *)bias_, (void *)weight_, (void *)weight_bias_, (void *)y_sq_sum_, (void *)normal_,
+                    (void *)depth_, (void *)denoised_, (void *)material_, (void *)srgb8_})
+        vrj_free_device(p);
+    colour_ = sum_ = bias_ = weight_ = weight_bias_ = y_sq_sum_ = normal_ = depth_ = denoised_ = nullptr;
+    material_ = nullptr, srgb8_ = nullptr;
+}
+void DeviceProgressiveBuffer::render(const Scene &scene, const RenderOptions &o, const ProgressiveOptions &pp) {
+    DeviceRenderParams dp(o);
+    dp.p.spp = 0;
+    VrjProgressiveParams vp{pp.min_samples, pp.max_samples, pp.pass_samples, pp.max_passes, pp.rel_error, pp.abs_floor};
+    VrjTile t{0, width_, 0, height_};
+    VrjAccumOut out{};
+    out.memory = VRJ_MEM_DEVICE, out.accumulate = started_ ? 1u : 0u;
+    out.colour = colour_, out.colour_sum = sum_, out.colour_bias = bias_, out.weight = weight_, out.weight_bias = weight_bias_;
+    out.stats = o.stats;
+    if (vrj_render_progressive(device_scene(scene, device_), &t, height_, width_, &dp.p, &vp, &out, y_sq_sum_, pp.stats) != VRJ_OK)
+        throw std::runtime_error(std::string("vrj_render_progressive: ") + vrj_last_error());
+    started_ = true;
+}
+ImageRgbU8 DeviceProgressiveBuffer::to_image_rgb_u8() const {
+    ImageRgbU8 image(width_, height_);
+    const size_t n = width_ * height_;
+    if (vrj_tone_map(device_, VRJ_MEM_DEVICE, VRJ_TONEMAP_XYZ, colour_, n, srgb8_) != VRJ_OK ||
+        vrj_copy_to_host(device_, image.pixel_data().data(), srgb8_, 3 * n) != VRJ_OK)
+        throw std::runtime_error(std::string("DeviceProgressiveBuffer::to_image_rgb_u8: ") + vrj_last_error());
+    return image;
+}
+ImageRgbU8 DeviceProgressiveBuffer::denoised_image_rgb_u8(const Scene &scene, const RenderOptions &options) {
+    if (!have_aux_) {
+        DeviceRenderParams dp(options);
+        VrjTile t{0, width_, 0, height_};
+        VrjAuxOut aux{};
+        aux.memory = VRJ_MEM_DEVICE, aux.normal = normal_, aux.depth = depth_, aux.material = material_;
+        if (vrj_render_aux(device_scene(scene, device_), &t, height_, width_, &dp.p, &aux) != VRJ_OK)
+            throw std::runtime_error(std::string("vrj_render_aux: ") + vrj_last_error());
+        have_aux_ = true;
+    }
+    const VrjDenoiseParams params{VRJ_DENOISE_DEFAULT_ITERATIONS, 0u, VRJ_DENOISE_DEFAULT_SIGMA_LUMINANCE, VRJ_DENOISE_DEFAULT_SIGMA_NORMAL,
+                                  VRJ_DENOISE_DEFAULT_SIGMA_DEPTH};
+    ImageRgbU8 image(width_, height_);
+    if (vrj_denoise(device_, VRJ_MEM_DEVICE, width_, height_, sum_, weight_, y_sq_sum_, normal_, depth_, material_, &params, denoised_, srgb8_,
+                    nullptr) != VRJ_OK ||
+        vrj_copy_to_host(device_, image.pixel_data().data(), srgb8_, 3 * width_ * height_) != VRJ_OK)
+        throw std::runtime_error(std::string("DeviceProgressiveBuffer::denoised_image_rgb_u8: ") + vrj_last_error());
+    return image;
+}
+AccumulationBuffer DeviceProgressiveBuffer::download() const {
+    AccumulationBuffer b(width_, height_, AccumulationBuffer::Uninitialized{});
+    const size_t n = width_ * height_;
+    const struct {
+        double *dst;
+        const double *src;
+        size_t count;
+    } copies[5] = {{b.colour.data(), colour_, 3 * n}, {b.colour_sum.data(), sum_, 3 * n}, {b.colour_bias.data(), bias_, 3 * n},
+                   {b.weight.data(), weight_, n}, {b.weight_bias.data(), weight_bias_, n}};
+    for (const auto &c : copies)
+        if (vrj_copy_to_host(device_, c.dst, c.src, c.count * 8) != VRJ_OK) throw std::runtime_error(std::string("vrj_copy_to_host: ") + vrj_last_error());
+    return b;
+}
+std::vector<double> DeviceProgressiveBuffer::download_y_sq_sum() const {
+    std::vector<double> q(width_ * height_);
+    if (vrj_copy_to_host(device_, q.data(), y_sq_sum_, q.size() * 8) != VRJ_OK) throw std::runtime_error(std::string("vrj_copy_to_host: ") + vrj_last_error());
+    return q;
 }
 
 } // namespace vanrijn

@@ -908,6 +908,14 @@ void fill_call_stats(VrjStats *st, const Scratch *s, const unsigned long long *h
     st->coalesced_calls = 1;
 }
 
+// VrjAccumOut.colour from (colour_sum, weight), as k_resolve computes it (vrj_render_sharded, vrj_render_progressive)
+__global__ void k_finalize(const double *sum, const double *weight, double *colour, uint32_t npix) {
+    uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= npix) return;
+    double inv = 1.0 / weight[p]; // accumulation_buffer.rs:59
+    colour[3 * p] = sum[3 * p] * inv, colour[3 * p + 1] = sum[3 * p + 1] * inv, colour[3 * p + 2] = sum[3 * p + 2] * inv;
+}
+
 // the tone-mapped colours of the block's accumulators to out->srgb8
 VrjStatus copy_srgb8(Scratch *s, uint64_t npix, uint8_t *dst, cudaMemcpyKind kind, uint64_t *launches) {
     if (s->srgb8.bytes < npix * 3) {
@@ -917,6 +925,18 @@ VrjStatus copy_srgb8(Scratch *s, uint64_t npix, uint8_t *dst, cudaMemcpyKind kin
     k_tone_map<<<(unsigned)((npix + 255) / 256), 256, 0, s->stream>>>(s->acc_colour.as<double>(), s->srgb8.as<unsigned char>(), npix, 0);
     (*launches)++;
     VRJ_CUDA(cudaMemcpyAsync(dst, s->srgb8.p, npix * 3, kind, s->stream));
+    return VRJ_OK;
+}
+
+// y_sq_sum, two pixel lists and a counter for npix pixels (vrj_render_adaptive, vrj_render_progressive)
+VrjStatus ensure_adaptive_buffers(Scratch *s, uint64_t npix) {
+    if (s->adapt_npix >= npix) return VRJ_OK;
+    s->adapt_npix = 0;
+    std::vector<std::pair<DeviceBuffer *, size_t>> want = {{&s->ysq, npix * 8}, {&s->alist[0], npix * 4}, {&s->alist[1], npix * 4},
+                                                           {&s->aconverged, 8}};
+    const VrjStatus st = alloc_group(s->adapt_slab, want, "adaptive sampling buffers");
+    if (st != VRJ_OK) return st;
+    s->adapt_npix = npix;
     return VRJ_OK;
 }
 
@@ -1546,14 +1566,8 @@ VrjStatus vrj_render_adaptive(const VrjScene *scene_c, const VrjTile *tile, uint
     const uint32_t filter = effective_filter(scene, p);
     st = ensure_call_scratch(s, p, call_wants_records(scene, p, filter), npix, &batch, n_light_samples);
     if (st != VRJ_OK) return st;
-    if (s->adapt_npix < npix) {
-        s->adapt_npix = 0;
-        std::vector<std::pair<DeviceBuffer *, size_t>> want = {{&s->ysq, npix * 8}, {&s->alist[0], npix * 4}, {&s->alist[1], npix * 4},
-                                                               {&s->aconverged, 8}};
-        st = alloc_group(s->adapt_slab, want, "adaptive sampling buffers");
-        if (st != VRJ_OK) return st;
-        s->adapt_npix = npix;
-    }
+    st = ensure_adaptive_buffers(s, npix);
+    if (st != VRJ_OK) return st;
     const size_t capacity = npix * batch; // paths per batch
     DeviceBuffer *zero[5] = {&s->acc_sum, &s->acc_bias, &s->acc_weight, &s->acc_wbias, &s->ysq};
     const size_t per[5] = {3, 3, 1, 1, 1};
@@ -1635,6 +1649,184 @@ VrjStatus vrj_render_adaptive(const VrjScene *scene_c, const VrjTile *tile, uint
     if (astats) {
         astats->passes = passes, astats->samples = samples;
         astats->pixels_converged = *host_converged, astats->pixels_unconverged = npix - *host_converged;
+    }
+    return VRJ_OK;
+}
+
+// Progressive rendering (the header states the schedule).  Before each pass k_progressive_select judges every pixel of the
+// tile on the state and writes the count it takes; the host reads back the counters (one 48-byte copy per pass).  When every
+// active pixel takes the same count c -- always, for a state this call's schedule produced with unchanged parameters -- the
+// pass is one sub-pass: the scan of the select's flags and k_progressive_compact list the active pixels with their first new
+// sample, and the LIST = 2 kernels render samples base .. base + c - 1 of each, resolved by k_resolve_adaptive.  Otherwise
+// the pass runs one such sub-pass per distinct count, largest first (k_progressive_group picks the pixels).  Pixel lists stay
+// row-major.  The state goes into the block once (copied from the host, or device to device) and comes back once.
+VrjStatus vrj_render_progressive(const VrjScene *scene_c, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p,
+                                 const VrjProgressiveParams *pp, VrjAccumOut *out, double *y_sq_sum, VrjProgressiveStats *pstats) {
+    VrjScene *scene = const_cast<VrjScene *>(scene_c);
+    size_t n_light_samples = 0;
+    VrjStatus st = check_render_args(scene, tile, height, width, p, out, &n_light_samples);
+    if (st != VRJ_OK) return st;
+    if (!pp) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (p->spp != 0) return fail(VRJ_ERR_INVALID_ARGUMENT, "params->spp must be 0: vrj_render_progressive takes its sample counts from VrjProgressiveParams");
+    if (pp->min_samples < 2) return fail(VRJ_ERR_INVALID_ARGUMENT, "min_samples must be >= 2 (the variance needs two samples)");
+    if (pp->max_samples < pp->min_samples) return fail(VRJ_ERR_INVALID_ARGUMENT, "max_samples must be >= min_samples");
+    if (pp->pass_samples < 1) return fail(VRJ_ERR_INVALID_ARGUMENT, "pass_samples must be >= 1");
+    if (!(pp->rel_error > 0.0) || !std::isfinite(pp->rel_error)) return fail(VRJ_ERR_INVALID_ARGUMENT, "rel_error must be > 0 and finite");
+    if (!(pp->abs_floor >= 0.0) || !std::isfinite(pp->abs_floor)) return fail(VRJ_ERR_INVALID_ARGUMENT, "abs_floor must be >= 0 and finite");
+    if (out->memory > VRJ_MEM_DEVICE) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown memory kind");
+    if (!out->colour_sum || !out->colour_bias || !out->weight || !out->weight_bias || !y_sq_sum)
+        return fail(VRJ_ERR_INVALID_ARGUMENT, "the state (colour_sum, colour_bias, weight, weight_bias, y_sq_sum) is required");
+    if (out->photons) return fail(VRJ_ERR_UNSUPPORTED, "vrj_render_progressive has no photons output");
+    const uint64_t npix = (tile->end_column - tile->start_column) * (tile->end_row - tile->start_row);
+    DeviceGuard device_guard;
+    VRJ_NVTX_RANGE(call_range, "vrj_render_progressive");
+    if (out->stats) std::memset(out->stats, 0, sizeof(VrjStats));
+    if (pstats) std::memset(pstats, 0, sizeof(VrjProgressiveStats));
+    if (npix == 0) return VRJ_OK;
+    VRJ_CUDA(cudaSetDevice(scene->device));
+
+    ActiveCall active(g_active_calls[(unsigned)scene->device % 64]);
+    // the widest pass is the whole tile at max(min, pass) samples (a fresh state's first pass, or a state that every pixel
+    // has to continue); the block is sized for it
+    const uint32_t widest = std::min(pp->max_samples, std::max(pp->min_samples, pp->pass_samples));
+    uint32_t batch = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(widest, call_path_budget(scene, active) / npix));
+    if (npix * (uint64_t)batch > 0xfffffff0ull) return fail(VRJ_ERR_UNSUPPORTED, "tile too large");
+    Scratch *s = acquire_scratch(scene, npix * batch);
+    struct Releaser {
+        VrjScene *sc;
+        Scratch *s;
+        ~Releaser() {
+            if (s->stream) cudaStreamSynchronize(s->stream);
+            release_scratch(sc, s);
+        }
+    } releaser{scene, s};
+    const uint32_t filter = effective_filter(scene, p);
+    st = ensure_call_scratch(s, p, call_wants_records(scene, p, filter), npix, &batch, n_light_samples);
+    if (st != VRJ_OK) return st;
+    st = ensure_adaptive_buffers(s, npix);
+    if (st != VRJ_OK) return st;
+    if (s->prog_npix < npix) {
+        s->prog_npix = 0;
+        std::vector<std::pair<DeviceBuffer *, size_t>> want = {{&s->pcount, npix * 4}, {&s->pcounters, sizeof(ProgressiveCounters)}};
+        st = alloc_group(s->prog_slab, want, "progressive rendering buffers");
+        if (st != VRJ_OK) return st;
+        s->prog_npix = npix;
+    }
+    const size_t capacity = npix * batch; // paths per batch
+    const cudaMemcpyKind in_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    const cudaMemcpyKind out_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    struct Arr {
+        double *user;
+        DeviceBuffer *dev;
+        size_t per;
+    } state[5] = {{out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3}, {out->weight, &s->acc_weight, 1},
+                  {out->weight_bias, &s->acc_wbias, 1}, {y_sq_sum, &s->ysq, 1}};
+    for (const Arr &a : state) {
+        if (out->accumulate) VRJ_CUDA(cudaMemcpyAsync(a.dev->p, a.user, npix * a.per * sizeof(double), in_kind, s->stream));
+        else VRJ_CUDA(cudaMemsetAsync(a.dev->p, 0, npix * a.per * sizeof(double), s->stream));
+    }
+    VRJ_CUDA(cudaMemsetAsync(s->stats.p, 0, ST_COUNT * sizeof(unsigned long long), s->stream));
+    st = stage_lights(s, p);
+    if (st != VRJ_OK) return st;
+
+    RenderConst rc = make_render_const(tile, height, width, p);
+    rc.lights = s->lights.as<LightDev>();
+    rc.light_samples = s->light_samples.as<double>();
+    rc.div_tile_w = FastDiv::make(rc.tile_w);
+    const uint32_t n = (uint32_t)npix;
+    // the flags and the scan's tile totals live in the photon buffer, as in vrj_render_adaptive
+    uint32_t *flags = s->photons.as<uint32_t>(), *count = s->pcount.as<uint32_t>();
+    uint32_t *list = s->alist[0].as<uint32_t>(), *base = s->alist[1].as<uint32_t>();
+    ProgressiveCounters *ctr = s->pcounters.as<ProgressiveCounters>();
+    // pinned slots (host_count: 0..3 drain check, 8.. sample table, 160.. stats, 192.. vrj_render_adaptive)
+    ProgressiveCounters *hctr = reinterpret_cast<ProgressiveCounters *>(s->host_count + 200);
+    uint32_t *host_listed = s->host_count + 216;
+    const unsigned grid = (n + 1 + 255) / 256;
+    uint64_t launches = 0, passes = 0, samples = 0;
+    s->n_marks = 0;
+    RenderTurn turn(scene->device); // declared after `releaser`: an early return gives the turn back before the block
+    turn.acquire();
+    VRJ_CUDA(cudaEventRecord(s->ev0, s->stream));
+    // the samples base[i] .. base[i] + c - 1 of the m listed pixels, in batches split to the path budget
+    auto render_listed = [&](uint32_t m, uint32_t c) -> VrjStatus {
+        const uint32_t b = (uint32_t)std::max<size_t>(1, std::min<size_t>(c, capacity / m));
+        rc.npix = m, rc.pixel_list = list, rc.pixel_base = base;
+        for (uint32_t done = 0; done < c; done += b) {
+            rc.batch_samples = std::min(b, c - done);
+            rc.div_batch = FastDiv::make(rc.batch_samples);
+            rc.first_sample = p->sample_offset + (uint64_t)done * rc.sample_stride;
+            const VrjStatus bst = dispatch_batch(scene, s, rc, p, filter, &launches, nullptr, s->ysq.as<double>());
+            if (bst != VRJ_OK) return bst;
+        }
+        samples += (uint64_t)m * c;
+        return VRJ_OK;
+    };
+    for (;;) {
+        VRJ_CUDA(cudaMemsetAsync(ctr, 0, sizeof(ProgressiveCounters), s->stream));
+        VRJ_CUDA(cudaMemsetAsync(&ctr->cmin, 0xff, sizeof(uint32_t), s->stream));
+        k_progressive_select<<<grid, 256, 0, s->stream>>>(s->acc_sum.as<double>(), s->acc_weight.as<double>(), s->ysq.as<double>(), n, pp->min_samples,
+                                                          pp->max_samples, pp->pass_samples, pp->rel_error, pp->abs_floor, count, flags, ctr);
+        launches++;
+        VRJ_CUDA(cudaGetLastError());
+        VRJ_CUDA(cudaMemcpyAsync(hctr, ctr, sizeof(ProgressiveCounters), cudaMemcpyDeviceToHost, s->stream));
+        VRJ_CUDA(cudaStreamSynchronize(s->stream));
+        if (hctr->bad) return fail(VRJ_ERR_INVALID_ARGUMENT, "a weight of the state is not a sample count (negative, fractional, not finite or >= 2^32)");
+        if (hctr->active == 0 || (pp->max_passes && passes == pp->max_passes)) break;
+        if (hctr->cmax == hctr->cmin) {
+            st = vrj_build::exclusive_scan_u32(flags, n + 1, flags + n + 1, s->stream);
+            if (st != VRJ_OK) return st;
+            k_progressive_compact<<<(n + 255) / 256, 256, 0, s->stream>>>(s->acc_weight.as<double>(), flags, n, list, base);
+            launches += 4;
+            VRJ_CUDA(cudaGetLastError());
+            st = render_listed((uint32_t)hctr->active, hctr->cmax);
+            if (st != VRJ_OK) return st;
+        } else {
+            for (uint32_t cur = hctr->cmax; cur != 0;) {
+                VRJ_CUDA(cudaMemsetAsync(&ctr->next, 0, sizeof(uint32_t), s->stream));
+                k_progressive_group<<<grid, 256, 0, s->stream>>>(count, n, cur, flags, ctr);
+                st = vrj_build::exclusive_scan_u32(flags, n + 1, flags + n + 1, s->stream);
+                if (st != VRJ_OK) return st;
+                k_progressive_compact<<<(n + 255) / 256, 256, 0, s->stream>>>(s->acc_weight.as<double>(), flags, n, list, base);
+                launches += 5;
+                VRJ_CUDA(cudaGetLastError());
+                VRJ_CUDA(cudaMemcpyAsync(host_listed, flags + n, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
+                VRJ_CUDA(cudaMemcpyAsync(&hctr->next, &ctr->next, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
+                VRJ_CUDA(cudaStreamSynchronize(s->stream));
+                const uint32_t m = *host_listed, next = hctr->next;
+                if (m) {
+                    st = render_listed(m, cur);
+                    if (st != VRJ_OK) return st;
+                }
+                cur = next;
+            }
+        }
+        passes++;
+    }
+    const ProgressiveCounters final_ctr = *hctr;
+    if (out->colour || out->srgb8) {
+        k_finalize<<<(n + 255) / 256, 256, 0, s->stream>>>(s->acc_sum.as<double>(), s->acc_weight.as<double>(), s->acc_colour.as<double>(), n);
+        launches++;
+        VRJ_CUDA(cudaGetLastError());
+    }
+    unsigned long long *hstats = reinterpret_cast<unsigned long long *>(s->host_count + 160);
+    VRJ_CUDA(cudaEventRecord(s->ev1, s->stream));
+    VRJ_CUDA(cudaMemcpyAsync(hstats, s->stats.p, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+    for (const Arr &a : state) VRJ_CUDA(cudaMemcpyAsync(a.user, a.dev->p, npix * a.per * sizeof(double), out_kind, s->stream));
+    if (out->colour) VRJ_CUDA(cudaMemcpyAsync(out->colour, s->acc_colour.p, npix * 3 * sizeof(double), out_kind, s->stream));
+    if (out->srgb8) {
+        st = copy_srgb8(s, npix, out->srgb8, out_kind, &launches);
+        if (st != VRJ_OK) return st;
+    }
+    VRJ_CUDA(cudaEventRecord(s->ev_done, s->stream));
+    VRJ_CUDA(wait_event(s->ev1, scene->device)); // the last kernel is done: the next caller may render while this one's copies run
+    turn.release();
+    VRJ_CUDA(wait_event(s->ev_done, scene->device));
+    float ms = 0.f;
+    VRJ_CUDA(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+    if (out->stats) fill_call_stats(out->stats, s, hstats, launches, ms);
+    if (pstats) {
+        pstats->passes = passes, pstats->samples = samples;
+        pstats->pixels_converged = final_ctr.converged, pstats->pixels_at_max = final_ctr.at_max, pstats->pixels_active = final_ctr.active;
     }
     return VRJ_OK;
 }
@@ -1920,12 +2112,6 @@ struct NcclApi {
 NcclApi g_nccl;
 const int kNcclDouble = 8, kNcclSum = 0; // nccl.h: ncclFloat64 = 8, ncclSum = 0
 
-__global__ void k_finalize(const double *sum, const double *weight, double *colour, uint32_t npix) {
-    uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= npix) return;
-    double inv = 1.0 / weight[p]; // accumulation_buffer.rs:59
-    colour[3 * p] = sum[3 * p] * inv, colour[3 * p + 1] = sum[3 * p + 1] * inv, colour[3 * p + 2] = sum[3 * p + 2] * inv;
-}
 } // namespace
 
 struct VrjComm {

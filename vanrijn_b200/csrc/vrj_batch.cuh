@@ -83,6 +83,8 @@ struct Scratch {
     DeviceBuffer lights, light_samples, srgb8;
     DeviceBuffer ysq, alist[2], aconverged, adapt_slab; // vrj_render_adaptive: y_sq_sum, this / next pass's pixel list, a counter
     size_t adapt_npix = 0;
+    DeviceBuffer pcount, pcounters, prog_slab; // vrj_render_progressive: per-pixel count of the pass, ProgressiveCounters
+    size_t prog_npix = 0;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr; // first / last kernel of a call
     cudaEvent_t ev_done = nullptr;             // behind the call's last copy
@@ -185,7 +187,7 @@ inline bool wants_records(const VrjScene *sc, int walk) {
 }
 
 // One batch with the integrator (WHITTED) and the scene's material kinds (MM, see vrj_device.cuh) fixed at compile time.
-template <typename NT, typename R, bool COUNT, bool WHITTED, int MM, bool LIST>
+template <typename NT, typename R, bool COUNT, bool WHITTED, int MM, int LIST>
 VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int walk, uint64_t *launches, const MultiCalls *multi,
                      const ResolveCopy *copy, double *ysq) {
     const bool quad = walk == 1, q16 = walk == 2; // 0: the 2-wide tree in NT boxes; 1: 4-wide f32; 2: 2-wide on the 16-bit grid
@@ -320,7 +322,7 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
 
 // kernel variants exist for "Lambertian only" (the reference's own scenes: main.rs, benches/simple_scene.rs) and for
 // "any material"; VRJ_MATERIAL_MASK=15 in the environment forces the general variant (experiments)
-template <typename NT, typename R, bool COUNT, bool LIST>
+template <typename NT, typename R, bool COUNT, int LIST>
 VrjStatus run_materials(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches, const MultiCalls *multi,
                         const ResolveCopy *copy, double *ysq) {
     const bool lambert_only = sc->kernel_material_mask == 1u;
@@ -330,13 +332,14 @@ VrjStatus run_materials(const VrjScene *sc, Scratch *s, const RenderConst &rc, b
     return lambert_only ? run_levels<NT, R, COUNT, false, 1, LIST>(sc, s, rc, walk, launches, multi, copy, ysq)
                         : run_levels<NT, R, COUNT, false, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches, multi, copy, ysq);
 }
-// `ysq` (vrj_render_adaptive): the batch is resolved by k_resolve_adaptive, which also keeps y_sq_sum; a batch over
-// rc.pixel_list runs the LIST variants of the kernels
+// `ysq` (vrj_render_adaptive, vrj_render_progressive): the batch is resolved by k_resolve_adaptive, which also keeps
+// y_sq_sum; a batch over rc.pixel_list runs the LIST variants of the kernels (LIST = 2 when rc.pixel_base is set too)
 template <typename NT, typename R, bool COUNT>
 VrjStatus run_batch(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches, const MultiCalls *multi = nullptr,
                     const ResolveCopy *copy = nullptr, double *ysq = nullptr) {
-    return rc.pixel_list ? run_materials<NT, R, COUNT, true>(sc, s, rc, whitted, walk, launches, multi, copy, ysq)
-                         : run_materials<NT, R, COUNT, false>(sc, s, rc, whitted, walk, launches, multi, copy, ysq);
+    if (rc.pixel_base) return run_materials<NT, R, COUNT, 2>(sc, s, rc, whitted, walk, launches, multi, copy, ysq);
+    return rc.pixel_list ? run_materials<NT, R, COUNT, 1>(sc, s, rc, whitted, walk, launches, multi, copy, ysq)
+                         : run_materials<NT, R, COUNT, 0>(sc, s, rc, whitted, walk, launches, multi, copy, ysq);
 }
 
 } // namespace vrjimpl

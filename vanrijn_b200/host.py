@@ -214,6 +214,40 @@ class HostScene:
         out["stats"], out["adaptive"] = st, ast
         return out
 
+    def render_progressive(self, tile, height, width, min_samples, max_samples, pass_samples, rel_error, abs_floor=0.0,
+                           max_passes=0, state=None, want=("colour",), device=0, **kw):
+        """vrj_render_progressive with host buffers: continues `state` (the dict a previous call returned; None: start from
+        zero) for at most `max_passes` passes (0: until no pixel is active) of the adaptive schedule.  `want` adds the optional
+        outputs ("colour", "srgb8"); `kw` are the render parameters of make_params (spp excepted).  Returns a dict with the
+        new state (colour_sum, colour_bias, weight, weight_bias, y_sq_sum: fresh arrays, `state` is not modified), the wanted
+        outputs, 'stats' (VrjStats) and 'progressive' (VrjProgressiveStats)."""
+        sc, ec, sr, er = tile
+        npix = (ec - sc) * (er - sr)
+        kw.setdefault("spp", 0)
+        p, keep = self.make_params(**kw)
+        pp = capi.ProgressiveParams(min_samples=min_samples, max_samples=max_samples, pass_samples=pass_samples,
+                                    max_passes=max_passes, rel_error=rel_error, abs_floor=abs_floor)
+        out = {}
+        ao = capi.AccumOut(memory=capi.MEM_HOST, accumulate=0 if state is None else 1)
+        for name, per in (("colour_sum", 3), ("colour_bias", 3), ("weight", 1), ("weight_bias", 1), ("y_sq_sum", 1)):
+            out[name] = np.zeros(npix * per) if state is None else np.array(state[name], np.float64, copy=True)
+            assert out[name].size == npix * per
+            if name != "y_sq_sum":
+                setattr(ao, name, out[name].ctypes.data)
+        if "colour" in want:
+            out["colour"] = np.zeros(npix * 3)
+            ao.colour = out["colour"].ctypes.data
+        if "srgb8" in want:
+            out["srgb8"] = np.zeros(npix * 3, np.uint8)
+            ao.srgb8 = out["srgb8"].ctypes.data
+        st, pst = capi.Stats(), capi.ProgressiveStats()
+        ao.stats = C.pointer(st)
+        t = capi.Tile(sc, ec, sr, er)
+        capi.check(capi.cuda().vrj_render_progressive(self.device_scene(device), C.byref(t), height, width, C.byref(p), C.byref(pp),
+                                                      C.byref(ao), out["y_sq_sum"].ctypes.data, C.byref(pst)))
+        out["stats"], out["progressive"] = st, pst
+        return out
+
     def render_aux(self, tile, height, width, spp=1, want=("normal", "depth", "object_id", "material"), device=0, **kw):
         """vrj_render_aux with host output buffers: the first-hit features of the camera rays that a render with the same
         spp, seed, sample_offset and sample_stride traces (`kw`: the other keywords of make_params).  Returns a dict of numpy

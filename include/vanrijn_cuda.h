@@ -298,11 +298,12 @@ VRJ_API VrjStatus vrj_render_tile(const VrjScene *scene, const VrjTile *tile, ui
  * y_sq_sum (optional, NULL: not returned): one double per pixel, memory of the kind out->memory says; q = q + y * y over the
  * pixel's samples in sample order, y being exactly the Y value the sample adds to colour_sum.
  * out: the arrays, layout and memory kinds of vrj_render_tile, srgb8 included; out->stats sums the passes (device_ms spans
- * the first to the last kernel, the per-pass readback of the active count -- 4 bytes -- included).  out->accumulate and
+ * the first to the last kernel, the readback of 48 bytes of pixel counts after each pass included).  out->accumulate and
  * out->photons: VRJ_ERR_UNSUPPORTED.  params: every field keeps its meaning (integrators, lights, filters, precisions,
  * sample_stride, count_traversal) except spp, which must be 0 (the counts come from `ap`).  astats may be NULL.
  * Scheduling: the call is never coalesced with others; it takes the device's render turn like any other call and uses a
- * scratch block from the pool (16 bytes per pixel more than vrj_render_tile: y_sq_sum and two pixel lists). */
+ * scratch block from the pool (20 bytes per pixel more than vrj_render_tile: y_sq_sum, two pixel lists and the first
+ * samples of one). */
 typedef struct VrjAdaptiveParams {
     uint32_t min_samples;   /* every pixel first takes samples 0..min_samples-1; >= 2 */
     uint32_t max_samples;   /* no pixel takes more; >= min_samples */
@@ -353,9 +354,10 @@ VRJ_API VrjStatus vrj_render_adaptive(const VrjScene *scene, const VrjTile *tile
  *  (e) calls with min_samples == max_samples = 4, 8, 12, ... are a uniform progressive frame, y_sq_sum included.
  * pstats (host, may be NULL): passes and samples run by this call; the three pixel counts describe the state at return and
  * add up to the tile's pixels.  out->stats sums the call's passes like vrj_render_adaptive's.
- * Scheduling: never coalesced; takes the device's render turn; uses a scratch block from the pool (y_sq_sum, two pixel
- * lists and a per-pixel count: 20 bytes per pixel more than vrj_render_tile).  Pixels of one pass that take different
- * counts are rendered in one sub-pass per distinct count. */
+ * Scheduling: never coalesced; takes the device's render turn; uses a scratch block from the pool (20 bytes per pixel more
+ * than vrj_render_tile, as vrj_render_adaptive).  The host reads back 48 bytes of pixel counts after each pass (and, for a
+ * continued state, before the first), and 8 more per distinct count when the pixels of one pass take different counts;
+ * those are rendered in one sub-pass per count. */
 typedef struct VrjProgressiveParams {
     uint32_t min_samples;   /* as VrjAdaptiveParams: >= 2 */
     uint32_t max_samples;   /* >= min_samples */

@@ -312,7 +312,7 @@ std::unordered_map<void *, size_t> g_host_pool_live;
 // Blocks are kept for concurrent callers (main.rs:197-209 drives the entry point from a pool of workers, each call needing
 // its own block): up to 16 per device as long as what the pool holds stays under 48 GB -- sixteen 1-spp 1080p blocks are
 // 14 GB, one 64-spp block is 45 GB.  A caller is handed the smallest pooled block that is large enough, else the largest.
-size_t scratch_bytes(const Scratch *s) { return s->capacity * 240 + s->rec_capacity * sizeof(TraceRec) + s->npix * 88 + s->adapt_npix * 16; }
+size_t scratch_bytes(const Scratch *s) { return s->capacity * 240 + s->rec_capacity * sizeof(TraceRec) + s->npix * 88 + s->pass_npix * 20; }
 std::atomic<int> g_active_calls[64];
 
 // Render gate: how many calls may have their wavefronts on one device at the same moment.  main.rs:197-209 drives the entry
@@ -399,6 +399,18 @@ void release_scratch(VrjScene *sc, Scratch *s) {
     if (same < 16 && (same < 2 || bytes <= (size_t(48) << 30))) g_pool.push_back({sc->device, s});
     else delete s;
 }
+// a call's block: whatever path leaves the call (an error in the middle of a batch loop included), nothing may still be
+// running on the block's streams when another caller is handed it
+struct BlockLease {
+    VrjScene *sc;
+    Scratch *s = nullptr;
+    ~BlockLease() {
+        if (!s) return;
+        if (s->stream) cudaStreamSynchronize(s->stream);
+        if (s->copy_stream) cudaStreamSynchronize(s->copy_stream);
+        release_scratch(sc, s);
+    }
+};
 
 // A group of a block's buffers is all-or-nothing: a failed allocation leaves the group empty with its size field at 0 (never
 // half-sized or stale), so the block can go back to the pool and the caller can retry
@@ -436,7 +448,7 @@ VrjStatus ensure_scratch(Scratch *s, size_t capacity, size_t rec_capacity, size_
         VRJ_CUDA(cudaEventCreateWithFlags(&s->copy_done, cudaEventDisableTiming));
         for (cudaEvent_t &e : s->piece_ev) VRJ_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         for (cudaEvent_t &e : s->drain_ev) VRJ_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        VRJ_CUDA(cudaMallocHost(&s->host_count, 256 * sizeof(uint32_t))); // drain-check slots + the sample table of coalesced calls
+        VRJ_CUDA(cudaMallocHost(reinterpret_cast<void **>(&s->pinned), sizeof(PinnedBlock)));
     }
     // every group below is all-or-nothing (alloc_group)
     if (s->capacity < capacity) {
@@ -533,250 +545,6 @@ void fill_stats(VrjStats *st, const unsigned long long *h, uint64_t launches, fl
     st->device_ms = ms;
 }
 
-
-// ---------------------------------------------------------------------------------------------- coalesced calls
-// main.rs:197-209 calls partial_render_scene once per one-sample pass from a pool of workers.  Each such call is a small
-// wavefront (2 M paths at 1080p) whose ~28 launches do not fill 148 SMs: 1.7 ms of device time against 0.52 ms per sample
-// when 64 samples share a wavefront.  Calls that arrive while the device is busy and differ only in their sample indices and
-// output buffers are therefore rendered TOGETHER: one of the waiting callers (the leader) takes its turn at the render gate,
-// collects every compatible caller that has queued up behind it, runs one wavefront over all their samples (the batch's slots
-// carry their sample indices in a table, RenderConst::sample_table), resolves each call's samples into that call's own
-// fresh buffer (k_resolve_multi) and copies every buffer back.  A sample is a pure function of (seed, pixel, sample index)
-// and each call's samples are applied to its buffer in sample order, so every caller receives bit for bit what it would have
-// received alone (tests/test_gpu_parity.py::test_coalesced_calls_bit_identical).  The ray counters of a shared wavefront are
-// split evenly over its calls (the remainder goes to the first; sums stay exact) and VrjStats.coalesced_calls says how many
-// shared it.  VRJ_COALESCE=0 turns this off (experiments).
-struct CoalesceRequest {
-    const VrjScene *scene;
-    VrjTile tile;
-    uint64_t height, width;
-    VrjRenderParams params;
-    VrjAccumOut *out;
-    VrjStatus status = VRJ_OK;
-    std::string error;
-    bool done = false;     // a leader failed before launching anything: `status` / `error` say why
-    bool launched = false; // rendered by a leader: stats are filled, the buffers are on their way, `wait_ev` fires on arrival
-    cudaEvent_t wait_ev = nullptr;
-    uint32_t wanted() const {
-        return (out->colour ? 1u : 0u) | (out->colour_sum ? 2u : 0u) | (out->colour_bias ? 4u : 0u) | (out->weight ? 8u : 0u) | (out->weight_bias ? 16u : 0u);
-    }
-    bool compatible(const CoalesceRequest &o) const {
-        return scene == o.scene && tile.start_column == o.tile.start_column && tile.end_column == o.tile.end_column &&
-               tile.start_row == o.tile.start_row && tile.end_row == o.tile.end_row && height == o.height && width == o.width &&
-               params.max_depth == o.params.max_depth && params.seed == o.params.seed && params.bvh_filter == o.params.bvh_filter &&
-               params.precision == o.params.precision && params.bias == o.params.bias &&
-               (params.sample_stride ? params.sample_stride : 1u) == (o.params.sample_stride ? o.params.sample_stride : 1u) && wanted() == o.wanted();
-    }
-};
-struct Coalescer {
-    std::mutex m;
-    std::condition_variable cv;
-    std::vector<CoalesceRequest *> waiting;
-    bool collecting = false; // a leader is waiting for its turn at the gate; arrivals pile up behind it
-};
-Coalescer g_coalescer[64];
-constexpr uint64_t kCoalesceMaxPaths = uint64_t(1) << 25; // 32 Mi paths = 11 GB of queue state per shared wavefront
-
-bool coalescing_enabled() {
-    static const bool on = [] {
-        const char *e = std::getenv("VRJ_COALESCE");
-        return !e || std::atoi(e) != 0;
-    }();
-    return on;
-}
-bool coalescable(const VrjRenderParams *p, const VrjAccumOut *out, uint64_t npix) {
-    return coalescing_enabled() && out->memory == VRJ_MEM_HOST && !out->accumulate && !out->photons && !out->srgb8 && out->colour &&
-           p->integrator == VRJ_INTEGRATOR_SIMPLE_RANDOM && p->n_lights == 0 && !p->ambient_light && !p->count_traversal &&
-           p->spp >= 1 && p->spp <= 4 && npix * p->spp * 2 <= kCoalesceMaxPaths;
-}
-
-// one wavefront for `n` compatible requests; fills their buffers and stats; the status applies to all of them
-VrjStatus render_group(Coalescer &co, CoalesceRequest *const *reqs, uint32_t n, RenderTurn &turn, bool *published) {
-    static const bool timing = std::getenv("VRJ_TIMING") != nullptr;
-    const auto t1 = std::chrono::steady_clock::now();
-    const CoalesceRequest &r0 = *reqs[0];
-    VrjScene *scene = const_cast<VrjScene *>(r0.scene);
-    const VrjRenderParams *p = &r0.params;
-    RenderConst rc = make_render_const(&r0.tile, r0.height, r0.width, p);
-    const uint64_t npix = rc.npix;
-    uint32_t total = 0;
-    MultiCalls mc{};
-    mc.n = n, mc.full = (r0.wanted() & ~1u) ? 1u : 0u;
-    std::vector<uint64_t> table;
-    for (uint32_t c = 0; c < n; c++) {
-        mc.first[c] = total, mc.count[c] = reqs[c]->params.spp;
-        for (uint32_t i = 0; i < reqs[c]->params.spp; i++) table.push_back(reqs[c]->params.sample_offset + (uint64_t)i * rc.sample_stride);
-        total += reqs[c]->params.spp;
-    }
-    VRJ_NVTX_RANGE(call_range, "vrj_render_tile (coalesced)");
-    // group sizes vary from wavefront to wavefront: blocks are sized in steps of eight 1-sample calls so that a block taken
-    // from the pool almost never has to grow (growing re-allocates every queue: tens of milliseconds)
-    const size_t capacity = npix * (size_t)((total + 7u) / 8u * 8u);
-    Scratch *s = acquire_scratch(scene, capacity);
-    struct Releaser {
-        VrjScene *sc;
-        Scratch *s;
-        ~Releaser() {
-            if (s->stream) cudaStreamSynchronize(s->stream);
-            release_scratch(sc, s);
-        }
-    } releaser{scene, s};
-    const uint32_t filter = effective_filter(scene, p);
-    const bool records = p->precision == VRJ_PRECISION_F64 && filter == VRJ_FILTER_F32 && scene->trace_records && scene->dev.n_bvh_items > 0;
-    VrjStatus st = ensure_scratch(s, capacity, records ? capacity : 0, 0, p->max_depth + 3, 0, 0);
-    if (st == VRJ_ERR_OUT_OF_MEMORY) { // fall back to exactly what this wavefront needs
-        vrj_pool_trim();
-        st = ensure_scratch(s, npix * total, records ? npix * total : 0, 0, p->max_depth + 3, 0, 0);
-    }
-    if (st != VRJ_OK) return st;
-    const auto t1b = std::chrono::steady_clock::now();
-    const size_t per_call = npix * (mc.full ? 11 : 3) * sizeof(double);
-    if (s->multi_out.bytes < per_call * n || !s->multi_out.p) {
-        // sized once for the largest group this tile size can form (1-sample calls up to the path limit)
-        const size_t max_calls = std::max<size_t>(n, std::min<size_t>(MULTI_MAX_CALLS, kCoalesceMaxPaths / std::max<uint64_t>(npix, 1)));
-        s->multi_out.release();
-        VRJ_CUDA(s->multi_out.alloc(per_call * max_calls));
-    }
-    if (!s->sample_table.p) VRJ_CUDA(s->sample_table.alloc(4 * MULTI_MAX_CALLS * sizeof(uint64_t)));
-    double *base = s->multi_out.as<double>();
-    mc.out.colour = base;
-    if (mc.full) {
-        mc.out.sum = base + 3 * npix * n, mc.out.bias = base + 6 * npix * n;
-        mc.out.weight = base + 9 * npix * n, mc.out.weight_bias = base + 10 * npix * n;
-    }
-    // the table goes through the block's pinned slot (entries 8.. of host_count; the drain check uses 0..3)
-    uint64_t *pinned_table = reinterpret_cast<uint64_t *>(s->host_count + 8);
-    std::memcpy(pinned_table, table.data(), table.size() * sizeof(uint64_t));
-    VRJ_CUDA(cudaMemcpyAsync(s->sample_table.p, pinned_table, table.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s->stream));
-    VRJ_CUDA(cudaMemsetAsync(s->stats.p, 0, ST_COUNT * sizeof(unsigned long long), s->stream));
-    rc.sample_table = s->sample_table.as<uint64_t>();
-    rc.lights = s->lights.as<LightDev>(), rc.light_samples = s->light_samples.as<double>();
-    rc.batch_samples = total;
-    rc.div_batch = FastDiv::make(total), rc.div_tile_w = FastDiv::make(rc.tile_w);
-    rc.first_sample = 0;
-    const int quad = filter == VRJ_FILTER_F32X4 ? 1 : filter == VRJ_FILTER_Q16 ? 2 : 0;
-    uint64_t launches = 0;
-    s->n_marks = 0;
-    VRJ_CUDA(cudaEventRecord(s->ev0, s->stream));
-    st = p->precision == VRJ_PRECISION_F32_FAST ? run_batch<float, float, false>(scene, s, rc, false, 0, &launches, &mc)
-         : filter == VRJ_FILTER_F64            ? run_batch<double, double, false>(scene, s, rc, false, 0, &launches, &mc)
-                                               : run_batch<float, double, false>(scene, s, rc, false, quad, &launches, &mc);
-    if (st != VRJ_OK) return st;
-    unsigned long long *hstats = reinterpret_cast<unsigned long long *>(s->host_count + 160); // pinned, see vrj_render_tile
-    VRJ_CUDA(cudaMemcpyAsync(hstats, s->stats.p, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-    VRJ_CUDA(cudaEventRecord(s->ev1, s->stream));
-    // every call's arrays cross PCIe behind an event of their own, the leader's (call 0) last: a caller returns as soon as ITS
-    // buffer has arrived, so the host's merge of the first buffer overlaps the copies of the others
-    const double *dev_arr[5] = {mc.out.colour, mc.out.sum, mc.out.bias, mc.out.weight, mc.out.weight_bias};
-    const size_t per[5] = {3, 3, 3, 1, 1};
-    for (uint32_t k = 0; k < n; k++) {
-        const uint32_t c = (k + 1) % n;
-        double *user[5] = {reqs[c]->out->colour, reqs[c]->out->colour_sum, reqs[c]->out->colour_bias, reqs[c]->out->weight, reqs[c]->out->weight_bias};
-        for (int i = 0; i < 5; i++)
-            if (user[i]) VRJ_CUDA(cudaMemcpyAsync(user[i], dev_arr[i] + (size_t)c * npix * per[i], npix * per[i] * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
-        VRJ_CUDA(cudaEventRecord(s->call_ev[c], s->stream));
-    }
-    const auto t2 = std::chrono::steady_clock::now();
-    VRJ_CUDA(wait_event(s->ev1, scene->device));
-    turn.release(); // the next wavefront may start while this one's buffers cross PCIe
-    float ms = 0.f;
-    VRJ_CUDA(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-    double cls_ms[6] = {0, 0, 0, 0, 0, 0};
-    uint64_t cls_n[6] = {0, 0, 0, 0, 0, 0};
-    for (size_t i = 1; i < s->n_marks; i++) {
-        int c = s->mark_class[i];
-        float seg = 0.f;
-        if (c >= 0 && cudaEventElapsedTime(&seg, s->marks[i - 1], s->marks[i]) == cudaSuccess) cls_ms[c] += seg, cls_n[c]++;
-    }
-    for (uint32_t c = 0; c < n; c++) {
-        VrjStats *o = reqs[c]->out->stats;
-        if (!o) continue;
-        unsigned long long share[ST_COUNT];
-        for (int k = 0; k < ST_COUNT; k++) share[k] = hstats[k] / n + (c == 0 ? hstats[k] % n : 0);
-        std::memset(o, 0, sizeof *o);
-        fill_stats(o, share, launches, ms / (float)n); // device time: the call's share of the wavefront
-        o->primary_ms = cls_ms[0] / n, o->bounce_ms = cls_ms[1] / n, o->resolve_ms = cls_ms[2] / n;
-        o->shade_ms = (cls_ms[3] + cls_ms[4]) / n, o->tail_ms = cls_ms[5] / n;
-        o->primary_launches = cls_n[0], o->bounce_launches = cls_n[1], o->resolve_launches = cls_n[2];
-        o->shade_launches = cls_n[3] + cls_n[4], o->tail_launches = cls_n[5];
-        o->coalesced_calls = n;
-    }
-    // the other callers wait for their own buffers from here on
-    {
-        std::lock_guard<std::mutex> lock(co.m);
-        for (uint32_t c = 1; c < n; c++) reqs[c]->wait_ev = s->call_ev[c], reqs[c]->launched = true;
-        *published = true; // from here on those requests belong to their callers again
-    }
-    co.cv.notify_all();
-    VRJ_CUDA(wait_event(s->call_ev[0], scene->device)); // recorded last: everything queued on the stream has finished
-    if (timing) {
-        auto msd = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
-            return std::chrono::duration<double, std::milli>(b - a).count();
-        };
-        std::fprintf(stderr, "vrj_render_tile (coalesced): %u calls, %u samples: scratch %.3f ms, enqueue %.3f ms, wait %.3f ms (device %.3f ms, %llu launches), mallocs %llu / %llu\n", n, total,
-                     msd(t1, t1b), msd(t1b, t2), msd(t2, std::chrono::steady_clock::now()), ms, (unsigned long long)launches,
-                     (unsigned long long)g_n_device_mallocs.load(), (unsigned long long)g_n_host_mallocs.load());
-    }
-    return VRJ_OK;
-}
-
-// entry of a coalescable call: queue up, then either be served by a leader or become one
-VrjStatus render_coalesced(const VrjScene *scene, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p, VrjAccumOut *out) {
-    CoalesceRequest req;
-    req.scene = scene, req.tile = *tile, req.height = height, req.width = width, req.params = *p, req.out = out;
-    Coalescer &co = g_coalescer[(unsigned)scene->device % 64];
-    const uint64_t npix = (tile->end_column - tile->start_column) * (tile->end_row - tile->start_row);
-    std::unique_lock<std::mutex> lock(co.m);
-    co.waiting.push_back(&req);
-    co.cv.wait(lock, [&] { return req.done || req.launched || (!co.collecting && !co.waiting.empty() && co.waiting.front() == &req); });
-    if (req.launched) { // a leader rendered this call with its own and will not touch `req` again: wait for the buffers
-        const cudaEvent_t ev = req.wait_ev;
-        lock.unlock();
-        const cudaError_t e = wait_event(ev, scene->device);
-        if (e != cudaSuccess) return fail(VRJ_ERR_CUDA, std::string("coalesced call: ") + cudaGetErrorString(e));
-        return VRJ_OK;
-    }
-    if (req.done) { // the leader failed before anything was launched
-        vrj_set_error(req.error);
-        return req.status;
-    }
-    co.collecting = true;
-    lock.unlock();
-    RenderTurn turn(scene->device);
-    turn.acquire(); // callers that arrive while this one waits for the device join its wavefront
-    lock.lock();
-    std::vector<CoalesceRequest *> group{&req};
-    uint64_t paths = npix * p->spp;
-    for (size_t i = 0; i < co.waiting.size();) {
-        CoalesceRequest *w = co.waiting[i];
-        if (w == &req) {
-            co.waiting.erase(co.waiting.begin() + i);
-            continue;
-        }
-        if (group.size() < (size_t)MULTI_MAX_CALLS && w->compatible(req) && paths + npix * w->params.spp <= kCoalesceMaxPaths) {
-            paths += npix * w->params.spp;
-            group.push_back(w);
-            co.waiting.erase(co.waiting.begin() + i);
-            continue;
-        }
-        i++;
-    }
-    co.collecting = false;
-    lock.unlock();
-    co.cv.notify_all(); // the next caller in line may start collecting
-    bool published = false; // true once the other callers have been told to wait for their buffers (they may return at any moment)
-    const VrjStatus st = render_group(co, group.data(), (uint32_t)group.size(), turn, &published);
-    turn.release();
-    if (!published) {
-        const std::string err = st != VRJ_OK ? std::string(vrj_last_error()) : std::string("coalesced call: not rendered");
-        lock.lock();
-        for (CoalesceRequest *g : group)
-            if (g != &req) g->status = st != VRJ_OK ? st : VRJ_ERR_CUDA, g->error = err, g->done = true;
-        lock.unlock();
-        co.cv.notify_all();
-    }
-    return st;
-}
 
 // ---------------------------------------------------------------------------------------------- shared by the render calls
 // a call in flight on a device: the path budget is shared between such calls, and wait_event sleeps instead of spinning
@@ -875,19 +643,19 @@ VrjStatus stage_lights(Scratch *s, const VrjRenderParams *p) {
 
 // one batch in the kernel variant the call's precision, walk and counting select
 VrjStatus dispatch_batch(const VrjScene *scene, Scratch *s, const RenderConst &rc, const VrjRenderParams *p, uint32_t filter, uint64_t *launches,
-                         const ResolveCopy *copy, double *ysq) {
+                         const MultiCalls *multi, const ResolveCopy *copy, double *ysq) {
     const bool whitted = p->integrator == VRJ_INTEGRATOR_WHITTED;
     // F32X4: the staged rays walk the 4-wide tree; inline any-hit queries (Whitted shadow rays, k_tail) use the 2-wide f32 tree
     const int quad = filter == VRJ_FILTER_F32X4 ? 1 : filter == VRJ_FILTER_Q16 ? 2 : 0;
     // VRJ_PRECISION_F32_FAST: the whole sample in binary32 over the 2-wide f32 tree (no reference counterpart; not a parity mode)
     const bool fast = p->precision == VRJ_PRECISION_F32_FAST;
     if (p->count_traversal)
-        return fast ? run_batch<float, float, true>(scene, s, rc, whitted, 0, launches, nullptr, copy, ysq)
-             : filter == VRJ_FILTER_F64 ? run_batch<double, double, true>(scene, s, rc, whitted, 0, launches, nullptr, copy, ysq)
-                                        : run_batch<float, double, true>(scene, s, rc, whitted, quad, launches, nullptr, copy, ysq);
-    return fast ? run_batch<float, float, false>(scene, s, rc, whitted, 0, launches, nullptr, copy, ysq)
-         : filter == VRJ_FILTER_F64 ? run_batch<double, double, false>(scene, s, rc, whitted, 0, launches, nullptr, copy, ysq)
-                                    : run_batch<float, double, false>(scene, s, rc, whitted, quad, launches, nullptr, copy, ysq);
+        return fast ? run_batch<float, float, true>(scene, s, rc, whitted, 0, launches, multi, copy, ysq)
+             : filter == VRJ_FILTER_F64 ? run_batch<double, double, true>(scene, s, rc, whitted, 0, launches, multi, copy, ysq)
+                                        : run_batch<float, double, true>(scene, s, rc, whitted, quad, launches, multi, copy, ysq);
+    return fast ? run_batch<float, float, false>(scene, s, rc, whitted, 0, launches, multi, copy, ysq)
+         : filter == VRJ_FILTER_F64 ? run_batch<double, double, false>(scene, s, rc, whitted, 0, launches, multi, copy, ysq)
+                                    : run_batch<float, double, false>(scene, s, rc, whitted, quad, launches, multi, copy, ysq);
 }
 
 // VrjStats of a call from its counters and the boundary events run_levels recorded
@@ -908,7 +676,7 @@ void fill_call_stats(VrjStats *st, const Scratch *s, const unsigned long long *h
     st->coalesced_calls = 1;
 }
 
-// VrjAccumOut.colour from (colour_sum, weight), as k_resolve computes it (vrj_render_sharded, vrj_render_progressive)
+// VrjAccumOut.colour from (colour_sum, weight), as k_resolve computes it (vrj_render_sharded, render_passes)
 __global__ void k_finalize(const double *sum, const double *weight, double *colour, uint32_t npix) {
     uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= npix) return;
@@ -928,16 +696,469 @@ VrjStatus copy_srgb8(Scratch *s, uint64_t npix, uint8_t *dst, cudaMemcpyKind kin
     return VRJ_OK;
 }
 
-// y_sq_sum, two pixel lists and a counter for npix pixels (vrj_render_adaptive, vrj_render_progressive)
-VrjStatus ensure_adaptive_buffers(Scratch *s, uint64_t npix) {
-    if (s->adapt_npix >= npix) return VRJ_OK;
-    s->adapt_npix = 0;
-    std::vector<std::pair<DeviceBuffer *, size_t>> want = {{&s->ysq, npix * 8}, {&s->alist[0], npix * 4}, {&s->alist[1], npix * 4},
-                                                           {&s->aconverged, 8}};
-    const VrjStatus st = alloc_group(s->adapt_slab, want, "adaptive sampling buffers");
-    if (st != VRJ_OK) return st;
-    s->adapt_npix = npix;
+// one of a call's arrays: the caller's (NULL: not wanted), the block's, doubles per pixel
+struct Arr {
+    double *user;
+    DeviceBuffer *dev;
+    size_t per;
+};
+
+// the arrays of a state into the block: from the caller's arrays when `load` (a NULL array starts at zero), else zero
+VrjStatus load_state(Scratch *s, const Arr *arrs, int n, bool load, cudaMemcpyKind kind, uint64_t npix) {
+    for (int i = 0; i < n; i++) {
+        if (load && arrs[i].user) VRJ_CUDA(cudaMemcpyAsync(arrs[i].dev->p, arrs[i].user, npix * arrs[i].per * sizeof(double), kind, s->stream));
+        else VRJ_CUDA(cudaMemsetAsync(arrs[i].dev->p, 0, npix * arrs[i].per * sizeof(double), s->stream));
+    }
     return VRJ_OK;
+}
+
+// What every render call (vrj_render_tile, render_passes) does around its kernels.  prepare(): a block from the pool for
+// batches of up to `widest` samples of the tile; start(): the call's counters, lights and constants, the render turn and
+// ev0; finish(): ev1, the counters, the copies of the outputs and the sRGB preview, the waits, VrjStats.  `turn` is declared
+// after `block`: an early return gives the turn back before the block.
+struct RenderCall {
+    VrjScene *scene;
+    const VrjRenderParams *p;
+    uint64_t npix;
+    BlockLease block;
+    RenderTurn turn;
+    Scratch *s = nullptr;
+    uint32_t filter = 0, batch = 0;
+    RenderConst rc{};
+    uint64_t launches = 0;
+    bool pieces_copied = false; // the arrays went out with the last resolve's pieces (ResolveCopy): wait for those copies
+    float ms = 0.f;             // device time, ev0 .. ev1
+    std::chrono::steady_clock::time_point t_start, t_enqueued, t_done; // turn taken, last copy enqueued, copies arrived
+    RenderCall(VrjScene *sc, const VrjRenderParams *params, uint64_t n) : scene(sc), p(params), npix(n), block{sc}, turn(sc->device) {}
+
+    VrjStatus prepare(uint32_t widest, const ActiveCall &active, size_t n_light_samples) {
+        batch = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(widest, call_path_budget(scene, active) / npix));
+        if (npix * (uint64_t)batch > 0xfffffff0ull) return fail(VRJ_ERR_UNSUPPORTED, "tile too large");
+        s = block.s = acquire_scratch(scene, npix * batch);
+        filter = effective_filter(scene, p);
+        return ensure_call_scratch(s, p, call_wants_records(scene, p, filter), npix, &batch, n_light_samples);
+    }
+    VrjStatus start(const VrjTile *tile, uint64_t height, uint64_t width) {
+        VRJ_CUDA(cudaMemsetAsync(s->stats.p, 0, ST_COUNT * sizeof(unsigned long long), s->stream));
+        const VrjStatus st = stage_lights(s, p);
+        if (st != VRJ_OK) return st;
+        rc = make_render_const(tile, height, width, p);
+        rc.lights = s->lights.as<LightDev>();
+        rc.light_samples = s->light_samples.as<double>();
+        rc.div_tile_w = FastDiv::make(rc.tile_w);
+        s->n_marks = 0;
+        turn.acquire();
+        t_start = std::chrono::steady_clock::now();
+        VRJ_CUDA(cudaEventRecord(s->ev0, s->stream));
+        return VRJ_OK;
+    }
+    VrjStatus finish(const Arr *arrs, int n, uint8_t *srgb8, cudaMemcpyKind kind, VrjStats *stats) {
+        VRJ_CUDA(cudaEventRecord(s->ev1, s->stream)); // before the counters' copy: that one queues up behind the pieces' copies on the copy engine
+        VRJ_CUDA(cudaMemcpyAsync(s->pinned->stats, s->stats.p, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+        if (pieces_copied) {
+            VRJ_CUDA(cudaStreamWaitEvent(s->stream, s->copy_done, 0)); // ev_done below then stands behind the pieces' copies too
+        } else {
+            for (int i = 0; i < n; i++)
+                if (arrs[i].user) VRJ_CUDA(cudaMemcpyAsync(arrs[i].user, arrs[i].dev->p, npix * arrs[i].per * sizeof(double), kind, s->stream));
+        }
+        if (srgb8) {
+            const VrjStatus st = copy_srgb8(s, npix, srgb8, kind, &launches);
+            if (st != VRJ_OK) return st;
+        }
+        t_enqueued = std::chrono::steady_clock::now();
+        VRJ_CUDA(cudaEventRecord(s->ev_done, s->stream));
+        VRJ_CUDA(wait_event(s->ev1, scene->device)); // the last kernel is done: the next caller may render while this one's copies run
+        turn.release();
+        VRJ_CUDA(wait_event(s->ev_done, scene->device));
+        t_done = std::chrono::steady_clock::now();
+        VRJ_CUDA(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+        if (stats) fill_call_stats(stats, s, s->pinned->stats, launches, ms);
+        return VRJ_OK;
+    }
+};
+
+// y_sq_sum, two pixel lists, the first samples of one and the selects' counters for npix pixels (render_passes)
+VrjStatus ensure_pass_buffers(Scratch *s, uint64_t npix) {
+    if (s->pass_npix >= npix) return VRJ_OK;
+    s->pass_npix = 0;
+    std::vector<std::pair<DeviceBuffer *, size_t>> want = {{&s->ysq, npix * 8}, {&s->pass_list[0], npix * 4}, {&s->pass_list[1], npix * 4},
+                                                           {&s->pass_base, npix * 4}, {&s->pass_counters, sizeof(ProgressiveCounters)}};
+    const VrjStatus st = alloc_group(s->pass_slab, want, "adaptive sampling buffers");
+    if (st != VRJ_OK) return st;
+    s->pass_npix = npix;
+    return VRJ_OK;
+}
+
+// the fields VrjAdaptiveParams and VrjProgressiveParams share, and params->spp, which must be 0
+template <typename P>
+VrjStatus check_pass_rule(const VrjRenderParams *p, const P *ap, const char *call, const char *type, PassRule *rule) {
+    if (!ap) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (p->spp != 0) return fail(VRJ_ERR_INVALID_ARGUMENT, std::string("params->spp must be 0: ") + call + " takes its sample counts from " + type);
+    if (ap->min_samples < 2) return fail(VRJ_ERR_INVALID_ARGUMENT, "min_samples must be >= 2 (the variance needs two samples)");
+    if (ap->max_samples < ap->min_samples) return fail(VRJ_ERR_INVALID_ARGUMENT, "max_samples must be >= min_samples");
+    if (ap->pass_samples < 1) return fail(VRJ_ERR_INVALID_ARGUMENT, "pass_samples must be >= 1");
+    if (!(ap->rel_error > 0.0) || !std::isfinite(ap->rel_error)) return fail(VRJ_ERR_INVALID_ARGUMENT, "rel_error must be > 0 and finite");
+    if (!(ap->abs_floor >= 0.0) || !std::isfinite(ap->abs_floor)) return fail(VRJ_ERR_INVALID_ARGUMENT, "abs_floor must be >= 0 and finite");
+    *rule = PassRule{ap->min_samples, ap->max_samples, ap->pass_samples, 0u, ap->rel_error, ap->abs_floor};
+    return VRJ_OK;
+}
+
+struct PassResult {
+    uint64_t passes = 0, samples = 0;
+    ProgressiveCounters counts{}; // converged and at_max over the call, active at return
+};
+
+// The passes of vrj_render_adaptive and vrj_render_progressive (the header states the schedule) on a tile of npix >= 1
+// pixels.  The state starts at zero, or (out->accumulate) comes from out's four state arrays and y_sq_sum; every output array
+// may be NULL.  A pass renders its pixels' samples in batches split to the path budget like vrj_render_tile's, and
+// k_resolve_adaptive applies them to the tile's accumulators and y_sq_sum.
+//  - A fresh state's pass 0 is known on the host (every pixel takes samples 0 .. min_samples-1): it runs over the tile on
+//    the tile's kernels, with no select before it.  A continued state is first judged over the whole tile, which is also
+//    where weights that are no sample counts are found.
+//  - Before every further pass k_progressive_select judges the pixels the previous pass rendered (an inactive pixel stays
+//    inactive) and the host reads back its counters.  When every active pixel takes the same count -- always, for a state
+//    this schedule produced with unchanged parameters -- an exclusive scan (vrj_build::exclusive_scan_u32) of its flags and
+//    k_progressive_compact list the active pixels in tile order with their first new sample, and the LIST kernels render
+//    them.  Otherwise k_progressive_group lists the pixels of each count, largest first, in a segment of the list of its own,
+//    and each segment is rendered as a sub-pass once all are listed.
+//  - colour: a fresh state's pixels were all resolved, which writes it; a continued state's comes from k_finalize.
+VrjStatus render_passes(VrjScene *scene, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p, const PassRule &rule,
+                        uint32_t max_passes, size_t n_light_samples, VrjAccumOut *out, double *y_sq_sum, PassResult *res) {
+    const uint64_t npix = (tile->end_column - tile->start_column) * (tile->end_row - tile->start_row);
+    const bool fresh = !out->accumulate;
+    ActiveCall active(g_active_calls[(unsigned)scene->device % 64]);
+    RenderCall call(scene, p, npix);
+    // the widest pass is the whole tile at max(min, pass) samples (a fresh state's first pass, or a state that every pixel
+    // has to continue); the block is sized for it
+    VrjStatus st = call.prepare(std::min(rule.max_samples, std::max(rule.min_samples, rule.pass_samples)), active, n_light_samples);
+    if (st != VRJ_OK) return st;
+    Scratch *s = call.s;
+    st = ensure_pass_buffers(s, npix);
+    if (st != VRJ_OK) return st;
+    const cudaMemcpyKind in_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    const cudaMemcpyKind out_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    const Arr arrs[6] = {{out->colour, &s->acc_colour, 3}, {out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3},
+                         {out->weight, &s->acc_weight, 1}, {out->weight_bias, &s->acc_wbias, 1}, {y_sq_sum, &s->ysq, 1}};
+    st = load_state(s, arrs + 1, 5, !fresh, in_kind, npix);
+    if (st != VRJ_OK) return st;
+    ProgressiveCounters *ctr = s->pass_counters.as<ProgressiveCounters>(), *hctr = &s->pinned->pass;
+    VRJ_CUDA(cudaMemsetAsync(ctr, 0, sizeof(ProgressiveCounters), s->stream));
+    st = call.start(tile, height, width);
+    if (st != VRJ_OK) return st;
+
+    RenderConst &rc = call.rc;
+    const size_t capacity = npix * call.batch; // paths per batch
+    const double *sum = s->acc_sum.as<double>(), *weight = s->acc_weight.as<double>(), *ysq = s->ysq.as<double>();
+    // the flags and the scan's tile totals live in the photon buffer, which is free between a pass's resolve and the next
+    // batch: (n + 1) + (n / 2048 + 2) uint32 fit the 16 bytes per path of a block that holds at least one path per pixel
+    uint32_t *flags = s->photons.as<uint32_t>(), *base = s->pass_base.as<uint32_t>();
+    // samples base[i] .. base[i] + c - 1 of the m pixels of `list` (the tile's samples 0 .. c - 1 when `list` is NULL)
+    auto render = [&](const uint32_t *list, const uint32_t *first, uint32_t m, uint32_t c) -> VrjStatus {
+        const uint32_t b = (uint32_t)std::max<size_t>(1, std::min<size_t>(c, capacity / m));
+        rc.npix = m, rc.pixel_list = list, rc.pixel_base = first;
+        for (uint32_t done = 0; done < c; done += b) {
+            rc.batch_samples = std::min(b, c - done);
+            rc.div_batch = FastDiv::make(rc.batch_samples);
+            rc.first_sample = p->sample_offset + (uint64_t)done * rc.sample_stride;
+            const VrjStatus bst = dispatch_batch(scene, s, rc, p, call.filter, &call.launches, nullptr, nullptr, s->ysq.as<double>());
+            if (bst != VRJ_OK) return bst;
+        }
+        res->samples += (uint64_t)m * c;
+        return VRJ_OK;
+    };
+    auto compact = [&](const uint32_t *list, uint32_t n, uint32_t *to, uint32_t *first) -> VrjStatus {
+        const VrjStatus sst = vrj_build::exclusive_scan_u32(flags, n + 1, flags + n + 1, s->stream);
+        if (sst != VRJ_OK) return sst;
+        k_progressive_compact<<<(n + 255) / 256, 256, 0, s->stream>>>(list, weight, flags, n, to, first);
+        call.launches += 4;
+        VRJ_CUDA(cudaGetLastError());
+        return VRJ_OK;
+    };
+    if (fresh) {
+        st = render(nullptr, nullptr, (uint32_t)npix, rule.min_samples);
+        if (st != VRJ_OK) return st;
+        res->passes = 1;
+    }
+    const uint32_t *list = nullptr; // the pixels the last select judges (NULL: the tile)
+    uint32_t n = (uint32_t)npix, next = 0, held = rule.min_samples; // held: what every pixel of a fresh state's list holds
+    for (;;) {
+        VRJ_CUDA(cudaMemsetAsync(ctr, 0, offsetof(ProgressiveCounters, converged), s->stream)); // active, cmax, cmin_not
+        k_progressive_select<<<(n + 1 + 255) / 256, 256, 0, s->stream>>>(sum, weight, ysq, list, n, rule, flags, ctr);
+        call.launches++;
+        VRJ_CUDA(cudaGetLastError());
+        VRJ_CUDA(cudaMemcpyAsync(hctr, ctr, sizeof(ProgressiveCounters), cudaMemcpyDeviceToHost, s->stream));
+        // the last select only counts, and nothing waits for it (its counters arrive with the outputs): the pass limit is
+        // reached, or a fresh state's pixels all hold max_samples (no weight can be invalid in either case)
+        if ((max_passes && res->passes == max_passes) || (fresh && held >= rule.max_samples)) break;
+        VRJ_CUDA(cudaStreamSynchronize(s->stream));
+        if (hctr->bad) return fail(VRJ_ERR_INVALID_ARGUMENT, "a weight of the state is not a sample count (negative, fractional, not finite or >= 2^32)");
+        if (hctr->active == 0) break;
+        const uint32_t m = (uint32_t)hctr->active, cmax = hctr->cmax;
+        held += cmax;
+        uint32_t *to = s->pass_list[next].as<uint32_t>();
+        if (cmax == ~hctr->cmin_not) {
+            st = compact(list, n, to, base);
+            if (st == VRJ_OK) st = render(to, base, m, cmax);
+            if (st != VRJ_OK) return st;
+        } else {
+            // every segment is listed before any is rendered: rendering changes the state the counts are computed from
+            std::vector<std::pair<uint32_t, uint32_t>> segments; // (count, length)
+            uint32_t listed = 0;
+            for (uint32_t c = cmax; c != 0;) {
+                VRJ_CUDA(cudaMemsetAsync(&ctr->next, 0, sizeof(uint32_t), s->stream));
+                k_progressive_group<<<(n + 1 + 255) / 256, 256, 0, s->stream>>>(sum, weight, ysq, list, n, rule, c, flags, ctr);
+                call.launches++;
+                st = compact(list, n, to + listed, base + listed);
+                if (st != VRJ_OK) return st;
+                VRJ_CUDA(cudaMemcpyAsync(&s->pinned->listed, flags + n, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
+                VRJ_CUDA(cudaMemcpyAsync(&hctr->next, &ctr->next, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
+                VRJ_CUDA(cudaStreamSynchronize(s->stream));
+                if (s->pinned->listed) segments.push_back({c, s->pinned->listed}), listed += s->pinned->listed;
+                c = hctr->next;
+            }
+            listed = 0;
+            for (const auto &seg : segments) {
+                st = render(to + listed, base + listed, seg.second, seg.first);
+                if (st != VRJ_OK) return st;
+                listed += seg.second;
+            }
+        }
+        list = to, n = m, next ^= 1u;
+        res->passes++;
+    }
+    if (!fresh && (out->colour || out->srgb8)) {
+        k_finalize<<<(unsigned)((npix + 255) / 256), 256, 0, s->stream>>>(sum, weight, s->acc_colour.as<double>(), (uint32_t)npix);
+        call.launches++;
+        VRJ_CUDA(cudaGetLastError());
+    }
+    st = call.finish(arrs, 6, out->srgb8, out_kind, out->stats);
+    if (st != VRJ_OK) return st;
+    res->counts = *hctr;
+    return VRJ_OK;
+}
+
+// ---------------------------------------------------------------------------------------------- coalesced calls
+// main.rs:197-209 calls partial_render_scene once per one-sample pass from a pool of workers.  Each such call is a small
+// wavefront (2 M paths at 1080p) whose ~28 launches do not fill 148 SMs: 1.7 ms of device time against 0.52 ms per sample
+// when 64 samples share a wavefront.  Calls that arrive while the device is busy and differ only in their sample indices and
+// output buffers are therefore rendered TOGETHER: one of the waiting callers (the leader) takes its turn at the render gate,
+// collects every compatible caller that has queued up behind it, runs one wavefront over all their samples (the batch's slots
+// carry their sample indices in a table, RenderConst::sample_table), resolves each call's samples into that call's own
+// fresh buffer (k_resolve_multi) and copies every buffer back.  A sample is a pure function of (seed, pixel, sample index)
+// and each call's samples are applied to its buffer in sample order, so every caller receives bit for bit what it would have
+// received alone (tests/test_gpu_parity.py::test_coalesced_calls_bit_identical).  The ray counters of a shared wavefront are
+// split evenly over its calls (the remainder goes to the first; sums stay exact) and VrjStats.coalesced_calls says how many
+// shared it.  VRJ_COALESCE=0 turns this off (experiments).
+struct CoalesceRequest {
+    const VrjScene *scene;
+    VrjTile tile;
+    uint64_t height, width;
+    VrjRenderParams params;
+    VrjAccumOut *out;
+    VrjStatus status = VRJ_OK;
+    std::string error;
+    bool done = false;     // a leader failed before launching anything: `status` / `error` say why
+    bool launched = false; // rendered by a leader: stats are filled, the buffers are on their way, `wait_ev` fires on arrival
+    cudaEvent_t wait_ev = nullptr;
+    uint32_t wanted() const {
+        return (out->colour ? 1u : 0u) | (out->colour_sum ? 2u : 0u) | (out->colour_bias ? 4u : 0u) | (out->weight ? 8u : 0u) | (out->weight_bias ? 16u : 0u);
+    }
+    bool compatible(const CoalesceRequest &o) const {
+        return scene == o.scene && tile.start_column == o.tile.start_column && tile.end_column == o.tile.end_column &&
+               tile.start_row == o.tile.start_row && tile.end_row == o.tile.end_row && height == o.height && width == o.width &&
+               params.max_depth == o.params.max_depth && params.seed == o.params.seed && params.bvh_filter == o.params.bvh_filter &&
+               params.precision == o.params.precision && params.bias == o.params.bias &&
+               (params.sample_stride ? params.sample_stride : 1u) == (o.params.sample_stride ? o.params.sample_stride : 1u) && wanted() == o.wanted();
+    }
+};
+struct Coalescer {
+    std::mutex m;
+    std::condition_variable cv;
+    std::vector<CoalesceRequest *> waiting;
+    bool collecting = false; // a leader is waiting for its turn at the gate; arrivals pile up behind it
+};
+Coalescer g_coalescer[64];
+constexpr uint64_t kCoalesceMaxPaths = uint64_t(1) << 25; // 32 Mi paths = 11 GB of queue state per shared wavefront
+
+bool coalescing_enabled() {
+    static const bool on = [] {
+        const char *e = std::getenv("VRJ_COALESCE");
+        return !e || std::atoi(e) != 0;
+    }();
+    return on;
+}
+static_assert(sizeof(PinnedBlock::sample_table) == 4 * MULTI_MAX_CALLS * sizeof(uint64_t),
+              "the sample table of a coalesced wavefront holds MULTI_MAX_CALLS calls of up to 4 samples (coalescable)");
+bool coalescable(const VrjRenderParams *p, const VrjAccumOut *out, uint64_t npix) {
+    return coalescing_enabled() && out->memory == VRJ_MEM_HOST && !out->accumulate && !out->photons && !out->srgb8 && out->colour &&
+           p->integrator == VRJ_INTEGRATOR_SIMPLE_RANDOM && p->n_lights == 0 && !p->ambient_light && !p->count_traversal &&
+           p->spp >= 1 && p->spp <= 4 && npix * p->spp * 2 <= kCoalesceMaxPaths;
+}
+
+// one wavefront for `n` compatible requests; fills their buffers and stats; the status applies to all of them
+VrjStatus render_group(Coalescer &co, CoalesceRequest *const *reqs, uint32_t n, RenderTurn &turn, bool *published) {
+    static const bool timing = std::getenv("VRJ_TIMING") != nullptr;
+    const auto t1 = std::chrono::steady_clock::now();
+    const CoalesceRequest &r0 = *reqs[0];
+    VrjScene *scene = const_cast<VrjScene *>(r0.scene);
+    const VrjRenderParams *p = &r0.params;
+    RenderConst rc = make_render_const(&r0.tile, r0.height, r0.width, p);
+    const uint64_t npix = rc.npix;
+    uint32_t total = 0;
+    MultiCalls mc{};
+    mc.n = n, mc.full = (r0.wanted() & ~1u) ? 1u : 0u;
+    std::vector<uint64_t> table;
+    for (uint32_t c = 0; c < n; c++) {
+        mc.first[c] = total, mc.count[c] = reqs[c]->params.spp;
+        for (uint32_t i = 0; i < reqs[c]->params.spp; i++) table.push_back(reqs[c]->params.sample_offset + (uint64_t)i * rc.sample_stride);
+        total += reqs[c]->params.spp;
+    }
+    VRJ_NVTX_RANGE(call_range, "vrj_render_tile (coalesced)");
+    // group sizes vary from wavefront to wavefront: blocks are sized in steps of eight 1-sample calls so that a block taken
+    // from the pool almost never has to grow (growing re-allocates every queue: tens of milliseconds)
+    const size_t capacity = npix * (size_t)((total + 7u) / 8u * 8u);
+    const BlockLease lease{scene, acquire_scratch(scene, capacity)};
+    Scratch *s = lease.s;
+    const uint32_t filter = effective_filter(scene, p);
+    const bool records = call_wants_records(scene, p, filter);
+    VrjStatus st = ensure_scratch(s, capacity, records ? capacity : 0, 0, p->max_depth + 3, 0, 0);
+    if (st == VRJ_ERR_OUT_OF_MEMORY) { // fall back to exactly what this wavefront needs
+        vrj_pool_trim();
+        st = ensure_scratch(s, npix * total, records ? npix * total : 0, 0, p->max_depth + 3, 0, 0);
+    }
+    if (st != VRJ_OK) return st;
+    const auto t1b = std::chrono::steady_clock::now();
+    const size_t per_call = npix * (mc.full ? 11 : 3) * sizeof(double);
+    if (s->multi_out.bytes < per_call * n || !s->multi_out.p) {
+        // sized once for the largest group this tile size can form (1-sample calls up to the path limit)
+        const size_t max_calls = std::max<size_t>(n, std::min<size_t>(MULTI_MAX_CALLS, kCoalesceMaxPaths / std::max<uint64_t>(npix, 1)));
+        s->multi_out.release();
+        VRJ_CUDA(s->multi_out.alloc(per_call * max_calls));
+    }
+    if (!s->sample_table.p) VRJ_CUDA(s->sample_table.alloc(sizeof(PinnedBlock::sample_table)));
+    double *base = s->multi_out.as<double>();
+    mc.out.colour = base;
+    if (mc.full) {
+        mc.out.sum = base + 3 * npix * n, mc.out.bias = base + 6 * npix * n;
+        mc.out.weight = base + 9 * npix * n, mc.out.weight_bias = base + 10 * npix * n;
+    }
+    std::memcpy(s->pinned->sample_table, table.data(), table.size() * sizeof(uint64_t));
+    VRJ_CUDA(cudaMemcpyAsync(s->sample_table.p, s->pinned->sample_table, table.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s->stream));
+    VRJ_CUDA(cudaMemsetAsync(s->stats.p, 0, ST_COUNT * sizeof(unsigned long long), s->stream));
+    rc.sample_table = s->sample_table.as<uint64_t>();
+    rc.lights = s->lights.as<LightDev>(), rc.light_samples = s->light_samples.as<double>();
+    rc.batch_samples = total;
+    rc.div_batch = FastDiv::make(total), rc.div_tile_w = FastDiv::make(rc.tile_w);
+    rc.first_sample = 0;
+    uint64_t launches = 0;
+    s->n_marks = 0;
+    VRJ_CUDA(cudaEventRecord(s->ev0, s->stream));
+    st = dispatch_batch(scene, s, rc, p, filter, &launches, &mc, nullptr, nullptr);
+    if (st != VRJ_OK) return st;
+    unsigned long long *hstats = s->pinned->stats;
+    VRJ_CUDA(cudaMemcpyAsync(hstats, s->stats.p, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+    VRJ_CUDA(cudaEventRecord(s->ev1, s->stream));
+    // every call's arrays cross PCIe behind an event of their own, the leader's (call 0) last: a caller returns as soon as ITS
+    // buffer has arrived, so the host's merge of the first buffer overlaps the copies of the others
+    const double *dev_arr[5] = {mc.out.colour, mc.out.sum, mc.out.bias, mc.out.weight, mc.out.weight_bias};
+    const size_t per[5] = {3, 3, 3, 1, 1};
+    for (uint32_t k = 0; k < n; k++) {
+        const uint32_t c = (k + 1) % n;
+        double *user[5] = {reqs[c]->out->colour, reqs[c]->out->colour_sum, reqs[c]->out->colour_bias, reqs[c]->out->weight, reqs[c]->out->weight_bias};
+        for (int i = 0; i < 5; i++)
+            if (user[i]) VRJ_CUDA(cudaMemcpyAsync(user[i], dev_arr[i] + (size_t)c * npix * per[i], npix * per[i] * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+        VRJ_CUDA(cudaEventRecord(s->call_ev[c], s->stream));
+    }
+    const auto t2 = std::chrono::steady_clock::now();
+    VRJ_CUDA(wait_event(s->ev1, scene->device));
+    turn.release(); // the next wavefront may start while this one's buffers cross PCIe
+    float ms = 0.f;
+    VRJ_CUDA(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+    for (uint32_t c = 0; c < n; c++) {
+        VrjStats *o = reqs[c]->out->stats;
+        if (!o) continue;
+        unsigned long long share[ST_COUNT];
+        for (int k = 0; k < ST_COUNT; k++) share[k] = hstats[k] / n + (c == 0 ? hstats[k] % n : 0);
+        std::memset(o, 0, sizeof *o);
+        fill_call_stats(o, s, share, launches, ms / (float)n); // device time: the call's share of the wavefront
+        o->primary_ms /= n, o->bounce_ms /= n, o->resolve_ms /= n, o->shade_ms /= n, o->tail_ms /= n;
+        o->coalesced_calls = n;
+    }
+    // the other callers wait for their own buffers from here on
+    {
+        std::lock_guard<std::mutex> lock(co.m);
+        for (uint32_t c = 1; c < n; c++) reqs[c]->wait_ev = s->call_ev[c], reqs[c]->launched = true;
+        *published = true; // from here on those requests belong to their callers again
+    }
+    co.cv.notify_all();
+    VRJ_CUDA(wait_event(s->call_ev[0], scene->device)); // recorded last: everything queued on the stream has finished
+    if (timing) {
+        auto msd = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
+            return std::chrono::duration<double, std::milli>(b - a).count();
+        };
+        std::fprintf(stderr, "vrj_render_tile (coalesced): %u calls, %u samples: scratch %.3f ms, enqueue %.3f ms, wait %.3f ms (device %.3f ms, %llu launches), mallocs %llu / %llu\n", n, total,
+                     msd(t1, t1b), msd(t1b, t2), msd(t2, std::chrono::steady_clock::now()), ms, (unsigned long long)launches,
+                     (unsigned long long)g_n_device_mallocs.load(), (unsigned long long)g_n_host_mallocs.load());
+    }
+    return VRJ_OK;
+}
+
+// entry of a coalescable call: queue up, then either be served by a leader or become one
+VrjStatus render_coalesced(const VrjScene *scene, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p, VrjAccumOut *out) {
+    CoalesceRequest req;
+    req.scene = scene, req.tile = *tile, req.height = height, req.width = width, req.params = *p, req.out = out;
+    Coalescer &co = g_coalescer[(unsigned)scene->device % 64];
+    const uint64_t npix = (tile->end_column - tile->start_column) * (tile->end_row - tile->start_row);
+    std::unique_lock<std::mutex> lock(co.m);
+    co.waiting.push_back(&req);
+    co.cv.wait(lock, [&] { return req.done || req.launched || (!co.collecting && !co.waiting.empty() && co.waiting.front() == &req); });
+    if (req.launched) { // a leader rendered this call with its own and will not touch `req` again: wait for the buffers
+        const cudaEvent_t ev = req.wait_ev;
+        lock.unlock();
+        const cudaError_t e = wait_event(ev, scene->device);
+        if (e != cudaSuccess) return fail(VRJ_ERR_CUDA, std::string("coalesced call: ") + cudaGetErrorString(e));
+        return VRJ_OK;
+    }
+    if (req.done) { // the leader failed before anything was launched
+        vrj_set_error(req.error);
+        return req.status;
+    }
+    co.collecting = true;
+    lock.unlock();
+    RenderTurn turn(scene->device);
+    turn.acquire(); // callers that arrive while this one waits for the device join its wavefront
+    lock.lock();
+    std::vector<CoalesceRequest *> group{&req};
+    uint64_t paths = npix * p->spp;
+    for (size_t i = 0; i < co.waiting.size();) {
+        CoalesceRequest *w = co.waiting[i];
+        if (w == &req) {
+            co.waiting.erase(co.waiting.begin() + i);
+            continue;
+        }
+        if (group.size() < (size_t)MULTI_MAX_CALLS && w->compatible(req) && paths + npix * w->params.spp <= kCoalesceMaxPaths) {
+            paths += npix * w->params.spp;
+            group.push_back(w);
+            co.waiting.erase(co.waiting.begin() + i);
+            continue;
+        }
+        i++;
+    }
+    co.collecting = false;
+    lock.unlock();
+    co.cv.notify_all(); // the next caller in line may start collecting
+    bool published = false; // true once the other callers have been told to wait for their buffers (they may return at any moment)
+    const VrjStatus st = render_group(co, group.data(), (uint32_t)group.size(), turn, &published);
+    turn.release();
+    if (!published) {
+        const std::string err = st != VRJ_OK ? std::string(vrj_last_error()) : std::string("coalesced call: not rendered");
+        lock.lock();
+        for (CoalesceRequest *g : group)
+            if (g != &req) g->status = st != VRJ_OK ? st : VRJ_ERR_CUDA, g->error = err, g->done = true;
+        lock.unlock();
+        co.cv.notify_all();
+    }
+    return st;
 }
 
 } // namespace
@@ -1410,52 +1631,21 @@ VrjStatus vrj_render_tile(const VrjScene *scene_c, const VrjTile *tile, uint64_t
     // batch: as many samples of the whole tile in flight as fit the path budget
     ActiveCall active(g_active_calls[(unsigned)scene->device % 64]);
     if (coalescable(p, out, npix)) return render_coalesced(scene, tile, height, width, p, out);
-    uint32_t batch = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(p->spp, call_path_budget(scene, active) / npix));
-    if (npix * (uint64_t)batch > 0xfffffff0ull) return fail(VRJ_ERR_UNSUPPORTED, "tile too large");
-    Scratch *s = acquire_scratch(scene, npix * batch);
-    struct Releaser {
-        VrjScene *sc;
-        Scratch *s;
-        // whatever path leaves this function (an error in the middle of the batch loop included), nothing may still be
-        // running on the block's stream when another caller is handed the block
-        ~Releaser() {
-            if (s->stream) cudaStreamSynchronize(s->stream);
-            if (s->copy_stream) cudaStreamSynchronize(s->copy_stream);
-            release_scratch(sc, s);
-        }
-    } releaser{scene, s};
-    const uint32_t filter = effective_filter(scene, p);
-    st = ensure_call_scratch(s, p, call_wants_records(scene, p, filter), npix, &batch, n_light_samples);
+    RenderCall call(scene, p, npix);
+    st = call.prepare(p->spp, active, n_light_samples);
     if (st != VRJ_OK) return st;
+    Scratch *s = call.s;
+    const uint32_t batch = call.batch;
 
     const cudaMemcpyKind in_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
     const cudaMemcpyKind out_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-    struct Arr {
-        double *user;
-        DeviceBuffer *dev;
-        size_t per;
-    } arrs[5] = {{out->colour, &s->acc_colour, 3}, {out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3},
-                 {out->weight, &s->acc_weight, 1}, {out->weight_bias, &s->acc_wbias, 1}};
-    for (int i = 1; i < 5; i++) {
-        if (out->accumulate && arrs[i].user)
-            VRJ_CUDA(cudaMemcpyAsync(arrs[i].dev->p, arrs[i].user, npix * arrs[i].per * sizeof(double), in_kind, s->stream));
-        else
-            VRJ_CUDA(cudaMemsetAsync(arrs[i].dev->p, 0, npix * arrs[i].per * sizeof(double), s->stream));
-    }
-    VRJ_CUDA(cudaMemsetAsync(s->stats.p, 0, ST_COUNT * sizeof(unsigned long long), s->stream));
-    st = stage_lights(s, p);
+    const Arr arrs[5] = {{out->colour, &s->acc_colour, 3}, {out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3},
+                         {out->weight, &s->acc_weight, 1}, {out->weight_bias, &s->acc_wbias, 1}};
+    st = load_state(s, arrs + 1, 4, out->accumulate, in_kind, npix);
     if (st != VRJ_OK) return st;
-
-    RenderConst rc = make_render_const(tile, height, width, p);
-    rc.lights = s->lights.as<LightDev>();
-    rc.light_samples = s->light_samples.as<double>();
-
-    uint64_t launches = 0;
-    s->n_marks = 0;
-    RenderTurn turn(scene->device); // declared after `releaser`: an early return gives the turn back before the block
-    turn.acquire();
-    const auto t_call1 = std::chrono::steady_clock::now();
-    VRJ_CUDA(cudaEventRecord(s->ev0, s->stream));
+    st = call.start(tile, height, width);
+    if (st != VRJ_OK) return st;
+    RenderConst &rc = call.rc;
     // the last batch's resolve runs in pieces whose parts of the arrays start for the host at once (ResolveCopy); small tiles
     // and device-memory outputs (copies at HBM speed) keep the single resolve
     ResolveCopy rcopy{{arrs[0].user, arrs[1].user, arrs[2].user, arrs[3].user, arrs[4].user}, out_kind, 4u};
@@ -1466,14 +1656,13 @@ VrjStatus vrj_render_tile(const VrjScene *scene_c, const VrjTile *tile, uint64_t
         if (arrs[i].user && (cudaPointerGetAttributes(&attr, arrs[i].user) != cudaSuccess || attr.type != cudaMemoryTypeHost)) piecewise = false;
     }
     cudaGetLastError();
-    bool copied = false;
     for (uint32_t done = 0; done < p->spp; done += batch) {
         rc.batch_samples = std::min(batch, p->spp - done);
         const ResolveCopy *copy = piecewise && done + batch >= p->spp ? &rcopy : nullptr;
-        copied = copied || copy != nullptr;
-        rc.div_batch = FastDiv::make(rc.batch_samples), rc.div_tile_w = FastDiv::make(rc.tile_w);
+        call.pieces_copied = call.pieces_copied || copy != nullptr;
+        rc.div_batch = FastDiv::make(rc.batch_samples);
         rc.first_sample = p->sample_offset + (uint64_t)done * rc.sample_stride;
-        st = dispatch_batch(scene, s, rc, p, filter, &launches, copy, nullptr);
+        st = dispatch_batch(scene, s, rc, p, call.filter, &call.launches, nullptr, copy, nullptr);
         if (st != VRJ_OK) return st;
         if (out->photons) {
             // debug output, batch-major: [(sample * npix + pixel) * 2]; the device keeps the batch pixel-major, so transpose
@@ -1481,64 +1670,34 @@ VrjStatus vrj_render_tile(const VrjScene *scene_c, const VrjTile *tile, uint64_t
             double2 *tmp = s->queues[0][0].as<double2>();
             const size_t count = (size_t)rc.batch_samples * npix;
             k_photons_sample_major<<<(unsigned)((count + 255) / 256), 256, 0, s->stream>>>(s->photons.as<double2>(), tmp, (uint32_t)npix, rc.batch_samples);
-            launches++;
+            call.launches++;
             VRJ_CUDA(cudaMemcpyAsync(out->photons + (size_t)done * npix * 2, tmp, count * sizeof(double2), out_kind, s->stream));
         }
     }
-    // the counters go through the block's pinned slot: a copy into pageable memory would hold this thread until everything
-    // queued before it -- the copies of the result included -- had finished, and the gate could not open early
-    unsigned long long *hstats = reinterpret_cast<unsigned long long *>(s->host_count + 160);
-    VRJ_CUDA(cudaEventRecord(s->ev1, s->stream)); // before the counters' copy: that one queues up behind the pieces' copies on the copy engine
-    VRJ_CUDA(cudaMemcpyAsync(hstats, s->stats.p, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-    if (copied) {
-        VRJ_CUDA(cudaStreamWaitEvent(s->stream, s->copy_done, 0)); // ev_done below then stands behind the pieces' copies too
-    } else {
-        for (int i = 0; i < 5; i++)
-            if (arrs[i].user)
-                VRJ_CUDA(cudaMemcpyAsync(arrs[i].user, arrs[i].dev->p, npix * arrs[i].per * sizeof(double), out_kind, s->stream));
-    }
-    if (out->srgb8) {
-        st = copy_srgb8(s, npix, out->srgb8, out_kind, &launches);
-        if (st != VRJ_OK) return st;
-    }
-    const auto t_call2 = std::chrono::steady_clock::now();
-    VRJ_CUDA(cudaEventRecord(s->ev_done, s->stream));
-    VRJ_CUDA(wait_event(s->ev1, scene->device)); // the last kernel is done: the next caller may render while this one's copies run
-    turn.release();
-    VRJ_CUDA(wait_event(s->ev_done, scene->device));
-    const auto t_call3 = std::chrono::steady_clock::now();
-    float ms = 0.f;
-    VRJ_CUDA(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+    st = call.finish(arrs, 5, out->srgb8, out_kind, out->stats);
+    if (st != VRJ_OK) return st;
     if (timing) {
         auto msd = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
             return std::chrono::duration<double, std::milli>(b - a).count();
         };
         std::fprintf(stderr, "vrj_render_tile: setup %.3f ms, enqueue %.3f ms, wait %.3f ms (device %.3f ms, %llu launches)\n",
-                     msd(t_call0, t_call1), msd(t_call1, t_call2), msd(t_call2, t_call3), ms, (unsigned long long)launches);
+                     msd(t_call0, call.t_start), msd(call.t_start, call.t_enqueued), msd(call.t_enqueued, call.t_done), call.ms,
+                     (unsigned long long)call.launches);
     }
-    if (out->stats) fill_call_stats(out->stats, s, hstats, launches, ms);
     return VRJ_OK;
 }
 
-// Adaptive sampling (the header states the passes and the stopping rule).  Pass j renders its `count` samples for the pixels of
-// its list -- the whole tile in pass 0, RenderConst::pixel_list after that -- in batches split to the path budget like
-// vrj_render_tile's, and k_resolve_adaptive applies them to the tile's accumulators and y_sq_sum.  k_adaptive_select then
-// judges the list's pixels, an exclusive scan (vrj_build::exclusive_scan_u32) of its flags gives every continuing pixel its
-// place, and k_adaptive_compact writes the next list in tile order.  The host reads back one count per pass and copies the
-// arrays out once, at the end.
+// Adaptive sampling (the header states the passes and the stopping rule): render_passes from a zero state, until no pixel is
+// active.
 VrjStatus vrj_render_adaptive(const VrjScene *scene_c, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p,
                               const VrjAdaptiveParams *ap, VrjAccumOut *out, double *y_sq_sum, VrjAdaptiveStats *astats) {
     VrjScene *scene = const_cast<VrjScene *>(scene_c);
     size_t n_light_samples = 0;
     VrjStatus st = check_render_args(scene, tile, height, width, p, out, &n_light_samples);
     if (st != VRJ_OK) return st;
-    if (!ap) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
-    if (p->spp != 0) return fail(VRJ_ERR_INVALID_ARGUMENT, "params->spp must be 0: vrj_render_adaptive takes its sample counts from VrjAdaptiveParams");
-    if (ap->min_samples < 2) return fail(VRJ_ERR_INVALID_ARGUMENT, "min_samples must be >= 2 (the variance needs two samples)");
-    if (ap->max_samples < ap->min_samples) return fail(VRJ_ERR_INVALID_ARGUMENT, "max_samples must be >= min_samples");
-    if (ap->pass_samples < 1) return fail(VRJ_ERR_INVALID_ARGUMENT, "pass_samples must be >= 1");
-    if (!(ap->rel_error > 0.0) || !std::isfinite(ap->rel_error)) return fail(VRJ_ERR_INVALID_ARGUMENT, "rel_error must be > 0 and finite");
-    if (!(ap->abs_floor >= 0.0) || !std::isfinite(ap->abs_floor)) return fail(VRJ_ERR_INVALID_ARGUMENT, "abs_floor must be >= 0 and finite");
+    PassRule rule;
+    st = check_pass_rule(p, ap, "vrj_render_adaptive", "VrjAdaptiveParams", &rule);
+    if (st != VRJ_OK) return st;
     if (out->accumulate) return fail(VRJ_ERR_UNSUPPORTED, "vrj_render_adaptive does not continue from a previous state (accumulate)");
     if (out->photons) return fail(VRJ_ERR_UNSUPPORTED, "vrj_render_adaptive has no photons output");
     const uint64_t npix = (tile->end_column - tile->start_column) * (tile->end_row - tile->start_row);
@@ -1548,131 +1707,26 @@ VrjStatus vrj_render_adaptive(const VrjScene *scene_c, const VrjTile *tile, uint
     if (astats) std::memset(astats, 0, sizeof(VrjAdaptiveStats));
     if (npix == 0) return VRJ_OK;
     VRJ_CUDA(cudaSetDevice(scene->device));
-
-    ActiveCall active(g_active_calls[(unsigned)scene->device % 64]);
-    // the largest pass renders every pixel (min_samples) or a subset (pass_samples): the block is sized for the larger of the two
-    const uint32_t widest = std::min(ap->max_samples, std::max(ap->min_samples, ap->pass_samples));
-    uint32_t batch = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(widest, call_path_budget(scene, active) / npix));
-    if (npix * (uint64_t)batch > 0xfffffff0ull) return fail(VRJ_ERR_UNSUPPORTED, "tile too large");
-    Scratch *s = acquire_scratch(scene, npix * batch);
-    struct Releaser {
-        VrjScene *sc;
-        Scratch *s;
-        ~Releaser() {
-            if (s->stream) cudaStreamSynchronize(s->stream);
-            release_scratch(sc, s);
-        }
-    } releaser{scene, s};
-    const uint32_t filter = effective_filter(scene, p);
-    st = ensure_call_scratch(s, p, call_wants_records(scene, p, filter), npix, &batch, n_light_samples);
+    PassResult res;
+    st = render_passes(scene, tile, height, width, p, rule, 0, n_light_samples, out, y_sq_sum, &res);
     if (st != VRJ_OK) return st;
-    st = ensure_adaptive_buffers(s, npix);
-    if (st != VRJ_OK) return st;
-    const size_t capacity = npix * batch; // paths per batch
-    DeviceBuffer *zero[5] = {&s->acc_sum, &s->acc_bias, &s->acc_weight, &s->acc_wbias, &s->ysq};
-    const size_t per[5] = {3, 3, 1, 1, 1};
-    for (int i = 0; i < 5; i++) VRJ_CUDA(cudaMemsetAsync(zero[i]->p, 0, npix * per[i] * sizeof(double), s->stream));
-    VRJ_CUDA(cudaMemsetAsync(s->aconverged.p, 0, sizeof(unsigned long long), s->stream));
-    VRJ_CUDA(cudaMemsetAsync(s->stats.p, 0, ST_COUNT * sizeof(unsigned long long), s->stream));
-    st = stage_lights(s, p);
-    if (st != VRJ_OK) return st;
-
-    RenderConst rc = make_render_const(tile, height, width, p);
-    rc.lights = s->lights.as<LightDev>();
-    rc.light_samples = s->light_samples.as<double>();
-    rc.div_tile_w = FastDiv::make(rc.tile_w);
-    // the flags and the scan's tile totals live in the photon buffer, which is free between a pass's resolve and the next
-    // batch: (n + 1) + (n / 2048 + 2) uint32 fit the 16 bytes per path of a block that holds at least one path per pixel
-    uint32_t *flags = s->photons.as<uint32_t>();
-    uint32_t *host_active = s->host_count + 192; // pinned slots (host_count: 0..3 drain check, 8.. sample table, 160.. stats)
-    unsigned long long *host_converged = reinterpret_cast<unsigned long long *>(s->host_count + 194);
-    uint64_t launches = 0, passes = 0, samples = 0;
-    uint32_t n_active = (uint32_t)npix, held = 0, count = ap->min_samples, cur = 0;
-    const uint32_t *list = nullptr; // pass 0: the whole tile
-    s->n_marks = 0;
-    RenderTurn turn(scene->device); // declared after `releaser`: an early return gives the turn back before the block
-    turn.acquire();
-    VRJ_CUDA(cudaEventRecord(s->ev0, s->stream));
-    for (;;) {
-        const uint32_t b = (uint32_t)std::max<size_t>(1, std::min<size_t>(count, capacity / n_active));
-        rc.npix = n_active, rc.pixel_list = list;
-        for (uint32_t done = 0; done < count; done += b) {
-            rc.batch_samples = std::min(b, count - done);
-            rc.div_batch = FastDiv::make(rc.batch_samples);
-            rc.first_sample = p->sample_offset + (uint64_t)(held + done) * rc.sample_stride;
-            st = dispatch_batch(scene, s, rc, p, filter, &launches, nullptr, s->ysq.as<double>());
-            if (st != VRJ_OK) return st;
-        }
-        held += count, passes++, samples += (uint64_t)n_active * count;
-        const uint32_t more = held < ap->max_samples ? 1u : 0u;
-        k_adaptive_select<<<(n_active + 1 + 255) / 256, 256, 0, s->stream>>>(s->acc_sum.as<double>(), s->acc_weight.as<double>(), s->ysq.as<double>(), list, n_active,
-                                                                          ap->rel_error, ap->abs_floor, more, flags, s->aconverged.as<unsigned long long>());
-        launches++;
-        VRJ_CUDA(cudaGetLastError());
-        if (!more) break;
-        st = vrj_build::exclusive_scan_u32(flags, n_active + 1, flags + n_active + 1, s->stream);
-        if (st != VRJ_OK) return st;
-        launches += 3;
-        k_adaptive_compact<<<(n_active + 255) / 256, 256, 0, s->stream>>>(list, flags, n_active, s->alist[cur].as<uint32_t>());
-        launches++;
-        VRJ_CUDA(cudaGetLastError());
-        VRJ_CUDA(cudaMemcpyAsync(host_active, flags + n_active, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
-        VRJ_CUDA(cudaStreamSynchronize(s->stream));
-        if (*host_active == 0) break;
-        n_active = *host_active, list = s->alist[cur].as<uint32_t>(), cur ^= 1u;
-        count = std::min(ap->pass_samples, ap->max_samples - held);
-    }
-    unsigned long long *hstats = reinterpret_cast<unsigned long long *>(s->host_count + 160);
-    VRJ_CUDA(cudaEventRecord(s->ev1, s->stream));
-    VRJ_CUDA(cudaMemcpyAsync(hstats, s->stats.p, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-    VRJ_CUDA(cudaMemcpyAsync(host_converged, s->aconverged.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-    const cudaMemcpyKind out_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-    struct Arr {
-        double *user;
-        DeviceBuffer *dev;
-        size_t per;
-    } arrs[6] = {{out->colour, &s->acc_colour, 3}, {out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3},
-                 {out->weight, &s->acc_weight, 1}, {out->weight_bias, &s->acc_wbias, 1}, {y_sq_sum, &s->ysq, 1}};
-    for (const Arr &a : arrs)
-        if (a.user) VRJ_CUDA(cudaMemcpyAsync(a.user, a.dev->p, npix * a.per * sizeof(double), out_kind, s->stream));
-    if (out->srgb8) {
-        st = copy_srgb8(s, npix, out->srgb8, out_kind, &launches);
-        if (st != VRJ_OK) return st;
-    }
-    VRJ_CUDA(cudaEventRecord(s->ev_done, s->stream));
-    VRJ_CUDA(wait_event(s->ev1, scene->device)); // the last kernel is done: the next caller may render while this one's copies run
-    turn.release();
-    VRJ_CUDA(wait_event(s->ev_done, scene->device));
-    float ms = 0.f;
-    VRJ_CUDA(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-    if (out->stats) fill_call_stats(out->stats, s, hstats, launches, ms);
     if (astats) {
-        astats->passes = passes, astats->samples = samples;
-        astats->pixels_converged = *host_converged, astats->pixels_unconverged = npix - *host_converged;
+        astats->passes = res.passes, astats->samples = res.samples;
+        astats->pixels_converged = res.counts.converged, astats->pixels_unconverged = res.counts.at_max;
     }
     return VRJ_OK;
 }
 
-// Progressive rendering (the header states the schedule).  Before each pass k_progressive_select judges every pixel of the
-// tile on the state and writes the count it takes; the host reads back the counters (one 48-byte copy per pass).  When every
-// active pixel takes the same count c -- always, for a state this call's schedule produced with unchanged parameters -- the
-// pass is one sub-pass: the scan of the select's flags and k_progressive_compact list the active pixels with their first new
-// sample, and the LIST = 2 kernels render samples base .. base + c - 1 of each, resolved by k_resolve_adaptive.  Otherwise
-// the pass runs one such sub-pass per distinct count, largest first (k_progressive_group picks the pixels).  Pixel lists stay
-// row-major.  The state goes into the block once (copied from the host, or device to device) and comes back once.
+// Progressive rendering (the header states the schedule): render_passes on the caller's state.
 VrjStatus vrj_render_progressive(const VrjScene *scene_c, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p,
                                  const VrjProgressiveParams *pp, VrjAccumOut *out, double *y_sq_sum, VrjProgressiveStats *pstats) {
     VrjScene *scene = const_cast<VrjScene *>(scene_c);
     size_t n_light_samples = 0;
     VrjStatus st = check_render_args(scene, tile, height, width, p, out, &n_light_samples);
     if (st != VRJ_OK) return st;
-    if (!pp) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
-    if (p->spp != 0) return fail(VRJ_ERR_INVALID_ARGUMENT, "params->spp must be 0: vrj_render_progressive takes its sample counts from VrjProgressiveParams");
-    if (pp->min_samples < 2) return fail(VRJ_ERR_INVALID_ARGUMENT, "min_samples must be >= 2 (the variance needs two samples)");
-    if (pp->max_samples < pp->min_samples) return fail(VRJ_ERR_INVALID_ARGUMENT, "max_samples must be >= min_samples");
-    if (pp->pass_samples < 1) return fail(VRJ_ERR_INVALID_ARGUMENT, "pass_samples must be >= 1");
-    if (!(pp->rel_error > 0.0) || !std::isfinite(pp->rel_error)) return fail(VRJ_ERR_INVALID_ARGUMENT, "rel_error must be > 0 and finite");
-    if (!(pp->abs_floor >= 0.0) || !std::isfinite(pp->abs_floor)) return fail(VRJ_ERR_INVALID_ARGUMENT, "abs_floor must be >= 0 and finite");
+    PassRule rule;
+    st = check_pass_rule(p, pp, "vrj_render_progressive", "VrjProgressiveParams", &rule);
+    if (st != VRJ_OK) return st;
     if (out->memory > VRJ_MEM_DEVICE) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown memory kind");
     if (!out->colour_sum || !out->colour_bias || !out->weight || !out->weight_bias || !y_sq_sum)
         return fail(VRJ_ERR_INVALID_ARGUMENT, "the state (colour_sum, colour_bias, weight, weight_bias, y_sq_sum) is required");
@@ -1684,149 +1738,12 @@ VrjStatus vrj_render_progressive(const VrjScene *scene_c, const VrjTile *tile, u
     if (pstats) std::memset(pstats, 0, sizeof(VrjProgressiveStats));
     if (npix == 0) return VRJ_OK;
     VRJ_CUDA(cudaSetDevice(scene->device));
-
-    ActiveCall active(g_active_calls[(unsigned)scene->device % 64]);
-    // the widest pass is the whole tile at max(min, pass) samples (a fresh state's first pass, or a state that every pixel
-    // has to continue); the block is sized for it
-    const uint32_t widest = std::min(pp->max_samples, std::max(pp->min_samples, pp->pass_samples));
-    uint32_t batch = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(widest, call_path_budget(scene, active) / npix));
-    if (npix * (uint64_t)batch > 0xfffffff0ull) return fail(VRJ_ERR_UNSUPPORTED, "tile too large");
-    Scratch *s = acquire_scratch(scene, npix * batch);
-    struct Releaser {
-        VrjScene *sc;
-        Scratch *s;
-        ~Releaser() {
-            if (s->stream) cudaStreamSynchronize(s->stream);
-            release_scratch(sc, s);
-        }
-    } releaser{scene, s};
-    const uint32_t filter = effective_filter(scene, p);
-    st = ensure_call_scratch(s, p, call_wants_records(scene, p, filter), npix, &batch, n_light_samples);
+    PassResult res;
+    st = render_passes(scene, tile, height, width, p, rule, pp->max_passes, n_light_samples, out, y_sq_sum, &res);
     if (st != VRJ_OK) return st;
-    st = ensure_adaptive_buffers(s, npix);
-    if (st != VRJ_OK) return st;
-    if (s->prog_npix < npix) {
-        s->prog_npix = 0;
-        std::vector<std::pair<DeviceBuffer *, size_t>> want = {{&s->pcount, npix * 4}, {&s->pcounters, sizeof(ProgressiveCounters)}};
-        st = alloc_group(s->prog_slab, want, "progressive rendering buffers");
-        if (st != VRJ_OK) return st;
-        s->prog_npix = npix;
-    }
-    const size_t capacity = npix * batch; // paths per batch
-    const cudaMemcpyKind in_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-    const cudaMemcpyKind out_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-    struct Arr {
-        double *user;
-        DeviceBuffer *dev;
-        size_t per;
-    } state[5] = {{out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3}, {out->weight, &s->acc_weight, 1},
-                  {out->weight_bias, &s->acc_wbias, 1}, {y_sq_sum, &s->ysq, 1}};
-    for (const Arr &a : state) {
-        if (out->accumulate) VRJ_CUDA(cudaMemcpyAsync(a.dev->p, a.user, npix * a.per * sizeof(double), in_kind, s->stream));
-        else VRJ_CUDA(cudaMemsetAsync(a.dev->p, 0, npix * a.per * sizeof(double), s->stream));
-    }
-    VRJ_CUDA(cudaMemsetAsync(s->stats.p, 0, ST_COUNT * sizeof(unsigned long long), s->stream));
-    st = stage_lights(s, p);
-    if (st != VRJ_OK) return st;
-
-    RenderConst rc = make_render_const(tile, height, width, p);
-    rc.lights = s->lights.as<LightDev>();
-    rc.light_samples = s->light_samples.as<double>();
-    rc.div_tile_w = FastDiv::make(rc.tile_w);
-    const uint32_t n = (uint32_t)npix;
-    // the flags and the scan's tile totals live in the photon buffer, as in vrj_render_adaptive
-    uint32_t *flags = s->photons.as<uint32_t>(), *count = s->pcount.as<uint32_t>();
-    uint32_t *list = s->alist[0].as<uint32_t>(), *base = s->alist[1].as<uint32_t>();
-    ProgressiveCounters *ctr = s->pcounters.as<ProgressiveCounters>();
-    // pinned slots (host_count: 0..3 drain check, 8.. sample table, 160.. stats, 192.. vrj_render_adaptive)
-    ProgressiveCounters *hctr = reinterpret_cast<ProgressiveCounters *>(s->host_count + 200);
-    uint32_t *host_listed = s->host_count + 216;
-    const unsigned grid = (n + 1 + 255) / 256;
-    uint64_t launches = 0, passes = 0, samples = 0;
-    s->n_marks = 0;
-    RenderTurn turn(scene->device); // declared after `releaser`: an early return gives the turn back before the block
-    turn.acquire();
-    VRJ_CUDA(cudaEventRecord(s->ev0, s->stream));
-    // the samples base[i] .. base[i] + c - 1 of the m listed pixels, in batches split to the path budget
-    auto render_listed = [&](uint32_t m, uint32_t c) -> VrjStatus {
-        const uint32_t b = (uint32_t)std::max<size_t>(1, std::min<size_t>(c, capacity / m));
-        rc.npix = m, rc.pixel_list = list, rc.pixel_base = base;
-        for (uint32_t done = 0; done < c; done += b) {
-            rc.batch_samples = std::min(b, c - done);
-            rc.div_batch = FastDiv::make(rc.batch_samples);
-            rc.first_sample = p->sample_offset + (uint64_t)done * rc.sample_stride;
-            const VrjStatus bst = dispatch_batch(scene, s, rc, p, filter, &launches, nullptr, s->ysq.as<double>());
-            if (bst != VRJ_OK) return bst;
-        }
-        samples += (uint64_t)m * c;
-        return VRJ_OK;
-    };
-    for (;;) {
-        VRJ_CUDA(cudaMemsetAsync(ctr, 0, sizeof(ProgressiveCounters), s->stream));
-        VRJ_CUDA(cudaMemsetAsync(&ctr->cmin, 0xff, sizeof(uint32_t), s->stream));
-        k_progressive_select<<<grid, 256, 0, s->stream>>>(s->acc_sum.as<double>(), s->acc_weight.as<double>(), s->ysq.as<double>(), n, pp->min_samples,
-                                                          pp->max_samples, pp->pass_samples, pp->rel_error, pp->abs_floor, count, flags, ctr);
-        launches++;
-        VRJ_CUDA(cudaGetLastError());
-        VRJ_CUDA(cudaMemcpyAsync(hctr, ctr, sizeof(ProgressiveCounters), cudaMemcpyDeviceToHost, s->stream));
-        VRJ_CUDA(cudaStreamSynchronize(s->stream));
-        if (hctr->bad) return fail(VRJ_ERR_INVALID_ARGUMENT, "a weight of the state is not a sample count (negative, fractional, not finite or >= 2^32)");
-        if (hctr->active == 0 || (pp->max_passes && passes == pp->max_passes)) break;
-        if (hctr->cmax == hctr->cmin) {
-            st = vrj_build::exclusive_scan_u32(flags, n + 1, flags + n + 1, s->stream);
-            if (st != VRJ_OK) return st;
-            k_progressive_compact<<<(n + 255) / 256, 256, 0, s->stream>>>(s->acc_weight.as<double>(), flags, n, list, base);
-            launches += 4;
-            VRJ_CUDA(cudaGetLastError());
-            st = render_listed((uint32_t)hctr->active, hctr->cmax);
-            if (st != VRJ_OK) return st;
-        } else {
-            for (uint32_t cur = hctr->cmax; cur != 0;) {
-                VRJ_CUDA(cudaMemsetAsync(&ctr->next, 0, sizeof(uint32_t), s->stream));
-                k_progressive_group<<<grid, 256, 0, s->stream>>>(count, n, cur, flags, ctr);
-                st = vrj_build::exclusive_scan_u32(flags, n + 1, flags + n + 1, s->stream);
-                if (st != VRJ_OK) return st;
-                k_progressive_compact<<<(n + 255) / 256, 256, 0, s->stream>>>(s->acc_weight.as<double>(), flags, n, list, base);
-                launches += 5;
-                VRJ_CUDA(cudaGetLastError());
-                VRJ_CUDA(cudaMemcpyAsync(host_listed, flags + n, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
-                VRJ_CUDA(cudaMemcpyAsync(&hctr->next, &ctr->next, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
-                VRJ_CUDA(cudaStreamSynchronize(s->stream));
-                const uint32_t m = *host_listed, next = hctr->next;
-                if (m) {
-                    st = render_listed(m, cur);
-                    if (st != VRJ_OK) return st;
-                }
-                cur = next;
-            }
-        }
-        passes++;
-    }
-    const ProgressiveCounters final_ctr = *hctr;
-    if (out->colour || out->srgb8) {
-        k_finalize<<<(n + 255) / 256, 256, 0, s->stream>>>(s->acc_sum.as<double>(), s->acc_weight.as<double>(), s->acc_colour.as<double>(), n);
-        launches++;
-        VRJ_CUDA(cudaGetLastError());
-    }
-    unsigned long long *hstats = reinterpret_cast<unsigned long long *>(s->host_count + 160);
-    VRJ_CUDA(cudaEventRecord(s->ev1, s->stream));
-    VRJ_CUDA(cudaMemcpyAsync(hstats, s->stats.p, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
-    for (const Arr &a : state) VRJ_CUDA(cudaMemcpyAsync(a.user, a.dev->p, npix * a.per * sizeof(double), out_kind, s->stream));
-    if (out->colour) VRJ_CUDA(cudaMemcpyAsync(out->colour, s->acc_colour.p, npix * 3 * sizeof(double), out_kind, s->stream));
-    if (out->srgb8) {
-        st = copy_srgb8(s, npix, out->srgb8, out_kind, &launches);
-        if (st != VRJ_OK) return st;
-    }
-    VRJ_CUDA(cudaEventRecord(s->ev_done, s->stream));
-    VRJ_CUDA(wait_event(s->ev1, scene->device)); // the last kernel is done: the next caller may render while this one's copies run
-    turn.release();
-    VRJ_CUDA(wait_event(s->ev_done, scene->device));
-    float ms = 0.f;
-    VRJ_CUDA(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-    if (out->stats) fill_call_stats(out->stats, s, hstats, launches, ms);
     if (pstats) {
-        pstats->passes = passes, pstats->samples = samples;
-        pstats->pixels_converged = final_ctr.converged, pstats->pixels_at_max = final_ctr.at_max, pstats->pixels_active = final_ctr.active;
+        pstats->passes = res.passes, pstats->samples = res.samples;
+        pstats->pixels_converged = res.counts.converged, pstats->pixels_at_max = res.counts.at_max, pstats->pixels_active = res.counts.active;
     }
     return VRJ_OK;
 }

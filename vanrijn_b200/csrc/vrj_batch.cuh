@@ -68,6 +68,17 @@ struct ResolveCopy {
     uint32_t pieces;
 };
 
+// The block's page-locked slots.  Counters come back and the sample table goes out through them: a copy between the device and
+// pageable memory holds the enqueueing thread until everything queued before it has finished (the render gate could not
+// open before the result's copies).
+struct PinnedBlock {
+    uint32_t drain[4];                          // run_levels' drain check: (queue length, tail flag) of two groups of levels
+    uint64_t sample_table[4 * MULTI_MAX_CALLS]; // coalesced calls: the wavefront's sample indices
+    unsigned long long stats[ST_COUNT];         // the call's ray counters
+    ProgressiveCounters pass;                   // render_passes: the last select's counters
+    uint32_t listed;                            // render_passes: the length of a sub-pass's pixel list
+};
+
 // per-call scratch: path queues, photon results, accumulators, counters
 struct Scratch {
     size_t capacity = 0; // paths
@@ -81,10 +92,9 @@ struct Scratch {
     DeviceBuffer queue_slab, rec_slab, acc_slab; // the groups above live in one allocation each (see ensure_scratch)
     DeviceBuffer multi_out, sample_table; // coalesced calls: their output arrays (call-major pieces) and the batch's sample indices
     DeviceBuffer lights, light_samples, srgb8;
-    DeviceBuffer ysq, alist[2], aconverged, adapt_slab; // vrj_render_adaptive: y_sq_sum, this / next pass's pixel list, a counter
-    size_t adapt_npix = 0;
-    DeviceBuffer pcount, pcounters, prog_slab; // vrj_render_progressive: per-pixel count of the pass, ProgressiveCounters
-    size_t prog_npix = 0;
+    // render_passes: y_sq_sum, the previous / next pass's pixel list, the next pass's first samples, the selects' counters
+    DeviceBuffer ysq, pass_list[2], pass_base, pass_counters, pass_slab;
+    size_t pass_npix = 0;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr; // first / last kernel of a call
     cudaEvent_t ev_done = nullptr;             // behind the call's last copy
@@ -96,7 +106,7 @@ struct Scratch {
     std::vector<cudaEvent_t> marks; // per-launch boundaries, reused across calls
     std::vector<int> mark_class;    // class of the launch that ENDS at mark i (-1: start of a batch)
     size_t n_marks = 0;
-    uint32_t *host_count = nullptr; // pinned
+    PinnedBlock *pinned = nullptr;
     ~Scratch() {
         if (stream) cudaStreamDestroy(stream);
         if (ev0) cudaEventDestroy(ev0);
@@ -111,7 +121,7 @@ struct Scratch {
         for (cudaEvent_t e : drain_ev)
             if (e) cudaEventDestroy(e);
         for (cudaEvent_t e : marks) cudaEventDestroy(e);
-        if (host_count) cudaFreeHost(host_count);
+        if (pinned) cudaFreeHost(pinned);
     }
     // record a boundary event on the stream; cls = class of the launch it closes
     cudaError_t mark(int cls) {
@@ -187,7 +197,7 @@ inline bool wants_records(const VrjScene *sc, int walk) {
 }
 
 // One batch with the integrator (WHITTED) and the scene's material kinds (MM, see vrj_device.cuh) fixed at compile time.
-template <typename NT, typename R, bool COUNT, bool WHITTED, int MM, int LIST>
+template <typename NT, typename R, bool COUNT, bool WHITTED, int MM, bool LIST>
 VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int walk, uint64_t *launches, const MultiCalls *multi,
                      const ResolveCopy *copy, double *ysq) {
     const bool quad = walk == 1, q16 = walk == 2; // 0: the 2-wide tree in NT boxes; 1: 4-wide f32; 2: 2-wide on the 16-bit grid
@@ -276,10 +286,10 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
             const int slot = (int)(k / 4) & 1;
             if (drain_pending) {
                 VRJ_CUDA(cudaEventSynchronize(s->drain_ev[slot ^ 1]));
-                if (s->host_count[2 * (slot ^ 1)] == 0 || s->host_count[2 * (slot ^ 1) + 1] != 0) break;
+                if (s->pinned->drain[2 * (slot ^ 1)] == 0 || s->pinned->drain[2 * (slot ^ 1) + 1] != 0) break;
             }
-            VRJ_CUDA(cudaMemcpyAsync(s->host_count + 2 * slot, qcount + k + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
-            VRJ_CUDA(cudaMemcpyAsync(s->host_count + 2 * slot + 1, tail_done, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
+            VRJ_CUDA(cudaMemcpyAsync(s->pinned->drain + 2 * slot, qcount + k + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
+            VRJ_CUDA(cudaMemcpyAsync(s->pinned->drain + 2 * slot + 1, tail_done, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
             VRJ_CUDA(cudaEventRecord(s->drain_ev[slot], s->stream));
             drain_pending = true;
         }
@@ -322,7 +332,7 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
 
 // kernel variants exist for "Lambertian only" (the reference's own scenes: main.rs, benches/simple_scene.rs) and for
 // "any material"; VRJ_MATERIAL_MASK=15 in the environment forces the general variant (experiments)
-template <typename NT, typename R, bool COUNT, int LIST>
+template <typename NT, typename R, bool COUNT, bool LIST>
 VrjStatus run_materials(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches, const MultiCalls *multi,
                         const ResolveCopy *copy, double *ysq) {
     const bool lambert_only = sc->kernel_material_mask == 1u;
@@ -332,14 +342,13 @@ VrjStatus run_materials(const VrjScene *sc, Scratch *s, const RenderConst &rc, b
     return lambert_only ? run_levels<NT, R, COUNT, false, 1, LIST>(sc, s, rc, walk, launches, multi, copy, ysq)
                         : run_levels<NT, R, COUNT, false, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches, multi, copy, ysq);
 }
-// `ysq` (vrj_render_adaptive, vrj_render_progressive): the batch is resolved by k_resolve_adaptive, which also keeps
-// y_sq_sum; a batch over rc.pixel_list runs the LIST variants of the kernels (LIST = 2 when rc.pixel_base is set too)
+// `ysq` (render_passes): the batch is resolved by k_resolve_adaptive, which also keeps y_sq_sum; a batch over rc.pixel_list
+// (and rc.pixel_base) runs the LIST variants of the kernels
 template <typename NT, typename R, bool COUNT>
 VrjStatus run_batch(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches, const MultiCalls *multi = nullptr,
                     const ResolveCopy *copy = nullptr, double *ysq = nullptr) {
-    if (rc.pixel_base) return run_materials<NT, R, COUNT, 2>(sc, s, rc, whitted, walk, launches, multi, copy, ysq);
-    return rc.pixel_list ? run_materials<NT, R, COUNT, 1>(sc, s, rc, whitted, walk, launches, multi, copy, ysq)
-                         : run_materials<NT, R, COUNT, 0>(sc, s, rc, whitted, walk, launches, multi, copy, ysq);
+    return rc.pixel_list ? run_materials<NT, R, COUNT, true>(sc, s, rc, whitted, walk, launches, multi, copy, ysq)
+                         : run_materials<NT, R, COUNT, false>(sc, s, rc, whitted, walk, launches, multi, copy, ysq);
 }
 
 } // namespace vrjimpl

@@ -16,7 +16,7 @@ struct DenoiseGuides {
     const int32_t *material;
 };
 
-// c = s * (1/n), var = v * (1/n) with k_adaptive_select's v
+// c = s * (1/n), var = v * (1/n) with adaptive_converged's v
 static __global__ void k_denoise_init(const double *__restrict__ sum, const double *__restrict__ weight, const double *__restrict__ ysq,
                                uint32_t npix, double4 *__restrict__ out) {
     const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;

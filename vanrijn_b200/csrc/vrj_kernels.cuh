@@ -118,11 +118,11 @@ struct RenderConst {
     double film_w, film_h;
     const LightDev *lights;      // n_lights entries, then (if has_ambient) the ambient light's spectrum in entry n_lights
     const double *light_samples;
-    const uint32_t *pixel_list;  // kernels with LIST != 0: batch position p renders tile pixel pixel_list[p] and npix is the
-                                 // list's length (the still-active pixels of an adaptive pass, vrj_render_adaptive); slots and
-                                 // photons stay indexed by list position
-    const uint32_t *pixel_base;  // kernels with LIST == 2: batch position p renders samples pixel_base[p] + s, s < batch_samples,
-                                 // of its pixel (a progressive pass over pixels that hold different counts, vrj_render_progressive)
+    const uint32_t *pixel_list;  // kernels with LIST: batch position p renders tile pixel pixel_list[p] and npix is the list's
+                                 // length (the active pixels of a pass, render_passes); slots and photons stay indexed by list
+                                 // position
+    const uint32_t *pixel_base;  // set with pixel_list: batch position p renders samples pixel_base[p] + s, s < batch_samples,
+                                 // of its pixel (the samples the pixel already holds come first)
 };
 
 template <typename R>
@@ -188,19 +188,19 @@ __device__ __forceinline__ void biased_ray(V3<R> origin, V3<R> direction, R amou
 // same nodes (broadcast loads), hits the same primitive class, and the first bounces leave from neighbouring points
 // (k_trace on camera rays 3.5 -> 2.5 ms per 32-spp step, measured).  A sample is still a pure function of
 // (seed, pixel, sample index), so the order changes no result.
-// LIST (a compile-time switch, so the tile's kernels carry no trace of it): 0, the batch covers the tile; 1, the pixels of
-// rc.pixel_list, all at the same samples; 2, the pixels of rc.pixel_list, each from its own first sample rc.pixel_base[p].
-template <int LIST = 0>
+// LIST (a compile-time switch, so the tile's kernels carry no trace of it): the batch covers the pixels of rc.pixel_list, each
+// from its own first sample rc.pixel_base[p]; otherwise the tile.
+template <bool LIST = false>
 __device__ __forceinline__ void slot_to_pixel(const RenderConst &rc, uint32_t slot, uint32_t &pixel_global,
                                               uint64_t &sample, uint64_t &grow, uint64_t &gcol) {
     uint32_t p = rc.div_batch.div(slot), s = slot - p * rc.batch_samples;
     uint64_t k = s;
-    if (LIST == 2) k += __ldg(rc.pixel_base + p);
+    if (LIST) k += __ldg(rc.pixel_base + p);
     if (LIST) p = __ldg(rc.pixel_list + p);
     uint32_t row = rc.div_tile_w.div(p), col = p - row * rc.tile_w;
     grow = rc.start_row + row, gcol = rc.start_column + col;
     pixel_global = (uint32_t)(grow * rc.width + gcol);
-    if (LIST == 2) sample = rc.first_sample + k * rc.sample_stride;
+    if (LIST) sample = rc.first_sample + k * rc.sample_stride;
     else sample = rc.sample_table ? __ldg(rc.sample_table + s) : rc.first_sample + (uint64_t)s * rc.sample_stride;
 }
 
@@ -237,7 +237,7 @@ __device__ __forceinline__ void stage_ray(const DevScene &sc, bool have_ray, uin
 // The camera ray of a result slot (camera.rs:45-66): two Philox draws, the film point, Ray::new.  It is a pure function of
 // the slot, so the primary level never stores it: k_raygen, k_trace on camera rays and the first k_shade each form it again
 // (one Philox block + one normalisation) instead of moving 48 bytes per ray through HBM three times.
-template <typename R, int LIST = 0>
+template <typename R, bool LIST = false>
 __device__ __forceinline__ void camera_ray(const DevScene &sc, const RenderConst &rc, uint32_t slot, V3<R> &o, V3<R> &d) {
     uint32_t pixel;
     uint64_t sample, grow, gcol;
@@ -253,7 +253,7 @@ __device__ __forceinline__ void camera_ray(const DevScene &sc, const RenderConst
 }
 
 // ---- k_raygen: camera rays (camera.rs:45-66), staged for traversal ----
-template <typename R, bool COUNT, int LIST = 0>
+template <typename R, bool COUNT, bool LIST = false>
 __global__ void __launch_bounds__(128, sizeof(R) == 4 ? VRJ_SHADE_MINB_F32 : VRJ_RAYGEN_MINB) k_raygen(DevScene sc, RenderConst rc, PathQueue q, TraceBuffers tb, uint32_t *list_count,
                                                 uint32_t *work, unsigned long long *stats) {
     const uint32_t n = rc.npix * rc.batch_samples;
@@ -318,7 +318,7 @@ struct RecHitSink {
     }
 };
 // the same for the camera rays of a batch: the ray is formed from its slot, nothing is read from the queue
-template <int LIST = 0>
+template <bool LIST = false>
 struct PrimaryRaySource {
     const DevScene &sc;
     const RenderConst &rc;
@@ -368,7 +368,7 @@ __global__ void VRJ_TRACE_BOUNDS(R) k_trace(DevScene sc, PathQueue q, TraceBuffe
 }
 
 // k_trace for the camera rays of a batch
-template <typename NT, typename R, bool COUNT, int LIST = 0>
+template <typename NT, typename R, bool COUNT, bool LIST = false>
 __global__ void VRJ_TRACE_BOUNDS(R) k_trace_primary(DevScene sc, RenderConst rc, TraceBuffers tb, const uint32_t *list_count, uint32_t *work,
                                                     unsigned long long *stats) {
     const uint32_t n = *list_count;
@@ -403,7 +403,7 @@ __global__ void VRJ_TRACE_BOUNDS(double) k_trace_rec(DevScene sc, TraceBuffers t
 }
 
 // the same launch over the 4-wide form of the tree (VRJ_FILTER_F32X4)
-template <bool COUNT, bool PRIMARY, int LIST = 0>
+template <bool COUNT, bool PRIMARY, bool LIST = false>
 __global__ void __launch_bounds__(128, VRJ_TRACE4_MINB) k_trace4(DevScene sc, RenderConst rc, PathQueue q, TraceBuffers tb, const uint32_t *list_count,
                                                                  uint32_t *work, unsigned long long *stats, const uint32_t *tail_done) {
     if (tail_done && *tail_done) return;
@@ -426,7 +426,7 @@ __global__ void __launch_bounds__(128, VRJ_TRACE4_MINB) k_trace4(DevScene sc, Re
 }
 
 // the same launch over 16-bit nodes (VRJ_FILTER_Q16)
-template <bool COUNT, bool PRIMARY, int LIST = 0>
+template <bool COUNT, bool PRIMARY, bool LIST = false>
 __global__ void __launch_bounds__(128, VRJ_TRACE_MINB) k_traceq(DevScene sc, RenderConst rc, PathQueue q, TraceBuffers tb, const uint32_t *list_count,
                                                                 uint32_t *work, unsigned long long *stats, const uint32_t *tail_done) {
     if (tail_done && *tail_done) return;
@@ -464,7 +464,7 @@ __device__ __forceinline__ double2 photon_out(R wavelength, R intensity) { retur
 // shadow rays), update the affine accumulator -- leaves the bounce ray and the new state in p and returns true.
 // `first`: p.slot is set, the rest of the state is initialised here (camera.rs:108-119).
 // `load_ray(o, d)` fetches the ray only when it is needed.
-template <typename NT, bool COUNT, bool WHITTED, int MM, int LIST, typename R, typename RayLoader>
+template <typename NT, bool COUNT, bool WHITTED, int MM, bool LIST, typename R, typename RayLoader>
 __device__ __forceinline__ bool shade_entry(const DevScene &sc, const RenderConst &rc, PathRegsT<R> &p, int2 hit, R hit_t, bool first,
                                             RayLoader load_ray, double2 *photons, LocalStats &ls) {
     const R span = R(740.0) - R(380.0); // photon.rs:18-24, colour/mod.rs:13-14
@@ -579,7 +579,7 @@ __device__ __forceinline__ bool shade_entry(const DevScene &sc, const RenderCons
 }
 
 // ---- k_shade: consume the hits of a queue; survivors are enqueued warp-ballot compacted and staged ----
-template <typename NT, typename R, bool COUNT, bool WHITTED, bool FIRST, int MM, int LIST = 0>
+template <typename NT, typename R, bool COUNT, bool WHITTED, bool FIRST, int MM, bool LIST = false>
 __global__ void VRJ_SHADE_BOUNDS(R) k_shade(DevScene sc, RenderConst rc, PathQueue in, const uint32_t *in_count,
                                                TraceBuffers tb_in, PathQueue out, uint32_t *out_count, TraceBuffers tb_out,
                                                uint32_t *list_count, uint32_t *work, double2 *photons,
@@ -695,7 +695,7 @@ __global__ void __launch_bounds__(128, VRJ_STAGE_MINB) k_stage(DevScene sc, Path
 // run for dozens), so a lane whose path has ended takes the next queue entry at once (one warp-aggregated atomic) instead
 // of idling until the longest path of its warp is done -- in the one-path-per-thread form a warp ran ~6 bounces for ~1.7
 // useful ones per lane.
-template <typename NT, typename R, bool COUNT, bool WHITTED, int MM, int LIST = 0>
+template <typename NT, typename R, bool COUNT, bool WHITTED, int MM, bool LIST = false>
 __global__ void __launch_bounds__(128, 2) k_tail(DevScene sc, RenderConst rc, PathQueue in, const uint32_t *in_count,
                                               uint32_t tail_max, double2 *photons, unsigned long long *stats,
                                               uint32_t *tail_done, uint32_t *work) {
@@ -785,10 +785,10 @@ __global__ void k_resolve(AccumDev acc, const double2 *photons, uint32_t first, 
     acc.colour[3 * p] = sx * inv, acc.colour[3 * p + 1] = sy * inv, acc.colour[3 * p + 2] = sz * inv;
 }
 
-// k_resolve for one pass of an adaptive render (vrj_render_adaptive): list position i holds tile pixel list[i] (pixel i when
+// k_resolve for one pass of an adaptive render (render_passes): list position i holds tile pixel list[i] (pixel i when
 // `list` is NULL) and its samples are the batch's slots i * batch_samples + s.  Besides the Kahan update it keeps
 // ysq[pixel] = ysq + y * y in sample order, y being the sample's Y exactly as it enters colour_sum (the noise estimate of
-// k_adaptive_select).
+// pass_count).
 template <typename R>
 __global__ void k_resolve_adaptive(AccumDev acc, double *ysq, const uint32_t *list, const double2 *photons, uint32_t n, uint32_t batch_samples) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -820,11 +820,15 @@ __global__ void k_resolve_adaptive(AccumDev acc, double *ysq, const uint32_t *li
     acc.colour[3 * p] = sx * inv, acc.colour[3 * p + 1] = sy * inv, acc.colour[3 * p + 2] = sz * inv;
 }
 
-// The stopping rule of vrj_render_adaptive on the n pixels of the pass just resolved (list as in k_resolve_adaptive), in the
-// order the header states it so a caller can replay it bit for bit: n = weight, s = colour_sum.y, q = y_sq_sum,
-// m = s / n (as s * (1/n)), v = max(0, (q - s m) / (n - 1)), t = rel_error * max(m, abs_floor); converged iff v <= t t n.
-// A NaN anywhere fails the comparison: such a pixel keeps sampling.  flag[i] = 1 if pixel i takes another pass (`more` is 0
-// when the pass reached max_samples); flag[n] = 0, so the exclusive scan of flag[0..n] ends in the next pass's length.
+// ---- the passes of vrj_render_adaptive and vrj_render_progressive (render_passes; the header states the schedule) ----
+struct PassRule {
+    uint32_t min_samples, max_samples, pass_samples, pad;
+    double rel_error, abs_floor;
+};
+
+// The stopping rule in the order the header states it, so a caller can replay it bit for bit: n = weight, s = colour_sum.y,
+// q = y_sq_sum, m = s / n (as s * (1/n)), v = max(0, (q - s m) / (n - 1)), t = rel_error * max(m, abs_floor); converged iff
+// v <= t t n.  A NaN anywhere fails the comparison: such a pixel keeps sampling.
 __device__ __forceinline__ bool adaptive_converged(double w, double s, double q, double rel_error, double abs_floor) {
     const double m = s * (1.0 / w);
     double v = (q - s * m) / (w - 1.0);
@@ -832,91 +836,102 @@ __device__ __forceinline__ bool adaptive_converged(double w, double s, double q,
     const double t = rel_error * (m > abs_floor ? m : abs_floor);
     return v <= t * t * w;
 }
-static __global__ void k_adaptive_select(const double *sum, const double *weight, const double *ysq, const uint32_t *list, uint32_t n,
-                                         double rel_error, double abs_floor, uint32_t more, uint32_t *flag, unsigned long long *converged) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    bool conv = false;
-    if (i < n) {
-        const uint32_t p = list ? list[i] : i;
-        conv = adaptive_converged(weight[p], sum[3 * p + 1], ysq[p], rel_error, abs_floor);
-        flag[i] = !conv && more ? 1u : 0u;
-    } else if (i == n) {
-        flag[n] = 0u;
+
+// The samples a pixel with state (w, s, q) takes in the coming pass; 0 when it is not active, and then `conv` / `at_max` say
+// why.  A weight that is no sample count (negative, fractional, not finite, >= 2^32) sets `bad` and takes nothing.
+__device__ __forceinline__ uint32_t pass_count(const PassRule &r, double w, double s, double q, bool &conv, bool &at_max, bool &bad) {
+    if (!(w >= 0.0 && w < 4294967296.0) || w != floor(w)) {
+        bad = true;
+        return 0;
     }
-    const uint32_t c = __reduce_add_sync(0xffffffffu, conv ? 1u : 0u);
-    if ((threadIdx.x & 31) == 0 && c) atomicAdd(converged, (unsigned long long)c);
+    const uint32_t held = (uint32_t)w;
+    const bool rule = adaptive_converged(w, s, q, r.rel_error, r.abs_floor);
+    if (held < r.min_samples) return r.min_samples - held;
+    if (held < r.max_samples && !rule) return min(r.pass_samples, r.max_samples - held);
+    if (rule) conv = true;
+    else at_max = true;
+    return 0;
 }
 
-// order-preserving compaction behind the scan of k_adaptive_select's flags: the next pass's list stays row-major, so its
-// camera rays stay as coherent as the tile's
-static __global__ void k_adaptive_compact(const uint32_t *list, const uint32_t *offset, uint32_t n, uint32_t *next) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n && offset[i + 1] != offset[i]) next[offset[i]] = list ? list[i] : i;
-}
-
-// ---- vrj_render_progressive (the header states the schedule) ----
-// What k_progressive_select reports to the host before each pass: the pixel counts of the state it judged, how many weights
-// were not sample counts, and the largest / smallest count an active pixel takes
+// What the selects of a call report to the host.  A pixel found inactive stays so for the rest of the call (its state no
+// longer changes), so each select judges only the pixels the previous pass rendered: `converged` and `at_max` sum over the
+// call's selects, the other fields describe the last one.
 struct ProgressiveCounters {
-    unsigned long long active, converged, at_max, bad;
-    uint32_t cmax, cmin; // cmin starts at 0xffffffff
-    uint32_t next;       // k_progressive_group: the largest count below the current sub-pass's (0: none)
+    unsigned long long active; // per select, like cmax / cmin_not (all three start at zero)
+    uint32_t cmax;             // the largest count an active pixel takes
+    uint32_t cmin_not;         // ~(the smallest), so that it too starts at zero and takes a maximum
+    unsigned long long converged, at_max, bad;
+    uint32_t next; // k_progressive_group: the largest count below the current sub-pass's (0: none)
     uint32_t pad;
 };
 
-// One thread per tile pixel: judges (n, s, q) with the rule of k_adaptive_select and writes the samples the pixel takes in
-// the coming pass to count[i] (0: inactive) and count[i] != 0 to flag[i]; flag[n] = 0 as in k_adaptive_select.  A weight
-// that is no sample count (negative, fractional, not finite, >= 2^32) is counted in `bad` and takes nothing.
-static __global__ void k_progressive_select(const double *sum, const double *weight, const double *ysq, uint32_t n, uint32_t min_samples,
-                                            uint32_t max_samples, uint32_t pass_samples, double rel_error, double abs_floor,
-                                            uint32_t *count, uint32_t *flag, ProgressiveCounters *ctr) {
+// One thread per position i of `list` (tile pixel list[i]; pixel i when `list` is NULL): flag[i] = 1 if the pixel takes
+// samples in the coming pass; flag[n] = 0, so the exclusive scan of flag[0..n] ends in the number of active pixels.  The
+// counters are summed per block before they go to `ctr`: with atomics from every warp on that one line of L2 the selects of
+// a 1080p adaptive render took 0.9 ms more (B200).
+static __global__ void k_progressive_select(const double *sum, const double *weight, const double *ysq, const uint32_t *list, uint32_t n,
+                                            PassRule rule, uint32_t *flag, ProgressiveCounters *ctr) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     uint32_t c = 0;
     bool conv = false, at_max = false, bad = false;
     if (i < n) {
-        const double w = weight[i];
-        if (!(w >= 0.0 && w < 4294967296.0) || w != floor(w)) {
-            bad = true;
-        } else {
-            const uint32_t held = (uint32_t)w;
-            const bool rule = adaptive_converged(w, sum[3 * i + 1], ysq[i], rel_error, abs_floor);
-            if (held < min_samples) c = min_samples - held;
-            else if (held < max_samples && !rule) c = min(pass_samples, max_samples - held);
-            else if (rule) conv = true;
-            else at_max = true;
-        }
-        count[i] = c;
+        const uint32_t p = list ? list[i] : i;
+        c = pass_count(rule, weight[p], sum[3 * p + 1], ysq[p], conv, at_max, bad);
         flag[i] = c ? 1u : 0u;
     } else if (i == n) {
         flag[n] = 0u;
     }
-    const uint32_t full = 0xffffffffu;
-    const uint32_t n_active = __reduce_add_sync(full, c ? 1u : 0u), n_conv = __reduce_add_sync(full, conv ? 1u : 0u);
-    const uint32_t n_max = __reduce_add_sync(full, at_max ? 1u : 0u), n_bad = __reduce_add_sync(full, bad ? 1u : 0u);
-    const uint32_t cmax = __reduce_max_sync(full, c), cmin = __reduce_min_sync(full, c ? c : full);
-    if ((threadIdx.x & 31) == 0) {
-        if (n_active) atomicAdd(&ctr->active, (unsigned long long)n_active), atomicMax(&ctr->cmax, cmax), atomicMin(&ctr->cmin, cmin);
-        if (n_conv) atomicAdd(&ctr->converged, (unsigned long long)n_conv);
-        if (n_max) atomicAdd(&ctr->at_max, (unsigned long long)n_max);
-        if (n_bad) atomicAdd(&ctr->bad, (unsigned long long)n_bad);
+    // 0 active, 1 converged, 2 at max, 3 bad (sums); 4 cmax, 5 cmin_not (maxima)
+    __shared__ uint32_t part[6][32];
+    const uint32_t full = 0xffffffffu, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint32_t v[6] = {__reduce_add_sync(full, c ? 1u : 0u), __reduce_add_sync(full, conv ? 1u : 0u), __reduce_add_sync(full, at_max ? 1u : 0u),
+                     __reduce_add_sync(full, bad ? 1u : 0u), __reduce_max_sync(full, c), __reduce_max_sync(full, c ? ~c : 0u)};
+    if (lane == 0)
+        for (int k = 0; k < 6; k++) part[k][warp] = v[k];
+    __syncthreads();
+    if (warp != 0) return;
+    const bool mine = lane < (blockDim.x >> 5);
+    for (int k = 0; k < 6; k++) {
+        const uint32_t x = mine ? part[k][lane] : 0u;
+        v[k] = k < 4 ? __reduce_add_sync(full, x) : __reduce_max_sync(full, x);
+    }
+    if (lane == 0) {
+        if (v[0]) atomicAdd(&ctr->active, (unsigned long long)v[0]), atomicMax(&ctr->cmax, v[4]), atomicMax(&ctr->cmin_not, v[5]);
+        if (v[1]) atomicAdd(&ctr->converged, (unsigned long long)v[1]);
+        if (v[2]) atomicAdd(&ctr->at_max, (unsigned long long)v[2]);
+        if (v[3]) atomicAdd(&ctr->bad, (unsigned long long)v[3]);
     }
 }
 
-// a pass whose active pixels take different counts runs one sub-pass per count, largest first: flag[i] = 1 for the pixels
-// that take `cur`, and ctr->next becomes the largest count below it
-static __global__ void k_progressive_group(const uint32_t *count, uint32_t n, uint32_t cur, uint32_t *flag, ProgressiveCounters *ctr) {
+// a pass whose active pixels take different counts runs one sub-pass per count, largest first: over the select's positions,
+// flag[i] = 1 for the pixels that take `cur` (the count recomputed from the state, which no sub-pass has changed yet), and
+// ctr->next becomes the largest count below it
+static __global__ void k_progressive_group(const double *sum, const double *weight, const double *ysq, const uint32_t *list, uint32_t n,
+                                           PassRule rule, uint32_t cur, uint32_t *flag, ProgressiveCounters *ctr) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    const uint32_t c = i < n ? count[i] : 0u;
-    if (i < n) flag[i] = c == cur ? 1u : 0u;
-    else if (i == n) flag[n] = 0u;
+    uint32_t c = 0;
+    if (i < n) {
+        const uint32_t p = list ? list[i] : i;
+        bool conv = false, at_max = false, bad = false;
+        c = pass_count(rule, weight[p], sum[3 * p + 1], ysq[p], conv, at_max, bad);
+        flag[i] = c == cur ? 1u : 0u;
+    } else if (i == n) {
+        flag[n] = 0u;
+    }
     const uint32_t below = __reduce_max_sync(0xffffffffu, c < cur ? c : 0u);
     if ((threadIdx.x & 31) == 0 && below) atomicMax(&ctr->next, below);
 }
 
-// k_adaptive_compact over the tile that also carries each listed pixel's first new sample (its weight) for LIST = 2
-static __global__ void k_progressive_compact(const double *weight, const uint32_t *offset, uint32_t n, uint32_t *list, uint32_t *base) {
+// order-preserving compaction behind the scan of the flags (list as in k_progressive_select): the flagged pixels go to `out`
+// with their first new sample (their weight) in `base`.  A list made from the tile is row-major, so its camera rays stay as
+// coherent as the tile's.
+static __global__ void k_progressive_compact(const uint32_t *list, const double *weight, const uint32_t *offset, uint32_t n, uint32_t *out,
+                                             uint32_t *base) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n && offset[i + 1] != offset[i]) list[offset[i]] = i, base[offset[i]] = (uint32_t)weight[i];
+    if (i < n && offset[i + 1] != offset[i]) {
+        const uint32_t p = list ? list[i] : i;
+        out[offset[i]] = p, base[offset[i]] = (uint32_t)weight[p];
+    }
 }
 
 // Several calls rendered as ONE wavefront (vanrijn_cuda.cu, "coalesced calls"): the batch's samples [first[c], first[c] +

@@ -407,6 +407,11 @@ class DeviceProgressiveBuffer {
     size_t height() const { return height_; }
     // continues the frame's state with up to pp.max_passes passes (options.spp is ignored: the counts come from pp)
     void render(const Scene &scene, const RenderOptions &options, const ProgressiveOptions &pp);
+    // the planned loop (vrj_plan_counts, vrj_render_counts): plan_counts() writes the frame's count map from its state with
+    // pp's rule (pp.max_passes is not used) and returns the plan; render_counts() renders that map -- or `counts`, a
+    // device map of width * height counts on this buffer's GPU -- in full wavefronts.  Loop until the plan's samples is 0.
+    VrjPlanStats plan_counts(const ProgressiveOptions &pp);
+    VrjCountsStats render_counts(const Scene &scene, const RenderOptions &options, const uint32_t *counts = nullptr);
     ImageRgbU8 to_image_rgb_u8() const; // ClampingToneMapper on the device
     // vrj_denoise (the header's defaults) of the frame as it stands, on the device; the first-hit features come from one
     // vrj_render_aux of options.spp camera rays per pixel, traced at the first call and kept for the frame
@@ -418,6 +423,7 @@ class DeviceProgressiveBuffer {
     double *colour_ = nullptr, *sum_ = nullptr, *bias_ = nullptr, *weight_ = nullptr, *weight_bias_ = nullptr, *y_sq_sum_ = nullptr;
     double *normal_ = nullptr, *depth_ = nullptr, *denoised_ = nullptr;
     int32_t *material_ = nullptr;
+    uint32_t *counts_ = nullptr;
     uint8_t *srgb8_ = nullptr;
     size_t width_, height_;
     int device_;

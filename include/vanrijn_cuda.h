@@ -378,6 +378,70 @@ VRJ_API VrjStatus vrj_render_progressive(const VrjScene *scene, const VrjTile *t
                                          const VrjRenderParams *params, const VrjProgressiveParams *pp,
                                          VrjAccumOut *out, double *y_sq_sum, VrjProgressiveStats *pstats);
 
+/* ---- per-pixel sample counts in full wavefronts, and a planner for them ----
+ * vrj_render_counts gives each pixel of `tile` its own number of new samples, counts[p], and renders all of them as full
+ * wavefronts: the call's samples are laid out one per slot (a pixel's samples in neighbouring slots) and rendered in batches
+ * of up to the call's path budget, whatever the counts are.  A count map can come from vrj_plan_counts below, or from the
+ * caller: a region of interest, foveation, refinement of pixels the caller picks.
+ *
+ * State: as vrj_render_progressive's.  out->accumulate == 0 starts from zero; otherwise colour_sum, colour_bias, weight and
+ * weight_bias (all four required) hold the state to continue, and y_sq_sum (may be NULL: not kept) its sum of Y squared.
+ * counts: one uint32 per tile pixel, row-major like the arrays; every pointer is memory of the kind out->memory says.
+ *
+ * Sampling.  Pixel p, holding n = weight[p] samples, takes its samples n .. n + counts[p] - 1: the sample indices
+ * sample_offset + k * stride, applied in sample order.  On return the four state arrays (and y_sq_sum) hold the new state;
+ * out->colour and out->srgb8 (optional) are formed for EVERY pixel of the tile (colour = colour_sum * (1/weight): NaN where
+ * the weight is 0).
+ * Guarantee: a pixel that ends with N samples holds, bit for bit, the colour_sum, colour_bias, weight and weight_bias that
+ * vrj_render_tile with spp = N gives it, and the y_sq_sum of vrj_render_adaptive / vrj_render_progressive (q = q + y * y in
+ * sample order).  An all-zero map returns the state unchanged, bit for bit.
+ * Errors: params->spp != 0 or a NULL counts: VRJ_ERR_INVALID_ARGUMENT; out->photons: VRJ_ERR_UNSUPPORTED.  A weight that is
+ * no sample count (negative, not an integer, not finite, >= 2^32; every pixel is checked), or n + counts[p] >= 2^32:
+ * VRJ_ERR_INVALID_ARGUMENT.  More than 2^32 - 1 samples in the call: VRJ_ERR_UNSUPPORTED.  In these cases nothing is
+ * rendered and the state is left as it was.
+ * cstats (host, may be NULL): samples rendered, pixels with counts[p] > 0, wavefront batches.  out->stats sums the batches.
+ * Scheduling: never coalesced; takes the device's render turn; uses a scratch block from the pool, with 24 bytes per pixel
+ * more than vrj_render_tile (vrj_render_adaptive's 20 and the map's scan) and 8 bytes per path in flight (the pixel and
+ * sample of every slot).  The host reads back 32 bytes of sums of the map before rendering. */
+typedef struct VrjCountsStats {
+    uint64_t samples;  /* rendered: the sum of counts */
+    uint64_t pixels;   /* pixels with counts[p] > 0 */
+    uint64_t batches;  /* wavefront batches */
+} VrjCountsStats;
+
+VRJ_API VrjStatus vrj_render_counts(const VrjScene *scene, const VrjTile *tile, uint64_t height, uint64_t width,
+                                    const VrjRenderParams *params, const uint32_t *counts, VrjAccumOut *out,
+                                    double *y_sq_sum, VrjCountsStats *cstats);
+
+/* vrj_plan_counts: a count map from a state's noise estimate, on the device.  Inputs: npix pixels of a state (weight,
+ * colour_sum: 3 per pixel, y_sq_sum), memory of the kind `memory` says, on `device`; `rule`: as vrj_render_adaptive's
+ * (min_samples >= 2, max_samples >= min_samples, pass_samples >= 1, rel_error > 0, abs_floor >= 0).  Output: counts[p].
+ * Per pixel, in binary64 in exactly this order, with n = weight, s = colour_sum.y, q = y_sq_sum and the m, v, t of
+ * vrj_render_adaptive's stopping rule (m = s * (1/n); v = max(0, (q - s*m) / (n - 1)); t = rel_error * max(m, abs_floor)):
+ *     n < min_samples                           ->  c = min_samples - n
+ *     n >= max_samples, or v <= t * t * n       ->  c = 0
+ *     otherwise  need = v / (t * t);  target = (need < max_samples) ? ceil(need) : max_samples   (NaN: max_samples)
+ *                c = min(max_samples - n, max(pass_samples, target - n))
+ * ceil(v / t^2) is the count at which today's variance estimate would pass the rule; pass_samples is the least an
+ * unconverged pixel takes, so an underestimate still moves.  The plan depends only on the state, so the loop
+ *     plan -> vrj_render_counts -> plan -> ...  (the first round is the uniform pilot at min_samples)
+ * ends when a plan's samples is 0, with every pixel converged or at max_samples, and any split of its rounds into calls gives
+ * the same bits.  pstats (host, may be NULL): samples (the sum of counts, so a caller can cap a round to a budget),
+ * pixels_planned (c > 0), pixels_converged and pixels_at_max (c = 0, by the rule / at max_samples without meeting it); the
+ * three pixel counts add up to npix.  Integer sums: deterministic.
+ * Errors: a NULL pointer, an invalid rule or an unknown memory kind, and a weight that is no sample count:
+ * VRJ_ERR_INVALID_ARGUMENT (counts is then left as it was).  npix >= 2^32: VRJ_ERR_UNSUPPORTED.  npix == 0: no work.
+ * Runs on a stream of its own and takes no render turn. */
+typedef struct VrjPlanStats {
+    uint64_t samples;           /* sum of counts */
+    uint64_t pixels_planned;    /* c > 0 */
+    uint64_t pixels_converged;  /* c = 0: the rule holds */
+    uint64_t pixels_at_max;     /* c = 0: n >= max_samples and the rule does not hold */
+} VrjPlanStats;
+
+VRJ_API VrjStatus vrj_plan_counts(int32_t device, uint32_t memory, uint64_t npix, const double *weight, const double *colour_sum,
+                                  const double *y_sq_sum, const VrjAdaptiveParams *rule, uint32_t *counts, VrjPlanStats *pstats);
+
 /* ---- first-hit features for a denoiser ----
  * vrj_render_aux traces params->spp (>= 1) camera rays per pixel of `tile`: the rays of samples sample_offset + k * stride,
  * k = 0 .. spp-1, with params->seed -- exactly the camera rays vrj_render_tile / vrj_render_adaptive trace with the same

@@ -155,6 +155,25 @@ impl Default for VrjProgressiveParams {
     }
 }
 
+/// What `vrj_render_counts` rendered: samples (the sum of the map), pixels with a count above 0, wavefront batches.
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct VrjCountsStats {
+    pub samples: u64,
+    pub pixels: u64,
+    pub batches: u64,
+}
+
+/// What `vrj_plan_counts` planned: samples (the sum of the map) and the pixels planned / converged / at `max_samples`.
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct VrjPlanStats {
+    pub samples: u64,
+    pub pixels_planned: u64,
+    pub pixels_converged: u64,
+    pub pixels_at_max: u64,
+}
+
 /// What `vrj_render_progressive` did (passes, samples) and the state it left: pixels converged / at `max_samples` / active.
 #[repr(C)]
 #[derive(Clone, Copy, Debug, Default)]
@@ -222,6 +241,15 @@ extern "C" {
     pub fn vrj_render_progressive(scene: *const VrjScene, tile: *const VrjTile, height: u64, width: u64,
                                   params: *const VrjRenderParams, pp: *const VrjProgressiveParams, out: *mut VrjAccumOut,
                                   y_sq_sum: *mut f64, pstats: *mut VrjProgressiveStats) -> i32;
+    /// Gives pixel p `counts[p]` new samples (its samples n .. n + counts[p] - 1, n = weight[p]) rendered in full
+    /// wavefronts, from a zero state or (`out.accumulate`) the state in `out`; `y_sq_sum` may be null; `params.spp` must be 0.
+    pub fn vrj_render_counts(scene: *const VrjScene, tile: *const VrjTile, height: u64, width: u64,
+                             params: *const VrjRenderParams, counts: *const u32, out: *mut VrjAccumOut,
+                             y_sq_sum: *mut f64, cstats: *mut VrjCountsStats) -> i32;
+    /// The count map the header's rule gives each of `npix` pixels of a state (weight, colour_sum, y_sq_sum).
+    pub fn vrj_plan_counts(device: i32, memory: u32, npix: u64, weight: *const f64, colour_sum: *const f64,
+                           y_sq_sum: *const f64, rule: *const VrjAdaptiveParams, counts: *mut u32,
+                           pstats: *mut VrjPlanStats) -> i32;
     /// First-hit normal, depth, object id and material of the camera rays a render with the same
     /// spp / seed / sample_offset / sample_stride traces.
     pub fn vrj_render_aux(scene: *const VrjScene, tile: *const VrjTile, height: u64, width: u64,

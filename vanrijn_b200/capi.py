@@ -28,7 +28,7 @@ CUDA_SYMBOLS = ["vrj_last_error", "vrj_abi_version", "vrj_device_count", "vrj_sc
                 "vrj_scene_device_bytes", "vrj_scene_upload_bytes", "vrj_render_tile", "vrj_trace_rays", "vrj_release_scratch", "vrj_alloc_host",
                 "vrj_free_host", "vrj_alloc_device", "vrj_free_device", "vrj_copy_to_host", "vrj_comm_create", "vrj_comm_destroy", "vrj_comm_scene_create", "vrj_comm_scene_destroy",
                 "vrj_render_sharded", "vrj_tone_map", "vrj_bvh_build", "vrj_render_adaptive", "vrj_render_aux", "vrj_denoise",
-                "vrj_render_progressive"]
+                "vrj_render_progressive", "vrj_render_counts", "vrj_plan_counts"]
 
 
 class VrjError(RuntimeError):
@@ -148,6 +148,20 @@ class ProgressiveStats(C.Structure):
         return {n: int(getattr(self, n)) for n, _ in self._fields_}
 
 
+class CountsStats(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("samples", "pixels", "batches")]
+
+    def as_dict(self):
+        return {n: int(getattr(self, n)) for n, _ in self._fields_}
+
+
+class PlanStats(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("samples", "pixels_planned", "pixels_converged", "pixels_at_max")]
+
+    def as_dict(self):
+        return {n: int(getattr(self, n)) for n, _ in self._fields_}
+
+
 class AuxOut(C.Structure):
     _fields_ = [("memory", C.c_uint32), ("pad", C.c_uint32), ("normal", C.c_void_p), ("depth", C.c_void_p),
                 ("object_id", C.c_void_p), ("material", C.c_void_p), ("stats", C.POINTER(Stats))]
@@ -203,6 +217,12 @@ def cuda():
         L.vrj_render_progressive.argtypes = [C.c_void_p, C.POINTER(Tile), C.c_uint64, C.c_uint64, C.POINTER(RenderParams),
                                              C.POINTER(ProgressiveParams), C.POINTER(AccumOut), C.c_void_p,
                                              C.POINTER(ProgressiveStats)]
+        L.vrj_render_counts.restype = C.c_int32
+        L.vrj_render_counts.argtypes = [C.c_void_p, C.POINTER(Tile), C.c_uint64, C.c_uint64, C.POINTER(RenderParams), C.c_void_p,
+                                        C.POINTER(AccumOut), C.c_void_p, C.POINTER(CountsStats)]
+        L.vrj_plan_counts.restype = C.c_int32
+        L.vrj_plan_counts.argtypes = [C.c_int32, C.c_uint32, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.POINTER(AdaptiveParams), C.c_void_p, C.POINTER(PlanStats)]
         L.vrj_render_aux.restype = C.c_int32
         L.vrj_render_aux.argtypes = [C.c_void_p, C.POINTER(Tile), C.c_uint64, C.c_uint64, C.POINTER(RenderParams), C.POINTER(AuxOut)]
         L.vrj_denoise.restype = C.c_int32

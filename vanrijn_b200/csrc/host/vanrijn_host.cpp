@@ -1119,7 +1119,9 @@ DeviceProgressiveBuffer::DeviceProgressiveBuffer(size_t width, size_t height, in
     colour_ = f64(3 * n), sum_ = f64(3 * n), bias_ = f64(3 * n), weight_ = f64(n), weight_bias_ = f64(n), y_sq_sum_ = f64(n);
     normal_ = f64(3 * n), depth_ = f64(n), denoised_ = f64(3 * n);
     material_ = static_cast<int32_t *>(vrj_alloc_device(device, n * 4)), srgb8_ = static_cast<uint8_t *>(vrj_alloc_device(device, 3 * n));
-    if (!colour_ || !sum_ || !bias_ || !weight_ || !weight_bias_ || !y_sq_sum_ || !normal_ || !depth_ || !denoised_ || !material_ || !srgb8_) {
+    counts_ = static_cast<uint32_t *>(vrj_alloc_device(device, n * 4));
+    if (!colour_ || !sum_ || !bias_ || !weight_ || !weight_bias_ || !y_sq_sum_ || !normal_ || !depth_ || !denoised_ || !material_ || !srgb8_ ||
+        !counts_) {
         const std::string why = vrj_last_error();
         this->~DeviceProgressiveBuffer();
         throw std::runtime_error("DeviceProgressiveBuffer: " + why);
@@ -1127,10 +1129,10 @@ DeviceProgressiveBuffer::DeviceProgressiveBuffer(size_t width, size_t height, in
 }
 DeviceProgressiveBuffer::~DeviceProgressiveBuffer() {
     for (void *p : {(void *)colour_, (void *)sum_, (void *)bias_, (void *)weight_, (void *)weight_bias_, (void *)y_sq_sum_, (void *)normal_,
-                    (void *)depth_, (void *)denoised_, (void *)material_, (void *)srgb8_})
+                    (void *)depth_, (void *)denoised_, (void *)material_, (void *)srgb8_, (void *)counts_})
         vrj_free_device(p);
     colour_ = sum_ = bias_ = weight_ = weight_bias_ = y_sq_sum_ = normal_ = depth_ = denoised_ = nullptr;
-    material_ = nullptr, srgb8_ = nullptr;
+    material_ = nullptr, srgb8_ = nullptr, counts_ = nullptr;
 }
 void DeviceProgressiveBuffer::render(const Scene &scene, const RenderOptions &o, const ProgressiveOptions &pp) {
     DeviceRenderParams dp(o);
@@ -1144,6 +1146,28 @@ void DeviceProgressiveBuffer::render(const Scene &scene, const RenderOptions &o,
     if (vrj_render_progressive(device_scene(scene, device_), &t, height_, width_, &dp.p, &vp, &out, y_sq_sum_, pp.stats) != VRJ_OK)
         throw std::runtime_error(std::string("vrj_render_progressive: ") + vrj_last_error());
     started_ = true;
+}
+VrjPlanStats DeviceProgressiveBuffer::plan_counts(const ProgressiveOptions &pp) {
+    // a buffer that has not rendered yet holds the zero state (vrj_alloc_device zero-fills): its plan is the uniform pilot
+    const VrjAdaptiveParams rule{pp.min_samples, pp.max_samples, pp.pass_samples, 0u, pp.rel_error, pp.abs_floor};
+    VrjPlanStats ps{};
+    if (vrj_plan_counts(device_, VRJ_MEM_DEVICE, width_ * height_, weight_, sum_, y_sq_sum_, &rule, counts_, &ps) != VRJ_OK)
+        throw std::runtime_error(std::string("vrj_plan_counts: ") + vrj_last_error());
+    return ps;
+}
+VrjCountsStats DeviceProgressiveBuffer::render_counts(const Scene &scene, const RenderOptions &o, const uint32_t *counts) {
+    DeviceRenderParams dp(o);
+    dp.p.spp = 0;
+    VrjTile t{0, width_, 0, height_};
+    VrjAccumOut out{};
+    out.memory = VRJ_MEM_DEVICE, out.accumulate = started_ ? 1u : 0u;
+    out.colour = colour_, out.colour_sum = sum_, out.colour_bias = bias_, out.weight = weight_, out.weight_bias = weight_bias_;
+    out.stats = o.stats;
+    VrjCountsStats cs{};
+    if (vrj_render_counts(device_scene(scene, device_), &t, height_, width_, &dp.p, counts ? counts : counts_, &out, y_sq_sum_, &cs) != VRJ_OK)
+        throw std::runtime_error(std::string("vrj_render_counts: ") + vrj_last_error());
+    started_ = true;
+    return cs;
 }
 ImageRgbU8 DeviceProgressiveBuffer::to_image_rgb_u8() const {
     ImageRgbU8 image(width_, height_);

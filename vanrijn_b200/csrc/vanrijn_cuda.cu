@@ -33,12 +33,12 @@ thread_local std::string g_error;
 
 // the six instantiations live in vrj_batch_inst.cu (one object file each)
 namespace vrjimpl {
-extern template VrjStatus run_batch<float, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
-extern template VrjStatus run_batch<float, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
-extern template VrjStatus run_batch<double, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
-extern template VrjStatus run_batch<double, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
-extern template VrjStatus run_batch<float, float, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
-extern template VrjStatus run_batch<float, float, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *);
+extern template VrjStatus run_batch<float, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
+extern template VrjStatus run_batch<float, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
+extern template VrjStatus run_batch<double, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
+extern template VrjStatus run_batch<double, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
+extern template VrjStatus run_batch<float, float, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
+extern template VrjStatus run_batch<float, float, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
 } // namespace vrjimpl
 // NVTX ranges (SURVEY section 5) through the header-only NVTX 3: no library to link or load -- the calls are no-ops until a
 // tool (ncu --nvtx, nsys) injects itself
@@ -599,11 +599,12 @@ bool call_wants_records(const VrjScene *scene, const VrjRenderParams *p, uint32_
     return p->precision == VRJ_PRECISION_F64 && filter == VRJ_FILTER_F32 && scene->trace_records && scene->dev.n_bvh_items > 0;
 }
 
-// the block for batches of *batch samples of npix pixels
-VrjStatus ensure_call_scratch(Scratch *s, const VrjRenderParams *p, bool records, uint64_t npix, uint32_t *batch, size_t n_light_samples) {
+// the block for accumulators of npix pixels and batches of *batch units of `unit` paths each (a tile's batch: samples of
+// unit = npix pixels; vrj_render_counts: unit = 1 path per slot)
+VrjStatus ensure_call_scratch(Scratch *s, const VrjRenderParams *p, bool records, uint64_t npix, uint64_t unit, uint32_t *batch, size_t n_light_samples) {
     bool queue_oom = false;
     auto ensure = [&] {
-        return ensure_scratch(s, npix * *batch, records ? npix * *batch : 0, npix, p->max_depth + 3, p->n_lights, n_light_samples, &queue_oom);
+        return ensure_scratch(s, unit * *batch, records ? unit * *batch : 0, npix, p->max_depth + 3, p->n_lights, n_light_samples, &queue_oom);
     };
     VrjStatus st = ensure();
     while (st == VRJ_ERR_OUT_OF_MEMORY && queue_oom && *batch > 1) { // 240 bytes per path in flight: halve the batch until the queues fit
@@ -643,19 +644,19 @@ VrjStatus stage_lights(Scratch *s, const VrjRenderParams *p) {
 
 // one batch in the kernel variant the call's precision, walk and counting select
 VrjStatus dispatch_batch(const VrjScene *scene, Scratch *s, const RenderConst &rc, const VrjRenderParams *p, uint32_t filter, uint64_t *launches,
-                         const MultiCalls *multi, const ResolveCopy *copy, double *ysq) {
+                         const MultiCalls *multi, const ResolveCopy *copy, double *ysq, const CountsBatch *counts = nullptr) {
     const bool whitted = p->integrator == VRJ_INTEGRATOR_WHITTED;
     // F32X4: the staged rays walk the 4-wide tree; inline any-hit queries (Whitted shadow rays, k_tail) use the 2-wide f32 tree
     const int quad = filter == VRJ_FILTER_F32X4 ? 1 : filter == VRJ_FILTER_Q16 ? 2 : 0;
     // VRJ_PRECISION_F32_FAST: the whole sample in binary32 over the 2-wide f32 tree (no reference counterpart; not a parity mode)
     const bool fast = p->precision == VRJ_PRECISION_F32_FAST;
     if (p->count_traversal)
-        return fast ? run_batch<float, float, true>(scene, s, rc, whitted, 0, launches, multi, copy, ysq)
-             : filter == VRJ_FILTER_F64 ? run_batch<double, double, true>(scene, s, rc, whitted, 0, launches, multi, copy, ysq)
-                                        : run_batch<float, double, true>(scene, s, rc, whitted, quad, launches, multi, copy, ysq);
-    return fast ? run_batch<float, float, false>(scene, s, rc, whitted, 0, launches, multi, copy, ysq)
-         : filter == VRJ_FILTER_F64 ? run_batch<double, double, false>(scene, s, rc, whitted, 0, launches, multi, copy, ysq)
-                                    : run_batch<float, double, false>(scene, s, rc, whitted, quad, launches, multi, copy, ysq);
+        return fast ? run_batch<float, float, true>(scene, s, rc, whitted, 0, launches, multi, copy, ysq, counts)
+             : filter == VRJ_FILTER_F64 ? run_batch<double, double, true>(scene, s, rc, whitted, 0, launches, multi, copy, ysq, counts)
+                                        : run_batch<float, double, true>(scene, s, rc, whitted, quad, launches, multi, copy, ysq, counts);
+    return fast ? run_batch<float, float, false>(scene, s, rc, whitted, 0, launches, multi, copy, ysq, counts)
+         : filter == VRJ_FILTER_F64 ? run_batch<double, double, false>(scene, s, rc, whitted, 0, launches, multi, copy, ysq, counts)
+                                    : run_batch<float, double, false>(scene, s, rc, whitted, quad, launches, multi, copy, ysq, counts);
 }
 
 // VrjStats of a call from its counters and the boundary events run_levels recorded
@@ -712,9 +713,9 @@ VrjStatus load_state(Scratch *s, const Arr *arrs, int n, bool load, cudaMemcpyKi
     return VRJ_OK;
 }
 
-// What every render call (vrj_render_tile, render_passes) does around its kernels.  prepare(): a block from the pool for
-// batches of up to `widest` samples of the tile; start(): the call's counters, lights and constants, the render turn and
-// ev0; finish(): ev1, the counters, the copies of the outputs and the sRGB preview, the waits, VrjStats.  `turn` is declared
+// What every render call (vrj_render_tile, render_passes, vrj_render_counts) does around its kernels.  prepare(): a block from
+// the pool for batches of up to `widest` samples of the tile (prepare_paths: of up to `widest` units of `unit` paths);
+// start(): the call's counters, lights and constants, the render turn and ev0;finish(): ev1, the counters, the copies of the outputs and the sRGB preview, the waits, VrjStats.  `turn` is declared
 // after `block`: an early return gives the turn back before the block.
 struct RenderCall {
     VrjScene *scene;
@@ -731,12 +732,13 @@ struct RenderCall {
     std::chrono::steady_clock::time_point t_start, t_enqueued, t_done; // turn taken, last copy enqueued, copies arrived
     RenderCall(VrjScene *sc, const VrjRenderParams *params, uint64_t n) : scene(sc), p(params), npix(n), block{sc}, turn(sc->device) {}
 
-    VrjStatus prepare(uint32_t widest, const ActiveCall &active, size_t n_light_samples) {
-        batch = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(widest, call_path_budget(scene, active) / npix));
-        if (npix * (uint64_t)batch > 0xfffffff0ull) return fail(VRJ_ERR_UNSUPPORTED, "tile too large");
-        s = block.s = acquire_scratch(scene, npix * batch);
+    VrjStatus prepare(uint32_t widest, const ActiveCall &active, size_t n_light_samples) { return prepare_paths(npix, widest, active, n_light_samples); }
+    VrjStatus prepare_paths(uint64_t unit, uint32_t widest, const ActiveCall &active, size_t n_light_samples) {
+        batch = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(widest, call_path_budget(scene, active) / unit));
+        if (unit * (uint64_t)batch > 0xfffffff0ull) return fail(VRJ_ERR_UNSUPPORTED, "tile too large");
+        s = block.s = acquire_scratch(scene, unit * batch);
         filter = effective_filter(scene, p);
-        return ensure_call_scratch(s, p, call_wants_records(scene, p, filter), npix, &batch, n_light_samples);
+        return ensure_call_scratch(s, p, call_wants_records(scene, p, filter), npix, unit, &batch, n_light_samples);
     }
     VrjStatus start(const VrjTile *tile, uint64_t height, uint64_t width) {
         VRJ_CUDA(cudaMemsetAsync(s->stats.p, 0, ST_COUNT * sizeof(unsigned long long), s->stream));
@@ -777,23 +779,28 @@ struct RenderCall {
     }
 };
 
-// y_sq_sum, two pixel lists, the first samples of one and the selects' counters for npix pixels (render_passes)
-VrjStatus ensure_pass_buffers(Scratch *s, uint64_t npix) {
-    if (s->pass_npix >= npix) return VRJ_OK;
-    s->pass_npix = 0;
+// y_sq_sum, two pixel lists, the first samples of one and the selects' counters for npix pixels (render_passes); with
+// slots > 0 (vrj_render_counts) also the scan of the count map (npix + 1 values and the scan's scratch), its counters, and
+// a pixel and a first sample for each of `slots` paths in flight: 8 bytes per path
+VrjStatus ensure_pass_buffers(Scratch *s, uint64_t npix, uint64_t slots = 0) {
+    if (s->pass_npix >= npix && s->pass_slots >= slots) return VRJ_OK;
+    npix = std::max<uint64_t>(npix, s->pass_npix), slots = std::max<uint64_t>(slots, s->pass_slots);
+    s->pass_npix = 0, s->pass_slots = 0;
     std::vector<std::pair<DeviceBuffer *, size_t>> want = {{&s->ysq, npix * 8}, {&s->pass_list[0], npix * 4}, {&s->pass_list[1], npix * 4},
                                                            {&s->pass_base, npix * 4}, {&s->pass_counters, sizeof(ProgressiveCounters)}};
+    if (slots)
+        want.insert(want.end(), {{&s->count_offset, (npix + npix / 2048 + 4) * 4}, {&s->count_counters, sizeof(CountsCounters)},
+                                 {&s->slot_pixel, slots * 4}, {&s->slot_base, slots * 4}});
     const VrjStatus st = alloc_group(s->pass_slab, want, "adaptive sampling buffers");
     if (st != VRJ_OK) return st;
-    s->pass_npix = npix;
+    s->pass_npix = npix, s->pass_slots = slots;
     return VRJ_OK;
 }
 
 // the fields VrjAdaptiveParams and VrjProgressiveParams share, and params->spp, which must be 0
 template <typename P>
-VrjStatus check_pass_rule(const VrjRenderParams *p, const P *ap, const char *call, const char *type, PassRule *rule) {
+VrjStatus check_rule(const P *ap, PassRule *rule) {
     if (!ap) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
-    if (p->spp != 0) return fail(VRJ_ERR_INVALID_ARGUMENT, std::string("params->spp must be 0: ") + call + " takes its sample counts from " + type);
     if (ap->min_samples < 2) return fail(VRJ_ERR_INVALID_ARGUMENT, "min_samples must be >= 2 (the variance needs two samples)");
     if (ap->max_samples < ap->min_samples) return fail(VRJ_ERR_INVALID_ARGUMENT, "max_samples must be >= min_samples");
     if (ap->pass_samples < 1) return fail(VRJ_ERR_INVALID_ARGUMENT, "pass_samples must be >= 1");
@@ -801,6 +808,12 @@ VrjStatus check_pass_rule(const VrjRenderParams *p, const P *ap, const char *cal
     if (!(ap->abs_floor >= 0.0) || !std::isfinite(ap->abs_floor)) return fail(VRJ_ERR_INVALID_ARGUMENT, "abs_floor must be >= 0 and finite");
     *rule = PassRule{ap->min_samples, ap->max_samples, ap->pass_samples, 0u, ap->rel_error, ap->abs_floor};
     return VRJ_OK;
+}
+template <typename P>
+VrjStatus check_pass_rule(const VrjRenderParams *p, const P *ap, const char *call, const char *type, PassRule *rule) {
+    if (!ap) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (p->spp != 0) return fail(VRJ_ERR_INVALID_ARGUMENT, std::string("params->spp must be 0: ") + call + " takes its sample counts from " + type);
+    return check_rule(ap, rule);
 }
 
 struct PassResult {
@@ -935,6 +948,115 @@ VrjStatus render_passes(VrjScene *scene, const VrjTile *tile, uint64_t height, u
     if (st != VRJ_OK) return st;
     res->counts = *hctr;
     return VRJ_OK;
+}
+
+// a stream and two events of a call's own (vrj_render_aux, vrj_denoise, vrj_plan_counts, the sums of a device count map:
+// short calls that take no render turn and no scratch block).  Declared after the call's DeviceBuffers: nothing may still
+// use them when they return to the pool.
+struct CallStream {
+    cudaStream_t s = nullptr;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    cudaError_t create() {
+        cudaError_t e = cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking);
+        if (e == cudaSuccess) e = cudaEventCreate(&e0);
+        if (e == cudaSuccess) e = cudaEventCreate(&e1);
+        return e;
+    }
+    ~CallStream() {
+        if (s) cudaStreamSynchronize(s), cudaStreamDestroy(s);
+        if (e0) cudaEventDestroy(e0);
+        if (e1) cudaEventDestroy(e1);
+    }
+};
+
+// vrj_render_counts (the header states it) on a tile of npix >= 1 pixels.  The count map goes into the block, and
+// k_counts_check sums it exactly in 64 bits and checks the state before anything is rendered: a refused call has written
+// nothing the caller sees.  The exclusive scan of the map (vrj_build::exclusive_scan_u32) gives each pixel its run of slots;
+// the call's samples are then rendered as wavefronts of up to the path budget's slots, each one sample (batch_samples = 1)
+// of the LIST kernels: k_counts_expand lists the (pixel, sample) of every slot of the batch and k_resolve_counts applies the
+// batch to the accumulators and y_sq_sum.  Batches are resolved in order, so a pixel's run that straddles two of them is
+// still applied in sample order.  colour comes from k_finalize.
+VrjStatus render_counts(VrjScene *scene, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p, const uint32_t *counts,
+                        size_t n_light_samples, VrjAccumOut *out, double *y_sq_sum, VrjCountsStats *cstats) {
+    const uint64_t npix = (tile->end_column - tile->start_column) * (tile->end_row - tile->start_row);
+    const uint32_t n32 = (uint32_t)npix;
+    // the map's total sizes the block: a batch is at most the path budget's slots, and no more than the call renders
+    uint64_t total = 0;
+    if (out->memory == VRJ_MEM_HOST) {
+        for (uint64_t i = 0; i < npix; i++) total += counts[i];
+    } else {
+        DeviceBuffer sums;
+        VRJ_CUDA(sums.alloc(sizeof(CountsCounters)));
+        CallStream cs;
+        VRJ_CUDA(cs.create());
+        CountsCounters h{};
+        VRJ_CUDA(cudaMemsetAsync(sums.p, 0, sizeof(CountsCounters), cs.s));
+        k_counts_check<<<(n32 + 255) / 256, 256, 0, cs.s>>>(nullptr, counts, n32, nullptr, sums.as<CountsCounters>());
+        VRJ_CUDA(cudaGetLastError());
+        VRJ_CUDA(cudaMemcpyAsync(&h, sums.p, sizeof(CountsCounters), cudaMemcpyDeviceToHost, cs.s));
+        VRJ_CUDA(cudaStreamSynchronize(cs.s));
+        total = h.samples;
+    }
+    if (total > 0xffffffffull) return fail(VRJ_ERR_UNSUPPORTED, "more than 2^32 - 1 samples in one call");
+    ActiveCall active(g_active_calls[(unsigned)scene->device % 64]);
+    RenderCall call(scene, p, npix);
+    VrjStatus st = call.prepare_paths(1, (uint32_t)std::min<uint64_t>(std::max<uint64_t>(total, 1), 0xffffffffull), active, n_light_samples);
+    if (st != VRJ_OK) return st;
+    Scratch *s = call.s;
+    st = ensure_pass_buffers(s, npix, call.batch);
+    if (st != VRJ_OK) return st;
+    const cudaMemcpyKind in_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    const cudaMemcpyKind out_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    const Arr arrs[6] = {{out->colour, &s->acc_colour, 3}, {out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3},
+                         {out->weight, &s->acc_weight, 1}, {out->weight_bias, &s->acc_wbias, 1}, {y_sq_sum, &s->ysq, 1}};
+    st = load_state(s, arrs + 1, 5, out->accumulate != 0, in_kind, npix);
+    if (st != VRJ_OK) return st;
+    uint32_t *offset = s->count_offset.as<uint32_t>(), *held = s->pass_base.as<uint32_t>();
+    CountsCounters *ctr = s->count_counters.as<CountsCounters>(), *hctr = &s->pinned->counts;
+    VRJ_CUDA(cudaMemcpyAsync(offset, counts, npix * sizeof(uint32_t), in_kind, s->stream));
+    VRJ_CUDA(cudaMemsetAsync(offset + npix, 0, sizeof(uint32_t), s->stream));
+    VRJ_CUDA(cudaMemsetAsync(ctr, 0, sizeof(CountsCounters), s->stream));
+    k_counts_check<<<(n32 + 255) / 256, 256, 0, s->stream>>>(s->acc_weight.as<double>(), offset, n32, held, ctr);
+    VRJ_CUDA(cudaGetLastError());
+    VRJ_CUDA(cudaMemcpyAsync(hctr, ctr, sizeof(CountsCounters), cudaMemcpyDeviceToHost, s->stream));
+    VRJ_CUDA(cudaStreamSynchronize(s->stream));
+    if (hctr->bad) return fail(VRJ_ERR_INVALID_ARGUMENT, "a weight of the state is not a sample count (negative, fractional, not finite or >= 2^32)");
+    if (hctr->over) return fail(VRJ_ERR_INVALID_ARGUMENT, "a pixel would hold 2^32 samples or more (weight + count)");
+    total = hctr->samples;
+    if (cstats) cstats->samples = total, cstats->pixels = hctr->pixels;
+    call.launches = 1; // k_counts_check
+    st = call.start(tile, height, width);
+    if (st != VRJ_OK) return st;
+
+    RenderConst &rc = call.rc;
+    double *ysq = s->ysq.as<double>();
+    if (total) {
+        st = vrj_build::exclusive_scan_u32(offset, n32 + 1, offset + npix + 1, s->stream);
+        if (st != VRJ_OK) return st;
+        call.launches += 3;
+        uint32_t *slot_pixel = s->slot_pixel.as<uint32_t>(), *slot_base = s->slot_base.as<uint32_t>();
+        rc.batch_samples = 1, rc.div_batch = FastDiv::make(1);
+        rc.first_sample = p->sample_offset;
+        rc.pixel_list = slot_pixel, rc.pixel_base = slot_base;
+        uint64_t batches = 0;
+        for (uint64_t b0 = 0; b0 < total; b0 += call.batch, batches++) {
+            const uint32_t b1 = (uint32_t)std::min<uint64_t>(total, b0 + call.batch), m = b1 - (uint32_t)b0;
+            k_counts_expand<<<(m + 255) / 256, 256, 0, s->stream>>>(offset, held, n32, (uint32_t)b0, b1, slot_pixel, slot_base);
+            call.launches++;
+            VRJ_CUDA(cudaGetLastError());
+            rc.npix = m;
+            const CountsBatch cb{offset, n32, (uint32_t)b0, b1};
+            st = dispatch_batch(scene, s, rc, p, call.filter, &call.launches, nullptr, nullptr, ysq, &cb);
+            if (st != VRJ_OK) return st;
+        }
+        if (cstats) cstats->batches = batches;
+    }
+    if (out->colour || out->srgb8) {
+        k_finalize<<<(n32 + 255) / 256, 256, 0, s->stream>>>(s->acc_sum.as<double>(), s->acc_weight.as<double>(), s->acc_colour.as<double>(), n32);
+        call.launches++;
+        VRJ_CUDA(cudaGetLastError());
+    }
+    return call.finish(arrs, 6, out->srgb8, out_kind, out->stats);
 }
 
 // ---------------------------------------------------------------------------------------------- coalesced calls
@@ -1748,23 +1870,73 @@ VrjStatus vrj_render_progressive(const VrjScene *scene_c, const VrjTile *tile, u
     return VRJ_OK;
 }
 
-// a stream and two events of a call's own (vrj_render_aux, vrj_denoise: short calls that take no render turn and no scratch
-// block).  Declared after the call's DeviceBuffers: nothing may still use them when they return to the pool.
-struct CallStream {
-    cudaStream_t s = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    cudaError_t create() {
-        cudaError_t e = cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking);
-        if (e == cudaSuccess) e = cudaEventCreate(&e0);
-        if (e == cudaSuccess) e = cudaEventCreate(&e1);
-        return e;
+// Per-pixel sample counts in full wavefronts (the header states the call): render_counts on the caller's state.
+VrjStatus vrj_render_counts(const VrjScene *scene_c, const VrjTile *tile, uint64_t height, uint64_t width, const VrjRenderParams *p,
+                            const uint32_t *counts, VrjAccumOut *out, double *y_sq_sum, VrjCountsStats *cstats) {
+    VrjScene *scene = const_cast<VrjScene *>(scene_c);
+    size_t n_light_samples = 0;
+    VrjStatus st = check_render_args(scene, tile, height, width, p, out, &n_light_samples);
+    if (st != VRJ_OK) return st;
+    if (p->spp != 0) return fail(VRJ_ERR_INVALID_ARGUMENT, "params->spp must be 0: vrj_render_counts takes its sample counts from `counts`");
+    if (out->memory > VRJ_MEM_DEVICE) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown memory kind");
+    if (out->accumulate && (!out->colour_sum || !out->colour_bias || !out->weight || !out->weight_bias))
+        return fail(VRJ_ERR_INVALID_ARGUMENT, "a continued state (accumulate) needs colour_sum, colour_bias, weight and weight_bias");
+    if (out->photons) return fail(VRJ_ERR_UNSUPPORTED, "vrj_render_counts has no photons output");
+    const uint64_t npix = (tile->end_column - tile->start_column) * (tile->end_row - tile->start_row);
+    if (npix && !counts) return fail(VRJ_ERR_INVALID_ARGUMENT, "counts is NULL");
+    DeviceGuard device_guard;
+    VRJ_NVTX_RANGE(call_range, "vrj_render_counts");
+    if (out->stats) std::memset(out->stats, 0, sizeof(VrjStats));
+    if (cstats) std::memset(cstats, 0, sizeof(VrjCountsStats));
+    if (npix == 0) return VRJ_OK;
+    VRJ_CUDA(cudaSetDevice(scene->device));
+    return render_counts(scene, tile, height, width, p, counts, n_light_samples, out, y_sq_sum, cstats);
+}
+
+// The planner (the header states the rule): k_plan_counts, one thread per pixel, on a stream of its own.  The counts go to a
+// pooled buffer first and reach the caller only when every weight was a sample count.
+VrjStatus vrj_plan_counts(int32_t device, uint32_t memory, uint64_t npix, const double *weight, const double *colour_sum, const double *y_sq_sum,
+                          const VrjAdaptiveParams *rule, uint32_t *counts, VrjPlanStats *pstats) {
+    PassRule r;
+    VrjStatus st = check_rule(rule, &r);
+    if (st != VRJ_OK) return st;
+    if (memory > VRJ_MEM_DEVICE) return fail(VRJ_ERR_INVALID_ARGUMENT, "unknown memory kind");
+    if (pstats) std::memset(pstats, 0, sizeof(VrjPlanStats));
+    if (npix == 0) return VRJ_OK;
+    if (!weight || !colour_sum || !y_sq_sum || !counts) return fail(VRJ_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (npix > 0xffffffffull) return fail(VRJ_ERR_UNSUPPORTED, "more than 2^32 - 1 pixels");
+    const uint32_t n32 = (uint32_t)npix;
+    DeviceGuard device_guard;
+    VRJ_NVTX_RANGE(call_range, "vrj_plan_counts");
+    VRJ_CUDA(cudaSetDevice(device));
+    DeviceBuffer d_in[3], d_counts, d_ctr;
+    const void *src[3] = {weight, colour_sum, y_sq_sum};
+    const size_t per[3] = {8, 24, 8};
+    const bool host = memory == VRJ_MEM_HOST;
+    if (host)
+        for (int i = 0; i < 3; i++) VRJ_CUDA(d_in[i].alloc(npix * per[i]));
+    VRJ_CUDA(d_counts.alloc(npix * 4));
+    VRJ_CUDA(d_ctr.alloc(5 * sizeof(unsigned long long)));
+    CallStream cs;
+    VRJ_CUDA(cs.create());
+    if (host) {
+        for (int i = 0; i < 3; i++) VRJ_CUDA(cudaMemcpyAsync(d_in[i].p, src[i], npix * per[i], cudaMemcpyHostToDevice, cs.s));
+        for (int i = 0; i < 3; i++) src[i] = d_in[i].p;
     }
-    ~CallStream() {
-        if (s) cudaStreamSynchronize(s), cudaStreamDestroy(s);
-        if (e0) cudaEventDestroy(e0);
-        if (e1) cudaEventDestroy(e1);
-    }
-};
+    unsigned long long h[5] = {0, 0, 0, 0, 0};
+    VRJ_CUDA(cudaMemsetAsync(d_ctr.p, 0, 5 * sizeof(unsigned long long), cs.s));
+    k_plan_counts<<<(n32 + 255) / 256, 256, 0, cs.s>>>(static_cast<const double *>(src[0]), static_cast<const double *>(src[1]),
+                                                       static_cast<const double *>(src[2]), n32, r, d_counts.as<uint32_t>(), d_ctr.as<unsigned long long>());
+    VRJ_CUDA(cudaGetLastError());
+    VRJ_CUDA(cudaMemcpyAsync(h, d_ctr.p, sizeof(h), cudaMemcpyDeviceToHost, cs.s));
+    VRJ_CUDA(cudaStreamSynchronize(cs.s));
+    if (h[4]) return fail(VRJ_ERR_INVALID_ARGUMENT, "a weight of the state is not a sample count (negative, fractional, not finite or >= 2^32)");
+    VRJ_CUDA(cudaMemcpyAsync(counts, d_counts.p, npix * 4, host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, cs.s));
+    VRJ_CUDA(cudaStreamSynchronize(cs.s));
+    if (pstats) pstats->samples = h[0], pstats->pixels_planned = h[1], pstats->pixels_converged = h[2], pstats->pixels_at_max = h[3];
+    return VRJ_OK;
+}
+
 
 // First-hit features (the header states them): k_aux, one thread per pixel, forms each pixel's camera rays from the render's
 // RenderConst.  Like vrj_trace_rays it runs on a stream of its own and takes no render turn.

@@ -77,6 +77,14 @@ struct PinnedBlock {
     unsigned long long stats[ST_COUNT];         // the call's ray counters
     ProgressiveCounters pass;                   // render_passes: the last select's counters
     uint32_t listed;                            // render_passes: the length of a sub-pass's pixel list
+    CountsCounters counts;                      // vrj_render_counts: what k_counts_check found
+};
+
+// One batch of vrj_render_counts: slots [b0, b1) of the call, slot j being one sample of the tile pixel whose run of the
+// exclusive scan `offset` (npix + 1 entries) holds it; k_resolve_counts applies them.
+struct CountsBatch {
+    const uint32_t *offset;
+    uint32_t npix, b0, b1;
 };
 
 // per-call scratch: path queues, photon results, accumulators, counters
@@ -94,7 +102,10 @@ struct Scratch {
     DeviceBuffer lights, light_samples, srgb8;
     // render_passes: y_sq_sum, the previous / next pass's pixel list, the next pass's first samples, the selects' counters
     DeviceBuffer ysq, pass_list[2], pass_base, pass_counters, pass_slab;
-    size_t pass_npix = 0;
+    // vrj_render_counts, in the same slab: the scan of the count map and its counters (per pixel), and the pixel and first
+    // sample of every slot of a batch (per path in flight)
+    DeviceBuffer count_offset, count_counters, slot_pixel, slot_base;
+    size_t pass_npix = 0, pass_slots = 0;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr; // first / last kernel of a call
     cudaEvent_t ev_done = nullptr;             // behind the call's last copy
@@ -199,7 +210,7 @@ inline bool wants_records(const VrjScene *sc, int walk) {
 // One batch with the integrator (WHITTED) and the scene's material kinds (MM, see vrj_device.cuh) fixed at compile time.
 template <typename NT, typename R, bool COUNT, bool WHITTED, int MM, bool LIST>
 VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int walk, uint64_t *launches, const MultiCalls *multi,
-                     const ResolveCopy *copy, double *ysq) {
+                     const ResolveCopy *copy, double *ysq, const CountsBatch *counts) {
     const bool quad = walk == 1, q16 = walk == 2; // 0: the 2-wide tree in NT boxes; 1: 4-wide f32; 2: 2-wide on the 16-bit grid
     // launch sequence: G T S_0 [X_k T_k S_k]*, k = 1..levels (X = k_tail, a no-op until the queue is short);
     // SimpleRandom needs max_depth levels, Whitted one more (its limit-0 level still shades and traces);
@@ -298,7 +309,10 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
     AccumDev acc;
     acc.colour = s->acc_colour.as<double>(), acc.sum = s->acc_sum.as<double>(), acc.bias = s->acc_bias.as<double>();
     acc.weight = s->acc_weight.as<double>(), acc.weight_bias = s->acc_wbias.as<double>();
-    if (multi) {
+    if (counts) {
+        k_resolve_counts<R><<<(counts->npix + 255) / 256, 256, 0, s->stream>>>(acc, ysq, counts->offset, photons, counts->npix, counts->b0, counts->b1);
+        (*launches)++;
+    } else if (multi) {
         k_resolve_multi<R><<<(rc.npix * multi->n + 255) / 256, 256, 0, s->stream>>>(*multi, photons, rc.npix, rc.batch_samples);
         (*launches)++;
     } else if (ysq) {
@@ -334,21 +348,21 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
 // "any material"; VRJ_MATERIAL_MASK=15 in the environment forces the general variant (experiments)
 template <typename NT, typename R, bool COUNT, bool LIST>
 VrjStatus run_materials(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches, const MultiCalls *multi,
-                        const ResolveCopy *copy, double *ysq) {
+                        const ResolveCopy *copy, double *ysq, const CountsBatch *counts) {
     const bool lambert_only = sc->kernel_material_mask == 1u;
     if (whitted)
-        return lambert_only ? run_levels<NT, R, COUNT, true, 1, LIST>(sc, s, rc, walk, launches, multi, copy, ysq)
-                            : run_levels<NT, R, COUNT, true, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches, multi, copy, ysq);
-    return lambert_only ? run_levels<NT, R, COUNT, false, 1, LIST>(sc, s, rc, walk, launches, multi, copy, ysq)
-                        : run_levels<NT, R, COUNT, false, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches, multi, copy, ysq);
+        return lambert_only ? run_levels<NT, R, COUNT, true, 1, LIST>(sc, s, rc, walk, launches, multi, copy, ysq, counts)
+                            : run_levels<NT, R, COUNT, true, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches, multi, copy, ysq, counts);
+    return lambert_only ? run_levels<NT, R, COUNT, false, 1, LIST>(sc, s, rc, walk, launches, multi, copy, ysq, counts)
+                        : run_levels<NT, R, COUNT, false, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches, multi, copy, ysq, counts);
 }
-// `ysq` (render_passes): the batch is resolved by k_resolve_adaptive, which also keeps y_sq_sum; a batch over rc.pixel_list
-// (and rc.pixel_base) runs the LIST variants of the kernels
+// `ysq` (render_passes): the batch is resolved by k_resolve_adaptive, which also keeps y_sq_sum; with `counts` as well
+// (vrj_render_counts) by k_resolve_counts.  A batch over rc.pixel_list (and rc.pixel_base) runs the LIST variants of the kernels
 template <typename NT, typename R, bool COUNT>
 VrjStatus run_batch(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches, const MultiCalls *multi = nullptr,
-                    const ResolveCopy *copy = nullptr, double *ysq = nullptr) {
-    return rc.pixel_list ? run_materials<NT, R, COUNT, true>(sc, s, rc, whitted, walk, launches, multi, copy, ysq)
-                         : run_materials<NT, R, COUNT, false>(sc, s, rc, whitted, walk, launches, multi, copy, ysq);
+                    const ResolveCopy *copy = nullptr, double *ysq = nullptr, const CountsBatch *counts = nullptr) {
+    return rc.pixel_list ? run_materials<NT, R, COUNT, true>(sc, s, rc, whitted, walk, launches, multi, copy, ysq, counts)
+                         : run_materials<NT, R, COUNT, false>(sc, s, rc, whitted, walk, launches, multi, copy, ysq, counts);
 }
 
 } // namespace vrjimpl

@@ -829,18 +829,25 @@ struct PassRule {
 // The stopping rule in the order the header states it, so a caller can replay it bit for bit: n = weight, s = colour_sum.y,
 // q = y_sq_sum, m = s / n (as s * (1/n)), v = max(0, (q - s m) / (n - 1)), t = rel_error * max(m, abs_floor); converged iff
 // v <= t t n.  A NaN anywhere fails the comparison: such a pixel keeps sampling.
-__device__ __forceinline__ bool adaptive_converged(double w, double s, double q, double rel_error, double abs_floor) {
+__device__ __forceinline__ void adaptive_estimate(double w, double s, double q, double rel_error, double abs_floor, double &v, double &t) {
     const double m = s * (1.0 / w);
-    double v = (q - s * m) / (w - 1.0);
+    v = (q - s * m) / (w - 1.0);
     if (v < 0.0) v = 0.0;
-    const double t = rel_error * (m > abs_floor ? m : abs_floor);
+    t = rel_error * (m > abs_floor ? m : abs_floor);
+}
+__device__ __forceinline__ bool adaptive_converged(double w, double s, double q, double rel_error, double abs_floor) {
+    double v, t;
+    adaptive_estimate(w, s, q, rel_error, abs_floor, v, t);
     return v <= t * t * w;
 }
+
+// a weight that is a sample count: not negative, an integer, finite and below 2^32 (NaN is none)
+__device__ __forceinline__ bool is_sample_count(double w) { return (w >= 0.0 && w < 4294967296.0) && w == floor(w); }
 
 // The samples a pixel with state (w, s, q) takes in the coming pass; 0 when it is not active, and then `conv` / `at_max` say
 // why.  A weight that is no sample count (negative, fractional, not finite, >= 2^32) sets `bad` and takes nothing.
 __device__ __forceinline__ uint32_t pass_count(const PassRule &r, double w, double s, double q, bool &conv, bool &at_max, bool &bad) {
-    if (!(w >= 0.0 && w < 4294967296.0) || w != floor(w)) {
+    if (!is_sample_count(w)) {
         bad = true;
         return 0;
     }
@@ -851,6 +858,31 @@ __device__ __forceinline__ uint32_t pass_count(const PassRule &r, double w, doub
     if (rule) conv = true;
     else at_max = true;
     return 0;
+}
+
+// vrj_plan_counts (the header states the rule): the samples a pixel with state (w, s, q) takes to reach the count at which
+// today's variance estimate would pass the stopping rule (v <= t t n  <=>  n >= v / t^2), at least pass_samples while it is
+// unconverged and below max_samples.  `conv`, `at_max` and `bad` as in pass_count.
+__device__ __forceinline__ uint32_t plan_count(const PassRule &r, double w, double s, double q, bool &conv, bool &at_max, bool &bad) {
+    if (!is_sample_count(w)) {
+        bad = true;
+        return 0;
+    }
+    const uint32_t held = (uint32_t)w;
+    if (held < r.min_samples) return r.min_samples - held;
+    const bool rule = adaptive_converged(w, s, q, r.rel_error, r.abs_floor);
+    if (held >= r.max_samples || rule) {
+        if (rule) conv = true;
+        else at_max = true;
+        return 0;
+    }
+    double v, t;
+    adaptive_estimate(w, s, q, r.rel_error, r.abs_floor, v, t);
+    const double need = v / (t * t);
+    const double target = need < (double)r.max_samples ? ceil(need) : (double)r.max_samples; // NaN: max_samples
+    const double extra = target - (double)held;
+    const uint32_t c = extra > (double)r.pass_samples ? (uint32_t)extra : r.pass_samples;
+    return min(r.max_samples - held, c);
 }
 
 // What the selects of a call report to the host.  A pixel found inactive stays so for the rest of the call (its state no
@@ -932,6 +964,116 @@ static __global__ void k_progressive_compact(const uint32_t *list, const double 
         const uint32_t p = list ? list[i] : i;
         out[offset[i]] = p, base[offset[i]] = (uint32_t)weight[p];
     }
+}
+
+// ---- vrj_render_counts and vrj_plan_counts (vanrijn_cuda.cu, render_counts; the header states both) ----
+// K 64-bit sums over the block into dst[0..K); every thread of the block calls it
+template <int K>
+__device__ __forceinline__ void block_add_u64(unsigned long long (&v)[K], unsigned long long *dst) {
+    __shared__ unsigned long long part[K][32];
+    const uint32_t full = 0xffffffffu, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int k = 0; k < K; k++) {
+        for (int o = 16; o; o >>= 1) v[k] += __shfl_xor_sync(full, v[k], o);
+        if (lane == 0) part[k][warp] = v[k];
+    }
+    __syncthreads();
+    if (warp != 0) return;
+#pragma unroll
+    for (int k = 0; k < K; k++) {
+        unsigned long long x = lane < (blockDim.x >> 5) ? part[k][lane] : 0ull;
+        for (int o = 16; o; o >>= 1) x += __shfl_xor_sync(full, x, o);
+        if (lane == 0 && x) atomicAdd(dst + k, x);
+    }
+}
+
+// what k_counts_check reports: samples (the exact 64-bit total), pixels with c > 0, weights that are no sample count, and
+// pixels whose n + c reaches 2^32
+struct CountsCounters {
+    unsigned long long samples, pixels, bad, over;
+};
+
+// One thread per tile pixel: checks the state and the count map before anything is rendered, and keeps each pixel's
+// starting count n in `held` (the state changes while the call's batches are resolved).  weight == NULL: only the sums of
+// the map (the call sizes its block with them), held may then be NULL too.
+static __global__ void k_counts_check(const double *weight, const uint32_t *counts, uint32_t npix, uint32_t *held, CountsCounters *ctr) {
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned long long v[4] = {0ull, 0ull, 0ull, 0ull};
+    if (p < npix) {
+        const double w = weight ? weight[p] : 0.0;
+        const uint32_t c = counts[p];
+        const bool ok = is_sample_count(w);
+        const uint32_t n = ok ? (uint32_t)w : 0u;
+        if (held) held[p] = n;
+        v[0] = c, v[1] = c ? 1ull : 0ull, v[2] = ok ? 0ull : 1ull;
+        v[3] = ok && (uint64_t)n + c >= (uint64_t(1) << 32) ? 1ull : 0ull;
+    }
+    block_add_u64<4>(v, &ctr->samples);
+}
+
+// One thread per slot j of the batch [b0, b1): slot j is one sample of the pixel p whose run [offset[p], offset[p+1]) holds
+// it (the last p with offset[p] <= j: zero-count pixels share their successor's offset), and that sample is the pixel's
+// held[p] + (j - offset[p])-th.  The LIST kernels read them from rc.pixel_list / rc.pixel_base with batch_samples = 1.
+static __global__ void k_counts_expand(const uint32_t *offset, const uint32_t *held, uint32_t npix, uint32_t b0, uint32_t b1,
+                                       uint32_t *pixel, uint32_t *base) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    const uint32_t j = b0 + i;
+    if (j >= b1) return;
+    uint32_t lo = 0, hi = npix; // offset[lo] <= j < offset[hi] (offset[npix] is the total, > j)
+    while (hi - lo > 1) {
+        const uint32_t mid = lo + ((hi - lo) >> 1);
+        if (offset[mid] <= j) lo = mid;
+        else hi = mid;
+    }
+    pixel[i] = lo, base[i] = held[lo] + (j - offset[lo]);
+}
+
+// The resolve of one batch of vrj_render_counts: one thread per tile pixel; a pixel whose run meets [b0, b1) applies the
+// photons of those slots (photon j - b0) in slot order, which is its sample order, with k_resolve_adaptive's Kahan update and
+// q = q + y * y.  Pixels with c = 0 write nothing; colour is formed at the end of the call (k_finalize).
+template <typename R>
+__global__ void k_resolve_counts(AccumDev acc, double *ysq, const uint32_t *offset, const double2 *photons, uint32_t npix, uint32_t b0, uint32_t b1) {
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= npix) return;
+    const uint32_t j0 = max(offset[p], b0), j1 = min(offset[p + 1], b1);
+    if (j0 >= j1) return;
+    double sx = acc.sum[3 * p], sy = acc.sum[3 * p + 1], sz = acc.sum[3 * p + 2];
+    double bx = acc.bias[3 * p], by = acc.bias[3 * p + 1], bz = acc.bias[3 * p + 2];
+    double w = acc.weight[p], wb = acc.weight_bias[p], q = ysq[p];
+    for (uint32_t j = j0; j < j1; j++) { // accumulation_buffer.rs:44-60, as in k_resolve
+        double2 ph = photons[j - b0];
+        D3 c = d3(0.0, 0.0, 0.0);
+        if (__double_as_longlong(ph.y) != 0ll) c = convert<double>(cmf<R>((R)ph.x) * (R)ph.y);
+        const double weight = 1.0;
+        double wy = weight - wb;
+        double wt = w + wy;
+        wb = (wt - w) - wy;
+        w = wt;
+        double yx = c.x * weight - bx, yy = c.y * weight - by, yz = c.z * weight - bz;
+        double tx = sx + yx, ty = sy + yy, tz = sz + yz;
+        bx = (tx - sx) - yx, by = (ty - sy) - yy, bz = (tz - sz) - yz;
+        sx = tx, sy = ty, sz = tz;
+        q = q + c.y * c.y;
+    }
+    acc.sum[3 * p] = sx, acc.sum[3 * p + 1] = sy, acc.sum[3 * p + 2] = sz;
+    acc.bias[3 * p] = bx, acc.bias[3 * p + 1] = by, acc.bias[3 * p + 2] = bz;
+    acc.weight[p] = w, acc.weight_bias[p] = wb;
+    ysq[p] = q;
+}
+
+// vrj_plan_counts: one thread per pixel, counts[p] = plan_count of its state; ctr: samples, pixels planned (c > 0),
+// converged, at max, bad weights.  Integer sums, so the counters do not depend on the order of the atomics.
+static __global__ void k_plan_counts(const double *weight, const double *sum, const double *ysq, uint32_t npix, PassRule rule, uint32_t *counts,
+                                     unsigned long long *ctr) {
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned long long v[5] = {0ull, 0ull, 0ull, 0ull, 0ull};
+    if (p < npix) {
+        bool conv = false, at_max = false, bad = false;
+        const uint32_t c = plan_count(rule, weight[p], sum[3 * p + 1], ysq[p], conv, at_max, bad);
+        counts[p] = c;
+        v[0] = c, v[1] = c ? 1ull : 0ull, v[2] = conv ? 1ull : 0ull, v[3] = at_max ? 1ull : 0ull, v[4] = bad ? 1ull : 0ull;
+    }
+    block_add_u64<5>(v, ctr);
 }
 
 // Several calls rendered as ONE wavefront (vanrijn_cuda.cu, "coalesced calls"): the batch's samples [first[c], first[c] +

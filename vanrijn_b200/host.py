@@ -248,6 +248,63 @@ class HostScene:
         out["stats"], out["progressive"] = st, pst
         return out
 
+    def render_counts(self, tile, height, width, counts, state=None, want=("colour",), device=0, **kw):
+        """vrj_render_counts with host buffers: pixel p of `tile` takes counts[p] (uint32, one per tile pixel, row-major) new
+        samples in full wavefronts, continuing `state` (a dict with colour_sum, colour_bias, weight, weight_bias and y_sq_sum,
+        as render_progressive / render_counts return it; None: start from zero).  `want` adds the optional outputs ("colour",
+        "srgb8"); `kw` are the render parameters of make_params (spp excepted).  Returns a dict with the new state (fresh
+        arrays; `state` is not modified), the wanted outputs, 'stats' (VrjStats) and 'counts' (VrjCountsStats)."""
+        sc, ec, sr, er = tile
+        npix = (ec - sc) * (er - sr)
+        kw.setdefault("spp", 0)
+        p, keep = self.make_params(**kw)
+        cmap = np.ascontiguousarray(counts, dtype=np.uint32).reshape(-1)
+        assert cmap.size == npix, (cmap.size, npix)
+        out = {}
+        ao = capi.AccumOut(memory=capi.MEM_HOST, accumulate=0 if state is None else 1)
+        for name, per in (("colour_sum", 3), ("colour_bias", 3), ("weight", 1), ("weight_bias", 1), ("y_sq_sum", 1)):
+            out[name] = np.zeros(npix * per) if state is None else np.array(state[name], np.float64, copy=True)
+            assert out[name].size == npix * per
+            if name != "y_sq_sum":
+                setattr(ao, name, out[name].ctypes.data)
+        if "colour" in want:
+            out["colour"] = np.zeros(npix * 3)
+            ao.colour = out["colour"].ctypes.data
+        if "srgb8" in want:
+            out["srgb8"] = np.zeros(npix * 3, np.uint8)
+            ao.srgb8 = out["srgb8"].ctypes.data
+        st, cst = capi.Stats(), capi.CountsStats()
+        ao.stats = C.pointer(st)
+        t = capi.Tile(sc, ec, sr, er)
+        capi.check(capi.cuda().vrj_render_counts(self.device_scene(device), C.byref(t), height, width, C.byref(p), cmap.ctypes.data,
+                                                 C.byref(ao), out["y_sq_sum"].ctypes.data, C.byref(cst)))
+        out["stats"], out["counts"] = st, cst
+        return out
+
+    def render_planned(self, tile, height, width, min_samples, max_samples, pass_samples, rel_error, abs_floor=0.0, rounds=0,
+                       state=None, want=("colour",), device=0, **kw):
+        """The planned loop: plan_counts -> render_counts, for at most `rounds` rounds (0: until a plan asks for no sample),
+        from `state` (None: zero, so the first round is the uniform pilot at min_samples).  Returns the last render_counts
+        dict (the state itself when no round ran) with 'rounds', 'samples' and 'batches' of this loop and 'plan' (the
+        VrjPlanStats of the last plan)."""
+        sc, ec, sr, er = tile
+        npix = (ec - sc) * (er - sr)
+        if state is None:
+            state = {"colour_sum": np.zeros(npix * 3), "colour_bias": np.zeros(npix * 3), "weight": np.zeros(npix),
+                     "weight_bias": np.zeros(npix), "y_sq_sum": np.zeros(npix)}
+        res, n, samples, batches = dict(state), 0, 0, 0
+        while rounds == 0 or n < rounds:
+            counts, plan = plan_counts(res["weight"], res["colour_sum"], res["y_sq_sum"], min_samples, max_samples, pass_samples,
+                                       rel_error, abs_floor, device=device)
+            res["plan"] = plan
+            if plan.samples == 0:
+                break
+            res = self.render_counts(tile, height, width, counts, state=res, want=want, device=device, **kw)
+            res["plan"] = plan
+            n, samples, batches = n + 1, samples + res["counts"].samples, batches + res["counts"].batches
+        res["rounds"], res["samples"], res["batches"] = n, samples, batches
+        return res
+
     def render_aux(self, tile, height, width, spp=1, want=("normal", "depth", "object_id", "material"), device=0, **kw):
         """vrj_render_aux with host output buffers: the first-hit features of the camera rays that a render with the same
         spp, seed, sample_offset and sample_stride traces (`kw`: the other keywords of make_params).  Returns a dict of numpy
@@ -357,6 +414,22 @@ def tone_map(colour, source=capi.TONEMAP_XYZ, device=0):
     out = np.zeros((c.shape[0], 3), np.uint8)
     capi.check(capi.cuda().vrj_tone_map(device, capi.MEM_HOST, source, c.ctypes.data_as(dp), c.shape[0], out.ctypes.data))
     return out
+
+
+def plan_counts(weight, colour_sum, y_sq_sum, min_samples, max_samples, pass_samples, rel_error, abs_floor=0.0, device=0):
+    """vrj_plan_counts on a host state: the count map (uint32, one per pixel) that the rule of the header gives each
+    pixel, and the VrjPlanStats."""
+    ins = [np.ascontiguousarray(weight, np.float64), np.ascontiguousarray(colour_sum, np.float64),
+           np.ascontiguousarray(y_sq_sum, np.float64)]
+    npix = ins[0].size
+    assert ins[1].size == 3 * npix and ins[2].size == npix
+    counts = np.zeros(npix, np.uint32)
+    rule = capi.AdaptiveParams(min_samples=min_samples, max_samples=max_samples, pass_samples=pass_samples,
+                               rel_error=rel_error, abs_floor=abs_floor)
+    ps = capi.PlanStats()
+    capi.check(capi.cuda().vrj_plan_counts(device, capi.MEM_HOST, npix, *[a.ctypes.data for a in ins], C.byref(rule),
+                                           counts.ctypes.data, C.byref(ps)))
+    return counts, ps
 
 
 # vrj_denoise's defaults (VRJ_DENOISE_DEFAULT_* in include/vanrijn_cuda.h), chosen with tools/denoise_quality.py

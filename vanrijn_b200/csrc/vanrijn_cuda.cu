@@ -559,7 +559,8 @@ struct ActiveCall {
 VrjStatus check_tile(const VrjTile *tile, uint64_t height, uint64_t width) {
     if (tile->end_column < tile->start_column || tile->end_row < tile->start_row || tile->end_column > width || tile->end_row > height)
         return fail(VRJ_ERR_INVALID_ARGUMENT, "tile outside the image");
-    if (width * height > 0xffffffffull) return fail(VRJ_ERR_UNSUPPORTED, "image larger than 2^32 pixels");
+    // width * height can wrap in 64 bits (2^32 x 2^32, 2^63 x 2): compare by division
+    if (height != 0 && width > 0xffffffffull / height) return fail(VRJ_ERR_UNSUPPORTED, "image larger than 2^32 - 1 pixels");
     return VRJ_OK;
 }
 

@@ -99,11 +99,13 @@ class HostScene:
     def spectrum_data(self, spectrum_id):
         """(SpectrumData, keepalive) for a spectrum of the spec, e.g. a light's."""
         lo, hi = C.c_double(), C.c_double()
-        buf = np.zeros(64)
-        n = self.H.vrjh_get_spectrum(self.h, spectrum_id, C.byref(lo), C.byref(hi), buf.ctypes.data_as(dp), 64)
+        # the first call only returns the count: a spectrum may hold any number of samples
+        n = self.H.vrjh_get_spectrum(self.h, spectrum_id, C.byref(lo), C.byref(hi), None, 0)
         if n < 0:
             raise capi.VrjError(self.H.vrjh_last_error().decode())
-        buf = buf[:n].copy()
+        buf = np.zeros(max(n, 1))
+        self.H.vrjh_get_spectrum(self.h, spectrum_id, C.byref(lo), C.byref(hi), buf.ctypes.data_as(dp), n)
+        buf = buf[:n]
         return capi.SpectrumData(lo.value, hi.value, n, 0, buf.ctypes.data_as(dp)), buf
 
     # ---- device ----

@@ -33,12 +33,12 @@ thread_local std::string g_error;
 
 // the six instantiations live in vrj_batch_inst.cu (one object file each)
 namespace vrjimpl {
-extern template VrjStatus run_batch<float, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
-extern template VrjStatus run_batch<float, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
-extern template VrjStatus run_batch<double, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
-extern template VrjStatus run_batch<double, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
-extern template VrjStatus run_batch<float, float, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
-extern template VrjStatus run_batch<float, float, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
+extern template VrjStatus run_batch<float, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *);
+extern template VrjStatus run_batch<float, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *);
+extern template VrjStatus run_batch<double, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *);
+extern template VrjStatus run_batch<double, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *);
+extern template VrjStatus run_batch<float, float, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *);
+extern template VrjStatus run_batch<float, float, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *);
 } // namespace vrjimpl
 // NVTX ranges (SURVEY section 5) through the header-only NVTX 3: no library to link or load -- the calls are no-ops until a
 // tool (ncu --nvtx, nsys) injects itself
@@ -644,20 +644,31 @@ VrjStatus stage_lights(Scratch *s, const VrjRenderParams *p) {
 }
 
 // one batch in the kernel variant the call's precision, walk and counting select
-VrjStatus dispatch_batch(const VrjScene *scene, Scratch *s, const RenderConst &rc, const VrjRenderParams *p, uint32_t filter, uint64_t *launches,
-                         const MultiCalls *multi, const ResolveCopy *copy, double *ysq, const CountsBatch *counts = nullptr) {
+VrjStatus dispatch_batch(const VrjScene *scene, Scratch *s, const RenderConst &rc, const VrjRenderParams *p, uint32_t filter, uint64_t *launches) {
     const bool whitted = p->integrator == VRJ_INTEGRATOR_WHITTED;
     // F32X4: the staged rays walk the 4-wide tree; inline any-hit queries (Whitted shadow rays, k_tail) use the 2-wide f32 tree
     const int quad = filter == VRJ_FILTER_F32X4 ? 1 : filter == VRJ_FILTER_Q16 ? 2 : 0;
     // VRJ_PRECISION_F32_FAST: the whole sample in binary32 over the 2-wide f32 tree (no reference counterpart; not a parity mode)
     const bool fast = p->precision == VRJ_PRECISION_F32_FAST;
     if (p->count_traversal)
-        return fast ? run_batch<float, float, true>(scene, s, rc, whitted, 0, launches, multi, copy, ysq, counts)
-             : filter == VRJ_FILTER_F64 ? run_batch<double, double, true>(scene, s, rc, whitted, 0, launches, multi, copy, ysq, counts)
-                                        : run_batch<float, double, true>(scene, s, rc, whitted, quad, launches, multi, copy, ysq, counts);
-    return fast ? run_batch<float, float, false>(scene, s, rc, whitted, 0, launches, multi, copy, ysq, counts)
-         : filter == VRJ_FILTER_F64 ? run_batch<double, double, false>(scene, s, rc, whitted, 0, launches, multi, copy, ysq, counts)
-                                    : run_batch<float, double, false>(scene, s, rc, whitted, quad, launches, multi, copy, ysq, counts);
+        return fast ? run_batch<float, float, true>(scene, s, rc, whitted, 0, launches)
+             : filter == VRJ_FILTER_F64 ? run_batch<double, double, true>(scene, s, rc, whitted, 0, launches)
+                                        : run_batch<float, double, true>(scene, s, rc, whitted, quad, launches);
+    return fast ? run_batch<float, float, false>(scene, s, rc, whitted, 0, launches)
+         : filter == VRJ_FILTER_F64 ? run_batch<double, double, false>(scene, s, rc, whitted, 0, launches)
+                                    : run_batch<float, double, false>(scene, s, rc, whitted, quad, launches);
+}
+
+// The resolve of the batch dispatch_batch left in s->photons: `launch` enqueues its kernels in the real type R of the call's
+// colour matching (run_batch's R: float for VRJ_PRECISION_F32_FAST), then the boundary that closes the resolve (resolve_ms).
+template <typename F>
+VrjStatus resolve_batch(Scratch *s, const VrjRenderParams *p, F &&launch) {
+    VRJ_NVTX_RANGE(resolve_range, "vrj resolve");
+    const VrjStatus st = p->precision == VRJ_PRECISION_F32_FAST ? launch(float{}) : launch(double{});
+    if (st != VRJ_OK) return st;
+    VRJ_CUDA(s->mark(2));
+    VRJ_CUDA(cudaGetLastError());
+    return VRJ_OK;
 }
 
 // VrjStats of a call from its counters and the boundary events run_levels recorded
@@ -682,8 +693,7 @@ void fill_call_stats(VrjStats *st, const Scratch *s, const unsigned long long *h
 __global__ void k_finalize(const double *sum, const double *weight, double *colour, uint32_t npix) {
     uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= npix) return;
-    double inv = 1.0 / weight[p]; // accumulation_buffer.rs:59
-    colour[3 * p] = sum[3 * p] * inv, colour[3 * p + 1] = sum[3 * p + 1] * inv, colour[3 * p + 2] = sum[3 * p + 2] * inv;
+    store_colour(colour, p, sum[3 * p], sum[3 * p + 1], sum[3 * p + 2], weight[p]);
 }
 
 // the tone-mapped colours of the block's accumulators to out->srgb8
@@ -705,19 +715,11 @@ struct Arr {
     size_t per;
 };
 
-// the arrays of a state into the block: from the caller's arrays when `load` (a NULL array starts at zero), else zero
-VrjStatus load_state(Scratch *s, const Arr *arrs, int n, bool load, cudaMemcpyKind kind, uint64_t npix) {
-    for (int i = 0; i < n; i++) {
-        if (load && arrs[i].user) VRJ_CUDA(cudaMemcpyAsync(arrs[i].dev->p, arrs[i].user, npix * arrs[i].per * sizeof(double), kind, s->stream));
-        else VRJ_CUDA(cudaMemsetAsync(arrs[i].dev->p, 0, npix * arrs[i].per * sizeof(double), s->stream));
-    }
-    return VRJ_OK;
-}
-
 // What every render call (vrj_render_tile, render_passes, vrj_render_counts) does around its kernels.  prepare(): a block from
 // the pool for batches of up to `widest` samples of the tile (prepare_paths: of up to `widest` units of `unit` paths);
-// start(): the call's counters, lights and constants, the render turn and ev0;finish(): ev1, the counters, the copies of the outputs and the sRGB preview, the waits, VrjStats.  `turn` is declared
-// after `block`: an early return gives the turn back before the block.
+// load_state(): the call's arrays and its state in the block; start(): the call's counters, lights and constants, the render
+// turn and ev0; finish(): ev1, the counters, the copies of the outputs and the sRGB preview, the waits, VrjStats.  `turn` is
+// declared after `block`: an early return gives the turn back before the block.
 struct RenderCall {
     VrjScene *scene;
     const VrjRenderParams *p;
@@ -728,7 +730,11 @@ struct RenderCall {
     uint32_t filter = 0, batch = 0;
     RenderConst rc{};
     uint64_t launches = 0;
-    bool pieces_copied = false; // the arrays went out with the last resolve's pieces (ResolveCopy): wait for those copies
+    VrjAccumOut *out = nullptr;
+    Arr arrs[6] = {}; // out's colour, colour_sum, colour_bias, weight, weight_bias, and y_sq_sum for the calls that keep it
+    int n_arrs = 0;
+    cudaMemcpyKind in_kind = cudaMemcpyHostToDevice, out_kind = cudaMemcpyDeviceToHost;
+    bool pieces_copied = false; // the arrays went out with the last resolve's pieces (vrj_render_tile): wait for those copies
     float ms = 0.f;             // device time, ev0 .. ev1
     std::chrono::steady_clock::time_point t_start, t_enqueued, t_done; // turn taken, last copy enqueued, copies arrived
     RenderCall(VrjScene *sc, const VrjRenderParams *params, uint64_t n) : scene(sc), p(params), npix(n), block{sc}, turn(sc->device) {}
@@ -740,6 +746,22 @@ struct RenderCall {
         s = block.s = acquire_scratch(scene, unit * batch);
         filter = effective_filter(scene, p);
         return ensure_call_scratch(s, p, call_wants_records(scene, p, filter), npix, unit, &batch, n_light_samples);
+    }
+    // The call's arrays: out's, and with `ysq` (render_passes, vrj_render_counts) y_sq_sum.  The state -- every array but
+    // colour -- comes into the block from the caller's arrays when `load` (a NULL array starts at zero), else it is zero.
+    VrjStatus load_state(VrjAccumOut *o, bool load, bool ysq = false, double *y_sq_sum = nullptr) {
+        out = o;
+        in_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+        out_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+        const Arr a[6] = {{out->colour, &s->acc_colour, 3}, {out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3},
+                          {out->weight, &s->acc_weight, 1}, {out->weight_bias, &s->acc_wbias, 1}, {y_sq_sum, &s->ysq, 1}};
+        n_arrs = ysq ? 6 : 5;
+        std::copy(a, a + n_arrs, arrs);
+        for (int i = 1; i < n_arrs; i++) {
+            if (load && arrs[i].user) VRJ_CUDA(cudaMemcpyAsync(arrs[i].dev->p, arrs[i].user, npix * arrs[i].per * sizeof(double), in_kind, s->stream));
+            else VRJ_CUDA(cudaMemsetAsync(arrs[i].dev->p, 0, npix * arrs[i].per * sizeof(double), s->stream));
+        }
+        return VRJ_OK;
     }
     VrjStatus start(const VrjTile *tile, uint64_t height, uint64_t width) {
         VRJ_CUDA(cudaMemsetAsync(s->stats.p, 0, ST_COUNT * sizeof(unsigned long long), s->stream));
@@ -755,17 +777,17 @@ struct RenderCall {
         VRJ_CUDA(cudaEventRecord(s->ev0, s->stream));
         return VRJ_OK;
     }
-    VrjStatus finish(const Arr *arrs, int n, uint8_t *srgb8, cudaMemcpyKind kind, VrjStats *stats) {
+    VrjStatus finish() {
         VRJ_CUDA(cudaEventRecord(s->ev1, s->stream)); // before the counters' copy: that one queues up behind the pieces' copies on the copy engine
         VRJ_CUDA(cudaMemcpyAsync(s->pinned->stats, s->stats.p, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
         if (pieces_copied) {
             VRJ_CUDA(cudaStreamWaitEvent(s->stream, s->copy_done, 0)); // ev_done below then stands behind the pieces' copies too
         } else {
-            for (int i = 0; i < n; i++)
-                if (arrs[i].user) VRJ_CUDA(cudaMemcpyAsync(arrs[i].user, arrs[i].dev->p, npix * arrs[i].per * sizeof(double), kind, s->stream));
+            for (int i = 0; i < n_arrs; i++)
+                if (arrs[i].user) VRJ_CUDA(cudaMemcpyAsync(arrs[i].user, arrs[i].dev->p, npix * arrs[i].per * sizeof(double), out_kind, s->stream));
         }
-        if (srgb8) {
-            const VrjStatus st = copy_srgb8(s, npix, srgb8, kind, &launches);
+        if (out->srgb8) {
+            const VrjStatus st = copy_srgb8(s, npix, out->srgb8, out_kind, &launches);
             if (st != VRJ_OK) return st;
         }
         t_enqueued = std::chrono::steady_clock::now();
@@ -775,7 +797,7 @@ struct RenderCall {
         VRJ_CUDA(wait_event(s->ev_done, scene->device));
         t_done = std::chrono::steady_clock::now();
         VRJ_CUDA(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-        if (stats) fill_call_stats(stats, s, s->pinned->stats, launches, ms);
+        if (out->stats) fill_call_stats(out->stats, s, s->pinned->stats, launches, ms);
         return VRJ_OK;
     }
 };
@@ -849,11 +871,7 @@ VrjStatus render_passes(VrjScene *scene, const VrjTile *tile, uint64_t height, u
     Scratch *s = call.s;
     st = ensure_pass_buffers(s, npix);
     if (st != VRJ_OK) return st;
-    const cudaMemcpyKind in_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-    const cudaMemcpyKind out_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-    const Arr arrs[6] = {{out->colour, &s->acc_colour, 3}, {out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3},
-                         {out->weight, &s->acc_weight, 1}, {out->weight_bias, &s->acc_wbias, 1}, {y_sq_sum, &s->ysq, 1}};
-    st = load_state(s, arrs + 1, 5, !fresh, in_kind, npix);
+    st = call.load_state(out, !fresh, true, y_sq_sum);
     if (st != VRJ_OK) return st;
     ProgressiveCounters *ctr = s->pass_counters.as<ProgressiveCounters>(), *hctr = &s->pinned->pass;
     VRJ_CUDA(cudaMemsetAsync(ctr, 0, sizeof(ProgressiveCounters), s->stream));
@@ -862,7 +880,9 @@ VrjStatus render_passes(VrjScene *scene, const VrjTile *tile, uint64_t height, u
 
     RenderConst &rc = call.rc;
     const size_t capacity = npix * call.batch; // paths per batch
-    const double *sum = s->acc_sum.as<double>(), *weight = s->acc_weight.as<double>(), *ysq = s->ysq.as<double>();
+    const AccumDev acc = s->accum();
+    const double *sum = acc.sum, *weight = acc.weight;
+    double *ysq = s->ysq.as<double>();
     // the flags and the scan's tile totals live in the photon buffer, which is free between a pass's resolve and the next
     // batch: (n + 1) + (n / 2048 + 2) uint32 fit the 16 bytes per path of a block that holds at least one path per pixel
     uint32_t *flags = s->photons.as<uint32_t>(), *base = s->pass_base.as<uint32_t>();
@@ -874,7 +894,13 @@ VrjStatus render_passes(VrjScene *scene, const VrjTile *tile, uint64_t height, u
             rc.batch_samples = std::min(b, c - done);
             rc.div_batch = FastDiv::make(rc.batch_samples);
             rc.first_sample = p->sample_offset + (uint64_t)done * rc.sample_stride;
-            const VrjStatus bst = dispatch_batch(scene, s, rc, p, call.filter, &call.launches, nullptr, nullptr, s->ysq.as<double>());
+            VrjStatus bst = dispatch_batch(scene, s, rc, p, call.filter, &call.launches);
+            if (bst == VRJ_OK)
+                bst = resolve_batch(s, p, [&](auto r) {
+                    k_resolve_adaptive<decltype(r)><<<(rc.npix + 255) / 256, 256, 0, s->stream>>>(acc, ysq, rc.pixel_list, s->photons.as<double2>(), rc.npix, rc.batch_samples);
+                    call.launches++;
+                    return VRJ_OK;
+                });
             if (bst != VRJ_OK) return bst;
         }
         res->samples += (uint64_t)m * c;
@@ -941,11 +967,11 @@ VrjStatus render_passes(VrjScene *scene, const VrjTile *tile, uint64_t height, u
         res->passes++;
     }
     if (!fresh && (out->colour || out->srgb8)) {
-        k_finalize<<<(unsigned)((npix + 255) / 256), 256, 0, s->stream>>>(sum, weight, s->acc_colour.as<double>(), (uint32_t)npix);
+        k_finalize<<<(unsigned)((npix + 255) / 256), 256, 0, s->stream>>>(sum, weight, acc.colour, (uint32_t)npix);
         call.launches++;
         VRJ_CUDA(cudaGetLastError());
     }
-    st = call.finish(arrs, 6, out->srgb8, out_kind, out->stats);
+    st = call.finish();
     if (st != VRJ_OK) return st;
     res->counts = *hctr;
     return VRJ_OK;
@@ -1006,15 +1032,11 @@ VrjStatus render_counts(VrjScene *scene, const VrjTile *tile, uint64_t height, u
     Scratch *s = call.s;
     st = ensure_pass_buffers(s, npix, call.batch);
     if (st != VRJ_OK) return st;
-    const cudaMemcpyKind in_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-    const cudaMemcpyKind out_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-    const Arr arrs[6] = {{out->colour, &s->acc_colour, 3}, {out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3},
-                         {out->weight, &s->acc_weight, 1}, {out->weight_bias, &s->acc_wbias, 1}, {y_sq_sum, &s->ysq, 1}};
-    st = load_state(s, arrs + 1, 5, out->accumulate != 0, in_kind, npix);
+    st = call.load_state(out, out->accumulate != 0, true, y_sq_sum);
     if (st != VRJ_OK) return st;
     uint32_t *offset = s->count_offset.as<uint32_t>(), *held = s->pass_base.as<uint32_t>();
     CountsCounters *ctr = s->count_counters.as<CountsCounters>(), *hctr = &s->pinned->counts;
-    VRJ_CUDA(cudaMemcpyAsync(offset, counts, npix * sizeof(uint32_t), in_kind, s->stream));
+    VRJ_CUDA(cudaMemcpyAsync(offset, counts, npix * sizeof(uint32_t), call.in_kind, s->stream));
     VRJ_CUDA(cudaMemsetAsync(offset + npix, 0, sizeof(uint32_t), s->stream));
     VRJ_CUDA(cudaMemsetAsync(ctr, 0, sizeof(CountsCounters), s->stream));
     k_counts_check<<<(n32 + 255) / 256, 256, 0, s->stream>>>(s->acc_weight.as<double>(), offset, n32, held, ctr);
@@ -1046,8 +1068,13 @@ VrjStatus render_counts(VrjScene *scene, const VrjTile *tile, uint64_t height, u
             call.launches++;
             VRJ_CUDA(cudaGetLastError());
             rc.npix = m;
-            const CountsBatch cb{offset, n32, (uint32_t)b0, b1};
-            st = dispatch_batch(scene, s, rc, p, call.filter, &call.launches, nullptr, nullptr, ysq, &cb);
+            st = dispatch_batch(scene, s, rc, p, call.filter, &call.launches);
+            if (st == VRJ_OK)
+                st = resolve_batch(s, p, [&](auto r) {
+                    k_resolve_counts<decltype(r)><<<(n32 + 255) / 256, 256, 0, s->stream>>>(s->accum(), ysq, offset, s->photons.as<double2>(), n32, (uint32_t)b0, b1);
+                    call.launches++;
+                    return VRJ_OK;
+                });
             if (st != VRJ_OK) return st;
         }
         if (cstats) cstats->batches = batches;
@@ -1057,7 +1084,7 @@ VrjStatus render_counts(VrjScene *scene, const VrjTile *tile, uint64_t height, u
         call.launches++;
         VRJ_CUDA(cudaGetLastError());
     }
-    return call.finish(arrs, 6, out->srgb8, out_kind, out->stats);
+    return call.finish();
 }
 
 // ---------------------------------------------------------------------------------------------- coalesced calls
@@ -1176,7 +1203,13 @@ VrjStatus render_group(Coalescer &co, CoalesceRequest *const *reqs, uint32_t n, 
     uint64_t launches = 0;
     s->n_marks = 0;
     VRJ_CUDA(cudaEventRecord(s->ev0, s->stream));
-    st = dispatch_batch(scene, s, rc, p, filter, &launches, &mc, nullptr, nullptr);
+    st = dispatch_batch(scene, s, rc, p, filter, &launches);
+    if (st == VRJ_OK)
+        st = resolve_batch(s, p, [&](auto r) {
+            k_resolve_multi<decltype(r)><<<(rc.npix * mc.n + 255) / 256, 256, 0, s->stream>>>(mc, s->photons.as<double2>(), rc.npix, rc.batch_samples);
+            launches++;
+            return VRJ_OK;
+        });
     if (st != VRJ_OK) return st;
     unsigned long long *hstats = s->pinned->stats;
     VRJ_CUDA(cudaMemcpyAsync(hstats, s->stats.p, ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
@@ -1760,44 +1793,70 @@ VrjStatus vrj_render_tile(const VrjScene *scene_c, const VrjTile *tile, uint64_t
     Scratch *s = call.s;
     const uint32_t batch = call.batch;
 
-    const cudaMemcpyKind in_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-    const cudaMemcpyKind out_kind = out->memory == VRJ_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-    const Arr arrs[5] = {{out->colour, &s->acc_colour, 3}, {out->colour_sum, &s->acc_sum, 3}, {out->colour_bias, &s->acc_bias, 3},
-                         {out->weight, &s->acc_weight, 1}, {out->weight_bias, &s->acc_wbias, 1}};
-    st = load_state(s, arrs + 1, 4, out->accumulate, in_kind, npix);
+    st = call.load_state(out, out->accumulate);
     if (st != VRJ_OK) return st;
     st = call.start(tile, height, width);
     if (st != VRJ_OK) return st;
     RenderConst &rc = call.rc;
-    // the last batch's resolve runs in pieces whose parts of the arrays start for the host at once (ResolveCopy); small tiles
-    // and device-memory outputs (copies at HBM speed) keep the single resolve
-    ResolveCopy rcopy{{arrs[0].user, arrs[1].user, arrs[2].user, arrs[3].user, arrs[4].user}, out_kind, 4u};
-    // (worth it when the resolve is long enough to hide a copy behind: with a sample or two per pixel it is 0.06 ms against 1.25 ms)
+    const AccumDev acc = s->accum();
+    const double2 *photons = s->photons.as<double2>();
+    // The last batch's resolve runs in `pieces` row-aligned pieces, and each piece's part of the arrays is copied to the caller
+    // on a second stream as soon as it is resolved: at 1080p the copy back (66 MB, 1.25 ms over PCIe) hides behind the 1.6 ms
+    // the seven exponentials per sample take, instead of following them.  Small tiles and device-memory outputs (copies at HBM
+    // speed) keep the single resolve (worth it when the resolve is long enough to hide a copy behind: with a sample or two per
+    // pixel it is 0.06 ms against 1.25 ms).
+    const uint32_t pieces = 4;
     bool piecewise = out->memory == VRJ_MEM_HOST && npix >= (uint64_t(1) << 18) && std::min(batch, p->spp) >= 8 && !std::getenv("VRJ_NO_PIECEWISE_COPY");
     for (int i = 0; i < 5 && piecewise; i++) { // page-locked destinations only: a copy into pageable memory holds the enqueueing thread
         cudaPointerAttributes attr{};
-        if (arrs[i].user && (cudaPointerGetAttributes(&attr, arrs[i].user) != cudaSuccess || attr.type != cudaMemoryTypeHost)) piecewise = false;
+        if (call.arrs[i].user && (cudaPointerGetAttributes(&attr, call.arrs[i].user) != cudaSuccess || attr.type != cudaMemoryTypeHost)) piecewise = false;
     }
     cudaGetLastError();
     for (uint32_t done = 0; done < p->spp; done += batch) {
         rc.batch_samples = std::min(batch, p->spp - done);
-        const ResolveCopy *copy = piecewise && done + batch >= p->spp ? &rcopy : nullptr;
-        call.pieces_copied = call.pieces_copied || copy != nullptr;
+        const bool copy = piecewise && done + batch >= p->spp;
+        call.pieces_copied = call.pieces_copied || copy;
         rc.div_batch = FastDiv::make(rc.batch_samples);
         rc.first_sample = p->sample_offset + (uint64_t)done * rc.sample_stride;
-        st = dispatch_batch(scene, s, rc, p, call.filter, &call.launches, nullptr, copy, nullptr);
+        st = dispatch_batch(scene, s, rc, p, call.filter, &call.launches);
+        if (st != VRJ_OK) return st;
+        st = resolve_batch(s, p, [&](auto r) -> VrjStatus {
+            using R = decltype(r);
+            if (!copy) {
+                k_resolve<R><<<(rc.npix + 255) / 256, 256, 0, s->stream>>>(acc, photons, 0u, rc.npix, rc.batch_samples);
+                call.launches++;
+                return VRJ_OK;
+            }
+            const uint32_t step = ((rc.npix + pieces - 1) / pieces + 255u) & ~255u; // whole CTAs per piece
+            uint32_t piece = 0;
+            for (uint32_t first = 0; first < rc.npix; first += step, piece++) {
+                const uint32_t end = std::min(rc.npix, first + step);
+                k_resolve<R><<<(end - first + 255) / 256, 256, 0, s->stream>>>(acc, photons, first, end, rc.batch_samples);
+                call.launches++;
+                VRJ_CUDA(cudaEventRecord(s->piece_ev[piece], s->stream));
+                VRJ_CUDA(cudaStreamWaitEvent(s->copy_stream, s->piece_ev[piece], 0));
+                for (int i = 0; i < 5; i++) {
+                    const Arr &a = call.arrs[i];
+                    if (a.user)
+                        VRJ_CUDA(cudaMemcpyAsync(a.user + (size_t)first * a.per, a.dev->as<double>() + (size_t)first * a.per, (size_t)(end - first) * a.per * sizeof(double),
+                                                 call.out_kind, s->copy_stream));
+                }
+            }
+            VRJ_CUDA(cudaEventRecord(s->copy_done, s->copy_stream));
+            return VRJ_OK;
+        });
         if (st != VRJ_OK) return st;
         if (out->photons) {
             // debug output, batch-major: [(sample * npix + pixel) * 2]; the device keeps the batch pixel-major, so transpose
             // into queue 0's storage (free at this point: 6 x 16 bytes per path >= 16 bytes per sample)
             double2 *tmp = s->queues[0][0].as<double2>();
             const size_t count = (size_t)rc.batch_samples * npix;
-            k_photons_sample_major<<<(unsigned)((count + 255) / 256), 256, 0, s->stream>>>(s->photons.as<double2>(), tmp, (uint32_t)npix, rc.batch_samples);
+            k_photons_sample_major<<<(unsigned)((count + 255) / 256), 256, 0, s->stream>>>(photons, tmp, (uint32_t)npix, rc.batch_samples);
             call.launches++;
-            VRJ_CUDA(cudaMemcpyAsync(out->photons + (size_t)done * npix * 2, tmp, count * sizeof(double2), out_kind, s->stream));
+            VRJ_CUDA(cudaMemcpyAsync(out->photons + (size_t)done * npix * 2, tmp, count * sizeof(double2), call.out_kind, s->stream));
         }
     }
-    st = call.finish(arrs, 5, out->srgb8, out_kind, out->stats);
+    st = call.finish();
     if (st != VRJ_OK) return st;
     if (timing) {
         auto msd = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {

@@ -59,15 +59,6 @@ struct DeviceBuffer {
     T *as() const { return static_cast<T *>(p); }
 };
 
-// Where the resolved arrays of a call's LAST batch go.  k_resolve then runs in `pieces` row-aligned pieces, and each piece's
-// part of the arrays is copied to the caller on a second stream as soon as it is resolved: at 1080p the copy back (66 MB,
-// 1.25 ms over PCIe) hides behind the 1.6 ms the seven exponentials per sample take, instead of following them.
-struct ResolveCopy {
-    double *user[5];      // colour, colour_sum, colour_bias, weight, weight_bias (NULL: not wanted)
-    cudaMemcpyKind kind;
-    uint32_t pieces;
-};
-
 // The block's page-locked slots.  Counters come back and the sample table goes out through them: a copy between the device and
 // pageable memory holds the enqueueing thread until everything queued before it has finished (the render gate could not
 // open before the result's copies).
@@ -78,13 +69,6 @@ struct PinnedBlock {
     ProgressiveCounters pass;                   // render_passes: the last select's counters
     uint32_t listed;                            // render_passes: the length of a sub-pass's pixel list
     CountsCounters counts;                      // vrj_render_counts: what k_counts_check found
-};
-
-// One batch of vrj_render_counts: slots [b0, b1) of the call, slot j being one sample of the tile pixel whose run of the
-// exclusive scan `offset` (npix + 1 entries) holds it; k_resolve_counts applies them.
-struct CountsBatch {
-    const uint32_t *offset;
-    uint32_t npix, b0, b1;
 };
 
 // per-call scratch: path queues, photon results, accumulators, counters
@@ -109,7 +93,7 @@ struct Scratch {
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr; // first / last kernel of a call
     cudaEvent_t ev_done = nullptr;             // behind the call's last copy
-    cudaStream_t copy_stream = nullptr;        // copies of resolved pieces (ResolveCopy) run here, next to the resolve kernels
+    cudaStream_t copy_stream = nullptr;        // copies of resolved pieces (vrj_render_tile) run here, next to the resolve kernels
     cudaEvent_t piece_ev[8] = {};              // behind the resolve of piece i
     cudaEvent_t copy_done = nullptr;           // behind the last of those copies
     cudaEvent_t call_ev[16] = {};              // coalesced calls: behind the copies of call c (MULTI_MAX_CALLS)
@@ -144,6 +128,12 @@ struct Scratch {
         }
         mark_class[n_marks] = cls;
         return cudaEventRecord(marks[n_marks++], stream);
+    }
+    AccumDev accum() const {
+        AccumDev a;
+        a.colour = acc_colour.as<double>(), a.sum = acc_sum.as<double>(), a.bias = acc_bias.as<double>();
+        a.weight = acc_weight.as<double>(), a.weight_bias = acc_wbias.as<double>();
+        return a;
     }
     TraceBuffers trace_buffers(int i, bool records = false) const {
         TraceBuffers t;
@@ -207,10 +197,10 @@ inline bool wants_records(const VrjScene *sc, int walk) {
     return sizeof(NT) == 4 && sizeof(R) == 8 && walk == 0 && sc->trace_records && sc->dev.n_bvh_items > 0;
 }
 
-// One batch with the integrator (WHITTED) and the scene's material kinds (MM, see vrj_device.cuh) fixed at compile time.
+// One batch with the integrator (WHITTED) and the scene's material kinds (MM, see vrj_device.cuh) fixed at compile time.  It
+// leaves the batch's photons in s->photons, pixel-major; the caller resolves them.
 template <typename NT, typename R, bool COUNT, bool WHITTED, int MM, bool LIST>
-VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int walk, uint64_t *launches, const MultiCalls *multi,
-                     const ResolveCopy *copy, double *ysq, const CountsBatch *counts) {
+VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int walk, uint64_t *launches) {
     const bool quad = walk == 1, q16 = walk == 2; // 0: the 2-wide tree in NT boxes; 1: 4-wide f32; 2: 2-wide on the 16-bit grid
     // launch sequence: G T S_0 [X_k T_k S_k]*, k = 1..levels (X = k_tail, a no-op until the queue is short);
     // SimpleRandom needs max_depth levels, Whitted one more (its limit-0 level still shades and traces);
@@ -305,41 +295,6 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
             drain_pending = true;
         }
     }
-    VRJ_NVTX_RANGE(resolve_range, "vrj resolve");
-    AccumDev acc;
-    acc.colour = s->acc_colour.as<double>(), acc.sum = s->acc_sum.as<double>(), acc.bias = s->acc_bias.as<double>();
-    acc.weight = s->acc_weight.as<double>(), acc.weight_bias = s->acc_wbias.as<double>();
-    if (counts) {
-        k_resolve_counts<R><<<(counts->npix + 255) / 256, 256, 0, s->stream>>>(acc, ysq, counts->offset, photons, counts->npix, counts->b0, counts->b1);
-        (*launches)++;
-    } else if (multi) {
-        k_resolve_multi<R><<<(rc.npix * multi->n + 255) / 256, 256, 0, s->stream>>>(*multi, photons, rc.npix, rc.batch_samples);
-        (*launches)++;
-    } else if (ysq) {
-        k_resolve_adaptive<R><<<(rc.npix + 255) / 256, 256, 0, s->stream>>>(acc, ysq, rc.pixel_list, photons, rc.npix, rc.batch_samples);
-        (*launches)++;
-    } else if (copy && copy->pieces > 1) {
-        const double *dev[5] = {acc.colour, acc.sum, acc.bias, acc.weight, acc.weight_bias};
-        const size_t per[5] = {3, 3, 3, 1, 1};
-        const uint32_t step = ((rc.npix + copy->pieces - 1) / copy->pieces + 255u) & ~255u; // whole CTAs per piece
-        uint32_t piece = 0;
-        for (uint32_t first = 0; first < rc.npix; first += step, piece++) {
-            const uint32_t end = std::min(rc.npix, first + step);
-            k_resolve<R><<<(end - first + 255) / 256, 256, 0, s->stream>>>(acc, photons, first, end, rc.batch_samples);
-            (*launches)++;
-            VRJ_CUDA(cudaEventRecord(s->piece_ev[piece], s->stream));
-            VRJ_CUDA(cudaStreamWaitEvent(s->copy_stream, s->piece_ev[piece], 0));
-            for (int i = 0; i < 5; i++)
-                if (copy->user[i])
-                    VRJ_CUDA(cudaMemcpyAsync(copy->user[i] + (size_t)first * per[i], dev[i] + (size_t)first * per[i], (size_t)(end - first) * per[i] * sizeof(double),
-                                             copy->kind, s->copy_stream));
-        }
-        VRJ_CUDA(cudaEventRecord(s->copy_done, s->copy_stream));
-    } else {
-        k_resolve<R><<<(rc.npix + 255) / 256, 256, 0, s->stream>>>(acc, photons, 0u, rc.npix, rc.batch_samples);
-        (*launches)++;
-    }
-    VRJ_CUDA(s->mark(2));
     VRJ_CUDA(cudaGetLastError());
     return VRJ_OK;
 }
@@ -347,22 +302,19 @@ VrjStatus run_levels(const VrjScene *sc, Scratch *s, const RenderConst &rc, int 
 // kernel variants exist for "Lambertian only" (the reference's own scenes: main.rs, benches/simple_scene.rs) and for
 // "any material"; VRJ_MATERIAL_MASK=15 in the environment forces the general variant (experiments)
 template <typename NT, typename R, bool COUNT, bool LIST>
-VrjStatus run_materials(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches, const MultiCalls *multi,
-                        const ResolveCopy *copy, double *ysq, const CountsBatch *counts) {
+VrjStatus run_materials(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches) {
     const bool lambert_only = sc->kernel_material_mask == 1u;
     if (whitted)
-        return lambert_only ? run_levels<NT, R, COUNT, true, 1, LIST>(sc, s, rc, walk, launches, multi, copy, ysq, counts)
-                            : run_levels<NT, R, COUNT, true, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches, multi, copy, ysq, counts);
-    return lambert_only ? run_levels<NT, R, COUNT, false, 1, LIST>(sc, s, rc, walk, launches, multi, copy, ysq, counts)
-                        : run_levels<NT, R, COUNT, false, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches, multi, copy, ysq, counts);
+        return lambert_only ? run_levels<NT, R, COUNT, true, 1, LIST>(sc, s, rc, walk, launches)
+                            : run_levels<NT, R, COUNT, true, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches);
+    return lambert_only ? run_levels<NT, R, COUNT, false, 1, LIST>(sc, s, rc, walk, launches)
+                        : run_levels<NT, R, COUNT, false, VRJ_MM_ALL, LIST>(sc, s, rc, walk, launches);
 }
-// `ysq` (render_passes): the batch is resolved by k_resolve_adaptive, which also keeps y_sq_sum; with `counts` as well
-// (vrj_render_counts) by k_resolve_counts.  A batch over rc.pixel_list (and rc.pixel_base) runs the LIST variants of the kernels
+// a batch over rc.pixel_list (and rc.pixel_base) runs the LIST variants of the kernels
 template <typename NT, typename R, bool COUNT>
-VrjStatus run_batch(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches, const MultiCalls *multi = nullptr,
-                    const ResolveCopy *copy = nullptr, double *ysq = nullptr, const CountsBatch *counts = nullptr) {
-    return rc.pixel_list ? run_materials<NT, R, COUNT, true>(sc, s, rc, whitted, walk, launches, multi, copy, ysq, counts)
-                         : run_materials<NT, R, COUNT, false>(sc, s, rc, whitted, walk, launches, multi, copy, ysq, counts);
+VrjStatus run_batch(const VrjScene *sc, Scratch *s, const RenderConst &rc, bool whitted, int walk, uint64_t *launches) {
+    return rc.pixel_list ? run_materials<NT, R, COUNT, true>(sc, s, rc, whitted, walk, launches)
+                         : run_materials<NT, R, COUNT, false>(sc, s, rc, whitted, walk, launches);
 }
 
 } // namespace vrjimpl

@@ -8,16 +8,16 @@
 
 namespace vrjimpl {
 #if VRJ_INST == 0
-template VrjStatus run_batch<float, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *); // the default path
+template VrjStatus run_batch<float, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *); // the default path
 #elif VRJ_INST == 1
-template VrjStatus run_batch<float, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
+template VrjStatus run_batch<float, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *);
 #elif VRJ_INST == 2
-template VrjStatus run_batch<double, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *); // VRJ_FILTER_F64
+template VrjStatus run_batch<double, double, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *); // VRJ_FILTER_F64
 #elif VRJ_INST == 3
-template VrjStatus run_batch<double, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
+template VrjStatus run_batch<double, double, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *);
 #elif VRJ_INST == 4
-template VrjStatus run_batch<float, float, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *); // VRJ_PRECISION_F32_FAST
+template VrjStatus run_batch<float, float, false>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *); // VRJ_PRECISION_F32_FAST
 #else
-template VrjStatus run_batch<float, float, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *, const MultiCalls *, const ResolveCopy *, double *, const CountsBatch *);
+template VrjStatus run_batch<float, float, true>(const VrjScene *, Scratch *, const RenderConst &, bool, int, uint64_t *);
 #endif
 } // namespace vrjimpl

@@ -752,17 +752,30 @@ struct AccumDev {
     double *weight, *weight_bias;
 };
 
-// accumulation_buffer.rs:44-60 applied for the batch's samples in sample order
-// R: precision of ColourXyz::from_photon (the colour matching functions); the accumulators are binary64 in both modes
-template <typename R>
-__global__ void k_resolve(AccumDev acc, const double2 *photons, uint32_t first, uint32_t npix, uint32_t batch_samples) {
-    uint32_t p = first + blockIdx.x * blockDim.x + threadIdx.x; // pixels [first, npix): a call's last batch resolves in pieces
-    if (p >= npix) return;
-    double sx = acc.sum[3 * p], sy = acc.sum[3 * p + 1], sz = acc.sum[3 * p + 2];
-    double bx = acc.bias[3 * p], by = acc.bias[3 * p + 1], bz = acc.bias[3 * p + 2];
-    double w = acc.weight[p], wb = acc.weight_bias[p];
-    for (uint32_t s = 0; s < batch_samples; s++) {
-        double2 ph = photons[(size_t)p * batch_samples + s]; // pixel-major: a thread walks its own 16 * batch_samples bytes
+// accumulation_buffer.rs:59: colour = sum * (1 / weight)
+template <typename I>
+__device__ __forceinline__ void store_colour(double *colour, I p, double sx, double sy, double sz, double w) {
+    double inv = 1.0 / w;
+    colour[3 * p] = sx * inv, colour[3 * p + 1] = sy * inv, colour[3 * p + 2] = sz * inv;
+}
+
+// One pixel's accumulator in registers: colour_sum (s), its Kahan compensation (b), weight (w), its compensation (wb), and
+// y_sq_sum (q) for the resolves that keep it.  Those load and store q themselves: a NULL-checked y_sq_sum pointer here
+// raises k_resolve_adaptive's register count.
+struct PixelAccum {
+    double sx, sy, sz, bx, by, bz, w, wb;
+    double q = 0.0;
+    template <typename I>
+    __device__ __forceinline__ void load(const AccumDev &acc, I p) {
+        sx = acc.sum[3 * p], sy = acc.sum[3 * p + 1], sz = acc.sum[3 * p + 2];
+        bx = acc.bias[3 * p], by = acc.bias[3 * p + 1], bz = acc.bias[3 * p + 2];
+        w = acc.weight[p], wb = acc.weight_bias[p];
+    }
+    // accumulation_buffer.rs:44-60 for one sample, and q = q + y * y, y being the sample's Y exactly as it enters colour_sum
+    // (the noise estimate of pass_count).  R: precision of ColourXyz::from_photon (the colour matching functions); the
+    // accumulators are binary64 in both modes.
+    template <typename R>
+    __device__ __forceinline__ void add(double2 ph) {
         // colour_xyz.rs:31-35.  A sample of intensity +0 (every primary miss and depth-limited path: 45 % of the bench frame)
         // contributes cmf * 0 = 0 whatever its wavelength; the seven exponentials are skipped and the Kahan update below,
         // which still runs, leaves the same sums (adding +0 or -0 to an accumulator that started at +0 is the identity)
@@ -777,47 +790,44 @@ __global__ void k_resolve(AccumDev acc, const double2 *photons, uint32_t first, 
         double tx = sx + yx, ty = sy + yy, tz = sz + yz;
         bx = (tx - sx) - yx, by = (ty - sy) - yy, bz = (tz - sz) - yz;
         sx = tx, sy = ty, sz = tz;
+        q = q + c.y * c.y;
     }
-    acc.sum[3 * p] = sx, acc.sum[3 * p + 1] = sy, acc.sum[3 * p + 2] = sz;
-    acc.bias[3 * p] = bx, acc.bias[3 * p + 1] = by, acc.bias[3 * p + 2] = bz;
-    acc.weight[p] = w, acc.weight_bias[p] = wb;
-    double inv = 1.0 / w;
-    acc.colour[3 * p] = sx * inv, acc.colour[3 * p + 1] = sy * inv, acc.colour[3 * p + 2] = sz * inv;
+    template <typename I>
+    __device__ __forceinline__ void store(const AccumDev &acc, I p) const {
+        acc.sum[3 * p] = sx, acc.sum[3 * p + 1] = sy, acc.sum[3 * p + 2] = sz;
+        acc.bias[3 * p] = bx, acc.bias[3 * p + 1] = by, acc.bias[3 * p + 2] = bz;
+        acc.weight[p] = w, acc.weight_bias[p] = wb;
+    }
+    template <typename I>
+    __device__ __forceinline__ void store_colour(double *colour, I p) const { vrj::store_colour(colour, p, sx, sy, sz, w); }
+};
+
+// the batch's samples applied in sample order
+template <typename R>
+__global__ void k_resolve(AccumDev acc, const double2 *photons, uint32_t first, uint32_t npix, uint32_t batch_samples) {
+    uint32_t p = first + blockIdx.x * blockDim.x + threadIdx.x; // pixels [first, npix): a call's last batch resolves in pieces
+    if (p >= npix) return;
+    PixelAccum a;
+    a.load(acc, p);
+    for (uint32_t s = 0; s < batch_samples; s++)
+        a.add<R>(photons[(size_t)p * batch_samples + s]); // pixel-major: a thread walks its own 16 * batch_samples bytes
+    a.store(acc, p);
+    a.store_colour(acc.colour, p);
 }
 
 // k_resolve for one pass of an adaptive render (render_passes): list position i holds tile pixel list[i] (pixel i when
 // `list` is NULL) and its samples are the batch's slots i * batch_samples + s.  Besides the Kahan update it keeps
-// ysq[pixel] = ysq + y * y in sample order, y being the sample's Y exactly as it enters colour_sum (the noise estimate of
-// pass_count).
+// ysq[pixel] = ysq + y * y in sample order.
 template <typename R>
 __global__ void k_resolve_adaptive(AccumDev acc, double *ysq, const uint32_t *list, const double2 *photons, uint32_t n, uint32_t batch_samples) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const uint32_t p = list ? list[i] : i;
-    double sx = acc.sum[3 * p], sy = acc.sum[3 * p + 1], sz = acc.sum[3 * p + 2];
-    double bx = acc.bias[3 * p], by = acc.bias[3 * p + 1], bz = acc.bias[3 * p + 2];
-    double w = acc.weight[p], wb = acc.weight_bias[p], q = ysq[p];
-    for (uint32_t s = 0; s < batch_samples; s++) { // accumulation_buffer.rs:44-60, as in k_resolve
-        double2 ph = photons[(size_t)i * batch_samples + s];
-        D3 c = d3(0.0, 0.0, 0.0);
-        if (__double_as_longlong(ph.y) != 0ll) c = convert<double>(cmf<R>((R)ph.x) * (R)ph.y);
-        const double weight = 1.0;
-        double wy = weight - wb;
-        double wt = w + wy;
-        wb = (wt - w) - wy;
-        w = wt;
-        double yx = c.x * weight - bx, yy = c.y * weight - by, yz = c.z * weight - bz;
-        double tx = sx + yx, ty = sy + yy, tz = sz + yz;
-        bx = (tx - sx) - yx, by = (ty - sy) - yy, bz = (tz - sz) - yz;
-        sx = tx, sy = ty, sz = tz;
-        q = q + c.y * c.y;
-    }
-    acc.sum[3 * p] = sx, acc.sum[3 * p + 1] = sy, acc.sum[3 * p + 2] = sz;
-    acc.bias[3 * p] = bx, acc.bias[3 * p + 1] = by, acc.bias[3 * p + 2] = bz;
-    acc.weight[p] = w, acc.weight_bias[p] = wb;
-    ysq[p] = q;
-    double inv = 1.0 / w;
-    acc.colour[3 * p] = sx * inv, acc.colour[3 * p + 1] = sy * inv, acc.colour[3 * p + 2] = sz * inv;
+    PixelAccum a;
+    a.load(acc, p), a.q = ysq[p];
+    for (uint32_t s = 0; s < batch_samples; s++) a.add<R>(photons[(size_t)i * batch_samples + s]);
+    a.store(acc, p), ysq[p] = a.q;
+    a.store_colour(acc.colour, p);
 }
 
 // ---- the passes of vrj_render_adaptive and vrj_render_progressive (render_passes; the header states the schedule) ----
@@ -1037,28 +1047,10 @@ __global__ void k_resolve_counts(AccumDev acc, double *ysq, const uint32_t *offs
     if (p >= npix) return;
     const uint32_t j0 = max(offset[p], b0), j1 = min(offset[p + 1], b1);
     if (j0 >= j1) return;
-    double sx = acc.sum[3 * p], sy = acc.sum[3 * p + 1], sz = acc.sum[3 * p + 2];
-    double bx = acc.bias[3 * p], by = acc.bias[3 * p + 1], bz = acc.bias[3 * p + 2];
-    double w = acc.weight[p], wb = acc.weight_bias[p], q = ysq[p];
-    for (uint32_t j = j0; j < j1; j++) { // accumulation_buffer.rs:44-60, as in k_resolve
-        double2 ph = photons[j - b0];
-        D3 c = d3(0.0, 0.0, 0.0);
-        if (__double_as_longlong(ph.y) != 0ll) c = convert<double>(cmf<R>((R)ph.x) * (R)ph.y);
-        const double weight = 1.0;
-        double wy = weight - wb;
-        double wt = w + wy;
-        wb = (wt - w) - wy;
-        w = wt;
-        double yx = c.x * weight - bx, yy = c.y * weight - by, yz = c.z * weight - bz;
-        double tx = sx + yx, ty = sy + yy, tz = sz + yz;
-        bx = (tx - sx) - yx, by = (ty - sy) - yy, bz = (tz - sz) - yz;
-        sx = tx, sy = ty, sz = tz;
-        q = q + c.y * c.y;
-    }
-    acc.sum[3 * p] = sx, acc.sum[3 * p + 1] = sy, acc.sum[3 * p + 2] = sz;
-    acc.bias[3 * p] = bx, acc.bias[3 * p + 1] = by, acc.bias[3 * p + 2] = bz;
-    acc.weight[p] = w, acc.weight_bias[p] = wb;
-    ysq[p] = q;
+    PixelAccum a;
+    a.load(acc, p), a.q = ysq[p];
+    for (uint32_t j = j0; j < j1; j++) a.add<R>(photons[j - b0]);
+    a.store(acc, p), ysq[p] = a.q;
 }
 
 // vrj_plan_counts: one thread per pixel, counts[p] = plan_count of its state; ctr: samples, pixels planned (c > 0),
@@ -1091,30 +1083,12 @@ __global__ void k_resolve_multi(MultiCalls mc, const double2 *photons, uint32_t 
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= npix * mc.n) return; // npix * n <= 2^32 is checked by the host
     const uint32_t p = i / mc.n, c = i - p * mc.n;
-    double sx = 0.0, sy = 0.0, sz = 0.0, bx = 0.0, by = 0.0, bz = 0.0, w = 0.0, wb = 0.0;
+    PixelAccum a{};
     const uint32_t s0 = mc.first[c], s1 = s0 + mc.count[c];
-    for (uint32_t s = s0; s < s1; s++) { // accumulation_buffer.rs:44-60, as in k_resolve
-        double2 ph = photons[(size_t)p * batch_samples + s];
-        D3 col = d3(0.0, 0.0, 0.0);
-        if (__double_as_longlong(ph.y) != 0ll) col = convert<double>(cmf<R>((R)ph.x) * (R)ph.y);
-        const double weight = 1.0;
-        double wy = weight - wb;
-        double wt = w + wy;
-        wb = (wt - w) - wy;
-        w = wt;
-        double yx = col.x * weight - bx, yy = col.y * weight - by, yz = col.z * weight - bz;
-        double tx = sx + yx, ty = sy + yy, tz = sz + yz;
-        bx = (tx - sx) - yx, by = (ty - sy) - yy, bz = (tz - sz) - yz;
-        sx = tx, sy = ty, sz = tz;
-    }
+    for (uint32_t s = s0; s < s1; s++) a.add<R>(photons[(size_t)p * batch_samples + s]);
     const size_t q = (size_t)c * npix + p;
-    double inv = 1.0 / w;
-    mc.out.colour[3 * q] = sx * inv, mc.out.colour[3 * q + 1] = sy * inv, mc.out.colour[3 * q + 2] = sz * inv;
-    if (mc.full) {
-        mc.out.sum[3 * q] = sx, mc.out.sum[3 * q + 1] = sy, mc.out.sum[3 * q + 2] = sz;
-        mc.out.bias[3 * q] = bx, mc.out.bias[3 * q + 1] = by, mc.out.bias[3 * q + 2] = bz;
-        mc.out.weight[q] = w, mc.out.weight_bias[q] = wb;
-    }
+    a.store_colour(mc.out.colour, q);
+    if (mc.full) a.store(mc.out, q);
 }
 
 // debug output (VrjAccumOut.photons) is sample-major: [(sample * npix + pixel)]

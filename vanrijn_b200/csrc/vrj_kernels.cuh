@@ -44,12 +44,6 @@
 #ifndef VRJ_FIRST_UNSORTED
 #define VRJ_FIRST_UNSORTED 1
 #endif
-#ifndef VRJ_SHADOW_QUAD
-#define VRJ_SHADOW_QUAD 1
-#endif
-#ifndef VRJ_TAIL_QUAD
-#define VRJ_TAIL_QUAD 1
-#endif
 #ifndef VRJ_TRACE4_MINB
 #define VRJ_TRACE4_MINB 5
 #endif
@@ -283,6 +277,16 @@ __global__ void __launch_bounds__(128, sizeof(R) == 4 ? VRJ_SHADE_MINB_F32 : VRJ
 }
 
 // ---- k_trace: BVH traversal for the staged rays; updates hits / tbest where a triangle is closer ----
+// ListRaySource and PrimaryRaySource: the walk's constants are formed from the ray that the source's load() yields
+template <typename Format, typename Source, typename R>
+__device__ __forceinline__ uint32_t setup_from_ray(const DevScene &sc, Source &source, uint32_t r, TriRayT<R> &tr,
+                                                   typename Format::Ray &fr, HitT<R> &best) {
+    V3<R> o, d;
+    source.load(r, o, d, best);
+    tr = tri_ray(o, d);
+    fr = Format::ray(sc, o, d);
+    return r;
+}
 struct ListRaySource {
     const PathQueue &q;
     const TraceBuffers &tb;
@@ -293,19 +297,18 @@ struct ListRaySource {
         int2 h = tb.hits[j];
         best.item = h.x, best.tri = h.y, best.t = (R)tb.tbest[j];
     }
-    template <typename NT, typename R>
-    __device__ __forceinline__ uint32_t load_setup(uint32_t r, TriRayT<R> &tr, FilterRay<NT> &fr, HitT<R> &best) {
-        V3<R> o, d;
-        load(r, o, d, best);
-        tr = tri_ray(o, d);
-        fr = filter_ray<NT>(o, d);
-        return r;
+    template <typename Format, typename R>
+    __device__ __forceinline__ uint32_t load_setup(const DevScene &sc, uint32_t r, TriRayT<R> &tr, typename Format::Ray &fr, HitT<R> &best) {
+        return setup_from_ray<Format>(sc, *this, r, tr, fr, best);
     }
 };
-// rays staged as records: nothing to compute, three 256-bit loads; the handle is the queue entry itself
+// rays staged as records (the 2-wide f32 walk in binary64): nothing to compute, three 256-bit loads; the handle is the queue
+// entry itself
 struct RecRaySource {
     const TraceBuffers &tb;
-    __device__ __forceinline__ uint32_t load_setup(uint32_t r, TriRayT<double> &tr, FilterRay<float> &fr, HitT<double> &best) {
+    template <typename Format>
+    __device__ __forceinline__ uint32_t load_setup(const DevScene &, uint32_t r, TriRayT<double> &tr, FilterRay<float> &fr, HitT<double> &best) {
+        static_assert(std::is_same<Format, Nodes2<float>>::value, "records hold the constants of the 2-wide f32 walk");
         return load_trace_rec(tb.recs, r, tr, fr, best);
     }
 };
@@ -330,13 +333,9 @@ struct PrimaryRaySource {
         int2 h = tb.hits[j];
         best.item = h.x, best.tri = h.y, best.t = (R)tb.tbest[j];
     }
-    template <typename NT, typename R>
-    __device__ __forceinline__ uint32_t load_setup(uint32_t r, TriRayT<R> &tr, FilterRay<NT> &fr, HitT<R> &best) {
-        V3<R> o, d;
-        load(r, o, d, best);
-        tr = tri_ray(o, d);
-        fr = filter_ray<NT>(o, d);
-        return r;
+    template <typename Format, typename R>
+    __device__ __forceinline__ uint32_t load_setup(const DevScene &sc, uint32_t r, TriRayT<R> &tr, typename Format::Ray &fr, HitT<R> &best) {
+        return setup_from_ray<Format>(sc, *this, r, tr, fr, best);
     }
 };
 struct ListHitSink {
@@ -350,102 +349,57 @@ struct ListHitSink {
     }
 };
 
-template <typename NT, typename R, bool COUNT>
-__global__ void VRJ_TRACE_BOUNDS(R) k_trace(DevScene sc, PathQueue q, TraceBuffers tb, const uint32_t *list_count,
-                                               uint32_t *work, unsigned long long *stats, const uint32_t *tail_done) {
+// the body of every trace kernel: nothing to do when k_tail has already finished the level (tail_done set), else walk the
+// staged rays and add the traversal counters to the stats
+template <typename Format, typename R, bool COUNT, typename Source, typename Sink>
+__device__ __forceinline__ void trace_staged(const DevScene &sc, const uint32_t *list_count, uint32_t *work, unsigned long long *stats,
+                                             const uint32_t *tail_done, Source source, Sink sink) {
     if (tail_done && *tail_done) return;
     const uint32_t n = *list_count;
-    ListRaySource source{q, tb};
-    ListHitSink sink{tb};
     TraceCounters tc = {0, 0};
-    trace_persistent<NT, R, COUNT>(sc, n, work, source, sink, tc);
+    trace_persistent<Format, R, COUNT>(sc, n, work, source, sink, tc);
     if (COUNT) {
         LocalStats ls;
         ls.clear();
         ls.v[ST_NODES] = tc.node_visits, ls.v[ST_TRIS] = tc.tri_tests;
         ls.flush(stats);
     }
+}
+
+template <typename NT, typename R, bool COUNT>
+__global__ void VRJ_TRACE_BOUNDS(R) k_trace(DevScene sc, PathQueue q, TraceBuffers tb, const uint32_t *list_count,
+                                               uint32_t *work, unsigned long long *stats, const uint32_t *tail_done) {
+    trace_staged<Nodes2<NT>, R, COUNT>(sc, list_count, work, stats, tail_done, ListRaySource{q, tb}, ListHitSink{tb});
 }
 
 // k_trace for the camera rays of a batch
 template <typename NT, typename R, bool COUNT, bool LIST = false>
 __global__ void VRJ_TRACE_BOUNDS(R) k_trace_primary(DevScene sc, RenderConst rc, TraceBuffers tb, const uint32_t *list_count, uint32_t *work,
                                                     unsigned long long *stats) {
-    const uint32_t n = *list_count;
-    PrimaryRaySource<LIST> source{sc, rc, tb};
-    ListHitSink sink{tb};
-    TraceCounters tc = {0, 0};
-    trace_persistent<NT, R, COUNT>(sc, n, work, source, sink, tc);
-    if (COUNT) {
-        LocalStats ls;
-        ls.clear();
-        ls.v[ST_NODES] = tc.node_visits, ls.v[ST_TRIS] = tc.tri_tests;
-        ls.flush(stats);
-    }
+    trace_staged<Nodes2<NT>, R, COUNT>(sc, list_count, work, stats, nullptr, PrimaryRaySource<LIST>{sc, rc, tb}, ListHitSink{tb});
 }
 
 // k_trace over ready-to-walk records (camera rays and bounce rays alike): the default walk of the parity path
 template <bool COUNT>
 __global__ void VRJ_TRACE_BOUNDS(double) k_trace_rec(DevScene sc, TraceBuffers tb, const uint32_t *list_count, uint32_t *work,
                                                      unsigned long long *stats, const uint32_t *tail_done) {
-    if (tail_done && *tail_done) return;
-    const uint32_t n = *list_count;
-    RecRaySource source{tb};
-    RecHitSink sink{tb};
-    TraceCounters tc = {0, 0};
-    trace_persistent<float, double, COUNT>(sc, n, work, source, sink, tc);
-    if (COUNT) {
-        LocalStats ls;
-        ls.clear();
-        ls.v[ST_NODES] = tc.node_visits, ls.v[ST_TRIS] = tc.tri_tests;
-        ls.flush(stats);
-    }
+    trace_staged<Nodes2<float>, double, COUNT>(sc, list_count, work, stats, tail_done, RecRaySource{tb}, RecHitSink{tb});
 }
 
 // the same launch over the 4-wide form of the tree (VRJ_FILTER_F32X4)
 template <bool COUNT, bool PRIMARY, bool LIST = false>
 __global__ void __launch_bounds__(128, VRJ_TRACE4_MINB) k_trace4(DevScene sc, RenderConst rc, PathQueue q, TraceBuffers tb, const uint32_t *list_count,
                                                                  uint32_t *work, unsigned long long *stats, const uint32_t *tail_done) {
-    if (tail_done && *tail_done) return;
-    const uint32_t n = *list_count;
-    ListHitSink sink{tb};
-    TraceCounters tc = {0, 0};
-    if (PRIMARY) {
-        PrimaryRaySource<LIST> source{sc, rc, tb};
-        trace_persistent_quad<COUNT>(sc, n, work, source, sink, tc);
-    } else {
-        ListRaySource source{q, tb};
-        trace_persistent_quad<COUNT>(sc, n, work, source, sink, tc);
-    }
-    if (COUNT) {
-        LocalStats ls;
-        ls.clear();
-        ls.v[ST_NODES] = tc.node_visits, ls.v[ST_TRIS] = tc.tri_tests;
-        ls.flush(stats);
-    }
+    if (PRIMARY) trace_staged<Nodes4, double, COUNT>(sc, list_count, work, stats, tail_done, PrimaryRaySource<LIST>{sc, rc, tb}, ListHitSink{tb});
+    else trace_staged<Nodes4, double, COUNT>(sc, list_count, work, stats, tail_done, ListRaySource{q, tb}, ListHitSink{tb});
 }
 
 // the same launch over 16-bit nodes (VRJ_FILTER_Q16)
 template <bool COUNT, bool PRIMARY, bool LIST = false>
 __global__ void __launch_bounds__(128, VRJ_TRACE_MINB) k_traceq(DevScene sc, RenderConst rc, PathQueue q, TraceBuffers tb, const uint32_t *list_count,
                                                                 uint32_t *work, unsigned long long *stats, const uint32_t *tail_done) {
-    if (tail_done && *tail_done) return;
-    const uint32_t n = *list_count;
-    ListHitSink sink{tb};
-    TraceCounters tc = {0, 0};
-    if (PRIMARY) {
-        PrimaryRaySource<LIST> source{sc, rc, tb};
-        trace_persistent_q16<COUNT>(sc, n, work, source, sink, tc);
-    } else {
-        ListRaySource source{q, tb};
-        trace_persistent_q16<COUNT>(sc, n, work, source, sink, tc);
-    }
-    if (COUNT) {
-        LocalStats ls;
-        ls.clear();
-        ls.v[ST_NODES] = tc.node_visits, ls.v[ST_TRIS] = tc.tri_tests;
-        ls.flush(stats);
-    }
+    if (PRIMARY) trace_staged<NodesQ16, double, COUNT>(sc, list_count, work, stats, tail_done, PrimaryRaySource<LIST>{sc, rc, tb}, ListHitSink{tb});
+    else trace_staged<NodesQ16, double, COUNT>(sc, list_count, work, stats, tail_done, ListRaySource{q, tb}, ListHitSink{tb});
 }
 
 // ---- one level of the integrator for one path (shared by k_shade and k_tail) ----
@@ -528,7 +482,7 @@ __device__ __forceinline__ bool shade_entry(const DevScene &sc, const RenderCons
             V3<R> ldir = V3<R>{(R)Lt.dir[0], (R)Lt.dir[1], (R)Lt.dir[2]};
             V3<R> so, sd;
             biased_ray(h.location, ldir, (R)rc.bias, so, sd);
-            HitT<R> sh = trace_closest<NT, COUNT, true, R, VRJ_SHADOW_QUAD != 0>(sc, so, sd, tc);
+            HitT<R> sh = trace_closest<NT, COUNT, true, R, true>(sc, so, sd, tc);
             ls.v[ST_SHADOW]++;
             R term;
             if (sh.item >= 0) {
@@ -737,7 +691,7 @@ __global__ void __launch_bounds__(128, 2) k_tail(DevScene sc, RenderConst rc, Pa
         if (alive) {
             TraceCounters tc = {0, 0};
             // one lane, one path: what it waits on is the chain of dependent node fetches, and the 4-wide tree halves it
-            HitT<R> h = trace_closest<NT, COUNT, false, R, VRJ_TAIL_QUAD != 0>(sc, p.o, p.d, tc);
+            HitT<R> h = trace_closest<NT, COUNT, false, R, true>(sc, p.o, p.d, tc);
             if (COUNT) ls.v[ST_NODES] += tc.node_visits, ls.v[ST_TRIS] += tc.tri_tests;
             alive = shade_entry<NT, COUNT, WHITTED, MM, LIST>(sc, rc, p, make_int2(h.item, h.tri), h.t, false, [](V3<R> &, V3<R> &) {}, photons, ls);
         }

@@ -10,6 +10,8 @@
 #pragma once
 #include "vrj_device.cuh"
 
+#include <type_traits>
+
 namespace vrj {
 
 struct ItemDev {
@@ -47,17 +49,6 @@ struct DevScene {
     double cam[3];
 };
 
-#ifndef VRJ_TRACE_TRIRAY_SMEM
-#define VRJ_TRACE_TRIRAY_SMEM 0
-#endif
-// Experiment (north_star: "node loads staged through shared memory"): K > 0 keeps the top K levels of the first mesh's
-// tree (2^K - 1 wide nodes of 64 bytes, heap-ordered) in shared memory; each CTA copies them in at kernel start and the
-// walk reads those nodes with LDS instead of LDG.  Off by default: measured no faster (profiles/README.md, round 2) --
-// the top of the tree already hits L1, and both paths go through the same load/store unit.
-#ifndef VRJ_TRACE_SMEM_LEVELS
-#define VRJ_TRACE_SMEM_LEVELS 0
-#endif
-#define VRJ_SMEM_TAG 0x40000000
 template <typename R>
 struct HitT {
     R t;
@@ -141,6 +132,12 @@ __device__ __forceinline__ T filter_limit(R t) {
     typedef FilterTraits<T> F;
     return F::up(t * (R(1) + R(4) * (R)F::rel()));
 }
+// the constants of no ray (a lane that holds none)
+template <typename T>
+__device__ __forceinline__ void clear_filter(FilterRay<T> &f) {
+#pragma unroll
+    for (int k = 0; k < 3; k++) f.id[k] = f.cn[k] = f.cf[k] = (T)0;
+}
 template <typename T>
 __device__ __forceinline__ bool box_filter(const FilterRay<T> &f, T lox, T hix, T loy, T hiy, T loz, T hiz, T t_limit,
                                            T &enter) {
@@ -221,124 +218,229 @@ __device__ __forceinline__ void load_tri_nrm(const DevScene &sc, int tri, F3 &n0
     n0 = F3{a.x, a.y, a.z}, n1 = F3{a.w, b.x, b.y}, n2 = F3{b.z, b.w, c.x};
 }
 
-// One BoundingVolumeHierarchy::intersect: closest triangle with distance rule "later DFS leaf wins ties".
-// `t_limit` (distance of the best hit found in EARLIER objects) only prunes; the caller merges.
-template <typename NT, bool COUNT, bool ANY, typename R>
-__device__ __forceinline__ void bvh_closest(const DevScene &sc, int root, const TriRayT<R> &tr, const FilterRay<NT> &fr,
-                                            R t_limit, R &best_t, int &best_tri, TraceCounters &cnt) {
-    int stack[32];
-    int sp = 0;
-    int cur = root;
-    best_t = real_inf<R>(), best_tri = -1;
-    // prune bound in NodeT, rounded up, with the relative slack of the filter
-    NT limit = filter_limit<NT>(t_limit);
-    while (true) {
-        while (cur >= 0) {
-            WideNode<NT> n;
-            load_node(sc, cur, n);
-            if (COUNT) cnt.node_visits += 2;
-            NT e0, e1;
-            bool h0 = box_filter(fr, n.c0[0], n.c0[1], n.c0[2], n.c0[3], n.c0[4], n.c0[5], limit, e0);
-            bool h1 = box_filter(fr, n.c1[0], n.c1[1], n.c1[2], n.c1[3], n.c1[4], n.c1[5], limit, e1);
-            if (h0 && h1) {
-                bool swap = e1 < e0;
-                stack[sp++] = swap ? n.left : n.right;
-                cur = swap ? n.right : n.left;
-            } else if (h0 || h1) {
-                cur = h0 ? n.left : n.right;
-            } else {
-                cur = sp ? stack[--sp] : VRJ_LEAF_DONE;
-            }
-        }
-        if (cur == VRJ_LEAF_DONE) break;
-        {
-            int tri = ~cur;
-            V3<R> v0, v1, v2, loc;
-            uint32_t mat, pid;
-            load_tri_pos(sc, tri, v0, v1, v2, mat, pid);
-            if (COUNT) cnt.tri_tests += 1;
-            R dist, b0, b1, b2;
-            if (triangle_test(tr, v0, v1, v2, dist, b0, b1, b2, loc)) {
-                if (dist < best_t || (dist == best_t && tri > best_tri)) {
-                    best_t = dist, best_tri = tri;
-                    if (ANY) return;
-                    limit = filter_limit<NT>(fmin(best_t, t_limit));
-                }
-            }
-        }
-        cur = sp ? stack[--sp] : VRJ_LEAF_DONE;
-        if (cur == VRJ_LEAF_DONE) break;
-    }
-}
+// ------------------------------------------------------------------------------------------
+// The node formats.  Each gives the walks below its per-ray filter constants (Ray, formed by ray(sc, o, d)), its prune
+// bound for a best distance t (limit(t)), its stack depth, the node steps the persistent engine runs between warp votes
+// (batch(sc)), and one node step: fetch node `cur`, test its children, push the farther hit children and descend into the
+// nearest.  When no child is hit, step() calls `miss` instead, with `cur` still naming the node: the caller's pop or the
+// end of the BVH.
 
-// The same query over the 4-wide form of the tree: half the dependent fetches, which is what a single thread following one
-// path to its end (k_tail) waits on.  Same filter, same exact test, same tie rule.
-__device__ __forceinline__ void cswap4(float &ka, int &ra, float &kb, int &rb) {
+// 2-wide nodes over NT boxes (nodes32 / nodes64)
+template <typename NT>
+struct Nodes2 {
+    typedef FilterRay<NT> Ray;
+    typedef NT Limit;
+    static constexpr int STACK = 32;
+    static __device__ __forceinline__ int batch(const DevScene &sc) { return sc.node_batch; }
+    template <typename R>
+    static __device__ __forceinline__ Ray ray(const DevScene &, V3<R> o, V3<R> d) { return filter_ray<NT>(o, d); }
+    template <typename R>
+    static __device__ __forceinline__ NT limit(R t) { return filter_limit<NT>(t); }
+    template <bool COUNT, typename Miss>
+    static __device__ __forceinline__ void step(const DevScene &sc, const Ray &fr, NT limit, int &cur, int *stack, int &sp,
+                                                TraceCounters &cnt, Miss miss) {
+        WideNode<NT> n;
+        load_node(sc, cur, n);
+        if (COUNT) cnt.node_visits += 2;
+        NT e0, e1;
+        bool h0 = box_filter(fr, n.c0[0], n.c0[1], n.c0[2], n.c0[3], n.c0[4], n.c0[5], limit, e0);
+        bool h1 = box_filter(fr, n.c1[0], n.c1[1], n.c1[2], n.c1[3], n.c1[4], n.c1[5], limit, e1);
+        if (h0 && h1) {
+            bool swap = e1 < e0;
+            stack[sp++] = swap ? n.left : n.right;
+            cur = swap ? n.right : n.left;
+        } else if (h0 || h1) {
+            cur = h0 ? n.left : n.right;
+        } else {
+            miss();
+        }
+    }
+};
+
+// 4-wide nodes with f32 boxes (nodes4, vrj_scene_prep.cuh): one 128-byte fetch decides four boxes, the hit children are
+// ordered by entry distance with a 5-comparator network, the nearest is followed and the others are pushed farthest first.
+// Same filter as Nodes2<float>: results are identical to the 2-wide walk; only the number of dependent fetches per ray (about
+// half) differs.
+__device__ __forceinline__ void cswap(float &ka, int &ra, float &kb, int &rb) {
     const bool sw = kb < ka;
     const float k = sw ? kb : ka, K = sw ? ka : kb;
     const int r = sw ? rb : ra, R = sw ? ra : rb;
     ka = k, kb = K, ra = r, rb = R;
 }
-template <bool COUNT, bool ANY, typename R>
-__device__ __forceinline__ void bvh_closest_quad(const DevScene &sc, int root, const TriRayT<R> &tr, const FilterRay<float> &fr, R t_limit,
-                                                 R &best_t, int &best_tri, TraceCounters &cnt) {
-    int stack[48];
+struct Nodes4 {
+    typedef FilterRay<float> Ray;
+    typedef float Limit;
+    static constexpr int STACK = 48; // up to three pushes per 4-wide level, 16 levels
+    static __device__ __forceinline__ int batch(const DevScene &sc) { return sc.node_batch4; }
+    template <typename R>
+    static __device__ __forceinline__ Ray ray(const DevScene &, V3<R> o, V3<R> d) { return filter_ray<float>(o, d); }
+    template <typename R>
+    static __device__ __forceinline__ float limit(R t) { return filter_limit<float>(t); }
+    template <bool COUNT, typename Miss>
+    static __device__ __forceinline__ void step(const DevScene &sc, const Ray &fr, float limit, int &cur, int *stack, int &sp,
+                                                TraceCounters &cnt, Miss miss) {
+        const float4 *p = sc.nodes4 + (size_t)cur * 8;
+        float4 a, b, c, d, e, f, g, h;
+        ldg256(p, a, b);
+        ldg256(p + 2, c, d);
+        ldg256(p + 4, e, f);
+        ldg256(p + 6, g, h);
+        if (COUNT) cnt.node_visits += 4;
+        float k0, k1, k2, k3;
+        const bool h0 = box_filter(fr, a.x, a.y, a.z, a.w, b.x, b.y, limit, k0);
+        const bool h1 = box_filter(fr, b.z, b.w, c.x, c.y, c.z, c.w, limit, k1);
+        const bool h2 = box_filter(fr, d.x, d.y, d.z, d.w, e.x, e.y, limit, k2);
+        const bool h3 = box_filter(fr, e.z, e.w, f.x, f.y, f.z, f.w, limit, k3);
+        int r0 = __float_as_int(g.x), r1 = __float_as_int(g.y), r2 = __float_as_int(g.z), r3 = __float_as_int(g.w);
+        const float inf = CUDART_INF_F;
+        k0 = h0 ? k0 : inf, k1 = h1 ? k1 : inf, k2 = h2 ? k2 : inf, k3 = h3 ? k3 : inf;
+        const int nh = (int)h0 + (int)h1 + (int)h2 + (int)h3;
+        // misses carry +inf and sink to the end; a hit's key is finite (its box test passed ep <= limit)
+        cswap(k0, r0, k1, r1), cswap(k2, r2, k3, r3), cswap(k0, r0, k2, r2), cswap(k1, r1, k3, r3), cswap(k1, r1, k2, r2);
+        if (nh == 0) {
+            miss();
+        } else {
+            if (nh > 3) stack[sp++] = r3;
+            if (nh > 2) stack[sp++] = r2;
+            if (nh > 1) stack[sp++] = r1;
+            cur = r0;
+        }
+    }
+};
+
+// 2-wide nodes on a 16-bit grid (nodesq, VRJ_FILTER_Q16): half the bytes per step.  A box plane is qlo + q * qcell; with
+// A = qcell / d (binary32) and B = (qlo - o) / d - 2^23 * A (formed in binary64 from the ROUNDED A, then rounded to binary32
+// away from the ray's interval, with a pad for q * (A - qcell / d)), the parameter of the plane is fma(2^23 + q, A, B):
+// one PRMT builds the float 2^23 + q from a 16-bit field, the bias cancels inside the fused multiply-add.  The box a ray
+// sees is at most two cells larger per side than the real one (one from the outward quantisation, one from rounding B),
+// never smaller; every triangle is still decided by the exact binary64 test, so results do not change.  All meshes share
+// the scene's grid, so a ray's constants hold for every BVH it visits.
+struct FilterRayQ {
+    float A[3], Bn[3], Bf[3];
+    uint32_t neg; // bit k: the direction is negative on axis k (the near plane is the box's hi plane)
+};
+__device__ __forceinline__ FilterRayQ filter_ray_q(const DevScene &sc, D3 o, D3 d) {
+    FilterRayQ f;
+    const double oo[3] = {o.x, o.y, o.z}, dd[3] = {d.x, d.y, d.z};
+    f.neg = 0;
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+        double id = 1.0 / dd[k];
+        if (!(fabs(id) <= 1e18)) id = copysign(1e18, dd[k]);
+        const float A = __double2float_rn(sc.qcell[k] * id);
+        const double shift = (sc.qlo[k] - oo[k]) * id;
+        const double B = shift - 8388608.0 * (double)A;
+        // q * (A - cell/d) <= 65535 * 2^-24 * |A|;  binary64 rounding of `shift` and B;  a floor so the pad is never zero
+        const double pad = fabs((double)A) * 0.0079 + (fabs(shift) + fabs(B)) * 1e-15 + 1e-300;
+        f.A[k] = A, f.Bn[k] = __double2float_rd(B - pad), f.Bf[k] = __double2float_ru(B + pad);
+        if (id < 0.0) f.neg |= 1u << k;
+    }
+    return f;
+}
+__device__ __forceinline__ void clear_filter(FilterRayQ &f) {
+    f.neg = 0;
+#pragma unroll
+    for (int k = 0; k < 3; k++) f.A[k] = f.Bn[k] = f.Bf[k] = 0.f;
+}
+struct NodesQ16 {
+    typedef FilterRayQ Ray;
+    typedef float Limit;
+    static constexpr int STACK = 32;
+    static __device__ __forceinline__ int batch(const DevScene &sc) { return sc.node_batch; }
+    static __device__ __forceinline__ Ray ray(const DevScene &sc, D3 o, D3 d) { return filter_ray_q(sc, o, d); }
+    template <typename R>
+    static __device__ __forceinline__ float limit(R t) { return filter_limit<float>(t); }
+    // parameter interval of child `sel` (0x7610: low halves, 0x7632: high halves) of the node words
+    static __device__ __forceinline__ bool child_test(const Ray &fr, float limit, uint32_t nx, uint32_t fx, uint32_t ny, uint32_t fy,
+                                                      uint32_t nz, uint32_t fz, uint32_t sel, float &enter) {
+        typedef FilterTraits<float> F;
+        const float qnx = __uint_as_float(__byte_perm(nx, 0x4b000000u, sel)), qfx = __uint_as_float(__byte_perm(fx, 0x4b000000u, sel));
+        const float qny = __uint_as_float(__byte_perm(ny, 0x4b000000u, sel)), qfy = __uint_as_float(__byte_perm(fy, 0x4b000000u, sel));
+        const float qnz = __uint_as_float(__byte_perm(nz, 0x4b000000u, sel)), qfz = __uint_as_float(__byte_perm(fz, 0x4b000000u, sel));
+        const float tn = fmaxf(fmaxf(fmaf(qnx, fr.A[0], fr.Bn[0]), fmaf(qny, fr.A[1], fr.Bn[1])), fmaf(qnz, fr.A[2], fr.Bn[2]));
+        const float tf = fminf(fminf(fmaf(qfx, fr.A[0], fr.Bf[0]), fmaf(qfy, fr.A[1], fr.Bf[1])), fmaf(qfz, fr.A[2], fr.Bf[2]));
+        const float ep = fmaf(-F::rel(), fabsf(tn), tn), xp = fmaf(F::rel(), fabsf(tf), tf);
+        enter = ep;
+        return (ep <= xp) && (xp >= 0.f) && (ep <= limit);
+    }
+    template <bool COUNT, typename Miss>
+    static __device__ __forceinline__ void step(const DevScene &sc, const Ray &fr, float limit, int &cur, int *stack, int &sp,
+                                                TraceCounters &cnt, Miss miss) {
+        const uint4 *p = sc.nodesq + (size_t)cur * 2;
+        uint4 a, b;
+        asm volatile("ld.global.nc.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                     : "=r"(a.x), "=r"(a.y), "=r"(a.z), "=r"(a.w), "=r"(b.x), "=r"(b.y), "=r"(b.z), "=r"(b.w)
+                     : "l"(p));
+        if (COUNT) cnt.node_visits += 2;
+        const bool ngx = fr.neg & 1u, ngy = fr.neg & 2u, ngz = fr.neg & 4u;
+        const uint32_t nx = ngx ? a.y : a.x, fx = ngx ? a.x : a.y;
+        const uint32_t ny = ngy ? a.w : a.z, fy = ngy ? a.z : a.w;
+        const uint32_t nz = ngz ? b.y : b.x, fz = ngz ? b.x : b.y;
+        float e0, e1;
+        const bool h0 = child_test(fr, limit, nx, fx, ny, fy, nz, fz, 0x7610u, e0);
+        const bool h1 = child_test(fr, limit, nx, fx, ny, fy, nz, fz, 0x7632u, e1);
+        const int left = (int)b.z, right = (int)b.w;
+        if (h0 && h1) {
+            bool swap = e1 < e0;
+            stack[sp++] = swap ? left : right;
+            cur = swap ? right : left;
+        } else if (h0 || h1) {
+            cur = h0 ? left : right;
+        } else {
+            miss();
+        }
+    }
+};
+
+// The leaf of triangle `tri`: the exact Triangle::intersect, and the rule "later DFS leaf wins ties" inside one BVH
+// (bounding_volume_hierarchy.rs:77-92).  Returns true when the triangle became the best.
+template <bool COUNT, typename R>
+__device__ __forceinline__ bool leaf_test(const DevScene &sc, const TriRayT<R> &tr, int tri, R &best_t, int &best_tri,
+                                          TraceCounters &cnt) {
+    V3<R> v0, v1, v2, loc;
+    uint32_t mat, pid;
+    load_tri_pos(sc, tri, v0, v1, v2, mat, pid);
+    if (COUNT) cnt.tri_tests += 1;
+    R dist, b0, b1, b2;
+    if (triangle_test(tr, v0, v1, v2, dist, b0, b1, b2, loc)) {
+        if (dist < best_t || (dist == best_t && tri > best_tri)) {
+            best_t = dist, best_tri = tri;
+            return true;
+        }
+    }
+    return false;
+}
+
+// One BoundingVolumeHierarchy::intersect by one thread: closest triangle with distance rule "later DFS leaf wins ties".
+// `t_limit` (distance of the best hit found in EARLIER objects) only prunes; the caller merges.
+template <typename Format, bool COUNT, bool ANY, typename R>
+__device__ __forceinline__ void bvh_closest(const DevScene &sc, int root, const TriRayT<R> &tr, const typename Format::Ray &fr,
+                                            R t_limit, R &best_t, int &best_tri, TraceCounters &cnt) {
+    int stack[Format::STACK];
     int sp = 0;
     int cur = root;
     best_t = real_inf<R>(), best_tri = -1;
-    float limit = filter_limit<float>(t_limit);
+    // prune bound in the node type, rounded up, with the relative slack of the filter
+    typename Format::Limit limit = Format::limit(t_limit);
     while (true) {
         while (cur >= 0) {
-            const float4 *p = sc.nodes4 + (size_t)cur * 8;
-            float4 a, b, c, d, e, f, g, h;
-            ldg256(p, a, b);
-            ldg256(p + 2, c, d);
-            ldg256(p + 4, e, f);
-            ldg256(p + 6, g, h);
-            if (COUNT) cnt.node_visits += 4;
-            float k0, k1, k2, k3;
-            const bool h0 = box_filter(fr, a.x, a.y, a.z, a.w, b.x, b.y, limit, k0);
-            const bool h1 = box_filter(fr, b.z, b.w, c.x, c.y, c.z, c.w, limit, k1);
-            const bool h2 = box_filter(fr, d.x, d.y, d.z, d.w, e.x, e.y, limit, k2);
-            const bool h3 = box_filter(fr, e.z, e.w, f.x, f.y, f.z, f.w, limit, k3);
-            int r0 = __float_as_int(g.x), r1 = __float_as_int(g.y), r2 = __float_as_int(g.z), r3 = __float_as_int(g.w);
-            const float inf = CUDART_INF_F;
-            k0 = h0 ? k0 : inf, k1 = h1 ? k1 : inf, k2 = h2 ? k2 : inf, k3 = h3 ? k3 : inf;
-            const int nh = (int)h0 + (int)h1 + (int)h2 + (int)h3;
-            cswap4(k0, r0, k1, r1), cswap4(k2, r2, k3, r3), cswap4(k0, r0, k2, r2), cswap4(k1, r1, k3, r3), cswap4(k1, r1, k2, r2);
-            if (nh == 0) {
-                cur = sp ? stack[--sp] : VRJ_LEAF_DONE;
-            } else {
-                if (nh > 3) stack[sp++] = r3;
-                if (nh > 2) stack[sp++] = r2;
-                if (nh > 1) stack[sp++] = r1;
-                cur = r0;
-            }
+            Format::template step<COUNT>(sc, fr, limit, cur, stack, sp, cnt, [&]() { cur = sp ? stack[--sp] : VRJ_LEAF_DONE; });
         }
         if (cur == VRJ_LEAF_DONE) break;
-        {
-            int tri = ~cur;
-            V3<R> v0, v1, v2, loc;
-            uint32_t mat, pid;
-            load_tri_pos(sc, tri, v0, v1, v2, mat, pid);
-            if (COUNT) cnt.tri_tests += 1;
-            R dist, b0, b1, b2;
-            if (triangle_test(tr, v0, v1, v2, dist, b0, b1, b2, loc)) {
-                if (dist < best_t || (dist == best_t && tri > best_tri)) {
-                    best_t = dist, best_tri = tri;
-                    if (ANY) return;
-                    limit = filter_limit<float>(fmin(best_t, t_limit));
-                }
-            }
+        if (leaf_test<COUNT>(sc, tr, ~cur, best_t, best_tri, cnt)) {
+            if (ANY) return;
+            limit = Format::limit(fmin(best_t, t_limit));
         }
         cur = sp ? stack[--sp] : VRJ_LEAF_DONE;
         if (cur == VRJ_LEAF_DONE) break;
     }
 }
 
-// Sampler::sample.  ANY = true stops at the first hit found (shadow rays: only Some/None is used).
+// Sampler::sample.  ANY = true stops at the first hit found (shadow rays: only Some/None is used).  QUAD walks the 4-wide
+// form of the tree: half the dependent fetches, which is what a single thread following one path to its end (k_tail) waits on.
 template <typename NT, bool COUNT, bool ANY, typename R, bool QUAD = false>
 __device__ __forceinline__ HitT<R> trace_closest(const DevScene &sc, V3<R> o, V3<R> d, TraceCounters &cnt) {
+    typedef typename std::conditional<QUAD, Nodes4, Nodes2<NT>>::type Format;
     HitT<R> best;
     best.t = real_inf<R>(), best.item = -1, best.tri = -1;
     bool have_tri_ray = false;
@@ -363,13 +465,8 @@ __device__ __forceinline__ HitT<R> trace_closest(const DevScene &sc, V3<R> o, V3
                 hit = triangle_test(tr, v0, v1, v2, t, b0, b1, b2, loc);
                 tri = (int)it.index;
             } else {
-                if (QUAD) {
-                    FilterRay<float> fr = filter_ray<float>(o, d);
-                    bvh_closest_quad<COUNT, ANY>(sc, (int)it.root, tr, fr, best.item < 0 ? real_inf<R>() : best.t, t, tri, cnt);
-                } else {
-                    FilterRay<NT> fr = filter_ray<NT>(o, d);
-                    bvh_closest<NT, COUNT, ANY>(sc, (int)it.root, tr, fr, best.item < 0 ? real_inf<R>() : best.t, t, tri, cnt);
-                }
+                typename Format::Ray fr = Format::ray(sc, o, d);
+                bvh_closest<Format, COUNT, ANY>(sc, (int)it.root, tr, fr, best.item < 0 ? real_inf<R>() : best.t, t, tri, cnt);
                 hit = tri >= 0;
             }
         }
@@ -469,49 +566,42 @@ __device__ __forceinline__ uint32_t load_trace_rec(const TraceRec *recs, uint32_
 }
 
 // ------------------------------------------------------------------------------------------
-// Closest hit, stage 2: the persistent-thread BVH engine.  Every lane owns one ray at a time; when
-// enough lanes of the warp have run dry they write their results and fetch new rays with ONE
-// warp-aggregated atomic, so short traversals do not hold the warp hostage to the longest one.  Box
-// steps run in small batches between warp votes; exact triangle tests are postponed until several lanes
-// are parked at a leaf (or nobody has box work left), so the expensive binary64 test runs with many lanes.
+// Closest hit, stage 2: the persistent-thread BVH engine, over any node format above.  Every lane owns one ray at a time;
+// when enough lanes of the warp have run dry they write their results and fetch new rays with ONE warp-aggregated atomic,
+// so short traversals do not hold the warp hostage to the longest one.  Box steps run in small batches between warp votes;
+// exact triangle tests are postponed until several lanes are parked at a leaf (or nobody has box work left), so the
+// expensive binary64 test runs with many lanes.
 //
 // Semantics: objects compete with "smaller distance wins, earlier object wins ties" (sampler.rs:14-19),
 // triangles inside one BVH with "later DFS leaf wins ties" (bounding_volume_hierarchy.rs:77-92).
 //
-// Source:  uint32_t load_setup(uint32_t r, TriRay &tr, FilterRay &fr, Hit &best) -- staged ray r: the constants of the exact
-//          triangle test and of the slab filter, and the best hit of the other objects; returns the sink's handle
-//          (the 4-wide and 16-bit engines below use  void load(uint32_t r, D3 &o, D3 &d, Hit &best)  and form the constants)
+// Source:  uint32_t load_setup<Format>(const DevScene &sc, uint32_t r, TriRay &tr, Format::Ray &fr, Hit &best) -- staged ray
+//          r: the constants of the exact triangle test and of the slab filter, and the best hit of the other objects;
+//          returns the sink's handle
 // Sink:    void store(uint32_t handle, const Hit &best, bool improved)
-template <typename NT, typename R, bool COUNT, typename Source, typename Sink>
+template <typename Format, typename R, bool COUNT, typename Source, typename Sink>
 __device__ __forceinline__ void trace_persistent(const DevScene &sc, uint32_t n, uint32_t *work, Source &source, Sink &sink,
                                                  TraceCounters &cnt) {
+    typedef typename Format::Limit Limit;
     const unsigned FULL = 0xffffffffu;
     const uint32_t NONE = 0xffffffffu;
     const uint32_t lane = threadIdx.x & 31;
     const int refill_threshold = sc.refill_threshold, leaf_threshold = sc.leaf_threshold;
-    const int node_batch = sc.node_batch, max_iters = sc.max_iters;
-    int stack[32];
+    const int node_batch = Format::batch(sc), max_iters = sc.max_iters;
+    int stack[Format::STACK];
     int sp = 0, cur = VRJ_LEAF_DONE;
     uint32_t r = NONE, bcur = 0;
     bool improved = false;
-#if VRJ_TRACE_TRIRAY_SMEM
-    // the triangle-test constants of the lane's ray live in shared memory: they are touched once per leaf, not per node
-    // step, and their 13 (binary64) registers are what keeps the kernel from 8 resident CTAs per SM
-    __shared__ TriRayT<R> s_tr[128];
-    TriRayT<R> &tr = s_tr[threadIdx.x];
-#else
     TriRayT<R> tr;
-#endif
-    FilterRay<NT> fr;
+    typename Format::Ray fr;
     HitT<R> best;
     R loc_t = real_inf<R>();
     int loc_tri = -1;
-    NT limit = (NT)0;
+    Limit limit = (Limit)0;
     bool exhausted = false;
     tr.o = V3<R>{R(0), R(0), R(0)}, tr.sx = tr.sy = tr.pdz = R(0), tr.perm = 0;
     best.t = real_inf<R>(), best.item = -1, best.tri = -1;
-#pragma unroll
-    for (int k = 0; k < 3; k++) fr.id[k] = fr.cn[k] = fr.cf[k] = (NT)0;
+    clear_filter(fr);
 
     // the current BVH's closest triangle competes with the best of the other objects, then the next BVH starts
     auto finish_bvh = [&]() {
@@ -522,72 +612,9 @@ __device__ __forceinline__ void trace_persistent(const DevScene &sc, uint32_t n,
         if (bcur < sc.n_bvh_items) {
             cur = (int)sc.items[sc.bvh_items[bcur]].root;
             sp = 0, loc_t = real_inf<R>(), loc_tri = -1;
-            limit = filter_limit<NT>(best.t);
+            limit = Format::limit(best.t);
         } else {
             cur = VRJ_LEAF_DONE;
-        }
-    };
-#if VRJ_TRACE_SMEM_LEVELS
-    constexpr int NTOP = (1 << VRJ_TRACE_SMEM_LEVELS) - 1;
-    __shared__ float4 s_top[sizeof(NT) == 4 ? NTOP * 4 : 1];
-    __shared__ int s_ref[sizeof(NT) == 4 ? NTOP * 2 : 1];
-    if (sizeof(NT) == 4) {
-        // heap-ordered copy of the top levels: node i has children 2i+1, 2i+2; s_ref holds their GLOBAL references
-        // (VRJ_LEAF_DONE = no such node), rewritten to tagged shared-memory references at the end
-        const float4 *nodes = reinterpret_cast<const float4 *>(sc.nodes32);
-        if (threadIdx.x == 0) {
-            const int root = (int)sc.items[sc.bvh_items[0]].root;
-            for (int q = 0; q < 4; q++) s_top[q] = nodes[(size_t)root * 4 + q];
-            s_ref[0] = __float_as_int(s_top[3].x), s_ref[1] = __float_as_int(s_top[3].y);
-        }
-        for (int level = 1; level < VRJ_TRACE_SMEM_LEVELS; level++) {
-            __syncthreads();
-            const int first = (1 << level) - 1, count = 1 << level;
-            for (int k = threadIdx.x; k < count; k += blockDim.x) {
-                const int i = first + k, parent = (i - 1) >> 1;
-                const int ref = s_ref[2 * parent + ((i - 1) & 1)];
-                if (ref >= 0) {
-                    for (int q = 0; q < 4; q++) s_top[i * 4 + q] = nodes[(size_t)ref * 4 + q];
-                    s_ref[2 * i] = __float_as_int(s_top[i * 4 + 3].x), s_ref[2 * i + 1] = __float_as_int(s_top[i * 4 + 3].y);
-                } else {
-                    s_ref[2 * i] = s_ref[2 * i + 1] = VRJ_LEAF_DONE;
-                }
-            }
-        }
-        __syncthreads();
-        for (int i = threadIdx.x; i < (NTOP >> 1); i += blockDim.x) { // nodes whose children are in the table too
-            if (s_ref[2 * i] >= 0) s_top[i * 4 + 3].x = __int_as_float(VRJ_SMEM_TAG | (2 * i + 1));
-            if (s_ref[2 * i + 1] >= 0) s_top[i * 4 + 3].y = __int_as_float(VRJ_SMEM_TAG | (2 * i + 2));
-        }
-        __syncthreads();
-    }
-#endif
-    auto node_step = [&]() {
-        WideNode<NT> nd;
-#if VRJ_TRACE_SMEM_LEVELS
-        if (sizeof(NT) == 4 && (cur & VRJ_SMEM_TAG)) {
-            const float4 *p = s_top + (cur & ~VRJ_SMEM_TAG) * 4;
-            const float4 a = p[0], b = p[1], c = p[2], kf = p[3];
-            nd.c0[0] = (NT)a.x, nd.c0[1] = (NT)a.y, nd.c0[2] = (NT)a.z, nd.c0[3] = (NT)a.w, nd.c0[4] = (NT)c.x, nd.c0[5] = (NT)c.y;
-            nd.c1[0] = (NT)b.x, nd.c1[1] = (NT)b.y, nd.c1[2] = (NT)b.z, nd.c1[3] = (NT)b.w, nd.c1[4] = (NT)c.z, nd.c1[5] = (NT)c.w;
-            nd.left = __float_as_int(kf.x), nd.right = __float_as_int(kf.y);
-        } else
-#endif
-            load_node(sc, cur, nd);
-        if (COUNT) cnt.node_visits += 2;
-        NT e0, e1;
-        bool h0 = box_filter(fr, nd.c0[0], nd.c0[1], nd.c0[2], nd.c0[3], nd.c0[4], nd.c0[5], limit, e0);
-        bool h1 = box_filter(fr, nd.c1[0], nd.c1[1], nd.c1[2], nd.c1[3], nd.c1[4], nd.c1[5], limit, e1);
-        if (h0 && h1) {
-            bool swap = e1 < e0;
-            stack[sp++] = swap ? nd.left : nd.right;
-            cur = swap ? nd.right : nd.left;
-        } else if (h0 || h1) {
-            cur = h0 ? nd.left : nd.right;
-        } else if (sp) {
-            cur = stack[--sp];
-        } else {
-            finish_bvh();
         }
     };
 
@@ -611,12 +638,12 @@ __device__ __forceinline__ void trace_persistent(const DevScene &sc, uint32_t n,
                 if (idle) {
                     uint32_t my = base + (uint32_t)__popc(idle_mask & ((1u << lane) - 1u));
                     if (my < n) {
-                        r = source.load_setup(my, tr, fr, best); // the handle the sink stores the result under
+                        r = source.template load_setup<Format>(sc, my, tr, fr, best); // the handle the sink stores the result under
                         improved = false;
                         bcur = 0;
-                        cur = (VRJ_TRACE_SMEM_LEVELS && sizeof(NT) == 4) ? VRJ_SMEM_TAG : (int)sc.items[sc.bvh_items[0]].root;
+                        cur = (int)sc.items[sc.bvh_items[0]].root;
                         sp = 0, loc_t = real_inf<R>(), loc_tri = -1;
-                        limit = filter_limit<NT>(best.t);
+                        limit = Format::limit(best.t);
                     }
                 }
             }
@@ -626,338 +653,16 @@ __device__ __forceinline__ void trace_persistent(const DevScene &sc, uint32_t n,
         for (int it = 0; it < max_iters; it++) {
 #pragma unroll 1
             for (int u = 0; u < node_batch; u++)
-                if (cur >= 0) node_step();
-            bool at_leaf = cur < 0 && cur != VRJ_LEAF_DONE;
-            unsigned leaf_mask = __ballot_sync(FULL, at_leaf);
-            unsigned node_mask = __ballot_sync(FULL, cur >= 0);
-            if (leaf_mask && (node_mask == 0 || __popc(leaf_mask) >= leaf_threshold)) {
-                if (at_leaf) {
-                    int tri = ~cur;
-                    V3<R> v0, v1, v2, loc;
-                    uint32_t mat, pid;
-                    load_tri_pos(sc, tri, v0, v1, v2, mat, pid);
-                    if (COUNT) cnt.tri_tests += 1;
-                    R dist, b0, b1, b2;
-                    if (triangle_test(tr, v0, v1, v2, dist, b0, b1, b2, loc)) {
-                        if (dist < loc_t || (dist == loc_t && tri > loc_tri)) {
-                            loc_t = dist, loc_tri = tri;
-                            limit = filter_limit<NT>(fmin(loc_t, best.t));
-                        }
-                    }
+                if (cur >= 0) Format::template step<COUNT>(sc, fr, limit, cur, stack, sp, cnt, [&]() {
                     if (sp) cur = stack[--sp];
                     else finish_bvh();
-                }
-            }
-            unsigned done_mask = __ballot_sync(FULL, cur == VRJ_LEAF_DONE);
-            if (done_mask == FULL || (!exhausted && __popc(done_mask) >= refill_threshold)) break;
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------------------
-// The same engine over 16-bit nodes (VRJ_FILTER_Q16): half the bytes per step.  A box plane is qlo + q * qcell; with
-// A = qcell / d (binary32) and B = (qlo - o) / d - 2^23 * A (formed in binary64 from the ROUNDED A, then rounded to binary32
-// away from the ray's interval, with a pad for q * (A - qcell / d)), the parameter of the plane is fma(2^23 + q, A, B):
-// one PRMT builds the float 2^23 + q from a 16-bit field, the bias cancels inside the fused multiply-add.  The box a ray
-// sees is at most two cells larger per side than the real one (one from the outward quantisation, one from rounding B),
-// never smaller; every triangle is still decided by the exact binary64 test, so results do not change.
-struct FilterRayQ {
-    float A[3], Bn[3], Bf[3];
-    uint32_t neg; // bit k: the direction is negative on axis k (the near plane is the box's hi plane)
-};
-__device__ __forceinline__ FilterRayQ filter_ray_q(const DevScene &sc, D3 o, D3 d) {
-    FilterRayQ f;
-    const double oo[3] = {o.x, o.y, o.z}, dd[3] = {d.x, d.y, d.z};
-    f.neg = 0;
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-        double id = 1.0 / dd[k];
-        if (!(fabs(id) <= 1e18)) id = copysign(1e18, dd[k]);
-        const float A = __double2float_rn(sc.qcell[k] * id);
-        const double shift = (sc.qlo[k] - oo[k]) * id;
-        const double B = shift - 8388608.0 * (double)A;
-        // q * (A - cell/d) <= 65535 * 2^-24 * |A|;  binary64 rounding of `shift` and B;  a floor so the pad is never zero
-        const double pad = fabs((double)A) * 0.0079 + (fabs(shift) + fabs(B)) * 1e-15 + 1e-300;
-        f.A[k] = A, f.Bn[k] = __double2float_rd(B - pad), f.Bf[k] = __double2float_ru(B + pad);
-        if (id < 0.0) f.neg |= 1u << k;
-    }
-    return f;
-}
-template <bool COUNT, typename Source, typename Sink>
-__device__ __forceinline__ void trace_persistent_q16(const DevScene &sc, uint32_t n, uint32_t *work, Source &source, Sink &sink,
-                                                     TraceCounters &cnt) {
-    typedef FilterTraits<float> F;
-    const unsigned FULL = 0xffffffffu;
-    const uint32_t NONE = 0xffffffffu;
-    const uint32_t lane = threadIdx.x & 31;
-    const int refill_threshold = sc.refill_threshold, leaf_threshold = sc.leaf_threshold;
-    const int node_batch = sc.node_batch, max_iters = sc.max_iters;
-    int stack[32];
-    int sp = 0, cur = VRJ_LEAF_DONE;
-    uint32_t r = NONE, bcur = 0;
-    bool improved = false;
-    TriRay tr;
-    FilterRayQ fr;
-    Hit best;
-    double loc_t = CUDART_INF;
-    int loc_tri = -1;
-    float limit = 0.f;
-    bool exhausted = false;
-    tr.o = d3(0, 0, 0), tr.sx = tr.sy = tr.pdz = 0.0, tr.perm = 0;
-    best.t = CUDART_INF, best.item = -1, best.tri = -1;
-    fr.neg = 0;
-#pragma unroll
-    for (int k = 0; k < 3; k++) fr.A[k] = fr.Bn[k] = fr.Bf[k] = 0.f;
-
-    auto finish_bvh = [&]() {
-        uint32_t item = sc.bvh_items[bcur];
-        if (loc_tri >= 0 && (best.item < 0 || loc_t < best.t || (loc_t == best.t && (int)item < best.item)))
-            best.t = loc_t, best.item = (int)item, best.tri = loc_tri, improved = true;
-        bcur++;
-        if (bcur < sc.n_bvh_items) {
-            cur = (int)sc.items[sc.bvh_items[bcur]].root; // all meshes share the scene's grid: the ray constants stay
-            sp = 0, loc_t = CUDART_INF, loc_tri = -1;
-            limit = filter_limit<float>(best.t);
-        } else {
-            cur = VRJ_LEAF_DONE;
-        }
-    };
-    // parameter interval of child `hi16` (0: low halves, 1: high halves) of the node words
-    auto child_test = [&](uint32_t nx, uint32_t fx, uint32_t ny, uint32_t fy, uint32_t nz, uint32_t fz, uint32_t sel, float &enter) {
-        const float qnx = __uint_as_float(__byte_perm(nx, 0x4b000000u, sel)), qfx = __uint_as_float(__byte_perm(fx, 0x4b000000u, sel));
-        const float qny = __uint_as_float(__byte_perm(ny, 0x4b000000u, sel)), qfy = __uint_as_float(__byte_perm(fy, 0x4b000000u, sel));
-        const float qnz = __uint_as_float(__byte_perm(nz, 0x4b000000u, sel)), qfz = __uint_as_float(__byte_perm(fz, 0x4b000000u, sel));
-        const float tn = fmaxf(fmaxf(fmaf(qnx, fr.A[0], fr.Bn[0]), fmaf(qny, fr.A[1], fr.Bn[1])), fmaf(qnz, fr.A[2], fr.Bn[2]));
-        const float tf = fminf(fminf(fmaf(qfx, fr.A[0], fr.Bf[0]), fmaf(qfy, fr.A[1], fr.Bf[1])), fmaf(qfz, fr.A[2], fr.Bf[2]));
-        const float ep = fmaf(-F::rel(), fabsf(tn), tn), xp = fmaf(F::rel(), fabsf(tf), tf);
-        enter = ep;
-        return (ep <= xp) && (xp >= 0.f) && (ep <= limit);
-    };
-    auto node_step = [&]() {
-        const uint4 *p = sc.nodesq + (size_t)cur * 2;
-        uint4 a, b;
-        asm volatile("ld.global.nc.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                     : "=r"(a.x), "=r"(a.y), "=r"(a.z), "=r"(a.w), "=r"(b.x), "=r"(b.y), "=r"(b.z), "=r"(b.w)
-                     : "l"(p));
-        if (COUNT) cnt.node_visits += 2;
-        const bool ngx = fr.neg & 1u, ngy = fr.neg & 2u, ngz = fr.neg & 4u;
-        const uint32_t nx = ngx ? a.y : a.x, fx = ngx ? a.x : a.y;
-        const uint32_t ny = ngy ? a.w : a.z, fy = ngy ? a.z : a.w;
-        const uint32_t nz = ngz ? b.y : b.x, fz = ngz ? b.x : b.y;
-        float e0, e1;
-        const bool h0 = child_test(nx, fx, ny, fy, nz, fz, 0x7610u, e0);
-        const bool h1 = child_test(nx, fx, ny, fy, nz, fz, 0x7632u, e1);
-        const int left = (int)b.z, right = (int)b.w;
-        if (h0 && h1) {
-            bool swap = e1 < e0;
-            stack[sp++] = swap ? left : right;
-            cur = swap ? right : left;
-        } else if (h0 || h1) {
-            cur = h0 ? left : right;
-        } else if (sp) {
-            cur = stack[--sp];
-        } else {
-            finish_bvh();
-        }
-    };
-
-    while (true) {
-        bool idle = cur == VRJ_LEAF_DONE;
-        unsigned idle_mask = __ballot_sync(FULL, idle);
-        if (idle_mask) {
-            if (idle && r != NONE) {
-                sink.store(r, best, improved);
-                r = NONE;
-            }
-            if (exhausted) {
-                if (idle_mask == FULL) break;
-            } else if (idle_mask == FULL || __popc(idle_mask) >= refill_threshold) {
-                uint32_t want = (uint32_t)__popc(idle_mask), base = 0;
-                int leader = __ffs(idle_mask) - 1;
-                if ((int)lane == leader) base = atomicAdd(work, want);
-                base = __shfl_sync(FULL, base, leader);
-                if (base + want >= n) exhausted = true;
-                if (idle) {
-                    uint32_t my = base + (uint32_t)__popc(idle_mask & ((1u << lane) - 1u));
-                    if (my < n) {
-                        D3 o, d;
-                        source.load(my, o, d, best);
-                        r = my, improved = false;
-                        tr = tri_ray(o, d);
-                        fr = filter_ray_q(sc, o, d);
-                        bcur = 0;
-                        cur = (int)sc.items[sc.bvh_items[0]].root;
-                        sp = 0, loc_t = CUDART_INF, loc_tri = -1;
-                        limit = filter_limit<float>(best.t);
-                    }
-                }
-            }
-        }
-#pragma unroll 1
-        for (int it = 0; it < max_iters; it++) {
-#pragma unroll 1
-            for (int u = 0; u < node_batch; u++)
-                if (cur >= 0) node_step();
+                });
             bool at_leaf = cur < 0 && cur != VRJ_LEAF_DONE;
             unsigned leaf_mask = __ballot_sync(FULL, at_leaf);
             unsigned node_mask = __ballot_sync(FULL, cur >= 0);
             if (leaf_mask && (node_mask == 0 || __popc(leaf_mask) >= leaf_threshold)) {
                 if (at_leaf) {
-                    int tri = ~cur;
-                    D3 v0, v1, v2, loc;
-                    uint32_t mat, pid;
-                    load_tri_pos(sc, tri, v0, v1, v2, mat, pid);
-                    if (COUNT) cnt.tri_tests += 1;
-                    double dist, b0, b1, b2;
-                    if (triangle_test(tr, v0, v1, v2, dist, b0, b1, b2, loc)) {
-                        if (dist < loc_t || (dist == loc_t && tri > loc_tri)) {
-                            loc_t = dist, loc_tri = tri;
-                            limit = filter_limit<float>(fmin(loc_t, best.t));
-                        }
-                    }
-                    if (sp) cur = stack[--sp];
-                    else finish_bvh();
-                }
-            }
-            unsigned done_mask = __ballot_sync(FULL, cur == VRJ_LEAF_DONE);
-            if (done_mask == FULL || (!exhausted && __popc(done_mask) >= refill_threshold)) break;
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------------------
-// The same engine over the 4-wide form of the tree (vrj_scene_prep.cuh): one 128-byte fetch decides four boxes, the
-// hit children are ordered by entry distance with a 5-comparator network, the nearest is followed and the others are
-// pushed farthest first.  Same filter, same exact triangle test, same tie rules: results are identical to the 2-wide
-// walk; only the number of dependent fetches per ray (about half) differs.
-__device__ __forceinline__ void cswap(float &ka, int &ra, float &kb, int &rb) {
-    const bool sw = kb < ka;
-    const float k = sw ? kb : ka, K = sw ? ka : kb;
-    const int r = sw ? rb : ra, R = sw ? ra : rb;
-    ka = k, kb = K, ra = r, rb = R;
-}
-template <bool COUNT, typename Source, typename Sink>
-__device__ __forceinline__ void trace_persistent_quad(const DevScene &sc, uint32_t n, uint32_t *work, Source &source, Sink &sink,
-                                                      TraceCounters &cnt) {
-    typedef FilterTraits<float> F;
-    const unsigned FULL = 0xffffffffu;
-    const uint32_t NONE = 0xffffffffu;
-    const uint32_t lane = threadIdx.x & 31;
-    const int refill_threshold = sc.refill_threshold, leaf_threshold = sc.leaf_threshold;
-    const int node_batch = sc.node_batch4, max_iters = sc.max_iters;
-    int stack[48]; // up to three pushes per 4-wide level, 16 levels
-    int sp = 0, cur = VRJ_LEAF_DONE;
-    uint32_t r = NONE, bcur = 0;
-    bool improved = false;
-    TriRay tr;
-    FilterRay<float> fr;
-    Hit best;
-    double loc_t = CUDART_INF;
-    int loc_tri = -1;
-    float limit = 0.f;
-    bool exhausted = false;
-    tr.o = d3(0, 0, 0), tr.sx = tr.sy = tr.pdz = 0.0, tr.perm = 0;
-    best.t = CUDART_INF, best.item = -1, best.tri = -1;
-#pragma unroll
-    for (int k = 0; k < 3; k++) fr.id[k] = fr.cn[k] = fr.cf[k] = 0.f;
-
-    auto finish_bvh = [&]() {
-        uint32_t item = sc.bvh_items[bcur];
-        if (loc_tri >= 0 && (best.item < 0 || loc_t < best.t || (loc_t == best.t && (int)item < best.item)))
-            best.t = loc_t, best.item = (int)item, best.tri = loc_tri, improved = true;
-        bcur++;
-        if (bcur < sc.n_bvh_items) {
-            cur = (int)sc.items[sc.bvh_items[bcur]].root;
-            sp = 0, loc_t = CUDART_INF, loc_tri = -1;
-            limit = filter_limit<float>(best.t);
-        } else {
-            cur = VRJ_LEAF_DONE;
-        }
-    };
-    auto node_step = [&]() {
-        const float4 *p = sc.nodes4 + (size_t)cur * 8;
-        float4 a, b, c, d, e, f, g, h;
-        ldg256(p, a, b);
-        ldg256(p + 2, c, d);
-        ldg256(p + 4, e, f);
-        ldg256(p + 6, g, h);
-        if (COUNT) cnt.node_visits += 4;
-        float k0, k1, k2, k3;
-        const bool h0 = box_filter(fr, a.x, a.y, a.z, a.w, b.x, b.y, limit, k0);
-        const bool h1 = box_filter(fr, b.z, b.w, c.x, c.y, c.z, c.w, limit, k1);
-        const bool h2 = box_filter(fr, d.x, d.y, d.z, d.w, e.x, e.y, limit, k2);
-        const bool h3 = box_filter(fr, e.z, e.w, f.x, f.y, f.z, f.w, limit, k3);
-        int r0 = __float_as_int(g.x), r1 = __float_as_int(g.y), r2 = __float_as_int(g.z), r3 = __float_as_int(g.w);
-        const float inf = CUDART_INF_F;
-        k0 = h0 ? k0 : inf, k1 = h1 ? k1 : inf, k2 = h2 ? k2 : inf, k3 = h3 ? k3 : inf;
-        const int nh = (int)h0 + (int)h1 + (int)h2 + (int)h3;
-        // misses carry +inf and sink to the end; a hit's key is finite (its box test passed ep <= limit)
-        cswap(k0, r0, k1, r1), cswap(k2, r2, k3, r3), cswap(k0, r0, k2, r2), cswap(k1, r1, k3, r3), cswap(k1, r1, k2, r2);
-        if (nh == 0) {
-            if (sp) cur = stack[--sp];
-            else finish_bvh();
-        } else {
-            if (nh > 3) stack[sp++] = r3;
-            if (nh > 2) stack[sp++] = r2;
-            if (nh > 1) stack[sp++] = r1;
-            cur = r0;
-        }
-    };
-
-    while (true) {
-        bool idle = cur == VRJ_LEAF_DONE;
-        unsigned idle_mask = __ballot_sync(FULL, idle);
-        if (idle_mask) {
-            if (idle && r != NONE) {
-                sink.store(r, best, improved);
-                r = NONE;
-            }
-            if (exhausted) {
-                if (idle_mask == FULL) break;
-            } else if (idle_mask == FULL || __popc(idle_mask) >= refill_threshold) {
-                uint32_t want = (uint32_t)__popc(idle_mask), base = 0;
-                int leader = __ffs(idle_mask) - 1;
-                if ((int)lane == leader) base = atomicAdd(work, want);
-                base = __shfl_sync(FULL, base, leader);
-                if (base + want >= n) exhausted = true;
-                if (idle) {
-                    uint32_t my = base + (uint32_t)__popc(idle_mask & ((1u << lane) - 1u));
-                    if (my < n) {
-                        D3 o, d;
-                        source.load(my, o, d, best);
-                        r = my, improved = false;
-                        tr = tri_ray(o, d);
-                        fr = filter_ray<float>(o, d);
-                        bcur = 0;
-                        cur = (int)sc.items[sc.bvh_items[0]].root;
-                        sp = 0, loc_t = CUDART_INF, loc_tri = -1;
-                        limit = F::up(best.t * (1.0 + 4.0 * (double)F::rel()));
-                    }
-                }
-            }
-        }
-#pragma unroll 1
-        for (int it = 0; it < max_iters; it++) {
-#pragma unroll 1
-            for (int u = 0; u < node_batch; u++)
-                if (cur >= 0) node_step();
-            bool at_leaf = cur < 0 && cur != VRJ_LEAF_DONE;
-            unsigned leaf_mask = __ballot_sync(FULL, at_leaf);
-            unsigned node_mask = __ballot_sync(FULL, cur >= 0);
-            if (leaf_mask && (node_mask == 0 || __popc(leaf_mask) >= leaf_threshold)) {
-                if (at_leaf) {
-                    int tri = ~cur;
-                    D3 v0, v1, v2, loc;
-                    uint32_t mat, pid;
-                    load_tri_pos(sc, tri, v0, v1, v2, mat, pid);
-                    if (COUNT) cnt.tri_tests += 1;
-                    double dist, b0, b1, b2;
-                    if (triangle_test(tr, v0, v1, v2, dist, b0, b1, b2, loc)) {
-                        if (dist < loc_t || (dist == loc_t && tri > loc_tri)) {
-                            loc_t = dist, loc_tri = tri;
-                            limit = F::up(fmin(loc_t, best.t) * (1.0 + 4.0 * (double)F::rel()));
-                        }
-                    }
+                    if (leaf_test<COUNT>(sc, tr, ~cur, loc_t, loc_tri, cnt)) limit = Format::limit(fmin(loc_t, best.t));
                     if (sp) cur = stack[--sp];
                     else finish_bvh();
                 }
